@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — agent-steps/s of the batched rollout hot path (env step + comm + comm-GNN policy forward).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--config c3] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--config c3] [--impl b200|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one rollout iteration over the whole batch: cm_policy_forward (forward + action sampling) followed by
@@ -12,8 +12,8 @@ GPU steps its own 65536 envs; the only collective of the rollout is the episode-
 region).  One JSON line is printed by rank 0:
 
   value      device-resident rollout: inputs live in HBM, steps replayed from one CUDA graph of `ring` iterations.  The
-             timed region is at least --min-seconds long whatever --steps says (the graph is replayed more often and the
-             real step count is reported), so it contains time-limit resets and several clock samples.
+             timed region is exactly --steps steps: the graph holds the largest divisor of --steps that is not above --ring.
+             The configs of the sweep have no step count of their own and are timed for at least --min-seconds.
   e2e        the same loop through the sampler-level host-buffer call (HostRollout = cm_rollout_step_host): one C call per
              env part and step runs policy -> env on device-resident state, copies the availability bytes host -> device
              and everything the sampler appends per step (next observation, masks, reward, done, counts, actions,
@@ -29,6 +29,9 @@ region).  One JSON line is printed by rank 0:
 
 `--impl reference` times that CPU port on all host cores (the reference itself is pure Python and is not present
 on the GPU box; oracle/ is its pinned restatement).
+
+`--dump-outputs DIR` writes what the timed loop of `value` handed back for its last step to DIR/<name>.npy (see
+dump_last_step), so that two builds run with the same arguments, hence the same inputs, can be compared output for output.
 """
 import argparse
 import json
@@ -217,12 +220,18 @@ class ClockSampler:
         for ln in self.proc.stdout:
             self.lines.append((time.time(), ln.strip()))
 
+    def close(self):
+        """ends the sampling loop: nvidia-smi -lms would otherwise outlive a run that fails before stop()"""
+        if self.proc is not None and self.proc.poll() is None:
+            self.proc.terminate()
+            self.proc.wait()
+
     def stop(self, t_lo, t_hi):
         """median SM clock and throttle reasons of the samples taken INSIDE [t_lo, t_hi] (the timed region)"""
         if self.proc is None:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"], "samples": 0}
         time.sleep(0.1)
-        self.proc.terminate()
+        self.close()
         sm, mx, reasons, power = [], None, set(), []
         for ts, ln in self.lines:
             f = [x.strip() for x in ln.split(",")]
@@ -286,9 +295,35 @@ class Ctx:
         return [float(x) for x in t]
 
 
-def measure_config(cx, cfg, steps_req, warm_req, min_seconds, full, clocks=None, e2e_seconds=0.5):
+DUMP_BYTES = 64 << 20
+DUMP_MAX_ENVS = 512
+
+
+def dump_last_step(eng, out_dir):
+    """Writes what RolloutEngine handed its caller for the last step it ran, as DIR/<name>.npy: the policy's actions and
+    probabilities and the env's reward, done, counts, prey_alive_out, success (ring slot K - 1), the next observation,
+    adjacency / channel bit rows and ave_deg (slot K), plus the episode-statistics sums of the whole run (episode_stats).
+    Rows are a fixed seeded sample of at most DUMP_MAX_ENVS envs (their indices in env_index), fewer if the files would pass
+    DUMP_BYTES.  float32 arrays stay float32; integers (bit rows included) become float64, which holds them exactly."""
+    import torch
+    t, K = eng.traj, eng.K
+    rows = {k: t[k][K - 1] for k in ("actions", "probs", "reward", "done", "counts", "prey_alive_out", "success")}
+    rows.update({k: t[k][K] for k in ("obs", "adj_bits", "chan_bits", "ave_deg")})
+    per_env = sum(v[0].numel() * (4 if v.dtype == torch.float32 else 8) for v in rows.values())
+    count = min(eng.B, DUMP_MAX_ENVS, (DUMP_BYTES - (1 << 20)) // per_env)
+    idx = np.sort(np.random.default_rng(0).choice(eng.B, size=count, replace=False))
+    sel = torch.as_tensor(idx, device=eng.device)
+    arrays = {k: v.index_select(0, sel).cpu().numpy() for k, v in rows.items()}
+    arrays["env_index"] = idx
+    arrays["episode_stats"] = eng.local_stats().cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f"{name}.npy"), a.astype(np.float32 if a.dtype == np.float32 else np.float64))
+
+
+def measure_config(cx, cfg, steps_req, warm_req, min_seconds, full, clocks=None, e2e_seconds=0.5, dump_dir=None):
     """rollout value / kernel rooflines / e2e of one BASELINE config on this rank's GPU; every rank runs it, all return the
-    same record (times are max over ranks)."""
+    same record (times are max over ranks).  steps_req > 0 times exactly that many steps, 0 at least min_seconds."""
     torch, args, dev = cx.torch, cx.args, cx.dev
     from com_marl_b200.rollout import HostRollout, RolloutEngine, make_policy
     from com_marl_b200.scenario import ScenarioSpec
@@ -297,7 +332,8 @@ def measure_config(cx, cfg, steps_req, warm_req, min_seconds, full, clocks=None,
     spec = ScenarioSpec.from_params(scen, params, seed=1, **spec_over)
     B = (args.envs if (args.envs and cfg == args.config) else CONFIGS[base_cfg][6])
     n, Dobs, L = spec.n_agents, spec.obs_dim, spec.n_layers
-    ring = args.ring
+    # the engine runs whole graphs of `ring` steps: a ring that divides the requested count times exactly that count
+    ring = max(k for k in range(1, min(args.ring, steps_req) + 1) if steps_req % k == 0) if steps_req > 0 else args.ring
     pol = make_policy(spec, device=dev)
     # independent env groups: 4 chains for teams up to 64 (8 when a chain still gets ~2000 policy tiles per launch — C3: measured
     # 849 -> 864 M agent-steps/s; smaller batches lose with 8), two chains for the three-launch pipeline of large teams (C5: 315 -> 320 M)
@@ -312,9 +348,7 @@ def measure_config(cx, cfg, steps_req, warm_req, min_seconds, full, clocks=None,
     ev0.record(); eng.run(ring); ev1.record()
     torch.cuda.synchronize(dev)
     pilot_ms, = cx.max_over_ranks(ev0.elapsed_time(ev1) / ring)
-    steps = max(ring, ((steps_req + ring - 1) // ring) * ring)
-    floor_steps = int(np.ceil(min_seconds * 1e3 / max(pilot_ms, 1e-6) / ring)) * ring
-    steps = max(steps, floor_steps)
+    steps = steps_req if steps_req > 0 else max(ring, int(np.ceil(min_seconds * 1e3 / max(pilot_ms, 1e-6) / ring)) * ring)
     # ---------------- value: device-resident rollout ----------------
     launches0 = eng.kernel_launches
     cx.barrier(); torch.cuda.synchronize(dev)
@@ -328,6 +362,8 @@ def measure_config(cx, cfg, steps_req, warm_req, min_seconds, full, clocks=None,
     launches = eng.kernel_launches - launches0
     eng.env.check_errors()
     pol.check_errors()
+    if dump_dir is not None and cx.rank == 0:
+        dump_last_step(eng, dump_dir)               # before the kernel timings below overwrite the ring
     clock_info = clocks.stop(t_lo, t_hi) if clocks is not None else None
     stats = cx.D.gather_stats(eng.local_stats())          # the rollout's only collective (NCCL over NVLink)
     # ---------------- per-kernel durations: CUDA events around a CUDA graph of launches of ONE kernel ----------------
@@ -631,7 +667,11 @@ def run_b200_arm(args):
     if clocks is not None:
         clocks.start()
         time.sleep(0.2)
-    main = measure_config(cx, args.config, args.steps, args.warmup, args.min_seconds, True, clocks)
+    try:
+        main = measure_config(cx, args.config, args.steps, args.warmup, args.min_seconds, True, clocks, dump_dir=args.dump_outputs)
+    finally:
+        if clocks is not None:
+            clocks.close()
     sweep = {}
     if not args.no_sweep:
         names = [c for c in (("c4",) if cx.world > 1 else ("c1", "c2", "c3", "c3_ge", "c4", "c5")) if c != args.config]
@@ -653,8 +693,8 @@ def run_b200_arm(args):
         "dtype": ("f32-equivalent: error-compensated fp16-split tcgen05 products (x = hi + 2^-12 lo) with fp32 accumulation in TMEM (policy)"
                   if tc else "f32 FFMA (policy)") + " + u8/u16/u64 bit rows (env, comm)",
         "data": "synthetic", "timed_region_s": main["timed_region_s"],
-        "steps_note": f"--steps {args.steps} / --warmup {args.warmup} were rounded up to whole {args.ring}-step graph replays and to a timed "
-                      f"region of at least {args.min_seconds} s",
+        "steps_note": f"the timed region is exactly --steps {args.steps} steps, replays of a {main['config']['ring_slots']}-step graph; "
+                      f"--warmup {args.warmup} was rounded up to whole replays (at least 3)",
         "config": main["config"], "e2e": main["e2e"], "gpu_launches": main["gpu_launches"],
         "roofline": main["roofline"], "roofline_env": main["roofline_env"], "clocks": main.get("clocks"),
         "episode_stats": main["episode_stats"], "host_affinity": cx.numa,
@@ -697,15 +737,20 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--config", default="c3", choices=sorted(CONFIGS))
     ap.add_argument("--envs", type=int, default=0, help="envs per GPU of --config (default: the config's)")
-    ap.add_argument("--ring", type=int, default=64, help="trajectory ring slots = steps per CUDA graph")
-    ap.add_argument("--min-seconds", type=float, default=0.25, help="floor on the timed region of `value`")
+    ap.add_argument("--ring", type=int, default=64, help="trajectory ring slots = steps per CUDA graph (at most; see `value`)")
+    ap.add_argument("--min-seconds", type=float, default=0.25, help="floor on the timed region of each config of the sweep")
     ap.add_argument("--e2e-steps", type=int, default=2000, help="cap on the steps of an e2e (host-buffer) loop")
     ap.add_argument("--e2e-batches", type=int, default=4, help="independent env parts of the e2e (host-buffer) loops")
     ap.add_argument("--groups", type=int, default=0, help="independent env groups, each a policy->step chain on its own stream (0: 4 or 8 for teams <= 64, else 2)")
     ap.add_argument("--ppo-envs", type=int, default=128, help="envs per GPU of the c5_ppo sub-record")
     ap.add_argument("--no-sweep", action="store_true", help="skip the configs sweep and the c5_ppo sub-record")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     args.out = _quiet_stdout()
     if args.impl == "reference":
         run_reference_arm(args)

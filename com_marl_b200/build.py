@@ -49,6 +49,20 @@ def build(force=False, verbose=False):
     return OUT
 
 
+TC_PROBE_SRC = os.path.join(ROOT, "tests", "native", "tc_gemm_probe.cu")
+TC_PROBE = os.path.join(ROOT, "tests", "native", "libtc_probe.so")
+
+
+def build_tc_probe(force=False):
+    """tests/native/libtc_probe.so: the tcgen05 GEMM probe over csrc/tc_common.cuh that tests/test_gpu_tc_probe.py loads"""
+    deps = (TC_PROBE_SRC, os.path.join(_HERE, "csrc", "tc_common.cuh"))
+    if force or not os.path.exists(TC_PROBE) or any(os.path.getmtime(d) > os.path.getmtime(TC_PROBE) for d in deps):
+        subprocess.check_call([nvcc_path(), "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
+                               "-Xcompiler", "-fPIC", "-shared", "-I", os.path.join(_HERE, "csrc"), "-I", os.path.join(ROOT, "include"),
+                               "-o", TC_PROBE, TC_PROBE_SRC])
+    return TC_PROBE
+
+
 if __name__ == "__main__":
     build(force="--force" in sys.argv, verbose="-v" in sys.argv)
     print(OUT)

@@ -1,25 +1,18 @@
 """tcgen05 building block (tests/native/tc_gemm_probe.cu over com_marl_b200/csrc/tc_common.cuh):
 C = A B^T on the 5th-gen tensor cores with error-compensated TF32 must reach fp32-level accuracy."""
 import ctypes as C
-import os
-import subprocess
 
 import numpy as np
 import pytest
 import torch
 
+from com_marl_b200 import build as cm_build
+
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-SO = os.path.join(ROOT, "tests", "native", "libtc_probe.so")
-SRC = os.path.join(ROOT, "tests", "native", "tc_gemm_probe.cu")
 
 
 def _lib():
-    if not os.path.exists(SO) or os.path.getmtime(SO) < os.path.getmtime(SRC):
-        subprocess.check_call(["nvcc", "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
-                               "-Xcompiler", "-fPIC", "-shared", "-I", os.path.join(ROOT, "com_marl_b200", "csrc"),
-                               "-I", os.path.join(ROOT, "include"), "-o", SO, SRC])
-    lib = C.CDLL(SO)
+    lib = C.CDLL(cm_build.build_tc_probe())        # built by __graft_entry__.build(); rebuilt here only when stale
     lib.tc_gemm_probe.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]
     lib.tc_gemm_probe.restype = C.c_int
     lib.tc_gemm_probe16.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p]
