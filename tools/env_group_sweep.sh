@@ -1,6 +1,7 @@
 #!/bin/bash
 # experiment: lanes per env of env_kernel (CM_ENV_GROUP; 0 = the library's own choice) at the team sizes of C3 / C4 / C5
 # usage: gpurun -- 'bash tools/env_group_sweep.sh'      (library builds are compared with tools/variant_sweep.sh)
+# measures speed only; bit-exactness under every group is tests/test_gpu_env_layouts.py (each group forced in its own process)
 mkdir -p gpurun_out
 run() {  # config group
   CM_ENV_GROUP=$2 python bench.py --config $1 --no-cpu-baseline --no-sweep --e2e-steps 4 2>/dev/null | python -c "
