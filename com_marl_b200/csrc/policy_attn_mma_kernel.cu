@@ -77,6 +77,7 @@ __device__ __forceinline__ float tanh_fast(float x)
 // multiply-add and one special-function instruction (__expf costs six: subtract, scale, denormal range test and fix-up).
 // The rounding of m log2(e) is common to a row's keys and to its rescaling factors, so it cancels in out / (d + 1e-12 z).
 static constexpr float kLog2e = 1.4426950408889634f;
+static constexpr float kLog2Eps = -39.863137138648348f;     // log2(1e-12): the renormalisation's epsilon (comm_base_net.py:102)
 __device__ __forceinline__ float ex2_fast(float x)
 {
     float r;
@@ -132,9 +133,10 @@ __device__ __forceinline__ void score_block(float (&s)[8][4], const __half *Qh, 
 }
 
 struct StripState {               // rows g (index 0) and g + 8 (index 1) of the strip
-    float m0, m1;                 // running maximum of the scores times log2(e): the reference point of the exponentials
+    float m0, m1;                 // running maximum of the scores times log2(e): the reference point of z
+    float q0, q1;                 // running maximum of the masked-in scores times log2(e): the reference point of d and out
     float z0, z1;                 // this lane's part of sum exp(s - m)
-    float d0, d1;                 // this lane's part of sum mask exp(s - m)
+    float d0, d1;                 // this lane's part of sum mask exp(s - q)
 };
 
 // one block of U key tiles of a strip: scores, running maximum + rescaling, exp, mask, aggregation into oacc
@@ -145,34 +147,45 @@ __device__ __forceinline__ void attn_block(StripState &st, float (&oacc)[8][4], 
 {
     float s[8][4];
     score_block<U>(s, Qh, Ql, Eh, El, nt0, g, t);
-    float bm0 = -1e30f, bm1 = -1e30f;
-#pragma unroll
-    for (int u = 0; u < U; ++u) {
-        const int key = 8 * (nt0 + u) + 2 * t;
-        if (key < n) { bm0 = fmaxf(bm0, s[u][0]); bm1 = fmaxf(bm1, s[u][2]); }
-        if (key + 1 < n) { bm0 = fmaxf(bm0, s[u][1]); bm1 = fmaxf(bm1, s[u][3]); }
-    }
-    // st.m0 / st.m1 hold the running maximum in the log2 domain (x -> fl(x log2(e)) is monotone: it commutes with the maximum)
-    const float ms0 = fmaxf(st.m0, quad_max(bm0) * kLog2e), ms1 = fmaxf(st.m1, quad_max(bm1) * kLog2e);
-    const float sc0 = ex2_fast(st.m0 - ms0), sc1 = ex2_fast(st.m1 - ms1);
-    st.m0 = ms0; st.m1 = ms1;
-    st.z0 *= sc0; st.d0 *= sc0; st.z1 *= sc1; st.d1 *= sc1;
-#pragma unroll
-    for (int ot = 0; ot < 8; ++ot) { oacc[ot][0] *= sc0; oacc[ot][1] *= sc0; oacc[ot][2] *= sc1; oacc[ot][3] *= sc1; }
-    // exp, mask (comm_base_net.py:101): the masked, un-normalised rows stay in the accumulators
+    float bm0 = -1e30f, bm1 = -1e30f, bq0 = -1e30f, bq1 = -1e30f;
+    uint32_t w0[U], w1[U];                                      // mask bits of keys 2t, 2t + 1 of each tile (beyond the team: 0)
 #pragma unroll
     for (int u = 0; u < U; ++u) {
         const int nt = nt0 + u, key = 8 * nt + 2 * t;
+        const uint32_t valid = key + 1 < n ? 3u : (key < n ? 1u : 0u);
+        w0[u] = (Mw[g * 8 + (nt >> 2)] >> (8 * (nt & 3) + 2 * t)) & valid;
+        w1[u] = (Mw[(g + 8) * 8 + (nt >> 2)] >> (8 * (nt & 3) + 2 * t)) & valid;
+        if (key < n) { bm0 = fmaxf(bm0, s[u][0]); bm1 = fmaxf(bm1, s[u][2]); }
+        if (key + 1 < n) { bm0 = fmaxf(bm0, s[u][1]); bm1 = fmaxf(bm1, s[u][3]); }
+        if (w0[u] & 1u) bq0 = fmaxf(bq0, s[u][0]);
+        if (w0[u] & 2u) bq0 = fmaxf(bq0, s[u][1]);
+        if (w1[u] & 1u) bq1 = fmaxf(bq1, s[u][2]);
+        if (w1[u] & 2u) bq1 = fmaxf(bq1, s[u][3]);
+    }
+    // the running maxima in the log2 domain (x -> fl(x log2(e)) is monotone: it commutes with the maximum)
+    const float ms0 = fmaxf(st.m0, quad_max(bm0) * kLog2e), ms1 = fmaxf(st.m1, quad_max(bm1) * kLog2e);
+    const float mq0 = fmaxf(st.q0, quad_max(bq0) * kLog2e), mq1 = fmaxf(st.q1, quad_max(bq1) * kLog2e);
+    const float sc0 = ex2_fast(st.m0 - ms0), sc1 = ex2_fast(st.m1 - ms1);
+    const float sq0 = ex2_fast(st.q0 - mq0), sq1 = ex2_fast(st.q1 - mq1);
+    // exp(s - m) -> exp(s - q) for the masked-in keys; capped at 2^126 (finite): a masked-in key 2^-126 below the maximum
+    // has flushed to zero already, and so then has every other masked-in key — their sum is nothing next to 1e-12
+    const float f0 = ex2_fast(fminf(ms0 - mq0, 126.0f)), f1 = ex2_fast(fminf(ms1 - mq1, 126.0f));
+    st.m0 = ms0; st.m1 = ms1; st.q0 = mq0; st.q1 = mq1;
+    st.z0 *= sc0; st.d0 *= sq0; st.z1 *= sc1; st.d1 *= sq1;
+#pragma unroll
+    for (int ot = 0; ot < 8; ++ot) { oacc[ot][0] *= sq0; oacc[ot][1] *= sq0; oacc[ot][2] *= sq1; oacc[ot][3] *= sq1; }
+    // exp, mask (comm_base_net.py:101): the masked, un-normalised rows stay in the accumulators
+#pragma unroll
+    for (int u = 0; u < U; ++u) {
+        const int key = 8 * (nt0 + u) + 2 * t;
         const float e00 = key < n ? ex2_fast(fmaf(s[u][0], kLog2e, -ms0)) : 0.0f, e01 = key + 1 < n ? ex2_fast(fmaf(s[u][1], kLog2e, -ms0)) : 0.0f;
         const float e10 = key < n ? ex2_fast(fmaf(s[u][2], kLog2e, -ms1)) : 0.0f, e11 = key + 1 < n ? ex2_fast(fmaf(s[u][3], kLog2e, -ms1)) : 0.0f;
         st.z0 += e00 + e01;
         st.z1 += e10 + e11;
-        const uint32_t w0 = Mw[g * 8 + (nt >> 2)] >> (8 * (nt & 3) + 2 * t);
-        const uint32_t w1 = Mw[(g + 8) * 8 + (nt >> 2)] >> (8 * (nt & 3) + 2 * t);
-        s[u][0] = (w0 & 1u) ? e00 : 0.0f;
-        s[u][1] = (w0 & 2u) ? e01 : 0.0f;
-        s[u][2] = (w1 & 1u) ? e10 : 0.0f;
-        s[u][3] = (w1 & 2u) ? e11 : 0.0f;
+        s[u][0] = (w0[u] & 1u) ? e00 * f0 : 0.0f;
+        s[u][1] = (w0[u] & 2u) ? e01 * f0 : 0.0f;
+        s[u][2] = (w1[u] & 1u) ? e10 * f1 : 0.0f;
+        s[u][3] = (w1[u] & 2u) ? e11 * f1 : 0.0f;
         st.d0 += s[u][0] + s[u][1];
         st.d1 += s[u][2] + s[u][3];
     }
@@ -228,10 +241,12 @@ __device__ __forceinline__ void attn_record_block(float *att0, float *att1, bool
 // A strip's n keys are walked in BLOCKS of 64 (flash-attention style) so that a warp holds 8 score tiles at a time instead
 // of n / 8: 16 warps of <= 128 registers share an env instead of 8 warps of 248 — the strip is a dependent chain of HMMAs
 // and shuffles, and the number of chains in flight is what the tensor pipe's utilisation follows.  Running per row:
-// m (max), z = sum exp(s - m), d = sum mask exp(s - m), out = sum mask exp(s - m) V; a larger maximum rescales z, d and out.
-// The reference's softmax -> mask -> renormalise (comm_base_net.py:101-103) is then
-//   A~ V = out / (d + 1e-12 z)        (p = exp(s - m) / z;  A~ = p mask / (sum p mask + 1e-12))
-// exactly, in fp32.  The unmasked softmax itself (agent_infos['attention_weights']) is written, when asked for, by a second
+// m (max), z = sum exp(s - m), q (max over the masked-in keys), d = sum mask exp(s - q), out = sum mask exp(s - q) V; a
+// larger maximum rescales z, or d and out.  The reference's softmax -> mask -> renormalise (comm_base_net.py:101-103) is then
+//   A~ V = out / (d + 1e-12 z 2^(m - q))        (p = exp(s - m) / z;  A~ = p mask / (sum p mask + 1e-12))
+// exactly, in fp32.  Taking the masked-in weights against their own maximum keeps the largest at 1: against m they can be
+// far below one once the masks remove the keys that carry the attention mass, and their fp16 hi / lo split would lose its
+// relative precision (or flush to zero) before the division by their small sum.  The unmasked softmax itself (agent_infos['attention_weights']) is written, when asked for, by a second
 // walk over the blocks with the final m and z.
 template <int NS, int WARPS>
 __global__ void __launch_bounds__(WARPS * 32, 1) policy_attn_mma_kernel(const AttnMmaArgs A)
@@ -337,7 +352,7 @@ __global__ void __launch_bounds__(WARPS * 32, 1) policy_attn_mma_kernel(const At
                 }
                 __syncwarp();
                 const bool v0 = i0 + g < n, v1 = i0 + g + 8 < n;
-                StripState st = {-1e30f, -1e30f, 0.0f, 0.0f, 0.0f, 0.0f};
+                StripState st = {-1e30f, -1e30f, -1e30f, -1e30f, 0.0f, 0.0f, 0.0f, 0.0f};
                 float oacc[8][4];
 #pragma unroll
                 for (int ot = 0; ot < 8; ++ot) oacc[ot][0] = oacc[ot][1] = oacc[ot][2] = oacc[ot][3] = 0.0f;
@@ -345,7 +360,9 @@ __global__ void __launch_bounds__(WARPS * 32, 1) policy_attn_mma_kernel(const At
                 for (int kb = 0; kb < NFULL; ++kb) attn_block<8>(st, oacc, Qh, Ql, Eh, El, Vh, Vl, HWP, Mw, 8 * kb, n, g, t);
                 if (TAIL) attn_block<TAIL ? TAIL : 2>(st, oacc, Qh, Ql, Eh, El, Vh, Vl, HWP, Mw, 8 * NFULL, n, g, t);
                 const float z0 = quad_sum(st.z0), z1 = quad_sum(st.z1);
-                const float den0 = 1.0f / fmaf(1e-12f, z0, quad_sum(st.d0)), den1 = 1.0f / fmaf(1e-12f, z1, quad_sum(st.d1));
+                // 1e-12 z 2^(m - q) = z 2^(m - q + log2(1e-12)); no masked-in key at all: q = -1e30, the term is inf, den = 0
+                const float den0 = 1.0f / fmaf(z0, ex2_fast(st.m0 - st.q0 + kLog2Eps), quad_sum(st.d0));
+                const float den1 = 1.0f / fmaf(z1, ex2_fast(st.m1 - st.q1 + kLog2Eps), quad_sum(st.d1));
                 // ---- the UNMASKED softmax (comm_base_net.py:93), when recorded: a second walk with the final m and z ----
                 if (l == 0 && A.attention) {
                     const float is0 = 1.0f / z0, is1 = 1.0f / z1;

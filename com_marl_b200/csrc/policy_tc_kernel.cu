@@ -424,10 +424,14 @@ __device__ __forceinline__ void softmax_tc(uint32_t lane_addr, float *red, float
     if constexpr (KT > 8) tmem_st<8>(lane_addr + kColM + (uint32_t)k0 + 8u, sc + 8);
 }
 
-// masked attention row of layer l -> B operand of the transposed aggregation (compact [128 rows][S keys], K-major) + this
-// thread's part of the row's masked sum
+// masked attention row of layer l -> B operand of the transposed aggregation (compact [128 rows][S keys], K-major), written
+// as p 2^e kPScale with 2^e the power of two that brings the row's masked maximum to [1, 2): once the masks remove the keys
+// that carry the attention mass, the remaining weights can be far below one, and without the rescaling their fp16 hi / lo
+// split loses its relative precision (or underflows to zero) before the division by their small sum.  Leaves this
+// thread's part of the row's masked sum (unscaled) in red rows 0..3 and returns 2^e in `pscale`.  Contains a CTA barrier.
 template <int KT>
-__device__ __forceinline__ float masked_p_operand(uint32_t lane_addr, unsigned char *pbuf, int S, int row, int sub, int n, uint32_t m0, uint32_t m1)
+__device__ __forceinline__ void masked_p_operand(uint32_t lane_addr, unsigned char *pbuf, float *red, int S, int row, int sub, int n,
+                                                  uint32_t m0, uint32_t m1, float &pscale)
 {
     const int k0 = sub * KT;
     float p[KT];
@@ -437,14 +441,21 @@ __device__ __forceinline__ float masked_p_operand(uint32_t lane_addr, unsigned c
     // the keys beyond the team are cleared in the mask word once (one bit test + select per key)
     const int left = n - k0;
     const uint32_t mbits = ((k0 < 32 ? m0 : m1) >> (k0 & 31)) & (left >= 32 ? 0xFFFFFFFFu : (left > 0 ? (1u << left) - 1u : 0u));
-    float den = 0.0f;
+    float den = 0.0f, mx = 0.0f;
 #pragma unroll
     for (int j = 0; j < KT; ++j) {
         p[j] = (mbits & (1u << j)) ? p[j] : 0.0f;
         den += p[j];
+        mx = fmaxf(mx, p[j]);
     }
-    write_unscaled<KT>(pbuf, S, (uint32_t)kTcRows * S * 2, row, k0, p, kPScale);
-    return den;
+    red[sub * kTPitch + row] = den;
+    red[(4 + sub) * kTPitch + row] = mx;
+    __syncthreads();
+    mx = fmaxf(fmaxf(red[4 * kTPitch + row], red[5 * kTPitch + row]), fmaxf(red[6 * kTPitch + row], red[7 * kTPitch + row]));
+    // 2^(127 - exponent of mx); rows whose masked weights are all below 2^-107 (a masked sum that is nothing next to the
+    // renormalisation's 1e-12) keep 2^107, so that 2^e kPScale stays finite
+    pscale = mx > 0.0f ? __int_as_float((254 - max(__float_as_int(mx) >> 23, 20)) << 23) : 1.0f;
+    write_unscaled<KT>(pbuf, S, (uint32_t)kTcRows * S * 2, row, k0, p, kPScale * pscale);
 }
 
 // bias offsets inside the shared-memory bias table
@@ -921,10 +932,10 @@ __global__ void __launch_bounds__(kTcThreads, 2) policy_tc_kernel(const TcArgs A
         const int n_slots = kTcRows >> slog;                                // envs per tile
         for (int l = 0; l < L; ++l) {
             // A_l = M * Range * chan_l (comm_base_net.py:101): this thread's keys -> B operand rows in ACT (E / H_l are dead
-            // there); the row's masked sum through one exchange
-            const float dpart = S == 32 ? masked_p_operand<8>(lane_addr, ACT, S, row, sub, n, m0, m1)
-                                        : masked_p_operand<16>(lane_addr, ACT, S, row, sub, n, m0, m1);
-            red[sub * kTPitch + row] = dpart;
+            // there); the row's masked sum and maximum through one exchange
+            float pscale;
+            if (S == 32) masked_p_operand<8>(lane_addr, ACT, red, S, row, sub, n, m0, m1, pscale);
+            else masked_p_operand<16>(lane_addr, ACT, red, S, row, sub, n, m0, m1, pscale);
             // out_e^T [64 x S] = V_e^T [64 x S keys] A_e^T [S keys x S rows] for every env slot e, three fp16 products each
             // into ONE accumulator (columns e S .. of R1; row c of the result = lane 32 (c / 16) + c % 16)
             run_slots(n_slots, [&](int e, uint32_t leader) {
@@ -964,8 +975,9 @@ __global__ void __launch_bounds__(kTcThreads, 2) policy_tc_kernel(const TcArgs A
                 __syncthreads();
                 fence_after_thread_sync();
             }
-            // H_{l+1} = tanh(out / (sum + 1e-12) + b) for this thread's 16 columns (graph_conv_module.py:51-72)
-            const float inv = __fdividef(kTanhScale * kPVUnscale, den + 1e-12f);
+            // H_{l+1} = tanh(out / (sum + 1e-12) + b) for this thread's 16 columns (graph_conv_module.py:51-72); out carries
+            // the row's scale 2^e, the sum does not (an exact power-of-two factor: (sum + 1e-12) 2^e <= 2 n + 2^107 1e-12)
+            const float inv = __fdividef(kTanhScale * kPVUnscale, (den + 1e-12f) * pscale);
             float v[16];
             const float4 *bp = reinterpret_cast<const float4 *>(bias_s + kBGcn + l * 64 + 16 * sub);
             const float4 *Tr = reinterpret_cast<const float4 *>(KV + row * 64);

@@ -282,9 +282,10 @@ class OracleVecEnv:
 # policy forward, numpy float32 (comm_categorical_mlp_policy.py:48-96, comm_base_net.py:80-108,
 # attention_module.py:38-49, graph_conv_module.py:51-72, categorical_mlp_module.py:64-80)
 # ------------------------------------------------------------------------------------------------
-def policy_forward(w, obs, avail, adj, chan, dtype=np.float32):
+def policy_forward(w, obs, avail, adj, chan, dtype=np.float32, residual=True):
     """w: dict keyed like the reference state_dict; obs (B,n,D); avail (B,n,5) or None;
-    adj (B,n,n); chan (B,L,n,n).  Returns logits, masked probs, attention (unmasked softmax)."""
+    adj (B,n,n); chan (B,L,n,n).  residual=False feeds H_L alone to the head (comm_base_net.py:105-106); a GCN layer
+    without a `bias` entry has no bias.  Returns logits, masked probs, attention (unmasked softmax)."""
     f = dtype
     g = lambda k: np.asarray(w[k], dtype=f)  # noqa: E731
     x = np.asarray(obs, dtype=f)
@@ -301,8 +302,9 @@ def policy_forward(w, obs, avail, adj, chan, dtype=np.float32):
     for l in range(L):
         A = M * np.asarray(adj, dtype=f) * np.asarray(chan[:, l], dtype=f)
         A = A / (A.sum(axis=-1, keepdims=True) + f(1e-12))
-        H = np.tanh(A @ (H @ g(f"gcn_layers.{l}.weight")) + g(f"gcn_layers.{l}.bias"))
-    X = E + H
+        bias = g(f"gcn_layers.{l}.bias") if f"gcn_layers.{l}.bias" in w else f(0)
+        H = np.tanh(A @ (H @ g(f"gcn_layers.{l}.weight")) + bias)
+    X = E + H if residual else H
     for i in range(3):
         X = np.tanh(X @ g(f"categorical_output_layer._layers.{i}.linear.weight").T
                     + g(f"categorical_output_layer._layers.{i}.linear.bias"))
