@@ -16,13 +16,15 @@ CH_FC, CH_FL, CH_IID, CH_GE = 0, 1, 2, 3
 POLICY_COMM, POLICY_DEC, POLICY_CENT = 0, 1, 2
 POLICY_FLAG_RELU = 1
 MAX_AGENTS, MAX_GRID, MAX_LAYERS = 256, 64, 4
-ABI_VERSION = 3
+ABI_VERSION = 4
 
 EXPORTS = ("cm_abi_version", "cm_strerror", "cm_last_cuda_error", "cm_device_count", "cm_env_reset", "cm_env_step",
            "cm_comm_update", "cm_policy_forward", "cm_policy_blob_floats", "cm_policy_cent_blob_floats", "cm_policy_cent_tc_blob_floats", "cm_policy_cent_workspace_bytes", "cm_policy_workspace_bytes", "cm_policy_tc_blob_floats", "cm_policy_tc_prepare", "cm_mask_pack",
            "cm_mask_unpack", "cm_policy_forward_host", "cm_env_step_host", "cm_env_reset_host", "cm_rollout_step_host", "cm_ppo_advantages",
-           "cm_adam_step", "cm_adam_step_dev", "cm_critic_blob_floats", "cm_ppo_net_workspace_floats", "cm_ppo_net")
-NET_POLICY, NET_CRITIC, NET_POLICY_DEC = 0, 1, 2
+           "cm_adam_step", "cm_adam_step_dev", "cm_critic_blob_floats", "cm_baseline_mlp_blob_floats", "cm_ppo_net_workspace_floats",
+           "cm_ppo_net")
+NET_POLICY, NET_CRITIC, NET_POLICY_DEC, NET_POLICY_CENT, NET_BASELINE_MLP = 0, 1, 2, 3, 4
+NET_FLAG_RELU = 1
 
 
 class EnvDesc(C.Structure):
@@ -66,7 +68,7 @@ class PolicyIO(C.Structure):
 
 class NetDesc(C.Structure):
     _fields_ = [(k, C.c_int32) for k in ("kind", "n_agents", "obs_dim", "n_layers", "residual")] + \
-               [(k, C.c_float) for k in ("ent_coeff", "clip_lo", "clip_hi")]
+               [(k, C.c_float) for k in ("ent_coeff", "clip_lo", "clip_hi")] + [("flags", C.c_int32)]
 
 
 class NetIO(C.Structure):
@@ -135,6 +137,8 @@ def lib():
                                    C.c_float, C.c_int32, C.c_void_p, C.c_void_p]
     L.cm_critic_blob_floats.restype = C.c_size_t
     L.cm_critic_blob_floats.argtypes = [C.c_int32, C.c_int32]
+    L.cm_baseline_mlp_blob_floats.restype = C.c_size_t
+    L.cm_baseline_mlp_blob_floats.argtypes = [C.c_int32]
     L.cm_ppo_net_workspace_floats.restype = C.c_size_t
     L.cm_ppo_net_workspace_floats.argtypes = [C.POINTER(NetDesc), C.c_int64, C.c_int32]
     L.cm_ppo_net.restype = C.c_int

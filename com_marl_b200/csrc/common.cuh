@@ -103,4 +103,36 @@ __device__ __forceinline__ void categorical_finish(const cm_policy_desc &d, cons
     io.actions[g] = (int8_t)act;
 }
 
+// acc[4][4*J] += A[rows 4ty..][k0..k0+kc) * Bs[k][cols], Bs pitch = 64*J, kc a multiple of 4 (zero padded): the register-tiled fp32
+// product of the CENT policy's layers (policy_cent_kernel.cu) and of the update's wide first layer (ppo_net_kernels.cu).  Thread (ty, tx)
+// of a 16 x 16 grid owns rows 4ty..4ty+3 and the columns {4tx..4tx+3} + 64j
+template <int J>
+__device__ __forceinline__ void cent_mac(const float *__restrict__ As, int lda, const float *__restrict__ Bs, int kc, int ty, int tx,
+                                         float (&acc)[4][4 * J])
+{
+#pragma unroll 2
+    for (int k = 0; k < kc; k += 4) {
+        float4 a[4];
+#pragma unroll
+        for (int i = 0; i < 4; ++i) a[i] = *reinterpret_cast<const float4 *>(As + (ty * 4 + i) * lda + k);
+#pragma unroll
+        for (int kk = 0; kk < 4; ++kk) {
+            float4 b[J];
+#pragma unroll
+            for (int j = 0; j < J; ++j) b[j] = *reinterpret_cast<const float4 *>(Bs + (k + kk) * (64 * J) + j * 64 + tx * 4);
+#pragma unroll
+            for (int i = 0; i < 4; ++i) {
+                const float av = kk == 0 ? a[i].x : (kk == 1 ? a[i].y : (kk == 2 ? a[i].z : a[i].w));
+#pragma unroll
+                for (int j = 0; j < J; ++j) {
+                    acc[i][4 * j + 0] = fmaf(av, b[j].x, acc[i][4 * j + 0]);
+                    acc[i][4 * j + 1] = fmaf(av, b[j].y, acc[i][4 * j + 1]);
+                    acc[i][4 * j + 2] = fmaf(av, b[j].z, acc[i][4 * j + 2]);
+                    acc[i][4 * j + 3] = fmaf(av, b[j].w, acc[i][4 * j + 3]);
+                }
+            }
+        }
+    }
+}
+
 }  // namespace cm

@@ -1,8 +1,10 @@
 // ppo_net_kernels.cu — hand-written forward + backward of the comm-GNN for the PPO update (SURVEY.md §8f.1): the policy
 // network of CommCategoricalMLPPolicy (comm_categorical_mlp_policy.py:48-96, comm_base_net.py:80-108) with the clipped
 // surrogate / entropy objective of CentralizedMAPPO._compute_loss (centralized_ma_ppo.py:390-438, 540-589), and the value
-// network of CommBaseCritic (comm_base_critic.py:11-120) with its Gaussian negative log-likelihood loss.  Replaces the torch
-// autograd graph (~150 library kernels per optimizer step) by ~30 launches of six kernels, all exact fp32 (FFMA):
+// network of CommBaseCritic (comm_base_critic.py:11-120) with its Gaussian negative log-likelihood loss; the same for the
+// Obs-DP policy, and for the CENT family: CentralizedCategoricalMLPPolicy (centralized_categorical_mlp_policy.py:61-97) and
+// GaussianMLPBaseline (gaussian_mlp_baseline.py:83-117), one MLP over the concatenated observation with rows = env steps.
+// Replaces the torch autograd graph (~150 library kernels per optimizer step) by ~30 launches of these kernels, all exact fp32 (FFMA):
 //
 //   net_dense_fwd     Y = act(X W + b)              rows x K x N register-tiled product, K <= 128, N in {32, 64, 128}
 //   net_dense_bwd     dZ = dY (1 - Y^2);  dX (+)= dZ W^T;  dW += X^T dZ;  db += sum dZ        (one pass over the rows)
@@ -12,6 +14,8 @@
 //   net_softmax_bwd   dS = M (dM - <dM, M>);  dQ = dS E;  dE += dS^T Q
 //   net_policy_head   logits = g3 W4 + b4 -> softmax -> availability mask -> log-likelihood, entropy, clipped objective,
 //                     d logits -> d g3, dW4, db4      net_critic_head: V(s) = sum_i (c1_i w2 + b2), Gaussian NLL, gradients
+//   net_wide_fwd      CENT first layer Y = act(X W1 + b1), K = n*D up to 32 768          net_wide_dw   dW1 += X^T dZ1, db1 (and dW4)
+//   net_cent_head     CENT logits [S][5n] = h3 W4 + b4 -> the per-agent tail of net_policy_head -> d logits, db4, dh3
 //
 // The n x n parts work on strips of 8 query rows per warp (register tiles of 8 rows x n/32 keys per lane for the dot
 // products; coefficient strips staged through shared memory for the aggregations); a CTA owns as many whole envs as fit
@@ -36,7 +40,7 @@ static constexpr int kNetThreads = 256; // head kernels: one thread per row
 // ------------------------------------------------------------------------------------------------------------------
 // ASYNC: the X tiles (rows of K floats, 16-byte aligned) arrive by one bulk async copy per row (cp.async.bulk, mbarrier
 // complete_tx) into a two-stage ring: the next tile is in flight while the products of the current one run.  Unaligned inputs
-// (the observation rows, D floats) take the synchronous load.
+// (the observation rows, D floats) take the synchronous load.  ACT: 0 none, 1 tanh, 2 relu.
 template <int N, int ACT, int ASYNC>
 __global__ void __launch_bounds__(256) net_dense_fwd_kernel(const float *__restrict__ X, int ldx, const float *__restrict__ W,
                                                             const float *__restrict__ bias, float *__restrict__ Y, int ldy, int64_t R, int K)
@@ -123,7 +127,8 @@ __global__ void __launch_bounds__(256) net_dense_fwd_kernel(const float *__restr
                 o.y = acc[i][4 * j + 1] + bj[4 * j + 1];
                 o.z = acc[i][4 * j + 2] + bj[4 * j + 2];
                 o.w = acc[i][4 * j + 3] + bj[4 * j + 3];
-                if (ACT) { o.x = tanhf(o.x); o.y = tanhf(o.y); o.z = tanhf(o.z); o.w = tanhf(o.w); }
+                if (ACT == 1) { o.x = tanhf(o.x); o.y = tanhf(o.y); o.z = tanhf(o.z); o.w = tanhf(o.w); }
+                if (ACT == 2) { o.x = fmaxf(o.x, 0.0f); o.y = fmaxf(o.y, 0.0f); o.z = fmaxf(o.z, 0.0f); o.w = fmaxf(o.w, 0.0f); }
                 *reinterpret_cast<float4 *>(Y + gr * ldy + 4 * tx + 64 * j) = o;
             }
         }
@@ -132,15 +137,16 @@ __global__ void __launch_bounds__(256) net_dense_fwd_kernel(const float *__restr
 }
 
 // One pass over the rows for the three gradients of Y = X W + b given dZ = dL/d(X W + b):
-//   dX[r][k] = ((accumulate ? dX[r][k] : 0) + sum_n dZ[r][n] W[k][n]) * (xact ? 1 - X[r][k]^2 : 1)
+//   dX[r][k] = ((accumulate ? dX[r][k] : 0) + sum_n dZ[r][n] W[k][n]) * (xact ? act'(X[r][k]) : 1),  act' = 1 - X^2 (tanh) or,
+//              with XRELU, [X > 0] (relu)
 //   dW[k][n] += sum_r X[r][k] dZ[r][n];   db[n] += sum_r dZ[r][n].
-// xact folds the tanh derivative of the layer BELOW into the hand-over (X is that layer's output and already sits in
+// xact folds the activation derivative of the layer BELOW into the hand-over (X is that layer's output and already sits in
 // shared memory), so every backward layer reads plain dZ rows.  16 warps: warps 0-7 form the dX tile while warps 8-15 reduce
 // dW / db over the same tile in shared memory (two independent FMA streams on one copy of the operands); dW / db stay in
 // registers over the tiles of a persistent CTA and are added to global memory once.  ASYNC: dZ and X tiles arrive by one bulk
 // async copy per row into a two-stage ring (the next tile is in flight during the products); unaligned X rows (the
 // observations) take the synchronous load.  ROWS = rows per tile (128, or 64 where two stages of 128 do not fit).
-template <int N, int KMAX, int ROWS, int ASYNC>
+template <int N, int KMAX, int ROWS, int ASYNC, int XRELU = 0>
 __global__ void __launch_bounds__(512) net_dense_bwd_kernel(const float *__restrict__ dZ, const float *__restrict__ X, int ldx,
                                                             const float *__restrict__ W, float *__restrict__ dX, int lddx, int accumulate,
                                                             int xact, float *__restrict__ dW, float *__restrict__ db, int64_t R, int K)
@@ -253,7 +259,7 @@ __global__ void __launch_bounds__(512) net_dense_bwd_kernel(const float *__restr
                         const int k = kx + 16 * j;
                         if (k < K) {
                             float v = old[i * KJ + j] + acc[i * KJ + j];
-                            if (xact) { const float x = Xs[r * KP + k]; v *= 1.0f - x * x; }
+                            if (xact) { const float x = Xs[r * KP + k]; if (XRELU) v = x > 0.0f ? v : 0.0f; else v *= 1.0f - x * x; }
                             dX[(r0 + r) * lddx + k] = v;
                         }
                     }
@@ -989,18 +995,97 @@ __global__ void __launch_bounds__(kSmallRows) net_small_softmax_bwd_kernel(const
 // heads + losses
 // ------------------------------------------------------------------------------------------------------------------
 struct PolicyHeadArgs {
-    const float *g3;             // [R][32] last hidden layer
-    const float *w4, *b4;        // [32][5], [5]
+    const float *g3;             // [R][32] last hidden layer (CENT: [S][32])
+    const float *w4, *b4;        // [32][5], [5]  (CENT: [32][5n], [5n])
     const uint8_t *avail_bits;   // [R] or NULL
     const int64_t *actions;      // [R] or NULL (forward only: no log-likelihood)
     const float *adv, *old_ll;   // [S]
     const uint8_t *valid;        // [S] or NULL
     float inv_count, ent_coeff, clip_lo, clip_hi;
     float *ll, *ent, *probs, *loss;
-    float *dg3, *dw4, *db4;      // NULL: forward only; dg3 receives dZ of the last hidden layer: d g3 (1 - g3^2)
+    float *dg3, *dw4, *db4;      // NULL: forward only; dg3 receives dZ of the last hidden layer: d g3 act'(g3)
+    float *dlogits;              // CENT: [S][5n] d logits for the dW4 product
+    int relu;                    // CENT: act = relu instead of tanh
     int n, G;
     int64_t S;
 };
+
+static constexpr float kProbEps = 1.1920928955078125e-07f;   // torch.finfo(float32).eps: probs_to_logits clamps to [eps, 1 - eps]
+
+// One agent's categorical tail from its five logits z: softmax p, availability mask, renormalisation q = masked / masked.sum()
+// (no + 1e-12), the clamped logs lc that Categorical(probs=q) uses, entropy and log-likelihood of `act`
+__device__ __forceinline__ void head_tail_fwd(const float (&z)[CM_ACTIONS], uint32_t av, int act, float (&p)[CM_ACTIONS],
+                                              float (&q)[CM_ACTIONS], float (&lc)[CM_ACTIONS], float &msum, float &ent, float &lp)
+{
+    float mx = -INFINITY;
+#pragma unroll
+    for (int j = 0; j < CM_ACTIONS; ++j) mx = fmaxf(mx, z[j]);
+    float sum = 0.0f;
+#pragma unroll
+    for (int j = 0; j < CM_ACTIONS; ++j) { p[j] = expf(z[j] - mx); sum += p[j]; }
+    msum = 0.0f;
+#pragma unroll
+    for (int j = 0; j < CM_ACTIONS; ++j) { p[j] = p[j] / sum; q[j] = ((av >> j) & 1u) ? p[j] : 0.0f; msum += q[j]; }
+    ent = 0.0f;
+#pragma unroll
+    for (int j = 0; j < CM_ACTIONS; ++j) {
+        q[j] = q[j] / msum;
+        lc[j] = logf(fminf(fmaxf(q[j], kProbEps), 1.0f - kProbEps));
+        ent -= q[j] * lc[j];
+    }
+    lp = 0.0f;
+#pragma unroll
+    for (int j = 0; j < CM_ACTIONS; ++j) if (j == act) lp = lc[j];
+}
+
+// d loss / d z of one agent, given gl = d loss / d ll and ge = d loss / d (its entropy term): through the clamp of probs_to_logits
+// (the gradient passes inside [eps, 1 - eps]), the renormalisation and the softmax
+__device__ __forceinline__ void head_tail_bwd(float gl, float ge, int act, uint32_t av, const float (&p)[CM_ACTIONS],
+                                              const float (&q)[CM_ACTIONS], const float (&lc)[CM_ACTIONS], float msum,
+                                              float (&gz)[CM_ACTIONS])
+{
+    float gq[CM_ACTIONS];
+    float proj = 0.0f;
+#pragma unroll
+    for (int j = 0; j < CM_ACTIONS; ++j) {
+        const float in = (q[j] >= kProbEps && q[j] <= 1.0f - kProbEps) ? 1.0f : 0.0f;
+        gq[j] = ge * (-lc[j] - in);
+        if (j == act) gq[j] += gl * (in > 0.0f ? 1.0f / q[j] : 0.0f);
+        proj = fmaf(gq[j], q[j], proj);
+    }
+    float dot = 0.0f;
+    float gp[CM_ACTIONS];
+#pragma unroll
+    for (int j = 0; j < CM_ACTIONS; ++j) {
+        gp[j] = ((av >> j) & 1u) ? (gq[j] - proj) / msum : 0.0f;
+        dot = fmaf(gp[j], p[j], dot);
+    }
+#pragma unroll
+    for (int j = 0; j < CM_ACTIONS; ++j) gz[j] = p[j] * (gp[j] - dot);
+}
+
+// One env step s with joint log-likelihood ll and mean entropy en: outputs, the clipped surrogate added to the loss and the
+// gradients gl = d loss / d ll, ge = d loss / d (one agent's entropy)
+__device__ __forceinline__ void head_step_objective(const PolicyHeadArgs &a, int64_t s, float ll, float en, int n, float &gl, float &ge)
+{
+    if (a.ll) a.ll[s] = ll;
+    if (a.ent) a.ent[s] = en;
+    gl = 0.0f;
+    ge = 0.0f;
+    const bool valid = a.valid ? a.valid[s] != 0 : true;
+    if (a.adv && valid) {
+        const float old = a.old_ll ? a.old_ll[s] : ll;
+        const float ratio = expf(ll - old), adv = a.adv[s];
+        const float rc = fminf(fmaxf(ratio, a.clip_lo), a.clip_hi);
+        const float s1 = ratio * adv, s2 = rc * adv;
+        const float in = (ratio >= a.clip_lo && ratio <= a.clip_hi) ? 1.0f : 0.0f;
+        // torch.min's gradient goes to the smaller argument, half to each on a tie; clamp passes it inside [lo, hi]
+        const float gr = s1 < s2 ? adv : (s1 > s2 ? adv * in : 0.5f * adv + 0.5f * adv * in);
+        if (a.loss) atomicAdd(a.loss, -(fminf(s1, s2) + a.ent_coeff * en) * a.inv_count);
+        gl = -a.inv_count * gr * ratio;
+        ge = -a.inv_count * a.ent_coeff / (float)n;
+    }
+}
 
 __global__ void __launch_bounds__(kNetThreads) net_policy_head_kernel(const PolicyHeadArgs a)
 {
@@ -1009,7 +1094,6 @@ __global__ void __launch_bounds__(kNetThreads) net_policy_head_kernel(const Poli
     __shared__ float red[32 * CM_ACTIONS + CM_ACTIONS];
     const int tid = threadIdx.x, lane = tid & 31;
     const int n = a.n;
-    const float eps = 1.1920928955078125e-07f;                   // torch.finfo(float32).eps: probs_to_logits clamps to [eps, 1 - eps]
     for (int i = tid; i < 32 * CM_ACTIONS + CM_ACTIONS; i += kNetThreads) {
         w4s[i] = i < 32 * CM_ACTIONS ? a.w4[i] : a.b4[i - 32 * CM_ACTIONS];
         red[i] = 0.0f;
@@ -1035,27 +1119,12 @@ __global__ void __launch_bounds__(kNetThreads) net_policy_head_kernel(const Poli
             for (int k = 0; k < 32; ++k)
 #pragma unroll
                 for (int j = 0; j < CM_ACTIONS; ++j) z[j] = fmaf(g[k], w4s[k * CM_ACTIONS + j], z[j]);
-            float mx = -INFINITY;
 #pragma unroll
-            for (int j = 0; j < CM_ACTIONS; ++j) { z[j] += w4s[32 * CM_ACTIONS + j]; mx = fmaxf(mx, z[j]); }
-            float sum = 0.0f;
-#pragma unroll
-            for (int j = 0; j < CM_ACTIONS; ++j) { p[j] = expf(z[j] - mx); sum += p[j]; }
+            for (int j = 0; j < CM_ACTIONS; ++j) z[j] += w4s[32 * CM_ACTIONS + j];
             if (a.avail_bits) av = a.avail_bits[row];
-            msum = 0.0f;
-#pragma unroll
-            for (int j = 0; j < CM_ACTIONS; ++j) { p[j] = p[j] / sum; q[j] = ((av >> j) & 1u) ? p[j] : 0.0f; msum += q[j]; }
-            float ent = 0.0f;
-#pragma unroll
-            for (int j = 0; j < CM_ACTIONS; ++j) {
-                q[j] = q[j] / msum;
-                lc[j] = logf(fminf(fmaxf(q[j], eps), 1.0f - eps));
-                ent -= q[j] * lc[j];
-            }
             if (a.actions) act = (int)a.actions[row];
-            float lp = 0.0f;
-#pragma unroll
-            for (int j = 0; j < CM_ACTIONS; ++j) if (j == act) lp = lc[j];
+            float ent, lp;
+            head_tail_fwd(z, av, act, p, q, lc, msum, ent, lp);
             if (active) {
                 ll_row[tid] = lp;
                 ent_row[tid] = ent;
@@ -1069,23 +1138,8 @@ __global__ void __launch_bounds__(kNetThreads) net_policy_head_kernel(const Poli
             float ll = 0.0f, en = 0.0f;
             for (int i = 0; i < n; ++i) { ll += ll_row[tid * n + i]; en += ent_row[tid * n + i]; }
             en = en / (float)n;
-            const int64_t s = eb.s0 + tid;
-            if (a.ll) a.ll[s] = ll;
-            if (a.ent) a.ent[s] = en;
-            float gl = 0.0f, ge = 0.0f;
-            const bool valid = a.valid ? a.valid[s] != 0 : true;
-            if (a.adv && valid) {
-                const float old = a.old_ll ? a.old_ll[s] : ll;
-                const float ratio = expf(ll - old), adv = a.adv[s];
-                const float rc = fminf(fmaxf(ratio, a.clip_lo), a.clip_hi);
-                const float s1 = ratio * adv, s2 = rc * adv;
-                const float in = (ratio >= a.clip_lo && ratio <= a.clip_hi) ? 1.0f : 0.0f;
-                // torch.min's gradient goes to the smaller argument, half to each on a tie; clamp passes it inside [lo, hi]
-                const float gr = s1 < s2 ? adv : (s1 > s2 ? adv * in : 0.5f * adv + 0.5f * adv * in);
-                if (a.loss) atomicAdd(a.loss, -(fminf(s1, s2) + a.ent_coeff * en) * a.inv_count);
-                gl = -a.inv_count * gr * ratio;
-                ge = -a.inv_count * a.ent_coeff / (float)n;
-            }
+            float gl, ge;
+            head_step_objective(a, eb.s0 + tid, ll, en, n, gl, ge);
             gll_env[tid] = gl;
             gent_env[tid] = ge;
         }
@@ -1095,24 +1149,10 @@ __global__ void __launch_bounds__(kNetThreads) net_policy_head_kernel(const Poli
         {
             const int e = active ? tid / n : 0;
             const float gl = active ? gll_env[e] : 0.0f, ge = active ? gent_env[e] : 0.0f;
-            float gq[CM_ACTIONS];
-            float proj = 0.0f;
+            float t[CM_ACTIONS];
+            head_tail_bwd(gl, ge, act, av, p, q, lc, msum, t);
 #pragma unroll
-            for (int j = 0; j < CM_ACTIONS; ++j) {
-                const float in = (q[j] >= eps && q[j] <= 1.0f - eps) ? 1.0f : 0.0f;
-                gq[j] = ge * (-lc[j] - in);
-                if (j == act) gq[j] += gl * (in > 0.0f ? 1.0f / q[j] : 0.0f);
-                proj = fmaf(gq[j], q[j], proj);
-            }
-            float dot = 0.0f;
-            float gp[CM_ACTIONS];
-#pragma unroll
-            for (int j = 0; j < CM_ACTIONS; ++j) {
-                gp[j] = ((av >> j) & 1u) ? (gq[j] - proj) / msum : 0.0f;
-                dot = fmaf(gp[j], p[j], dot);
-            }
-#pragma unroll
-            for (int j = 0; j < CM_ACTIONS; ++j) gz[j] = active ? p[j] * (gp[j] - dot) : 0.0f;
+            for (int j = 0; j < CM_ACTIONS; ++j) gz[j] = active ? t[j] : 0.0f;
         }
         if (active) {
             float4 *dst = reinterpret_cast<float4 *>(a.dg3 + row * 32);
@@ -1149,6 +1189,100 @@ __global__ void __launch_bounds__(kNetThreads) net_policy_head_kernel(const Poli
     }
 }
 
+// CENT head: the rows are env steps, logits [S][5n] = g3 W4 + b4 with W4 [32][5n].  Thread = (step, agent), the G = 256 / n steps
+// of a block with all their agents, like net_policy_head_kernel: a thread computes the five logits of its agent (the agent's W4
+// columns, shared by the block's steps, come through L1), the per-agent tail and, per step, the objective.  Backward: d logits go
+// to `dlogits` (dW4 is a product of its own), db4 is accumulated per thread over its blocks, and dg3 = dlogits W4^T is reduced
+// over the agents of a step in agent order through shared memory, times act'(g3).
+__global__ void __launch_bounds__(kNetThreads) net_cent_head_kernel(const PolicyHeadArgs a)
+{
+    __shared__ float ll_row[kRows], ent_row[kRows], gll_env[kRows], gent_env[kRows];
+    __shared__ float dgs[kRows * 33];
+    const int tid = threadIdx.x;
+    const int n = a.n, NO = n * CM_ACTIONS;
+    const int ia = tid % n;                                       // this thread's agent (the same in every block)
+    const float *__restrict__ w4 = a.w4 + ia * CM_ACTIONS;
+    float dbacc[CM_ACTIONS];
+#pragma unroll
+    for (int j = 0; j < CM_ACTIONS; ++j) dbacc[j] = 0.0f;
+    const int64_t nblk = (a.S + a.G - 1) / a.G;
+    for (int64_t blk = blockIdx.x; blk < nblk; blk += gridDim.x) {
+        const EnvBlock eb = env_block(blk, a.G, n, a.S);
+        __syncthreads();
+        const bool active = tid < eb.rows;
+        const int64_t s = eb.s0 + (active ? tid / n : 0), row = s * n + ia;
+        float p[CM_ACTIONS], q[CM_ACTIONS], lc[CM_ACTIONS];
+        float msum = 1.0f;
+        uint32_t av = 0x1Fu;
+        int act = 0;
+        {
+            const float4 *src = reinterpret_cast<const float4 *>(a.g3 + s * 32);
+            float z[CM_ACTIONS];
+#pragma unroll
+            for (int j = 0; j < CM_ACTIONS; ++j) z[j] = 0.0f;
+#pragma unroll
+            for (int k4 = 0; k4 < 8; ++k4) {
+                const float4 v = src[k4];
+                const float g[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+                for (int c = 0; c < 4; ++c)
+#pragma unroll
+                    for (int j = 0; j < CM_ACTIONS; ++j) z[j] = fmaf(g[c], __ldg(w4 + (size_t)(4 * k4 + c) * NO + j), z[j]);
+            }
+#pragma unroll
+            for (int j = 0; j < CM_ACTIONS; ++j) z[j] += __ldg(a.b4 + ia * CM_ACTIONS + j);
+            if (a.avail_bits) av = a.avail_bits[row];
+            if (a.actions) act = (int)a.actions[row];
+            float ent, lp;
+            head_tail_fwd(z, av, act, p, q, lc, msum, ent, lp);
+            if (active) {
+                ll_row[tid] = lp;
+                ent_row[tid] = ent;
+                if (a.probs)
+#pragma unroll
+                    for (int j = 0; j < CM_ACTIONS; ++j) a.probs[row * CM_ACTIONS + j] = q[j];
+            }
+        }
+        __syncthreads();
+        if (tid < eb.ne) {                                        // one thread per step: sums in agent order
+            float ll = 0.0f, en = 0.0f;
+            for (int i = 0; i < n; ++i) { ll += ll_row[tid * n + i]; en += ent_row[tid * n + i]; }
+            en = en / (float)n;
+            float gl, ge;
+            head_step_objective(a, eb.s0 + tid, ll, en, n, gl, ge);
+            gll_env[tid] = gl;
+            gent_env[tid] = ge;
+        }
+        if (!a.dg3) continue;
+        __syncthreads();
+        if (active) {
+            float gz[CM_ACTIONS];
+            head_tail_bwd(gll_env[tid / n], gent_env[tid / n], act, av, p, q, lc, msum, gz);
+#pragma unroll
+            for (int j = 0; j < CM_ACTIONS; ++j) { a.dlogits[s * NO + ia * CM_ACTIONS + j] = gz[j]; dbacc[j] += gz[j]; }
+#pragma unroll 4
+            for (int k = 0; k < 32; ++k) {
+                float v = 0.0f;
+#pragma unroll
+                for (int j = 0; j < CM_ACTIONS; ++j) v = fmaf(gz[j], __ldg(w4 + (size_t)k * NO + j), v);
+                dgs[tid * 33 + k] = v;
+            }
+        }
+        __syncthreads();
+        for (int e = tid; e < eb.ne * 32; e += kNetThreads) {       // (step, k): the step's agents in order
+            const int st = e >> 5, k = e & 31;
+            float v = 0.0f;
+            for (int i = 0; i < n; ++i) v += dgs[(st * n + i) * 33 + k];
+            const int64_t o = (eb.s0 + st) * 32 + k;
+            const float g = a.g3[o];
+            a.dg3[o] = a.relu ? (g > 0.0f ? v : 0.0f) : v * (1.0f - g * g);
+        }
+    }
+    if (a.dg3 && tid < a.G * n)
+#pragma unroll
+        for (int j = 0; j < CM_ACTIONS; ++j) atomicAdd(a.db4 + ia * CM_ACTIONS + j, dbacc[j]);
+}
+
 struct CriticHeadArgs {
     const float *c1;             // [R][64] decoder hidden layer
     const float *w2, *b2, *log_std;   // [64], [1], [1]
@@ -1156,6 +1290,7 @@ struct CriticHeadArgs {
     float inv_count;
     float *values, *loss;
     float *dc1, *dw2, *db2, *dlog_std;
+    int unclamped;               // 1: std = exp(log_std) without CommBaseCritic's clamp at log 1e-6 (GaussianMLPBaseline)
     int n, G;
     int64_t S;
 };
@@ -1168,7 +1303,7 @@ __global__ void __launch_bounds__(kNetThreads) net_critic_head_kernel(const Crit
     if (tid < 64) w2s[tid] = a.w2[tid];
     if (tid < 66) red[tid] = 0.0f;
     const float b2 = a.b2[0];
-    const float lmin = logf(1e-6f);
+    const float lmin = a.unclamped ? -INFINITY : logf(1e-6f);
     const float ls = a.log_std[0];
     const float lsc = fmaxf(ls, lmin), sd = expf(lsc);
     const int64_t nblk = (a.S + a.G - 1) / a.G;
@@ -1232,6 +1367,148 @@ __global__ void __launch_bounds__(kNetThreads) net_critic_head_kernel(const Crit
 }
 
 // ------------------------------------------------------------------------------------------------------------------
+// wide-K layers of the CENT family: rows are env steps, K = n*D grows with the team (87 .. 32 768)
+// ------------------------------------------------------------------------------------------------------------------
+static constexpr int kWRows = 64, kWK = 32, kWPA = kWK + 4;          // forward: rows per CTA, K chunk, pitch of the chunk
+
+// Y [R][64J] = act(X [R][K] W [K][64J] + b), act: 1 tanh, 2 relu.  The fp32 first layer of policy_cent_kernel: 64 rows per CTA, K
+// streamed through shared memory in chunks of 32 with the next chunk's global loads in flight (registers) while the current one
+// is multiplied (cent_mac).  The rows are read with 4-byte loads, one lane per k: rows K * 4 bytes apart need no alignment.
+template <int J, int ACT>
+__global__ void __launch_bounds__(256) net_wide_fwd_kernel(const float *__restrict__ X, const float *__restrict__ W,
+                                                           const float *__restrict__ bias, float *__restrict__ Y, int64_t R, int K)
+{
+    constexpr int N = 64 * J, BL = 2 * J;                            // BL: float4 of a weight chunk per thread
+    __shared__ __align__(16) float Ach[kWRows * kWPA];
+    __shared__ __align__(16) float Bch[kWK * N];
+    const int tid = threadIdx.x, ty = tid >> 4, tx = tid & 15, lane = tid & 31, warp = tid >> 5;
+    const int64_t row0 = (int64_t)blockIdx.x * kWRows;
+    const int rows = (int)min((int64_t)kWRows, R - row0);
+    const float *__restrict__ Xb = X + row0 * K;
+    float acc[4][4 * J];
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+#pragma unroll
+        for (int c = 0; c < 4 * J; ++c) acc[i][c] = 0.0f;
+    float ra[8];
+    float4 rb[BL];
+    auto fetch = [&](int k0) {
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {                                // lane = k, warp + 8j = row
+            const int r = warp + 8 * j;
+            ra[j] = (r < rows && k0 + lane < K) ? __ldg(Xb + (size_t)r * K + k0 + lane) : 0.0f;
+        }
+#pragma unroll
+        for (int j = 0; j < BL; ++j) {
+            const int e = tid + 256 * j, kk = e / (16 * J), c4 = e - kk * (16 * J);
+            rb[j] = (k0 + kk < K) ? __ldg(reinterpret_cast<const float4 *>(W + (size_t)(k0 + kk) * N + c4 * 4)) : make_float4(0.f, 0.f, 0.f, 0.f);
+        }
+    };
+    fetch(0);
+    for (int k0 = 0; k0 < K; k0 += kWK) {
+        __syncthreads();
+#pragma unroll
+        for (int j = 0; j < 8; ++j) Ach[(warp + 8 * j) * kWPA + lane] = ra[j];
+#pragma unroll
+        for (int j = 0; j < BL; ++j) {
+            const int e = tid + 256 * j, kk = e / (16 * J), c4 = e - kk * (16 * J);
+            *reinterpret_cast<float4 *>(Bch + kk * N + c4 * 4) = rb[j];
+        }
+        __syncthreads();
+        if (k0 + kWK < K) fetch(k0 + kWK);
+        cent_mac<J>(Ach, kWPA, Bch, kWK, ty, tx, acc);
+    }
+#pragma unroll
+    for (int j = 0; j < J; ++j) {
+        const float4 bv = __ldg(reinterpret_cast<const float4 *>(bias + j * 64 + tx * 4));
+#pragma unroll
+        for (int i = 0; i < 4; ++i) {
+            const int r = ty * 4 + i;
+            if (r >= rows) continue;
+            float4 v = make_float4(acc[i][4 * j + 0] + bv.x, acc[i][4 * j + 1] + bv.y, acc[i][4 * j + 2] + bv.z, acc[i][4 * j + 3] + bv.w);
+            if (ACT == 1) { v.x = tanhf(v.x); v.y = tanhf(v.y); v.z = tanhf(v.z); v.w = tanhf(v.w); }
+            if (ACT == 2) { v.x = fmaxf(v.x, 0.0f); v.y = fmaxf(v.y, 0.0f); v.z = fmaxf(v.z, 0.0f); v.w = fmaxf(v.w, 0.0f); }
+            *reinterpret_cast<float4 *>(Y + (row0 + r) * N + j * 64 + tx * 4) = v;
+        }
+    }
+}
+
+static constexpr int kWPanel = 64, kWTile = 32;                      // weight gradient: K panel per CTA, rows per staged tile
+
+// dW += X^T dZ over the rows [blockIdx.y * rows_per_cta, ...) and K panel blockIdx.x (64 k x all N columns); db += sum dZ (the CTAs
+// of panel 0).  X [R][K] (pitch ldx, rows unaligned: 4-byte loads), dZ [R][N].  X and dZ tiles of 32 rows are staged through shared
+// memory with the next tile's loads in flight (registers); thread (ty, tx) owns k = ty + TY i and the columns 4 tx .. 4 tx + 3, sums
+// in registers over all of the CTA's rows, and adds to global memory once.  TRANS: the result is stored transposed, dW[n][k]
+// (dW4 [32][5n] of the CENT head is (d logits)^T g3 with X = d logits, dZ = g3).
+template <int N, int TRANS>
+__global__ void __launch_bounds__(256) net_wide_dw_kernel(const float *__restrict__ X, int ldx, const float *__restrict__ dZ,
+                                                          float *__restrict__ dW, float *__restrict__ db, int64_t R, int K,
+                                                          int64_t rows_per_cta)
+{
+    constexpr int TX = N / 4, TY = 256 / TX, KI = kWPanel / TY, ZL = kWTile * N / 4 / 256;
+    __shared__ __align__(16) float Xs[kWTile * kWPanel];
+    __shared__ __align__(16) float Zs[kWTile * N];
+    const int tid = threadIdx.x, tx = tid % TX, ty = tid / TX, lane = tid & 31, warp = tid >> 5;
+    const int k0 = blockIdx.x * kWPanel;
+    const int64_t rb = (int64_t)blockIdx.y * rows_per_cta, re = min(R, rb + rows_per_cta);
+    const bool do_db = db && blockIdx.x == 0 && tid < N;
+    float acc[KI][4];
+#pragma unroll
+    for (int i = 0; i < KI; ++i) acc[i][0] = acc[i][1] = acc[i][2] = acc[i][3] = 0.0f;
+    float bacc = 0.0f;
+    float xr[8];
+    float4 zr[ZL];
+    auto fetch = [&](int64_t r0) {
+#pragma unroll
+        for (int j = 0; j < 8; ++j) {                                // rows warp + 8 (j / 2), k = lane + 32 (j % 2)
+            const int64_t r = r0 + warp + 8 * (j >> 1);
+            const int k = k0 + lane + 32 * (j & 1);
+            xr[j] = (r < re && k < K) ? __ldg(X + r * ldx + k) : 0.0f;
+        }
+#pragma unroll
+        for (int j = 0; j < ZL; ++j) {
+            const int e = tid + 256 * j, r = e / (N / 4), c4 = e - r * (N / 4);
+            zr[j] = r0 + r < re ? __ldg(reinterpret_cast<const float4 *>(dZ + (r0 + r) * N + 4 * c4)) : make_float4(0.f, 0.f, 0.f, 0.f);
+        }
+    };
+    if (rb < re) fetch(rb);
+    for (int64_t r0 = rb; r0 < re; r0 += kWTile) {
+        __syncthreads();
+#pragma unroll
+        for (int j = 0; j < 8; ++j) Xs[(warp + 8 * (j >> 1)) * kWPanel + lane + 32 * (j & 1)] = xr[j];
+#pragma unroll
+        for (int j = 0; j < ZL; ++j) reinterpret_cast<float4 *>(Zs)[tid + 256 * j] = zr[j];
+        __syncthreads();
+        if (r0 + kWTile < re) fetch(r0 + kWTile);
+#pragma unroll 4
+        for (int r = 0; r < kWTile; ++r) {                           // (rows past the end are zeros)
+            const float4 z = *reinterpret_cast<const float4 *>(Zs + r * N + 4 * tx);
+#pragma unroll
+            for (int i = 0; i < KI; ++i) {
+                const float x = Xs[r * kWPanel + ty + TY * i];
+                acc[i][0] = fmaf(x, z.x, acc[i][0]);
+                acc[i][1] = fmaf(x, z.y, acc[i][1]);
+                acc[i][2] = fmaf(x, z.z, acc[i][2]);
+                acc[i][3] = fmaf(x, z.w, acc[i][3]);
+            }
+        }
+        if (do_db) {
+            float sacc = 0.0f;
+            for (int r = 0; r < kWTile; ++r) sacc += Zs[r * N + tid];
+            bacc += sacc;
+        }
+    }
+#pragma unroll
+    for (int i = 0; i < KI; ++i) {
+        const int k = k0 + ty + TY * i;
+        if (k < K)
+#pragma unroll
+            for (int c = 0; c < 4; ++c) atomicAdd(TRANS ? dW + (size_t)(4 * tx + c) * K + k : dW + (size_t)k * N + 4 * tx + c, acc[i][c]);
+    }
+    if (do_db) atomicAdd(db + tid, bacc);
+}
+
+// ------------------------------------------------------------------------------------------------------------------
 // host side: launch helpers and the two entry points
 // ------------------------------------------------------------------------------------------------------------------
 struct CriticBlob { int enc_w1, enc_b1, enc_w2, enc_b2, att_w, gcn_w, gcn_b, dec_w1, dec_b1, dec_w2, dec_b2, log_std, total; };
@@ -1254,6 +1531,27 @@ static CriticBlob critic_blob_layout(int D, int L)
     o.total = p;
     return o;
 }
+
+// GaussianMLPBaseline(hidden_sizes <= (64, 64, 64)): w1 [K][64] b1 w2 [64][64] b2 w3 [64][64] b3 w4 [64] b4 [1] log_std [1]
+struct BaselineBlob { int w1, b1, w2, b2, w3, b3, w4, b4, log_std, total; };
+static BaselineBlob baseline_blob_layout(int K)
+{
+    BaselineBlob o;
+    int p = 0;
+    o.w1 = p; p += K * 64;
+    o.b1 = p; p += 64;
+    o.w2 = p; p += 64 * 64;
+    o.b2 = p; p += 64;
+    o.w3 = p; p += 64 * 64;
+    o.b3 = p; p += 64;
+    o.w4 = p; p += 64;
+    o.b4 = p; p += 1;
+    o.log_std = p; p += 1;
+    o.total = p;
+    return o;
+}
+
+static bool cent_kind(int kind) { return kind == CM_NET_POLICY_CENT || kind == CM_NET_BASELINE_MLP; }
 
 static int g_sms = 0;
 static int sm_count()
@@ -1302,46 +1600,80 @@ static cudaError_t dense_fwd_t(const float *X, int ldx, const float *W, const fl
 static cudaError_t dense_fwd(const float *X, int ldx, const float *W, const float *b, float *Y, int64_t R, int K, int N, int act,
                              cudaStream_t st)
 {
+    if (act == 2)                            // relu: the CENT policy's 128 -> 64 and 64 -> 32 layers
+        return N == 64 ? dense_fwd_t<64, 2>(X, ldx, W, b, Y, R, K, st) : dense_fwd_t<32, 2>(X, ldx, W, b, Y, R, K, st);
     if (N == 128) return act ? dense_fwd_t<128, 1>(X, ldx, W, b, Y, R, K, st) : dense_fwd_t<128, 0>(X, ldx, W, b, Y, R, K, st);
     if (N == 64) return act ? dense_fwd_t<64, 1>(X, ldx, W, b, Y, R, K, st) : dense_fwd_t<64, 0>(X, ldx, W, b, Y, R, K, st);
     return act ? dense_fwd_t<32, 1>(X, ldx, W, b, Y, R, K, st) : dense_fwd_t<32, 0>(X, ldx, W, b, Y, R, K, st);
 }
 
-template <int N, int KMAX, int ROWS, int ASYNC>
+template <int N, int KMAX, int ROWS, int ASYNC, int XRELU>
 static cudaError_t dense_bwd_a(const float *dZ, const float *X, int ldx, const float *W, float *dX, int accumulate, int xact, float *dW,
                                float *db, int64_t R, int K, cudaStream_t st)
 {
     const size_t smem = ((size_t)KMAX * (N + 4) + (ASYNC ? 2 : 1) * (size_t)ROWS * (N + 4 + KMAX + 4)) * sizeof(float) + 16;
-    NET_TRY(set_smem(net_dense_bwd_kernel<N, KMAX, ROWS, ASYNC>, smem));
+    NET_TRY(set_smem(net_dense_bwd_kernel<N, KMAX, ROWS, ASYNC, XRELU>, smem));
     int per_sm = 1;
-    NET_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, net_dense_bwd_kernel<N, KMAX, ROWS, ASYNC>, 512, smem));
+    NET_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, net_dense_bwd_kernel<N, KMAX, ROWS, ASYNC, XRELU>, 512, smem));
     if (per_sm < 1) per_sm = 1;
     const int64_t tiles = (R + ROWS - 1) / ROWS;
     const int grid = (int)(tiles < (int64_t)sm_count() * per_sm ? tiles : (int64_t)sm_count() * per_sm);
-    net_dense_bwd_kernel<N, KMAX, ROWS, ASYNC><<<grid, 512, smem, st>>>(dZ, X, ldx, W, dX, K, accumulate, xact, dW, db, R, K);
+    net_dense_bwd_kernel<N, KMAX, ROWS, ASYNC, XRELU><<<grid, 512, smem, st>>>(dZ, X, ldx, W, dX, K, accumulate, xact, dW, db, R, K);
     return cudaGetLastError();
 }
 
-template <int N, int KMAX>
+template <int N, int KMAX, int XRELU = 0>
 static cudaError_t dense_bwd_t(const float *dZ, const float *X, int ldx, const float *W, float *dX, int accumulate, int xact, float *dW,
                                float *db, int64_t R, int K, cudaStream_t st)
 {
     // two stages of 128-row tiles where they fit into shared memory, else of 64-row tiles
     constexpr bool fits = ((size_t)KMAX * (N + 4) + 2 * (size_t)128 * (N + 4 + KMAX + 4)) * sizeof(float) + 16 <= 227 * 1024;
-    if (!rows_aligned(X, ldx, K)) return dense_bwd_a<N, KMAX, 128, 0>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st);
-    return dense_bwd_a<N, KMAX, fits ? 128 : 64, 1>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st);
+    if (!rows_aligned(X, ldx, K)) return dense_bwd_a<N, KMAX, 128, 0, XRELU>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st);
+    return dense_bwd_a<N, KMAX, fits ? 128 : 64, 1, XRELU>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st);
 }
 
-// gradients of Y = X W + b from dZ [R][N]; dX [R][K] (lddx = K) may be NULL; xact: dX *= 1 - X^2
+// gradients of Y = X W + b from dZ [R][N]; dX [R][K] (lddx = K) may be NULL; xact: dX *= act'(X), 1 = tanh, 2 = relu (the CENT
+// policy's 64 -> 32 and 128 -> 64 layers, the only ones built for it)
 static cudaError_t dense_bwd(const float *dZ, const float *X, int ldx, const float *W, float *dX, int accumulate, int xact, float *dW,
                              float *db, int64_t R, int K, int N, cudaStream_t st)
 {
+    if (xact == 2) return N == 32 ? dense_bwd_t<32, 64, 1>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st)
+                                  : dense_bwd_t<64, 128, 1>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st);
     if (N == 128) return K <= 64 ? dense_bwd_t<128, 64>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st)
                                  : dense_bwd_t<128, 128>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st);
     if (N == 64) return K <= 64 ? dense_bwd_t<64, 64>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st)
                                 : dense_bwd_t<64, 128>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st);
     return K <= 64 ? dense_bwd_t<32, 64>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st)
                    : dense_bwd_t<32, 128>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st);
+}
+
+// wide-K layers (CENT family)
+template <int J, int ACT>
+static cudaError_t wide_fwd_t(const float *X, const float *W, const float *b, float *Y, int64_t R, int K, cudaStream_t st)
+{
+    net_wide_fwd_kernel<J, ACT><<<(unsigned)((R + kWRows - 1) / kWRows), 256, 0, st>>>(X, W, b, Y, R, K);
+    return cudaGetLastError();
+}
+// Y [R][N] = act(X [R][K] W + b), N in {64, 128}, act 1 tanh / 2 relu
+static cudaError_t wide_fwd(const float *X, const float *W, const float *b, float *Y, int64_t R, int K, int N, int act, cudaStream_t st)
+{
+    if (N == 128) return act == 2 ? wide_fwd_t<2, 2>(X, W, b, Y, R, K, st) : wide_fwd_t<2, 1>(X, W, b, Y, R, K, st);
+    return wide_fwd_t<1, 1>(X, W, b, Y, R, K, st);
+}
+// dW [K][N] (TRANS: [N][K]) += X^T dZ, db += sum dZ.  The rows are split across CTAs so that the K panels x row slices fill the SMs
+// about four CTAs deep even when K has few panels (C3: 1 696 / 64 = 27).
+template <int N, int TRANS>
+static cudaError_t wide_dw_t(const float *X, int ldx, const float *dZ, float *dW, float *db, int64_t R, int K, cudaStream_t st)
+{
+    const int panels = (K + kWPanel - 1) / kWPanel;
+    const int64_t tiles = (R + kWTile - 1) / kWTile;
+    int64_t split = ((int64_t)4 * sm_count() + panels - 1) / panels;
+    if (split > tiles) split = tiles;
+    if (split < 1) split = 1;
+    const int64_t per = (tiles + split - 1) / split * kWTile;
+    const dim3 grid((unsigned)panels, (unsigned)((R + per - 1) / per));
+    net_wide_dw_kernel<N, TRANS><<<grid, 256, 0, st>>>(X, ldx, dZ, dW, db, R, K, per);
+    return cudaGetLastError();
 }
 
 static int env_group(int n) { return n >= kRows ? 1 : kRows / n; }          // head kernels: one thread per row, 256 rows per CTA
@@ -1514,8 +1846,12 @@ static constexpr size_t kWsSlack = 160;      // alignment of the base pointer an
 struct NetWs {
     float *h1, *E, *Q, *M, *V[CM_MAX_LAYERS], *H[CM_MAX_LAYERS], *X, *g1, *g2, *g3, *t32, *t64a, *t64b, *t64c, *t128, *dM, *CT;
 };
-static size_t ws_floats_per_step(int n, int L, bool backward)
+static size_t ws_floats_per_step(const cm_net_desc &d, bool backward)
 {
+    const int n = d.n_agents, L = d.n_layers;
+    if (d.kind == CM_NET_POLICY_CENT)        // h1 h2 h3; backward: d logits, dZ3 dZ2 dZ1
+        return 128 + 64 + 32 + (backward ? 5 * (size_t)n + 32 + 64 + 128 : 0);
+    if (d.kind == CM_NET_BASELINE_MLP) return 3 * 64 + (backward ? 3 * 64 : 0);
     size_t rows = 128 + 64 + 64 + (size_t)L * 128 + 64 + 128 + 64 + 32;
     size_t sq = 1;
     if (backward) { rows += 32 + 3 * 64 + 128; sq += 1 + (size_t)L; }          // dM: one n x n array per layer
@@ -1597,8 +1933,80 @@ static Blob trunk_of(const CriticBlob &cb)
     return o;
 }
 
+// the CENT family: policy (CentralizedCategoricalMLPPolicy) or baseline (GaussianMLPBaseline) over `steps` env steps, one row per step
+static cudaError_t run_chunk_cent(const cm_net_desc &d, const cm_net_io &io, int64_t s0, int64_t steps, float *wsp, cudaStream_t st)
+{
+    const int n = d.n_agents, K = n * d.obs_dim, NO = n * CM_ACTIONS;
+    const bool backward = io.grad != nullptr;
+    const int64_t R = steps;
+    const float *obs = io.obs + s0 * K;
+    const float *wts = io.weights;
+    float *g = io.grad;
+    auto take = [&](size_t k) { float *q = wsp; wsp += (k + 3) & ~(size_t)3; return q; };      // every array 16-byte aligned
+    if (d.kind == CM_NET_BASELINE_MLP) {
+        const BaselineBlob o = baseline_blob_layout(K);
+        float *h1 = take(R * 64), *h2 = take(R * 64), *h3 = take(R * 64);
+        NET_TRY(wide_fwd(obs, wts + o.w1, wts + o.b1, h1, R, K, 64, 1, st));
+        NET_TRY(dense_fwd(h1, 64, wts + o.w2, wts + o.b2, h2, R, 64, 64, 1, st));
+        NET_TRY(dense_fwd(h2, 64, wts + o.w3, wts + o.b3, h3, R, 64, 64, 1, st));
+        CriticHeadArgs a = {};                   // the critic head with one "agent" per step: V = h3 w4 + b4
+        a.c1 = h3; a.w2 = wts + o.w4; a.b2 = wts + o.b4; a.log_std = wts + o.log_std;
+        a.returns = io.returns ? io.returns + s0 : nullptr;
+        a.inv_count = io.inv_count;
+        a.values = io.values ? io.values + s0 : nullptr;
+        a.loss = io.loss;
+        a.unclamped = 1;
+        a.n = 1; a.G = env_group(1); a.S = steps;
+        float *dz3 = nullptr, *dz2 = nullptr, *dz1 = nullptr;
+        if (backward) {
+            dz3 = take(R * 64); dz2 = take(R * 64); dz1 = take(R * 64);
+            a.dc1 = dz3; a.dw2 = g + o.w4; a.db2 = g + o.b4; a.dlog_std = g + o.log_std;
+        }
+        net_critic_head_kernel<<<env_grid(1, steps, 4), kNetThreads, 0, st>>>(a);
+        NET_TRY(cudaGetLastError());
+        if (!backward) return cudaSuccess;
+        NET_TRY(dense_bwd(dz3, h2, 64, wts + o.w3, dz2, 0, 1, g + o.w3, g + o.b3, R, 64, 64, st));
+        NET_TRY(dense_bwd(dz2, h1, 64, wts + o.w2, dz1, 0, 1, g + o.w2, g + o.b2, R, 64, 64, st));
+        return wide_dw_t<64, 0>(obs, K, dz1, g + o.w1, g + o.b1, R, K, st);
+    }
+    const CentBlob o = cent_blob_layout(n, d.obs_dim);
+    const int act = (d.flags & CM_NET_FLAG_RELU) ? 2 : 1;
+    float *h1 = take(R * 128), *h2 = take(R * 64), *h3 = take(R * 32);
+    NET_TRY(wide_fwd(obs, wts + o.w1, wts + o.b1, h1, R, K, 128, act, st));
+    NET_TRY(dense_fwd(h1, 128, wts + o.w2, wts + o.b2, h2, R, 128, 64, act, st));
+    NET_TRY(dense_fwd(h2, 64, wts + o.w3, wts + o.b3, h3, R, 64, 32, act, st));
+    PolicyHeadArgs a = {};
+    a.g3 = h3; a.w4 = wts + o.w4; a.b4 = wts + o.b4;
+    a.avail_bits = io.avail_bits ? io.avail_bits + s0 * n : nullptr;
+    a.actions = io.actions ? io.actions + s0 * n : nullptr;
+    a.adv = io.adv ? io.adv + s0 : nullptr;
+    a.old_ll = io.old_ll ? io.old_ll + s0 : nullptr;
+    a.valid = io.valid ? io.valid + s0 : nullptr;
+    a.inv_count = io.inv_count; a.ent_coeff = d.ent_coeff; a.clip_lo = d.clip_lo; a.clip_hi = d.clip_hi;
+    a.ll = io.ll ? io.ll + s0 : nullptr;
+    a.ent = io.entropy ? io.entropy + s0 : nullptr;
+    a.probs = io.probs ? io.probs + s0 * n * CM_ACTIONS : nullptr;
+    a.loss = io.loss;
+    a.relu = act == 2;
+    a.n = n; a.G = env_group(n); a.S = steps;
+    float *dz3 = nullptr, *dz2 = nullptr, *dz1 = nullptr;
+    if (backward) {
+        a.dlogits = take(R * NO);
+        dz3 = take(R * 32); dz2 = take(R * 64); dz1 = take(R * 128);
+        a.dg3 = dz3; a.db4 = g + o.b4;
+    }
+    net_cent_head_kernel<<<env_grid(n, steps, 4), kNetThreads, 0, st>>>(a);
+    NET_TRY(cudaGetLastError());
+    if (!backward) return cudaSuccess;
+    NET_TRY((wide_dw_t<32, 1>(a.dlogits, NO, h3, g + o.w4, nullptr, R, NO, st)));           // dW4 [32][5n] = h3^T d logits
+    NET_TRY(dense_bwd(dz3, h2, 64, wts + o.w3, dz2, 0, act, g + o.w3, g + o.b3, R, 64, 32, st));
+    NET_TRY(dense_bwd(dz2, h1, 128, wts + o.w2, dz1, 0, act, g + o.w2, g + o.b2, R, 128, 64, st));
+    return wide_dw_t<128, 0>(obs, K, dz1, g + o.w1, g + o.b1, R, K, st);
+}
+
 static cudaError_t run_chunk(const cm_net_desc &d, const cm_net_io &io, int64_t s0, int64_t steps, float *wsp, cudaStream_t st)
 {
+    if (cent_kind(d.kind)) return run_chunk_cent(d, io, s0, steps, wsp, st);
     const int n = d.n_agents, D = d.obs_dim, L = d.n_layers, W = (n + 31) / 32;
     const bool backward = io.grad != nullptr;
     const NetWs w = carve(wsp, n, L, steps, backward);
@@ -1681,10 +2089,15 @@ extern "C" size_t cm_critic_blob_floats(int32_t obs_dim, int32_t n_layers)
     return (size_t)cm::critic_blob_layout(obs_dim, n_layers).total;
 }
 
+extern "C" size_t cm_baseline_mlp_blob_floats(int32_t in_dim)
+{
+    return in_dim < 1 ? 0 : (size_t)cm::baseline_blob_layout(in_dim).total;
+}
+
 extern "C" size_t cm_ppo_net_workspace_floats(const cm_net_desc *desc, int64_t chunk_steps, int32_t backward)
 {
     if (!desc || chunk_steps < 1) return 0;
-    return cm::ws_floats_per_step(desc->n_agents, desc->n_layers, backward != 0) * (size_t)chunk_steps + cm::kWsSlack;
+    return cm::ws_floats_per_step(*desc, backward != 0) * (size_t)chunk_steps + cm::kWsSlack;
 }
 
 extern "C" int cm_ppo_net(const cm_net_desc *desc, const cm_net_io *io, cm_stream_t stream)
@@ -1692,15 +2105,17 @@ extern "C" int cm_ppo_net(const cm_net_desc *desc, const cm_net_io *io, cm_strea
     using namespace cm;
     if (!desc || !io || !io->weights || !io->obs || !io->workspace || io->n_steps < 0) return CM_EINVAL;
     const cm_net_desc &d = *desc;
-    if (d.kind != CM_NET_POLICY && d.kind != CM_NET_CRITIC && d.kind != CM_NET_POLICY_DEC) return CM_EINVAL;
-    if (d.n_agents < 1 || d.n_agents > CM_MAX_AGENTS || d.obs_dim < 1 || d.obs_dim > 128 || d.n_layers < 1 || d.n_layers > CM_MAX_LAYERS)
+    if (d.kind != CM_NET_POLICY && d.kind != CM_NET_CRITIC && d.kind != CM_NET_POLICY_DEC && !cent_kind(d.kind)) return CM_EINVAL;
+    if (d.n_agents < 1 || d.n_agents > CM_MAX_AGENTS || d.obs_dim < 1 || d.obs_dim > 128 ||
+        (!cent_kind(d.kind) && (d.n_layers < 1 || d.n_layers > CM_MAX_LAYERS)))
         return CM_EUNSUPPORTED;
-    if (io->grad && d.kind != CM_NET_CRITIC && (!io->actions || !io->adv)) return CM_EINVAL;
-    if (io->grad && d.kind == CM_NET_CRITIC && !io->returns) return CM_EINVAL;
+    const bool value_net = d.kind == CM_NET_CRITIC || d.kind == CM_NET_BASELINE_MLP;
+    if (io->grad && !value_net && (!io->actions || !io->adv)) return CM_EINVAL;
+    if (io->grad && value_net && !io->returns) return CM_EINVAL;
     if (io->n_steps == 0) return CM_OK;
     if (cm_device_count() <= 0) return CM_ENODEVICE;
     const bool backward = io->grad != nullptr;
-    const size_t per_step = ws_floats_per_step(d.n_agents, d.n_layers, backward);
+    const size_t per_step = ws_floats_per_step(d, backward);
     if (io->workspace_floats < per_step + kWsSlack) return CM_EINVAL;
     const int64_t chunk = (int64_t)((io->workspace_floats - kWsSlack) / per_step);
     float *wsp = reinterpret_cast<float *>((reinterpret_cast<uintptr_t>(io->workspace) + 15) & ~(uintptr_t)15);

@@ -625,16 +625,20 @@ class CentralizedCategoricalMLPPolicy(nn.Module):
     def uses_tensor_cores(self):
         return self.math == "tc"
 
+    def _pack_blob(self, sd):
+        """state dict -> w1 [n*D][128] b1 w2 [128][64] b2 w3 [64][32] b3 w4 [32][5n] b4 (include/commarl_b200.h), narrower layers
+        zero-padded; also the parameter <-> blob map of the fused PPO update (ppo_fused._BlobMap)"""
+        parts = []
+        for i, (k_in, k_out) in enumerate(((self._obs_dim, 128), (128, 64), (64, 32))):
+            parts += [_pad2(sd[f"_layers.{i}.linear.weight"].t(), k_in, k_out), _pad2(sd[f"_layers.{i}.linear.bias"], k_out, 0)]
+        parts += [_pad2(sd["_output_layers.0.linear.weight"].t(), 32, self._action_dim * self._n_agents), sd["_output_layers.0.linear.bias"]]
+        return torch.cat([p.detach().to(self.device, torch.float32).contiguous().reshape(-1) for p in parts])
+
     def weight_blob(self):
-        """w1 [n*D][128] b1 w2 [128][64] b2 w3 [64][32] b3 w4 [32][5n] b4 (include/commarl_b200.h), rebuilt when a parameter changed"""
+        """the kernels' fp32 blob (_pack_blob), rebuilt when a parameter changed"""
         sig = self._signature()
         if self._blob is None or sig != self._blob_sig:
-            sd = self.state_dict()
-            parts = []
-            for i, (k_in, k_out) in enumerate(((self._obs_dim, 128), (128, 64), (64, 32))):
-                parts += [_pad2(sd[f"_layers.{i}.linear.weight"].t(), k_in, k_out), _pad2(sd[f"_layers.{i}.linear.bias"], k_out, 0)]
-            parts += [_pad2(sd["_output_layers.0.linear.weight"].t(), 32, self._action_dim * self._n_agents), sd["_output_layers.0.linear.bias"]]
-            blob = torch.cat([p.detach().to(self.device, torch.float32).contiguous().reshape(-1) for p in parts])
+            blob = self._pack_blob(self.state_dict())
             assert blob.numel() == N.lib().cm_policy_cent_blob_floats(self._n_agents, self._dec_obs_dim)
             self._blob = _refresh_in_place(self._blob, blob)
             self._blob_sig = sig

@@ -14,7 +14,8 @@ Returns, GAE advantages and their per-path normalisation run in ``cm_ppo_advanta
 ``cm_adam_step`` (hand-written CUDA over flat parameter buckets, csrc/ppo_kernels.cu).  The network forward / backward of the
 Comm-DP and Obs-DP runner families (CommBaseCritic with a CommCategoricalMLPPolicy or a DecCategoricalMLPPolicy) runs on the
 hand-written kernels of csrc/ppo_net_kernels.cu (``cm_ppo_net`` through ppo_fused.FusedCommNets, ``fused='auto'``); the CENT
-family and ``fused=False`` (the kernels' cross-check) use torch autograd over the policies' differentiable ``forward``.  With
+family (CentralizedCategoricalMLPPolicy + GaussianMLPBaseline) runs on them with ``fused=True`` (ppo_fused.FusedCentNets) and on
+torch autograd otherwise; ``fused=False`` (the kernels' cross-check) uses torch autograd over the policies' differentiable ``forward``.  With
 more than one rank the flat gradient buckets are all-reduced (NCCL) before clipping — the only collective of the update
 (SURVEY.md §8e).
 """
@@ -129,7 +130,19 @@ class GaussianMLPBaseline(nn.Module):
         self.name, self.device = name, torch.device(device)
         self.input_dim = int(env_spec.observation_space.flat_dim)
         self.module = _GaussianMean(self.input_dim, hidden_sizes, init_std)
+        # the shape the hand-written update kernels hold (the runners' (64, 64, 64); narrower layers run exactly, zero-padded)
+        self._fusable = len(tuple(hidden_sizes)) == 3 and max(hidden_sizes) <= 64
         self.to(self.device)
+
+    def _pack_blob(self, sd):
+        """state dict -> the blob of cm_ppo_net's CM_NET_BASELINE_MLP (include/commarl_b200.h): w1 [K][64] b1 w2 [64][64] b2
+        w3 [64][64] b3 w4 [64] b4 [1] log_std [1], dense weights K-major, narrower layers zero-padded"""
+        m = "module._mean_module."
+        parts = []
+        for i, k_in in enumerate((self.input_dim, 64, 64)):
+            parts += [_pad2(sd[m + f"_layers.{i}.linear.weight"].t(), k_in, 64), _pad2(sd[m + f"_layers.{i}.linear.bias"], 64, 0)]
+        parts += [_pad2(sd[m + "_output_layers.0.linear.weight"].t(), 64, 1), sd[m + "_output_layers.0.linear.bias"], sd["module._init_std"]]
+        return torch.cat([p.detach().to(self.device, torch.float32).contiguous().reshape(-1) for p in parts])
 
     def forward(self, obs):
         """(P, T, O) -> (P, T) predicted values (:104-117)"""
@@ -286,14 +299,24 @@ class DevicePPO:
         self.group = process_group
         self.opt = FlatAdam(policy, lr=policy_lr, eps=adam_eps)
         self.baseline_opt = FlatAdam(baseline, lr=policy_lr, eps=adam_eps)
-        # fused = hand-written forward / backward kernels (cm_ppo_net) instead of torch autograd: the Comm-DP family
-        # (CommCategoricalMLPPolicy + CommBaseCritic); 'auto' = wherever they apply
-        from .ppo_fused import FusedCommNets
-        can = FusedCommNets.supports(policy, baseline) and getattr(baseline, "_fusable", False) and self.device.type == "cuda"
-        if fused is True and not can:
-            raise NotImplementedError("fused=True needs a CommCategoricalMLPPolicy with a CommBaseCritic of the kernel's shapes on a GPU")
-        self._fused = FusedCommNets(policy, baseline, self.opt, self.baseline_opt, self.ent_coeff, self.lr_clip_range) \
-            if (can and fused in (True, "auto")) else None
+        # fused = hand-written forward / backward kernels (cm_ppo_net) instead of torch autograd: the Comm-DP and Obs-DP
+        # families (with CommBaseCritic) and the CENT family (with GaussianMLPBaseline).  'auto' = the Comm-DP / Obs-DP kernels
+        # wherever they apply; CENT stays on autograd unless fused=True: its kernels are new and opt-in, and whether the default
+        # follows is decided on their measured update times against autograd (DESIGN.md §7.1 and §8 item 1,
+        # profiles/r03a_ppo_cent.jsonl)
+        from .ppo_fused import FusedCentNets, FusedCommNets
+        cuda = self.device.type == "cuda"
+        can_comm = cuda and FusedCommNets.supports(policy, baseline) and getattr(baseline, "_fusable", False)
+        can_cent = cuda and FusedCentNets.supports(policy, baseline)
+        if fused is True and not (can_comm or can_cent):
+            raise NotImplementedError("fused=True needs, of the kernels' shapes and on a GPU, a CommCategoricalMLPPolicy or "
+                                      "DecCategoricalMLPPolicy with a CommBaseCritic, or a CentralizedCategoricalMLPPolicy with a "
+                                      "GaussianMLPBaseline")
+        self._fused = None
+        if can_comm and fused in (True, "auto"):
+            self._fused = FusedCommNets(policy, baseline, self.opt, self.baseline_opt, self.ent_coeff, self.lr_clip_range)
+        elif can_cent and fused is True:
+            self._fused = FusedCentNets(policy, baseline, self.opt, self.baseline_opt, self.ent_coeff, self.lr_clip_range)
 
     # ---- process_samples ----------------------------------------------------------------------------------------
     def process_samples(self, paths):
@@ -471,7 +494,7 @@ class DevicePPO:
                     baseline_losses=bl_losses, grad_norms=gnorms, n_paths=P)
 
     def _train_once_fused(self, b, shuffled_ids=None):
-        """train_once on the hand-written kernels (ppo_fused.FusedCommNets): the same loop, losses, clipping, all-reduces and
+        """train_once on the hand-written kernels (ppo_fused.FusedCommNets / FusedCentNets): the same loop, losses, clipping, all-reduces and
         Adam steps; every network forward / backward is ONE cm_ppo_net call."""
         F = self._fused
         f = b.get("_flat") or F.prepare(b)

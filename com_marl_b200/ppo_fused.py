@@ -1,11 +1,12 @@
-"""Hand-written forward / backward of the PPO update for the Comm-DP family (csrc/ppo_net_kernels.cu, cm_ppo_net).
+"""Hand-written forward / backward of the PPO update for the three runner families (csrc/ppo_net_kernels.cu, cm_ppo_net).
 
 ``FusedCommNets`` is what ``DevicePPO`` drives instead of torch autograd when the baseline is a ``CommBaseCritic`` and the
-policy a ``CommCategoricalMLPPolicy`` (runner_*_comm.py) or a ``DecCategoricalMLPPolicy`` (runner_*_obsDP.py): per optimizer step ONE C call per network computes the loss of
-centralized_ma_ppo.py:390-438 / comm_base_critic.py and the gradient of every parameter, exact fp32.  The parameters stay
-torch tensors (views of FlatAdam's flat bucket): a precomputed index map turns the flat bucket into the kernels' weight blob
-(K-major, zero-padded to the kernel widths) with one gather, and the gradient blob back into the flat gradient bucket with
-another.  The CENT runner family keeps the autograd path.
+policy a ``CommCategoricalMLPPolicy`` (runner_*_comm.py) or a ``DecCategoricalMLPPolicy`` (runner_*_obsDP.py); ``FusedCentNets``
+when the policy is a ``CentralizedCategoricalMLPPolicy`` and the baseline a ``GaussianMLPBaseline`` (runner_*_cent.py, with
+``fused=True``).  Per optimizer step ONE C call per network computes the loss of centralized_ma_ppo.py:390-438 /
+comm_base_critic.py / gaussian_mlp_baseline.py and the gradient of every parameter, exact fp32.  The parameters stay torch
+tensors (views of FlatAdam's flat bucket): a precomputed index map turns the flat bucket into the kernels' weight blob (K-major,
+zero-padded to the kernel widths) with one gather, and the gradient blob back into the flat gradient bucket with another.
 """
 import ctypes as C
 
@@ -57,56 +58,28 @@ class _BlobMap:
         torch.index_select(self.grad, 0, self.inverse, out=flat_grad)
 
 
-class FusedCommNets:
-    """policy + critic of the Comm-DP runners on cm_ppo_net.  ``chunk_rows``: agent rows of activations kept in the workspace
-    at a time (the kernels walk a minibatch in chunks; gradients add up)."""
+class _FusedNets:
+    """policy + value network of one runner family on cm_ppo_net (the subclasses set the descriptors, blob maps and batch
+    layout).  ``chunk_rows``: agent rows of activations kept in the workspace at a time (the kernels walk a minibatch in
+    chunks; gradients add up)."""
+    _obs_keys = ("obs",)                 # per-step inputs of both networks besides the policy's avail / actions / valid
 
-    def __init__(self, policy, critic, opt, baseline_opt, ent_coeff, clip_range, chunk_rows=524288):
+    def _setup(self, policy, critic, opt, baseline_opt, chunk_rows):
         self.policy, self.critic = policy, critic
         self.device = policy.device
-        # L = layers of the communication masks in the batch (the critic's; the Obs-DP policy has none of its own)
-        self.n, self.D, self.L = policy._n_agents, policy._dec_obs_dim, len(critic.gcn_layers)
-        self.W = (self.n + 31) // 32
+        self.n, self.D = policy._n_agents, policy._dec_obs_dim
         self.pol_map = _BlobMap(policy, policy._pack_blob, opt.flat)
         self.cri_map = _BlobMap(critic, critic._pack_blob, baseline_opt.flat)
-        self.dec = not getattr(policy, "comm", False)
-        assert self.pol_map.const.numel() == N.lib().cm_policy_blob_floats(self.D, policy.n_gcn_layers)
-        assert self.cri_map.const.numel() == N.lib().cm_critic_blob_floats(self.D, self.L)
-        self.pol_desc = N.NetDesc(N.NET_POLICY_DEC if self.dec else N.NET_POLICY, self.n, self.D, policy.n_gcn_layers, int(policy.residual), float(ent_coeff),
-                                  1.0 - float(clip_range), 1.0 + float(clip_range))
-        self.cri_desc = N.NetDesc(N.NET_CRITIC, self.n, self.D, len(critic.gcn_layers), int(critic.residual), 0.0, 0.0, 0.0)
         import os
         chunk_rows = int(os.environ.get("CM_PPO_CHUNK_ROWS", chunk_rows))          # (experiments)
         self.chunk_steps = max(1, int(chunk_rows) // self.n)
-        if self.n > 64 and self.chunk_steps > 148:        # one env per CTA in the n x n kernels: whole waves of the 148 SMs
-            self.chunk_steps = self.chunk_steps // 148 * 148
         self._ws = None
-        self._scalar = torch.zeros(2, dtype=torch.float32, device=self.device)
 
-    @staticmethod
-    def supports(policy, critic):
-        from .policy import CommCategoricalMLPPolicy, DecCategoricalMLPPolicy
-        from .ppo import CommBaseCritic
-        if type(critic) is not CommBaseCritic or policy._dec_obs_dim > 128 or policy._n_agents != critic._n_agents:
-            return False
-        if type(policy) is DecCategoricalMLPPolicy:              # Obs-DP runners: no communication in the policy
-            return True
-        return type(policy) is CommCategoricalMLPPolicy and len(critic.gcn_layers) == policy.n_gcn_layers
-
-    # ---- batch ---------------------------------------------------------------------------------------------------
-    def prepare(self, b):
-        """flat (step-major) views of a padded [P, T, ...] batch; masks as bit rows, availability as bits"""
-        n, D, L, W = self.n, self.D, self.L, self.W
+    def _prepare_common(self, b):
+        n, D = self.n, self.D
         P, T = b["rewards"].shape
         S = P * T
         f = dict(P=P, T=T, obs=b["obs"].reshape(S, n, D).contiguous(), actions=b["actions"].reshape(S, n).contiguous())
-        if "adj_bits" in b:
-            f["adj"], f["chan"] = b["adj_bits"].reshape(S, n, W).contiguous(), b["chan_bits"].reshape(S, L, n, W).contiguous()
-        else:
-            from .policy import CommCategoricalMLPPolicy
-            pack = CommCategoricalMLPPolicy.pack_mask            # (static: cm_mask_pack)
-            f["adj"] = pack(b["dist_adjs"].reshape(S, n, n), n)
-            f["chan"] = pack(b["channels"].reshape(S, L, n, n), n)
         av = b["avail"].reshape(S, n, 5)
         wts = torch.tensor([1, 2, 4, 8, 16], dtype=torch.float32, device=av.device)
         f["avail"] = ((av != 0).to(torch.float32) * wts).sum(-1).to(torch.uint8).contiguous()
@@ -114,6 +87,7 @@ class FusedCommNets:
         f["valid"] = (torch.arange(T, device=self.device)[None, :] < b["valids"][:, None]).reshape(S).to(torch.uint8).contiguous()
         return f
 
+    # ---- batch ---------------------------------------------------------------------------------------------------
     def step_index(self, f, path_ids, valid_only):
         """flat step indices (device int64) of the given paths: every padded step, or the valid ones only"""
         T = f["T"]
@@ -129,7 +103,7 @@ class FusedCommNets:
     def subset(self, f, idx, policy=True):
         """the rows `idx` of the flat batch gathered ONCE (a minibatch is walked again in every mini-epoch): a flat batch of its
         own, to be passed to policy_call / critic_call with idx = None"""
-        keys = ("obs", "adj", "chan") + (("avail", "actions", "valid") if policy else ())
+        keys = self._obs_keys + (("avail", "actions", "valid") if policy else ())
         g = {k: f[k].index_select(0, idx) for k in keys}
         g["P"], g["T"] = 1, int(idx.numel())
         return g
@@ -149,7 +123,7 @@ class FusedCommNets:
 
     def _io(self, desc, f, idx, backward, wmap):
         sel = (lambda x: x) if idx is None else (lambda x: x.index_select(0, idx))
-        keep = dict(obs=sel(f["obs"]), adj=sel(f["adj"]), chan=sel(f["chan"]))
+        keep = {k: sel(f[k]) for k in self._obs_keys}
         S = keep["obs"].shape[0]
         if backward:
             (self.pol_map if desc is self.pol_desc else self.cri_map).grad.zero_()
@@ -157,7 +131,9 @@ class FusedCommNets:
         io.n_steps = S
         io.weights = N.ptr(wmap.blob)
         io.grad = N.ptr(wmap.grad) if backward else None
-        io.obs, io.adj_bits, io.chan_bits = N.ptr(keep["obs"]), N.ptr(keep["adj"]), N.ptr(keep["chan"])
+        io.obs = N.ptr(keep["obs"])
+        if "adj" in keep:
+            io.adj_bits, io.chan_bits = N.ptr(keep["adj"]), N.ptr(keep["chan"])
         ws = self._workspace(desc, S, backward)
         io.workspace, io.workspace_floats = N.ptr(ws), ws.numel()
         return io, keep, sel, S
@@ -206,3 +182,71 @@ class FusedCommNets:
         if S:
             self._run(self.cri_desc, io)
         return out
+
+
+class FusedCommNets(_FusedNets):
+    """policy + critic of the Comm-DP and Obs-DP runners (CommBaseCritic) on cm_ppo_net"""
+    _obs_keys = ("obs", "adj", "chan")
+
+    def __init__(self, policy, critic, opt, baseline_opt, ent_coeff, clip_range, chunk_rows=524288):
+        self._setup(policy, critic, opt, baseline_opt, chunk_rows)
+        # L = layers of the communication masks in the batch (the critic's; the Obs-DP policy has none of its own)
+        self.L = len(critic.gcn_layers)
+        self.W = (self.n + 31) // 32
+        self.dec = not getattr(policy, "comm", False)
+        assert self.pol_map.const.numel() == N.lib().cm_policy_blob_floats(self.D, policy.n_gcn_layers)
+        assert self.cri_map.const.numel() == N.lib().cm_critic_blob_floats(self.D, self.L)
+        self.pol_desc = N.NetDesc(N.NET_POLICY_DEC if self.dec else N.NET_POLICY, self.n, self.D, policy.n_gcn_layers, int(policy.residual), float(ent_coeff),
+                                  1.0 - float(clip_range), 1.0 + float(clip_range))
+        self.cri_desc = N.NetDesc(N.NET_CRITIC, self.n, self.D, len(critic.gcn_layers), int(critic.residual), 0.0, 0.0, 0.0)
+        if self.n > 64 and self.chunk_steps > 148:        # one env per CTA in the n x n kernels: whole waves of the 148 SMs
+            self.chunk_steps = self.chunk_steps // 148 * 148
+
+    @staticmethod
+    def supports(policy, critic):
+        from .policy import CommCategoricalMLPPolicy, DecCategoricalMLPPolicy
+        from .ppo import CommBaseCritic
+        if type(critic) is not CommBaseCritic or policy._dec_obs_dim > 128 or policy._n_agents != critic._n_agents:
+            return False
+        if type(policy) is DecCategoricalMLPPolicy:              # Obs-DP runners: no communication in the policy
+            return True
+        return type(policy) is CommCategoricalMLPPolicy and len(critic.gcn_layers) == policy.n_gcn_layers
+
+    def prepare(self, b):
+        """flat (step-major) views of a padded [P, T, ...] batch; masks as bit rows, availability as bits"""
+        n, L, W = self.n, self.L, self.W
+        f = self._prepare_common(b)
+        S = f["P"] * f["T"]
+        if "adj_bits" in b:
+            f["adj"], f["chan"] = b["adj_bits"].reshape(S, n, W).contiguous(), b["chan_bits"].reshape(S, L, n, W).contiguous()
+        else:
+            from .policy import CommCategoricalMLPPolicy
+            pack = CommCategoricalMLPPolicy.pack_mask            # (static: cm_mask_pack)
+            f["adj"] = pack(b["dist_adjs"].reshape(S, n, n), n)
+            f["chan"] = pack(b["channels"].reshape(S, L, n, n), n)
+        return f
+
+
+class FusedCentNets(_FusedNets):
+    """policy + baseline of the CENT runners (CentralizedCategoricalMLPPolicy + GaussianMLPBaseline) on cm_ppo_net: both
+    networks read the concatenated observation of the team, one row per env step; no communication masks"""
+
+    def __init__(self, policy, critic, opt, baseline_opt, ent_coeff, clip_range, chunk_rows=524288):
+        self._setup(policy, critic, opt, baseline_opt, chunk_rows)
+        assert self.pol_map.const.numel() == N.lib().cm_policy_cent_blob_floats(self.n, self.D)
+        assert self.cri_map.const.numel() == N.lib().cm_baseline_mlp_blob_floats(critic.input_dim)
+        self.pol_desc = N.NetDesc(N.NET_POLICY_CENT, self.n, self.D, 0, 0, float(ent_coeff), 1.0 - float(clip_range),
+                                  1.0 + float(clip_range), N.NET_FLAG_RELU if policy._relu else 0)
+        self.cri_desc = N.NetDesc(N.NET_BASELINE_MLP, self.n, self.D, 0, 0, 0.0, 0.0, 0.0, 0)
+
+    @staticmethod
+    def supports(policy, critic):
+        from .policy import CentralizedCategoricalMLPPolicy
+        from .ppo import GaussianMLPBaseline
+        return (type(policy) is CentralizedCategoricalMLPPolicy and type(critic) is GaussianMLPBaseline and critic._fusable
+                and policy._dec_obs_dim <= 128 and policy._n_agents <= N.MAX_AGENTS and critic.input_dim == policy._obs_dim
+                and policy._obs_dim == policy._n_agents * policy._dec_obs_dim)
+
+    def prepare(self, b):
+        """flat (step-major) views of a padded [P, T, ...] batch, availability as bits (no masks)"""
+        return self._prepare_common(b)

@@ -46,7 +46,8 @@
 extern "C" {
 #endif
 
-#define CM_ABI_VERSION 3   /* 2: host_arena / obs_bits members, cm_rollout_step_host; 3: cm_ppo_net */
+#define CM_ABI_VERSION 4   /* 2: host_arena / obs_bits members, cm_rollout_step_host; 3: cm_ppo_net; 4: CENT kinds of cm_ppo_net,
+                              cm_net_desc.flags */
 #define CM_MAX_AGENTS 256   /* n, p */
 #define CM_MAX_GRID 64      /* grid side incl. Coverage's wall border */
 #define CM_MAX_LAYERS 4     /* n_gcn_layers */
@@ -322,16 +323,32 @@ int cm_adam_step_dev(float *params, const float *grads, float *exp_avg, float *e
  *                         log-std (clamped at log 1e-6).  Blob (cm_critic_blob_floats): enc_w1 [D][128] enc_b1 enc_w2 [128][64]
  *                         enc_b2 att_w [64][64] gcn_w[l] [64][64] gcn_b[l] [64] dec_w1 [64][64] dec_b1 [64] dec_w2 [64] dec_b2 [1]
  *                         log_std [1], dense weights K-major like the policy blob.
+ *   kind = CM_NET_POLICY_CENT  CentralizedCategoricalMLPPolicy.forward (centralized_categorical_mlp_policy.py:61-97, 122-137: one MLP
+ *                         n*D -> 128 -> 64 -> 32 -> 5n over the concatenated observation of the team, act = tanh, or relu with
+ *                         CM_NET_FLAG_RELU) followed by _compute_loss / _compute_objective: logits [S][5n] reshaped per agent, softmax,
+ *                         availability mask, masked / masked.sum() (no + 1e-12), log-likelihood summed and entropy averaged over the
+ *                         agents; the joint ratio and the clipped surrogate as for CM_NET_POLICY.  Blob = the rollout blob of the CENT
+ *                         policy (cm_policy_cent_blob_floats).
+ *   kind = CM_NET_BASELINE_MLP  GaussianMLPBaseline.compute_loss (gaussian_mlp_baseline.py:83-117): V(s) = MLP(obs[S][n*D]), three
+ *                         tanh hidden layers of <= 64 units and a linear output of 1; loss = mean Gaussian negative log-likelihood over
+ *                         EVERY step passed, std = exp(log_std) with no clamp.  Blob (cm_baseline_mlp_blob_floats(n*D)): w1 [n*D][64]
+ *                         b1 [64] w2 [64][64] b2 [64] w3 [64][64] b3 [64] w4 [64] b4 [1] log_std [1], narrower layers zero-padded.
+ *   For the two CENT kinds the rows of every product are env steps, io.obs [S][n][D] is read as [S][n*D], adj_bits / chan_bits
+ *   and n_layers / residual are ignored, and n, D are limited as cm_policy_forward limits them for CM_POLICY_CENT.
  * grad == NULL: forward only (ll / entropy / probs / values / loss outputs).  grad != NULL: the parameter gradients of `loss`
  * are ADDED to grad (same layout as weights; the caller zeroes it) — exact fp32 like the autograd graph they replace.
  * Activations live in `workspace`; the steps are walked in chunks of as many steps as the workspace holds
  * (cm_ppo_net_workspace_floats(desc, chunk_steps, backward) floats hold one chunk).  Stream-ordered, capturable. */
-typedef enum cm_net_kind { CM_NET_POLICY = 0, CM_NET_CRITIC = 1, CM_NET_POLICY_DEC = 2 } cm_net_kind;
+typedef enum cm_net_kind {
+    CM_NET_POLICY = 0, CM_NET_CRITIC = 1, CM_NET_POLICY_DEC = 2, CM_NET_POLICY_CENT = 3, CM_NET_BASELINE_MLP = 4
+} cm_net_kind;
+#define CM_NET_FLAG_RELU 1     /* CM_NET_POLICY_CENT: hidden_nonlinearity = relu instead of tanh (runner_*_cent.py:49) */
 typedef struct cm_net_desc {
     int32_t kind;              /* cm_net_kind */
     int32_t n_agents, obs_dim, n_layers, residual;
     float ent_coeff;           /* policy_ent_coeff ('regularized'), 0 otherwise */
     float clip_lo, clip_hi;    /* 1 -/+ lr_clip_range (hard-coded 0.1 at centralized_ma_ppo.py:121) */
+    int32_t flags;             /* CM_NET_FLAG_* */
 } cm_net_desc;
 typedef struct cm_net_io {
     int64_t n_steps;           /* S */
@@ -355,6 +372,7 @@ typedef struct cm_net_io {
     size_t workspace_floats;
 } cm_net_io;
 size_t cm_critic_blob_floats(int32_t obs_dim, int32_t n_layers);
+size_t cm_baseline_mlp_blob_floats(int32_t in_dim);
 size_t cm_ppo_net_workspace_floats(const cm_net_desc *desc, int64_t chunk_steps, int32_t backward);
 int cm_ppo_net(const cm_net_desc *desc, const cm_net_io *io, cm_stream_t stream);
 

@@ -21,6 +21,7 @@ def main():
     ap.add_argument("--epochs", type=int, default=3)
     ap.add_argument("--mini-epochs", type=int, default=10)
     ap.add_argument("--minibatches", type=int, default=3)
+    ap.add_argument("--kind", default="comm", choices=["comm", "dec", "cent"], help="runner family (DeviceTrainer kind)")
     ap.add_argument("--fused", default="auto", choices=["auto", "0", "1"], help="hand-written update kernels (cm_ppo_net) or torch autograd")
     args = ap.parse_args()
     import bench
@@ -31,7 +32,7 @@ def main():
     torch.cuda.set_device(local_rank)
     scen, params = bench.params_for(args.config)
     spec = ScenarioSpec.from_params(scen, params, seed=1)
-    tr = DeviceTrainer(spec, args.envs, device=torch.device("cuda", local_rank), env_id0=rank * args.envs,
+    tr = DeviceTrainer(spec, args.envs, device=torch.device("cuda", local_rank), env_id0=rank * args.envs, kind=args.kind,
                        optimization_mini_epochs=args.mini_epochs, optimization_n_minibatches=args.minibatches,
                        fused={"auto": "auto", "0": False, "1": True}[args.fused])
     rounds = []
@@ -49,7 +50,7 @@ def main():
         sums = [float(cs)]
     if rank == 0:
         last = rounds[-1]
-        line = dict(config=args.config, n_gpus=world, envs_per_gpu=args.envs, n_agents=spec.n_agents, horizon=spec.max_steps,
+        line = dict(config=args.config, kind=args.kind, n_gpus=world, envs_per_gpu=args.envs, n_agents=spec.n_agents, horizon=spec.max_steps,
                     mini_epochs=args.mini_epochs, minibatches=args.minibatches, fused=tr.algo._fused is not None, optimizer_steps_per_round=len(last["losses"]),
                     rounds=[dict(rollout_ms=r["rollout_ms"], batch_ms=r["batch_ms"], update_ms=r["update_ms"], n_paths=r["n_paths"],
                                  loss_before=r["loss_before"], loss_after=r["loss_after"], kl=r["kl"], entropy=r["entropy"],
