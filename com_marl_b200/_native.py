@@ -16,7 +16,8 @@ CH_FC, CH_FL, CH_IID, CH_GE = 0, 1, 2, 3
 POLICY_COMM, POLICY_DEC, POLICY_CENT = 0, 1, 2
 POLICY_FLAG_RELU = 1
 MAX_AGENTS, MAX_GRID, MAX_LAYERS = 256, 64, 4
-ABI_VERSION = 4
+ABI_VERSION = 5
+MAX_CONDS = 256
 
 EXPORTS = ("cm_abi_version", "cm_strerror", "cm_last_cuda_error", "cm_device_count", "cm_env_reset", "cm_env_step",
            "cm_comm_update", "cm_policy_forward", "cm_policy_blob_floats", "cm_policy_cent_blob_floats", "cm_policy_cent_tc_blob_floats", "cm_policy_cent_workspace_bytes", "cm_policy_workspace_bytes", "cm_policy_tc_blob_floats", "cm_policy_tc_prepare", "cm_mask_pack",
@@ -34,7 +35,13 @@ class EnvDesc(C.Structure):
                [(k, C.c_float) for k in ("p_loss", "pgb", "pbg", "ge_bad_rate")] + \
                [(k, C.c_double) for k in ("capture_reward", "step_cost", "moving_cost", "penalty", "lazy_penalty",
                                           "revisit_penalty", "final_reward")] + \
-               [("seed", C.c_uint64), ("env_id0", C.c_int64), ("wall_rows", C.c_void_p), ("lut", C.c_void_p)]
+               [("seed", C.c_uint64), ("env_id0", C.c_int64), ("wall_rows", C.c_void_p), ("lut", C.c_void_p),
+                ("conds", C.c_void_p), ("cond_idx", C.c_void_p), ("n_conds", C.c_int32), ("conds_host", C.c_void_p)]
+
+
+class ChannelCond(C.Structure):
+    _fields_ = [("channel", C.c_int32), ("rcom2", C.c_int32)] + \
+               [(k, C.c_float) for k in ("p_loss", "pgb", "pbg", "ge_bad_rate")] + [("ge_init", C.c_int32)]
 
 
 class EnvState(C.Structure):

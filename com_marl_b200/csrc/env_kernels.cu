@@ -721,14 +721,16 @@ __device__ __forceinline__ int resolve_preys(const Scratch &S, const Grp &G, int
 // instruction FETCH (ncu: 1-3 warps per issue slot wait for instructions; every warp walks a long, divergent path through
 // the code of one env), so an instantiation carries only the code of its own scenario / channel / stream source — the
 // descriptor fields are overwritten with the template constants and the branches on them fold after inlining.
-// kChan: 0 = FC / FL (told apart at run time), CM_CH_IID, CM_CH_GE.
+// kChan: 0 = FC / FL (told apart at run time), CM_CH_IID, CM_CH_GE, or kChanTable: every env reads its own channel condition
+// (cm_env_desc.conds) and comm_update branches on its channel at run time; that code lives in its own instantiations only.
+static constexpr int kChanTable = 4;
 template <int kScen, int kChan, bool kInj>
 __global__ void __launch_bounds__(kWarpsPerCta * 32, 24 / kWarpsPerCta) env_kernel(const EnvArgs A_in)
 {
     EnvArgs A = A_in;
     A.d.scenario = kScen;
-    if (kChan != 0) A.d.channel = kChan;
-    else if (A.d.channel != CM_CH_FL) A.d.channel = CM_CH_FC;
+    if (kChan == 0) { if (A.d.channel != CM_CH_FL) A.d.channel = CM_CH_FC; }
+    else if (kChan != kChanTable) A.d.channel = kChan;
     if (kScen == CM_COVERAGE) { A.d.n_preys = 0; A.s.prey_pos = nullptr; A.s.prey_alive = nullptr; }
     if (!kInj) { A.io.prey_cand = nullptr; A.io.chan_u = nullptr; A.io.spawn_agent = nullptr; A.io.spawn_prey = nullptr; }
 #ifdef CM_ENV_TRACE
@@ -1081,6 +1083,21 @@ __global__ void __launch_bounds__(kWarpsPerCta * 32, 24 / kWarpsPerCta) env_kern
             write_obs(A, S, wall, b, G, t);
         }
         CM_ETP(9);
+        if (kChan == kChanTable) {                // this env's channel condition, loaded once
+            int k = A.d.cond_idx[b];
+            if (k >= A.d.n_conds) {
+                if (G.gl == 0 && A.io.error_flag) atomicExch(A.io.error_flag, (int)CM_EINVAL);
+                k = 0;
+            }
+            const cm_channel_cond c = A.d.conds[k];
+            A.d.channel = c.channel;
+            A.d.rcom2 = c.rcom2;
+            A.d.p_loss = c.p_loss;
+            A.d.pgb = c.pgb;
+            A.d.pbg = c.pbg;
+            A.d.ge_bad_rate = c.ge_bad_rate;
+            A.d.ge_init = c.ge_init;
+        }
         comm_update(A, S, b, G, key, A.mode == 2 ? (A.at_reset != 0) : did_reset);
         CM_ETP(10);
 #ifdef CM_ENV_TRACE
@@ -1097,6 +1114,7 @@ template <int kScen>
 static env_kernel_fn pick_env_kernel_s(int channel, bool inj)
 {
     switch (channel) {
+    case kChanTable: return inj ? env_kernel<kScen, kChanTable, true> : env_kernel<kScen, kChanTable, false>;
     case CM_CH_IID: return inj ? env_kernel<kScen, CM_CH_IID, true> : env_kernel<kScen, CM_CH_IID, false>;
     case CM_CH_GE: return inj ? env_kernel<kScen, CM_CH_GE, true> : env_kernel<kScen, CM_CH_GE, false>;
     default: return inj ? env_kernel<kScen, 0, true> : env_kernel<kScen, 0, false>;
@@ -1105,6 +1123,18 @@ static env_kernel_fn pick_env_kernel_s(int channel, bool inj)
 static env_kernel_fn pick_env_kernel(int scenario, int channel, bool inj)
 {
     return scenario == CM_COVERAGE ? pick_env_kernel_s<CM_COVERAGE>(channel, inj) : pick_env_kernel_s<CM_PREDATOR_PREY>(channel, inj);
+}
+
+// checks of one channel condition; *planes = injected channel planes it draws
+static int validate_channel(int channel, int ge_init, int loss_apply, int n_layers, const cm_env_state *s, int *planes)
+{
+    if (channel < CM_CH_FC || channel > CM_CH_GE) return CM_EINVAL;
+    if (channel == CM_CH_GE) {
+        if (ge_init == -1 && loss_apply == 0) return CM_EUNSUPPORTED;  // broken in the reference (env_communication.py:121)
+        if (!s->ge_state) return CM_EINVAL;
+    }
+    *planes = channel == CM_CH_IID ? n_layers : (channel == CM_CH_GE ? 2 * n_layers + 1 : 0);
+    return CM_OK;
 }
 
 static int validate(const cm_env_desc *d, const cm_env_state *s, const cm_step_io *io, int mode)
@@ -1121,19 +1151,25 @@ static int validate(const cm_env_desc *d, const cm_env_state *s, const cm_step_i
         if (d->n_preys != 0) return CM_EINVAL;
         if (!d->wall_rows || !s->visited || !s->total_capture) return CM_EINVAL;
     } else return CM_EINVAL;
-    if (d->channel < CM_CH_FC || d->channel > CM_CH_GE) return CM_EINVAL;
-    if (d->channel == CM_CH_GE) {
-        if (d->ge_init == -1 && d->loss_apply == 0) return CM_EUNSUPPORTED;  // broken in the reference (env_communication.py:121)
-        if (!s->ge_state) return CM_EINVAL;
+    int need = 0;   // channel planes an injected chan_u must hold
+    if (d->conds) {
+        if (!d->conds_host || !d->cond_idx || d->n_conds < 1 || d->n_conds > CM_MAX_CONDS) return CM_EINVAL;
+        for (int k = 0; k < d->n_conds; ++k) {
+            const cm_channel_cond &c = d->conds_host[k];
+            int planes = 0;
+            const int rc = validate_channel(c.channel, c.ge_init, d->loss_apply, d->n_layers, s, &planes);
+            if (rc) return rc;
+            need = planes > need ? planes : need;
+        }
+    } else {
+        const int rc = validate_channel(d->channel, d->ge_init, d->loss_apply, d->n_layers, s, &need);
+        if (rc) return rc;
     }
     if (!s->agent_pos || !s->step_count || !s->success || !s->episode || !s->tick) return CM_EINVAL;
     if (!d->lut && (io->obs || io->obs_bits)) return CM_EINVAL;
     if (mode == 0 && !io->actions) return CM_EINVAL;
     if (io->spawn_agent && (io->spawn_episodes < 1 || (d->n_preys > 0 && !io->spawn_prey))) return CM_EINVAL;
-    if (io->chan_u) {
-        int need = d->channel == CM_CH_IID ? d->n_layers : (d->channel == CM_CH_GE ? 2 * d->n_layers + 1 : 0);
-        if (io->chan_planes < need) return CM_EINVAL;
-    }
+    if (io->chan_u && io->chan_planes < need) return CM_EINVAL;
     return CM_OK;
 }
 
@@ -1166,7 +1202,7 @@ static int launch(const cm_env_desc *d, const cm_env_state *s, const cm_step_io 
     // (keeps the call CUDA-graph capturable)
     static thread_local struct { int dev; size_t smem; const void *kernel; int ctas_per_sm; int sms; } cache = {-1, 0, nullptr, 0, 0};
     const bool inj = io->prey_cand || io->chan_u || io->spawn_agent || io->spawn_prey;
-    void (*kernel)(const EnvArgs) = pick_env_kernel(d->scenario, d->channel, inj);
+    void (*kernel)(const EnvArgs) = pick_env_kernel(d->scenario, d->conds ? kChanTable : d->channel, inj);
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess) return set_cuda_error(cudaGetLastError(), CM_ENODEVICE);
     if (cache.dev != dev || cache.smem != smem || cache.kernel != (const void *)kernel) {

@@ -32,14 +32,36 @@ def unpack_positions(packed) -> np.ndarray:
     return np.stack([packed & 0xFF, packed >> 8], axis=-1).astype(np.int8)
 
 
+def check_conditions(spec: ScenarioSpec, conditions, n_envs: int):
+    """-> the validated list of channel conditions of a BatchedEnv (None when there are none); raises ValueError"""
+    if conditions is None:
+        return None
+    conditions = list(conditions)
+    if not 1 <= len(conditions) <= N.MAX_CONDS:
+        raise ValueError(f"between 1 and {N.MAX_CONDS} channel conditions are supported, got {len(conditions)}")
+    if int(n_envs) % len(conditions):
+        raise ValueError(f"n_envs = {n_envs} does not split evenly into {len(conditions)} conditions")
+    for k, c in enumerate(conditions):
+        if not spec.same_except_channel(c):
+            raise ValueError(f"condition {k} differs from the spec outside the channel fields {ScenarioSpec.CHANNEL_FIELDS}")
+        c.validate()
+    return conditions
+
+
 class BatchedEnv:
     """B environment instances of one scenario on one GPU."""
 
-    def __init__(self, spec: ScenarioSpec, n_envs: int, device="cuda", env_id0: int = 0, auto_reset: bool = True):
+    def __init__(self, spec: ScenarioSpec, n_envs: int, device="cuda", env_id0: int = 0, auto_reset: bool = True,
+                 conditions=None):
+        """``conditions``: optional list of specs that differ from ``spec`` in the channel fields only
+        (ScenarioSpec.CHANNEL_FIELDS, e.g. ``spec.with_channel(pl=..., rcom=...)``).  The envs are then split into equal
+        contiguous blocks in list order and block k communicates under ``conditions[k]`` (``spec``'s own channel is not
+        used); ``cond_idx`` [B] holds each env's condition.  Everything else — and the global env ids — stays as without."""
         N.lib()  # fail loudly if the CUDA library is missing; there is no CPU path
         if not torch.cuda.is_available():
             raise RuntimeError("com_marl_b200 needs a CUDA device: the rollout engine has no CPU fallback")
         spec.validate()
+        self.conditions = check_conditions(spec, conditions, n_envs)
         self.spec, self.B, self.auto_reset = spec, int(n_envs), bool(auto_reset)
         self.device = torch.device(device)
         self.env_id0 = int(env_id0)
@@ -62,7 +84,8 @@ class BatchedEnv:
         self.success = z((B,), torch.uint8)
         self.episode = z((B,), torch.int32)
         self.tick = z((B,), torch.int32)
-        self.ge_state = z((B, n, self.W), torch.int32) if spec.channel == N.CH_GE else None
+        chans = [c.channel for c in self.conditions] if self.conditions else [spec.channel]
+        self.ge_state = z((B, n, self.W), torch.int32) if N.CH_GE in chans else None
         # ---- outputs: one arena, in the order the host-buffer call copies them (one DMA transfer, csrc/host_abi.cu) ----
         for k, v in N.arena(self._out_specs(), device=dev).items():
             setattr(self, "_out_arena" if k == "_arena" else k, v)
@@ -71,7 +94,13 @@ class BatchedEnv:
         # ---- constants ----
         self._lut = torch.from_numpy(spec.lut()).to(dev)
         self._wall = torch.from_numpy(spec.wall_rows().view(np.int64)).to(dev) if spec.scenario == "co" else None
-        self.desc = spec.to_desc(N.ptr(self._wall), N.ptr(self._lut), env_id0=self.env_id0)
+        self.cond_idx = None
+        if self.conditions:
+            K = len(self.conditions)
+            self._conds_host = (N.ChannelCond * K)(*[c.channel_cond() for c in self.conditions])
+            self._conds = torch.frombuffer(bytearray(bytes(self._conds_host)), dtype=torch.uint8).to(dev)
+            self.cond_idx = torch.arange(K, dtype=torch.uint8, device=dev).repeat_interleave(B // K)
+        self.desc = self._desc()
         self.state = N.EnvState()
         self.state.n_envs = B
         for k in ("agent_pos", "prey_pos", "prey_alive", "visited", "step_count", "total_capture", "success",
@@ -80,6 +109,13 @@ class BatchedEnv:
         self._spawn_agent = self._spawn_prey = None
         self._spawn_episodes = 0
         self._io_cache = {}
+
+    def _desc(self):
+        d = self.spec.to_desc(N.ptr(self._wall), N.ptr(self._lut), env_id0=self.env_id0)
+        if self.cond_idx is not None:
+            d.conds, d.cond_idx, d.n_conds = N.ptr(self._conds), N.ptr(self.cond_idx), len(self.conditions)
+            d.conds_host = C.addressof(self._conds_host)
+        return d
 
     def _out_specs(self):
         B, n, p, L = self.B, self.n, self.p, self.L
@@ -99,7 +135,7 @@ class BatchedEnv:
 
     _SLICED = ("obs_bits", "agent_pos", "prey_pos", "prey_alive", "visited", "step_count", "total_capture", "success", "episode", "tick",
                "ge_state", "obs", "reward", "done", "counts", "prey_alive_out", "success_out", "adj_bits", "chan_bits", "ave_deg",
-               "stats", "_spawn_agent", "_spawn_prey")
+               "stats", "_spawn_agent", "_spawn_prey", "cond_idx")
 
     def slice(self, b0: int, b1: int) -> "BatchedEnv":
         """View of the envs [b0, b1): shares every buffer with this object (all arrays are env-major, so the slices are
@@ -112,7 +148,7 @@ class BatchedEnv:
         for k in self._SLICED:
             t = getattr(self, k, None)
             setattr(v, k, None if t is None else t[b0:b1])
-        v.desc = self.spec.to_desc(N.ptr(self._wall), N.ptr(self._lut), env_id0=v.env_id0)
+        v.desc = v._desc()
         v.state = N.EnvState()
         v.state.n_envs = v.B
         for k in ("agent_pos", "prey_pos", "prey_alive", "visited", "step_count", "total_capture", "success",

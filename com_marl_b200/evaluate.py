@@ -32,22 +32,48 @@ def _details(scenario: str, n: int, counts: np.ndarray, reward: float, ave_deg) 
 
 
 def eval_model(env, policy, itr=0, n_eval_episodes=100, max_env_steps=200, eval_greedy=True, render=False,
-               inspect_steps=False, seed=1, flag=None, groups: int = 4, chunk: int = 50, return_trajectory: bool = False):
+               inspect_steps=False, seed=1, flag=None, groups: int = 4, chunk: int = 50, return_trajectory: bool = False,
+               env_id0: int = 0):
     """``env``: a com_marl_b200 gym wrapper (or anything with ``spec_b200``) or a ScenarioSpec.  Returns the reference's
     ``(episode_data, epi_success, epi_rewards, bound_return)``: ``episode_data[i] = (step_success, {vec: [per step]})``,
     ``epi_rewards[vec][i]`` = sum over the episode's steps (mean for ``nodeDeg``), ``epi_success[i]`` = ``env.success``
-    when the episode ended."""
+    when the episode ended.  ``env_id0``: global id of the first episode's env (the random streams are keyed by it)."""
     if render:
         raise NotImplementedError("rendering is out of scope (DESIGN.md §8)")
     if flag is not None and flag[0]:
         return None, None, None, None
-    spec = copy.copy(getattr(env, "spec_b200", env))
+    spec = _eval_spec(getattr(env, "spec_b200", env), seed)
+    return _evaluate(spec, None, policy, int(n_eval_episodes), max_env_steps, eval_greedy, groups, chunk, return_trajectory,
+                     env_id0)[0]
+
+
+def eval_sweep(env, policy, conditions, n_eval_episodes=100, max_env_steps=200, eval_greedy=True, seed=1, groups: int = 4,
+               chunk: int = 50, return_trajectory: bool = False):
+    """``eval_model`` over many channel conditions in ONE engine: ``conditions`` are specs that differ from ``env``'s in the
+    channel fields only (``spec.with_channel(pl=..., rcom=..., channel_type=...)``).  Condition k plays its
+    ``n_eval_episodes`` episodes in the envs with global ids ``k * n_eval_episodes ...``, so its result equals
+    ``eval_model(conditions[k], ..., env_id0=k * n_eval_episodes)``.  Returns one ``eval_model`` tuple per condition, in
+    order."""
+    spec = _eval_spec(getattr(env, "spec_b200", env), seed)
+    conds = [_eval_spec(c, seed) for c in conditions]
+    return _evaluate(spec, conds, policy, int(n_eval_episodes), max_env_steps, eval_greedy, groups, chunk, return_trajectory, 0)
+
+
+def _eval_spec(spec, seed):
+    spec = copy.copy(spec)
     spec.seed = int(seed)
     spec.max_path_length = 0
-    n, B = spec.n_agents, int(n_eval_episodes)
+    return spec
+
+
+def _evaluate(spec, conditions, policy, E, max_env_steps, eval_greedy, groups, chunk, return_trajectory, env_id0):
+    """the eval loop of eval_model / eval_sweep: E episodes per condition (one condition: ``spec``'s own channel) in one
+    RolloutEngine; -> one eval_model result per condition"""
+    conds = conditions or [spec]
+    B = E * len(conds)
     K = max(1, min(int(chunk), int(max_env_steps)))
-    eng = RolloutEngine(spec, policy, B, device=policy.device, ring=K, greedy=bool(eval_greedy), use_graph=True,
-                        groups=groups, auto_reset=False)
+    eng = RolloutEngine(spec, policy, B, device=policy.device, env_id0=env_id0, ring=K, greedy=bool(eval_greedy),
+                        use_graph=True, groups=groups, auto_reset=False, conditions=conditions)
     eng.reset()
     length = np.zeros(B, dtype=np.int64)              # 0 = still running
     keep = {k: [] for k in ("reward", "done", "counts", "ave_deg", "success", "actions")}
@@ -73,6 +99,13 @@ def eval_model(env, policy, itr=0, n_eval_episodes=100, max_env_steps=200, eval_
     policy.check_errors()
     length[length == 0] = steps                          # cut by max_env_steps (eval_pp.py:71)
     cat = {k: np.concatenate(v) for k, v in keep.items() if v}
+    return [_results(c, {k: v[:, i * E:(i + 1) * E] for k, v in cat.items()}, length[i * E:(i + 1) * E], return_trajectory)
+            for i, c in enumerate(conds)]
+
+
+def _results(spec, cat, length, return_trajectory):
+    """eval_model's tuple for one condition's episodes (columns of the recorded steps)"""
+    n, B = spec.n_agents, len(length)
     episode_data: List[Tuple[list, dict]] = []
     epi_success: List[int] = []
     epi_rewards: Dict[str, list] = {vec: [] for vec in VECTORS}

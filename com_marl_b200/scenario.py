@@ -7,7 +7,8 @@ Mirrors (without copying) the host-side set-up of
   runner sizing rules                  exp_runners/env_uitils.py:171-217
 and turns it into the plain numbers ``cm_env_desc`` (include/commarl_b200.h) carries.
 """
-from dataclasses import dataclass, field
+import copy
+from dataclasses import dataclass, field, fields
 from typing import Optional
 
 import numpy as np
@@ -179,29 +180,62 @@ class ScenarioSpec:
                 raise ValueError("n_agents must be divisible by n_groups (coverage.py:53)")
         else:
             raise ValueError(f"unknown scenario {scenario!r}")
-        # --- init_communication (env_communication.py:26-75) ---
         pref = "tr" if params.get("mode", "train") in ("train", "restore") else "te"
         pl = params.get(f"{pref}pl")
         if pl is None:
             raise ValueError("Loss probability is not applied (env_communication.py:31-32)")
-        if pl == 0:
-            spec.channel = N.CH_FC
-        elif 0 < pl < 1:
-            spec.channel = N.CH_IID
-        elif pl == 1:
-            spec.channel = N.CH_FL
-        else:
-            raise ValueError(f"invalid Ploss value: pl={pl}")
-        spec.p_loss = float(pl)
-        rcom = int(params.get(f"{pref}Rcom", 9))
-        spec.rcom = 0 if rcom + 1 >= m else rcom                # :71-72
-        spec.pgb = float(params.get("Pgb", 0.0196))
-        spec.pbg = float(params.get("Pbg", 0.282))
-        spec.ge_init = int(params.get("GE_INIT", 1))
+        return spec.with_channel(pl=pl, rcom=params.get(f"{pref}Rcom", 9), channel_type=channel_type,
+                                 pgb=params.get("Pgb", 0.0196), pbg=params.get("Pbg", 0.282), ge_init=params.get("GE_INIT", 1))
+
+    CHANNEL_FIELDS = ("channel", "p_loss", "rcom", "pgb", "pbg", "ge_init")
+
+    def with_channel(self, pl=None, rcom=None, channel_type: Optional[str] = None, pgb=None, pbg=None, ge_init=None):
+        """A copy under another channel condition, by the rules of the reference's init_communication
+        (env_communication.py:26-75): ``pl`` 0 -> FC, 0 < pl < 1 -> IID, 1 -> FL; ``rcom`` collapses to fully connected when
+        Rcom + 1 >= map; ``channel_type`` ('FC', 'FL', 'IID', 'GE') is applied last, as setting ``env.channelType`` after
+        construction does.  Arguments left at None keep this spec's value."""
+        spec = copy.copy(self)
+        if pl is not None:
+            if pl == 0:
+                spec.channel = N.CH_FC
+            elif 0 < pl < 1:
+                spec.channel = N.CH_IID
+            elif pl == 1:
+                spec.channel = N.CH_FL
+            else:
+                raise ValueError(f"invalid Ploss value: pl={pl}")
+            spec.p_loss = float(pl)
+        if rcom is not None:
+            rcom = int(rcom)
+            spec.rcom = 0 if rcom + 1 >= spec.map_size else rcom     # :71-72
+        if pgb is not None:
+            spec.pgb = float(pgb)
+        if pbg is not None:
+            spec.pbg = float(pbg)
+        if ge_init is not None:
+            spec.ge_init = int(ge_init)
         if channel_type is not None:
             spec.channel = {"FC": N.CH_FC, "FL": N.CH_FL, "IID": N.CH_IID, "GE": N.CH_GE}[channel_type]
         spec.validate()
         return spec
+
+    def same_except_channel(self, other: "ScenarioSpec") -> bool:
+        """whether ``other`` differs from this spec in the channel fields (CHANNEL_FIELDS) at most"""
+        for f in fields(self):
+            if f.name in self.CHANNEL_FIELDS:
+                continue
+            a, b = getattr(self, f.name), getattr(other, f.name)
+            if isinstance(a, np.ndarray) or isinstance(b, np.ndarray):
+                if a is None or b is None or not np.array_equal(a, b):
+                    return False
+            elif a != b:
+                return False
+        return True
+
+    def channel_cond(self) -> "N.ChannelCond":
+        """this spec's channel as one entry of a cm_channel_cond table"""
+        d = self.to_desc(None, None)
+        return N.ChannelCond(d.channel, d.rcom2, d.p_loss, d.pgb, d.pbg, d.ge_bad_rate, d.ge_init)
 
     @classmethod
     def from_cli(cls, scenario: str, map_size: int, sen: int, den: float, cap: int = 2, loss: float = 0.0, **over):

@@ -46,8 +46,8 @@
 extern "C" {
 #endif
 
-#define CM_ABI_VERSION 4   /* 2: host_arena / obs_bits members, cm_rollout_step_host; 3: cm_ppo_net; 4: CENT kinds of cm_ppo_net,
-                              cm_net_desc.flags */
+#define CM_ABI_VERSION 5   /* 2: host_arena / obs_bits members, cm_rollout_step_host; 3: cm_ppo_net; 4: CENT kinds of cm_ppo_net,
+                              cm_net_desc.flags; 5: cm_channel_cond, per-env channel conditions (cm_env_desc.conds ...) */
 #define CM_MAX_AGENTS 256   /* n, p */
 #define CM_MAX_GRID 64      /* grid side incl. Coverage's wall border */
 #define CM_MAX_LAYERS 4     /* n_gcn_layers */
@@ -65,6 +65,17 @@ enum cm_error {
     CM_ENODEVICE = -4,
     CM_EACTION = -5       /* an action outside 0..4 was seen ('Action Not found!', predator_prey.py:255) */
 };
+
+/* One channel condition: the members of cm_env_desc of the same names, with the same meaning and float32 rounding. */
+typedef struct cm_channel_cond {
+    int32_t channel;           /* cm_channel */
+    int32_t rcom2;
+    float p_loss;
+    float pgb, pbg;
+    float ge_bad_rate;
+    int32_t ge_init;
+} cm_channel_cond;
+#define CM_MAX_CONDS 256
 
 /* Scenario description (host).  Replaces the attribute soup PredatorPrey.__init__ / Coverage.__init__ /
  * init_communication build from `params` (predator_prey.py:51-108, coverage.py:39-109,
@@ -93,6 +104,17 @@ typedef struct cm_env_desc {
     int64_t env_id0;           /* global id of env 0 of this shard: results do not depend on the sharding */
     const uint64_t *wall_rows; /* DEVICE u64 [G]: Coverage wall bitmap rows (border + obstacles); NULL for PredatorPrey */
     const float *lut;          /* DEVICE f32 [G + G + T + 1]: obs scalar features row[r], col[c], time[t] */
+    /* Per-env channel conditions (ABI 5; zero = NULL = one condition per launch, the members above).  Env b communicates
+     * under conds[cond_idx[b]] instead of the descriptor's channel, rcom2, p_loss, pgb, pbg, ge_bad_rate and ge_init; every
+     * other member stays uniform across the launch.  One launch may mix FC, FL, IID and GE (the reference's test-mode grid
+     * of loss rate x Rcom x channel model).  Every entry is validated like the descriptor's own channel (GE_INIT = -1 with
+     * loss_apply = 0 -> CM_EUNSUPPORTED; ge_state needed when an entry is GE; injected chan_u must hold the largest plane
+     * count of any entry).  Validation reads conds_host, which the caller keeps equal to the device table, so that the call
+     * never synchronises.  A cond_idx value >= n_conds reads entry 0 and sets io.error_flag to CM_EINVAL. */
+    const cm_channel_cond *conds;      /* DEVICE [n_conds] */
+    const uint8_t *cond_idx;           /* DEVICE [B] */
+    int32_t n_conds;                   /* 1 .. CM_MAX_CONDS */
+    const cm_channel_cond *conds_host; /* HOST copy of conds, read at call time */
 } cm_env_desc;
 
 typedef struct cm_env_state {
