@@ -1002,7 +1002,8 @@ struct PolicyHeadArgs {
     const float *adv, *old_ll;   // [S]
     const uint8_t *valid;        // [S] or NULL
     float inv_count, ent_coeff, clip_lo, clip_hi;
-    float *ll, *ent, *probs, *loss;
+    float *ll, *ent, *probs;
+    double *loss;                // the call's loss, summed in float64 (cm_ppo_net adds it to io.loss at the end)
     float *dg3, *dw4, *db4;      // NULL: forward only; dg3 receives dZ of the last hidden layer: d g3 act'(g3)
     float *dlogits;              // CENT: [S][5n] d logits for the dW4 product
     int relu;                    // CENT: act = relu instead of tanh
@@ -1064,9 +1065,24 @@ __device__ __forceinline__ void head_tail_bwd(float gl, float ge, int act, uint3
     for (int j = 0; j < CM_ACTIONS; ++j) gz[j] = p[j] * (gp[j] - dot);
 }
 
+// The loss terms of a CTA reach the call's sum in ONE float64 atomic add.  Added step by step into one fp32 value, 10^5 terms
+// of one sign lose ~1e-3 of the sum (each rounds against the growing total with the same bias), and even one fp32 add per CTA
+// loses ~1e-5: the running total must be float64 and see one term per CTA.
+// Called once by every thread after its last block; *red1 was zeroed before the kernel's first barrier.
+__device__ __forceinline__ void cta_loss_add(double *loss, float lsum, float *red1)
+{
+    const float v = warp_sumf(lsum);
+    if ((threadIdx.x & 31) == 0) atomicAdd(red1, v);
+    __syncthreads();
+    if (threadIdx.x == 0) atomicAdd(loss, (double)*red1);
+}
+
+__global__ void net_loss_store_kernel(float *loss, const double *sum) { *loss += (float)*sum; }
+
 // One env step s with joint log-likelihood ll and mean entropy en: outputs, the clipped surrogate added to the loss and the
 // gradients gl = d loss / d ll, ge = d loss / d (one agent's entropy)
-__device__ __forceinline__ void head_step_objective(const PolicyHeadArgs &a, int64_t s, float ll, float en, int n, float &gl, float &ge)
+__device__ __forceinline__ void head_step_objective(const PolicyHeadArgs &a, int64_t s, float ll, float en, int n, float &gl, float &ge,
+                                                    float &lsum)
 {
     if (a.ll) a.ll[s] = ll;
     if (a.ent) a.ent[s] = en;
@@ -1081,7 +1097,7 @@ __device__ __forceinline__ void head_step_objective(const PolicyHeadArgs &a, int
         const float in = (ratio >= a.clip_lo && ratio <= a.clip_hi) ? 1.0f : 0.0f;
         // torch.min's gradient goes to the smaller argument, half to each on a tie; clamp passes it inside [lo, hi]
         const float gr = s1 < s2 ? adv : (s1 > s2 ? adv * in : 0.5f * adv + 0.5f * adv * in);
-        if (a.loss) atomicAdd(a.loss, -(fminf(s1, s2) + a.ent_coeff * en) * a.inv_count);
+        lsum += -(fminf(s1, s2) + a.ent_coeff * en) * a.inv_count;
         gl = -a.inv_count * gr * ratio;
         ge = -a.inv_count * a.ent_coeff / (float)n;
     }
@@ -1091,9 +1107,11 @@ __global__ void __launch_bounds__(kNetThreads) net_policy_head_kernel(const Poli
 {
     __shared__ float w4s[32 * CM_ACTIONS + CM_ACTIONS];
     __shared__ float ll_row[kRows], ent_row[kRows], gll_env[kRows], gent_env[kRows];
-    __shared__ float red[32 * CM_ACTIONS + CM_ACTIONS];
+    __shared__ float red[32 * CM_ACTIONS + CM_ACTIONS], lred;
     const int tid = threadIdx.x, lane = tid & 31;
     const int n = a.n;
+    float lsum = 0.0f;
+    if (tid == 0) lred = 0.0f;
     for (int i = tid; i < 32 * CM_ACTIONS + CM_ACTIONS; i += kNetThreads) {
         w4s[i] = i < 32 * CM_ACTIONS ? a.w4[i] : a.b4[i - 32 * CM_ACTIONS];
         red[i] = 0.0f;
@@ -1139,7 +1157,7 @@ __global__ void __launch_bounds__(kNetThreads) net_policy_head_kernel(const Poli
             for (int i = 0; i < n; ++i) { ll += ll_row[tid * n + i]; en += ent_row[tid * n + i]; }
             en = en / (float)n;
             float gl, ge;
-            head_step_objective(a, eb.s0 + tid, ll, en, n, gl, ge);
+            head_step_objective(a, eb.s0 + tid, ll, en, n, gl, ge, lsum);
             gll_env[tid] = gl;
             gent_env[tid] = ge;
         }
@@ -1187,6 +1205,7 @@ __global__ void __launch_bounds__(kNetThreads) net_policy_head_kernel(const Poli
         for (int i = tid; i < 32 * CM_ACTIONS + CM_ACTIONS; i += kNetThreads)
             atomicAdd(i < 32 * CM_ACTIONS ? a.dw4 + i : a.db4 + (i - 32 * CM_ACTIONS), red[i]);
     }
+    if (a.loss) cta_loss_add(a.loss, lsum, &lred);
 }
 
 // CENT head: the rows are env steps, logits [S][5n] = g3 W4 + b4 with W4 [32][5n].  Thread = (step, agent), the G = 256 / n steps
@@ -1197,8 +1216,10 @@ __global__ void __launch_bounds__(kNetThreads) net_policy_head_kernel(const Poli
 __global__ void __launch_bounds__(kNetThreads) net_cent_head_kernel(const PolicyHeadArgs a)
 {
     __shared__ float ll_row[kRows], ent_row[kRows], gll_env[kRows], gent_env[kRows];
-    __shared__ float dgs[kRows * 33];
+    __shared__ float dgs[kRows * 33], lred;
     const int tid = threadIdx.x;
+    float lsum = 0.0f;
+    if (tid == 0) lred = 0.0f;
     const int n = a.n, NO = n * CM_ACTIONS;
     const int ia = tid % n;                                       // this thread's agent (the same in every block)
     const float *__restrict__ w4 = a.w4 + ia * CM_ACTIONS;
@@ -1249,7 +1270,7 @@ __global__ void __launch_bounds__(kNetThreads) net_cent_head_kernel(const Policy
             for (int i = 0; i < n; ++i) { ll += ll_row[tid * n + i]; en += ent_row[tid * n + i]; }
             en = en / (float)n;
             float gl, ge;
-            head_step_objective(a, eb.s0 + tid, ll, en, n, gl, ge);
+            head_step_objective(a, eb.s0 + tid, ll, en, n, gl, ge, lsum);
             gll_env[tid] = gl;
             gent_env[tid] = ge;
         }
@@ -1281,6 +1302,7 @@ __global__ void __launch_bounds__(kNetThreads) net_cent_head_kernel(const Policy
     if (a.dg3 && tid < a.G * n)
 #pragma unroll
         for (int j = 0; j < CM_ACTIONS; ++j) atomicAdd(a.db4 + ia * CM_ACTIONS + j, dbacc[j]);
+    if (a.loss) cta_loss_add(a.loss, lsum, &lred);
 }
 
 struct CriticHeadArgs {
@@ -1288,7 +1310,8 @@ struct CriticHeadArgs {
     const float *w2, *b2, *log_std;   // [64], [1], [1]
     const float *returns;        // [S] or NULL (forward only)
     float inv_count;
-    float *values, *loss;
+    float *values;
+    double *loss;                // (as PolicyHeadArgs::loss)
     float *dc1, *dw2, *db2, *dlog_std;
     int unclamped;               // 1: std = exp(log_std) without CommBaseCritic's clamp at log 1e-6 (GaussianMLPBaseline)
     int n, G;
@@ -1297,9 +1320,11 @@ struct CriticHeadArgs {
 
 __global__ void __launch_bounds__(kNetThreads) net_critic_head_kernel(const CriticHeadArgs a)
 {
-    __shared__ float w2s[64], v_row[kRows], gv_env[kRows], red[66];
+    __shared__ float w2s[64], v_row[kRows], gv_env[kRows], red[66], lred;
     const int tid = threadIdx.x, lane = tid & 31;
     const int n = a.n;
+    float lsum = 0.0f;
+    if (tid == 0) lred = 0.0f;
     if (tid < 64) w2s[tid] = a.w2[tid];
     if (tid < 66) red[tid] = 0.0f;
     const float b2 = a.b2[0];
@@ -1333,7 +1358,7 @@ __global__ void __launch_bounds__(kNetThreads) net_critic_head_kernel(const Crit
             float gv = 0.0f;
             if (a.returns) {
                 const float d = (a.returns[s] - V) / sd;
-                if (a.loss) atomicAdd(a.loss, (0.5f * d * d + logf(sd) + 0.91893853320467274178f) * a.inv_count);
+                lsum += (0.5f * d * d + logf(sd) + 0.91893853320467274178f) * a.inv_count;
                 gv = -d / sd * a.inv_count;
                 if (a.dlog_std && ls >= lmin) atomicAdd(&red[65], (1.0f - d * d) * a.inv_count);
             }
@@ -1364,6 +1389,7 @@ __global__ void __launch_bounds__(kNetThreads) net_critic_head_kernel(const Crit
         if (tid == 64) atomicAdd(a.db2, red[64]);
         if (tid == 65 && a.dlog_std) atomicAdd(a.dlog_std, red[65]);
     }
+    if (a.loss) cta_loss_add(a.loss, lsum, &lred);
 }
 
 // ------------------------------------------------------------------------------------------------------------------
@@ -1842,7 +1868,7 @@ static cudaError_t softmax_bwd(const EnvCall &c, const float *M, const float *dM
 }
 
 // workspace of one chunk of `steps` env steps (floats)
-static constexpr size_t kWsSlack = 160;      // alignment of the base pointer and of each of the <= 30 carved arrays
+static constexpr size_t kWsSlack = 164;      // alignment of the base pointer and of each of the <= 30 carved arrays; the loss sum
 struct NetWs {
     float *h1, *E, *Q, *M, *V[CM_MAX_LAYERS], *H[CM_MAX_LAYERS], *X, *g1, *g2, *g3, *t32, *t64a, *t64b, *t64c, *t128, *dM, *CT;
 };
@@ -1934,7 +1960,8 @@ static Blob trunk_of(const CriticBlob &cb)
 }
 
 // the CENT family: policy (CentralizedCategoricalMLPPolicy) or baseline (GaussianMLPBaseline) over `steps` env steps, one row per step
-static cudaError_t run_chunk_cent(const cm_net_desc &d, const cm_net_io &io, int64_t s0, int64_t steps, float *wsp, cudaStream_t st)
+static cudaError_t run_chunk_cent(const cm_net_desc &d, const cm_net_io &io, int64_t s0, int64_t steps, float *wsp, double *lacc,
+                                  cudaStream_t st)
 {
     const int n = d.n_agents, K = n * d.obs_dim, NO = n * CM_ACTIONS;
     const bool backward = io.grad != nullptr;
@@ -1954,7 +1981,7 @@ static cudaError_t run_chunk_cent(const cm_net_desc &d, const cm_net_io &io, int
         a.returns = io.returns ? io.returns + s0 : nullptr;
         a.inv_count = io.inv_count;
         a.values = io.values ? io.values + s0 : nullptr;
-        a.loss = io.loss;
+        a.loss = lacc;
         a.unclamped = 1;
         a.n = 1; a.G = env_group(1); a.S = steps;
         float *dz3 = nullptr, *dz2 = nullptr, *dz1 = nullptr;
@@ -1986,7 +2013,7 @@ static cudaError_t run_chunk_cent(const cm_net_desc &d, const cm_net_io &io, int
     a.ll = io.ll ? io.ll + s0 : nullptr;
     a.ent = io.entropy ? io.entropy + s0 : nullptr;
     a.probs = io.probs ? io.probs + s0 * n * CM_ACTIONS : nullptr;
-    a.loss = io.loss;
+    a.loss = lacc;
     a.relu = act == 2;
     a.n = n; a.G = env_group(n); a.S = steps;
     float *dz3 = nullptr, *dz2 = nullptr, *dz1 = nullptr;
@@ -2004,9 +2031,9 @@ static cudaError_t run_chunk_cent(const cm_net_desc &d, const cm_net_io &io, int
     return wide_dw_t<128, 0>(obs, K, dz1, g + o.w1, g + o.b1, R, K, st);
 }
 
-static cudaError_t run_chunk(const cm_net_desc &d, const cm_net_io &io, int64_t s0, int64_t steps, float *wsp, cudaStream_t st)
+static cudaError_t run_chunk(const cm_net_desc &d, const cm_net_io &io, int64_t s0, int64_t steps, float *wsp, double *lacc, cudaStream_t st)
 {
-    if (cent_kind(d.kind)) return run_chunk_cent(d, io, s0, steps, wsp, st);
+    if (cent_kind(d.kind)) return run_chunk_cent(d, io, s0, steps, wsp, lacc, st);
     const int n = d.n_agents, D = d.obs_dim, L = d.n_layers, W = (n + 31) / 32;
     const bool backward = io.grad != nullptr;
     const NetWs w = carve(wsp, n, L, steps, backward);
@@ -2044,7 +2071,7 @@ static cudaError_t run_chunk(const cm_net_desc &d, const cm_net_io &io, int64_t 
         a.ll = io.ll ? io.ll + s0 : nullptr;
         a.ent = io.entropy ? io.entropy + s0 : nullptr;
         a.probs = io.probs ? io.probs + r0 * CM_ACTIONS : nullptr;
-        a.loss = io.loss;
+        a.loss = lacc;
         a.n = n; a.G = G; a.S = steps;
         if (backward) { a.dg3 = w.t32; a.dw4 = io.grad + o.head_w4; a.db4 = io.grad + o.head_b4; }
         net_policy_head_kernel<<<env_grid(n, steps, 4), kNetThreads, 0, st>>>(a);
@@ -2072,7 +2099,7 @@ static cudaError_t run_chunk(const cm_net_desc &d, const cm_net_io &io, int64_t 
     a.returns = io.returns ? io.returns + s0 : nullptr;
     a.inv_count = io.inv_count;
     a.values = io.values ? io.values + s0 : nullptr;
-    a.loss = io.loss;
+    a.loss = lacc;
     a.n = n; a.G = G; a.S = steps;
     if (backward) { a.dc1 = w.t64a; a.dw2 = io.grad + cb.dec_w2; a.db2 = io.grad + cb.dec_b2; a.dlog_std = io.grad + cb.log_std; }
     net_critic_head_kernel<<<env_grid(n, steps, 4), kNetThreads, 0, st>>>(a);
@@ -2119,10 +2146,17 @@ extern "C" int cm_ppo_net(const cm_net_desc *desc, const cm_net_io *io, cm_strea
     if (io->workspace_floats < per_step + kWsSlack) return CM_EINVAL;
     const int64_t chunk = (int64_t)((io->workspace_floats - kWsSlack) / per_step);
     float *wsp = reinterpret_cast<float *>((reinterpret_cast<uintptr_t>(io->workspace) + 15) & ~(uintptr_t)15);
-    for (int64_t s0 = 0; s0 < io->n_steps; s0 += chunk) {
+    double *lacc = io->loss ? reinterpret_cast<double *>(wsp) : nullptr;      // the loss sum of every chunk (16-byte aligned)
+    wsp += 4;
+    const cudaStream_t st = (cudaStream_t)stream;
+    cudaError_t e = lacc ? cudaMemsetAsync(lacc, 0, sizeof(double), st) : cudaSuccess;
+    for (int64_t s0 = 0; e == cudaSuccess && s0 < io->n_steps; s0 += chunk) {
         int64_t steps = io->n_steps - s0 < chunk ? io->n_steps - s0 : chunk;
-        const cudaError_t e = run_chunk(d, *io, s0, steps, wsp, (cudaStream_t)stream);
-        if (e != cudaSuccess) return set_cuda_error(e, CM_ECUDA);
+        e = run_chunk(d, *io, s0, steps, wsp, lacc, st);
     }
-    return CM_OK;
+    if (e == cudaSuccess && lacc) {
+        net_loss_store_kernel<<<1, 1, 0, st>>>(io->loss, lacc);
+        e = cudaGetLastError();
+    }
+    return e == cudaSuccess ? CM_OK : set_cuda_error(e, CM_ECUDA);
 }

@@ -389,7 +389,7 @@ typedef struct cm_net_io {
     float *ll, *entropy;       /* policy outputs [S], optional */
     float *probs;              /* policy output [S][n][5], optional */
     float *values;             /* critic output [S], optional */
-    float *loss;               /* DEVICE f32[1], optional: the loss is ADDED to it */
+    float *loss;               /* DEVICE f32[1], optional: the loss (summed in float64 over the call) is ADDED to it */
     float *workspace;
     size_t workspace_floats;
 } cm_net_io;
