@@ -259,7 +259,7 @@ struct CentL1Args {
     int K, n_panels;
 };
 
-// W1 [K][128] fp32 -> per K panel of 64 the stacked [W1_hi ; W1_lo] (256 rows x 64 k) in the canonical K-major core-matrix layout
+// W1 [K][128] fp32 -> per K panel of kL1KP = 32 the stacked [W1_hi ; W1_lo] (256 rows x 32 k) in the canonical K-major core-matrix layout
 __global__ void cent_l1_prepare_kernel(const float *__restrict__ w1, __half *__restrict__ out, int K, int n_panels)
 {
     const int total = n_panels * kL1KP * kC1;

@@ -208,9 +208,13 @@ class CommCategoricalMLPPolicy(nn.Module):
                 self._tc_error = torch.zeros(1, dtype=torch.int32, device=self.device)
         return self._tc_blob
 
-    def refresh_weights(self):
+    def refresh_weights(self, force=False):
         """bring the kernel weight blobs up to date with the parameters (in place; cheap signature check when nothing
-        changed) — the rollout engine calls this before replaying a captured graph"""
+        changed) — the rollout engine calls this before replaying a captured graph.  The signature reads the parameters'
+        version counters, which every in-place op on a parameter, ``load_state_dict`` and FlatAdam bump; a write through
+        ``p.data`` (``p.data.add_``, optimizers and loaders written that way) does not: call with ``force=True`` after one."""
+        if force:
+            self._blob_sig = self._tc_sig = None
         if self.uses_tensor_cores():
             self.tc_weight_blob()
         else:
@@ -645,7 +649,7 @@ class CentralizedCategoricalMLPPolicy(nn.Module):
         return self._blob
 
     def tc_weight_blob(self):
-        """[W1_hi ; W1_lo] per K panel of 64 in the tensor cores' operand layout (cm_policy_tc_prepare); rebuilt when a parameter changed"""
+        """[W1_hi ; W1_lo] (256 x 32) per K panel of 32 in the tensor cores' operand layout (cm_policy_tc_prepare); rebuilt when a parameter changed"""
         blob = self.weight_blob()
         if self._tc_blob is None or self._tc_sig != self._blob_sig:
             out = self._tc_blob if self._tc_blob is not None else \

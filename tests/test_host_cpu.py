@@ -235,3 +235,29 @@ def test_channel_draw_integer_threshold_is_the_float_compare():
         assert np.array_equal(u < thr, words < tw), thr
         # the diagonal link: u + 1 lies in [1, 2), never below / always at or above a threshold inside (0, 1)
         assert np.all((u + np.float32(1.0)) >= thr) and not np.any((u + np.float32(1.0)) < thr)
+
+
+def test_action_stream_restatement_matches_oracle_philox():
+    """tests/policy_kinds_util.py restates categorical_finish's in-kernel draw for the GPU tests: its numpy Philox4x32-10 equals
+    the oracle's C implementation word for word (key = both halves of a 64-bit seed, counters near 2^32), u24 is (w >> 8) 2^-24
+    on [0, 1), and action_u picks word il & 3 of block il >> 2 with the stream id 4 | episode << 8"""
+    import policy_kinds_util as U
+    rng = np.random.default_rng(0)
+    for seed in (0, 7, 0x1234_5678_9ABC_DEF0, 2**64 - 1):
+        c = rng.integers(0, 2**32, (64, 4), dtype=np.uint64)
+        c[0] = 2**32 - 1
+        got = U.philox4x32_10(seed, c[:, 0], c[:, 1], c[:, 2], c[:, 3])
+        for i in range(len(c)):
+            assert np.array_equal(got[i], orc.philox(seed, *(int(x) for x in c[i]))), (seed, i)
+    w = np.array([0, 255, 256, 2**31, 2**32 - 1] + rng.integers(0, 2**32, 1000).tolist(), np.uint32)
+    u = U.u24(w)
+    assert u.dtype == np.float32 and (u >= 0).all() and (u < 1).all()
+    assert np.array_equal(u.astype(np.float64), (w >> 8).astype(np.float64) / 2**24)
+    assert u[1] == 0 and u[2] == 2**-24 and u[4] == 1 - 2**-24
+    seed, env_id0, n = 99, 2**32 - 3, 10
+    tick, episode = np.array([5, 2**31 - 1], np.int32), np.array([3, 2**24 - 1], np.int32)
+    got = U.action_u(seed, env_id0, [0, 1], tick, episode, n)
+    for e in range(2):
+        for il in range(n):
+            blk = orc.philox(seed, (env_id0 + e) % 2**32, int(tick[e]), (4 | int(episode[e]) << 8) % 2**32, il >> 2)
+            assert got[e, il] == np.float32((int(blk[il & 3]) >> 8) * 2.0**-24), (e, il)
