@@ -16,7 +16,7 @@ CH_FC, CH_FL, CH_IID, CH_GE = 0, 1, 2, 3
 POLICY_COMM, POLICY_DEC, POLICY_CENT = 0, 1, 2
 POLICY_FLAG_RELU = 1
 MAX_AGENTS, MAX_GRID, MAX_LAYERS = 256, 64, 4
-ABI_VERSION = 5
+ABI_VERSION = 6
 MAX_CONDS = 256
 
 EXPORTS = ("cm_abi_version", "cm_strerror", "cm_last_cuda_error", "cm_device_count", "cm_env_reset", "cm_env_step",
@@ -70,7 +70,8 @@ class PolicyIO(C.Structure):
                [(k, C.c_void_p) for k in ("weights", "obs", "adj_bits", "chan_bits", "avail_bits", "sample_u", "tick",
                                           "episode", "probs", "logits", "attention", "actions", "tc_weights",
                                           "error_flag", "workspace")] + \
-               [("workspace_bytes", C.c_size_t), ("obs_bits", C.c_void_p), ("obs_nbits", C.c_int32), ("host_arena", C.c_int32)]
+               [("workspace_bytes", C.c_size_t), ("obs_bits", C.c_void_p), ("obs_nbits", C.c_int32), ("host_arena", C.c_int32)] + \
+               [("n_policies", C.c_int32), ("envs_per_policy", C.c_int64), ("weights_stride", C.c_int64), ("tc_weights_stride", C.c_int64)]
 
 
 class NetDesc(C.Structure):

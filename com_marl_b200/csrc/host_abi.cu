@@ -80,6 +80,7 @@ extern "C" int cm_policy_forward_host(const cm_policy_desc *desc, const cm_polic
     using namespace cm;
     if (!desc || !dev || !host) return CM_EINVAL;
     if (desc->n_agents < 1 || desc->n_agents > CM_MAX_AGENTS || desc->obs_dim < 1 || dev->n_envs < 0) return CM_EINVAL;
+    if (dev->n_policies > 1 || host->n_policies > 1) return CM_EUNSUPPORTED;      // one policy per host-buffer call
     cudaStream_t s = (cudaStream_t)stream;
     const size_t B = (size_t)dev->n_envs, n = (size_t)desc->n_agents, D = (size_t)desc->obs_dim, L = (size_t)desc->n_layers;
     const size_t W = (n + 31) / 32, rows = B * n;
@@ -166,6 +167,7 @@ extern "C" int cm_rollout_step_host(const cm_policy_desc *pol_desc, const cm_pol
     if (!pol_dev->actions || pol_dev->actions != env_dev->actions) return CM_EINVAL;      // the step consumes the sampled actions
     if (!pol_dev->obs || pol_dev->obs != env_dev->obs) return CM_EINVAL;                  // ... and leaves the next observation there
     if (pol_dev->n_envs != state->n_envs || pol_desc->n_agents != env_desc->n_agents) return CM_EINVAL;
+    if (pol_dev->n_policies > 1 || pol_host->n_policies > 1) return CM_EUNSUPPORTED;
     cudaStream_t s = (cudaStream_t)stream;
     const size_t B = (size_t)state->n_envs, n = (size_t)env_desc->n_agents;
     if (B == 0) return CM_OK;

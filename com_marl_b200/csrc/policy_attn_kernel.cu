@@ -36,9 +36,10 @@ struct AttnArgs {
     float *scr_q;                         // [B n][64]  in: Q rows, out: X rows (in place, row by row)
     float *scr_hw;                        // [B n][64]  in: H_0 Wg_0; rewritten in place with H_l Wg_l of the later layers
     int64_t n_envs;
+    int64_t envs_per_policy, weights_stride;   // several policies (kMulti): env b reads the blob at weights + (b / envs_per_policy) * weights_stride
 };
 
-template <int RT, int KT>
+template <int RT, int KT, bool kMulti>
 __global__ void __launch_bounds__(kAThreads, (RT * KT <= 30) ? 2 : 1) policy_attn_kernel(const AttnArgs A)
 {
     constexpr int NK = 32 * KT, AP = NK + 4;
@@ -56,6 +57,7 @@ __global__ void __launch_bounds__(kAThreads, (RT * KT <= 30) ? 2 : 1) policy_att
 
     for (int64_t env = blockIdx.x; env < A.n_envs; env += gridDim.x) {
         const size_t r_env = (size_t)env * n;
+        const float *wts = kMulti ? A.weights + (env / A.envs_per_policy) * A.weights_stride : A.weights;
         __syncthreads();                         // the previous env's keys / values are dead
         for (int e = tid; e < NK * 16; e += kAThreads) {
             const int j = e >> 4, c = (e & 15) << 2;
@@ -72,7 +74,7 @@ __global__ void __launch_bounds__(kAThreads, (RT * KT <= 30) ? 2 : 1) policy_att
                 *reinterpret_cast<float4 *>(HWs + j * 64 + c) = v;
             }
             __syncthreads();
-            const float *bias = A.weights + o.gcn_b + l * kE;
+            const float *bias = wts + o.gcn_b + l * kE;
             const float4 b4 = __ldg(reinterpret_cast<const float4 *>(bias + cl));
             for (int grp = warp; grp < n_groups; grp += kAWarps) {
                 const int i0 = grp * RT;                             // first query row of this group
@@ -208,7 +210,7 @@ __global__ void __launch_bounds__(kAThreads, (RT * KT <= 30) ? 2 : 1) policy_att
                             *reinterpret_cast<float4 *>(Aw + r * AP + cl) = make_float4(acc[r][0], acc[r][1], acc[r][2], acc[r][3]);
                     }
                     __syncwarp();
-                    const float *wg = A.weights + o.gcn_w + (size_t)(l + 1) * kE * kE + 2 * lane;
+                    const float *wg = wts + o.gcn_w + (size_t)(l + 1) * kE * kE + 2 * lane;
                     float o2[RT][2];
 #pragma unroll
                     for (int r = 0; r < RT; ++r) o2[r][0] = o2[r][1] = 0.0f;
@@ -258,21 +260,24 @@ static int launch_attn_t(const AttnArgs &A, cudaStream_t stream)
 {
     constexpr int NK = 32 * KT;
     constexpr size_t smem = (size_t)(NK * kEPitch + NK * 64 + kAWarps * RT * (NK + 4)) * sizeof(float);
-    static thread_local struct { int dev; int slots; } cache = {-1, 0};
+    static thread_local struct { int dev; int slots; } caches[2] = {{-1, 0}, {-1, 0}};
+    const bool multi = A.weights_stride != 0;
+    auto &cache = caches[multi];
+    void (*kern)(const AttnArgs) = multi ? policy_attn_kernel<RT, KT, true> : policy_attn_kernel<RT, KT, false>;
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess) return set_cuda_error(cudaGetLastError(), CM_ENODEVICE);
     if (cache.dev != dev) {
         int sms = 0, ctas = 0;
         if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return set_cuda_error(cudaGetLastError(), CM_ECUDA);
-        cudaError_t e = cudaFuncSetAttribute(policy_attn_kernel<RT, KT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return set_cuda_error(e, CM_ECUDA);
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas, policy_attn_kernel<RT, KT>, kAThreads, smem) != cudaSuccess)
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas, kern, kAThreads, smem) != cudaSuccess)
             return set_cuda_error(cudaGetLastError(), CM_ECUDA);
         cache.dev = dev;
         cache.slots = sms * (ctas < 1 ? 1 : ctas);
     }
     const int grid = (int)(A.n_envs < cache.slots ? A.n_envs : cache.slots);
-    policy_attn_kernel<RT, KT><<<grid, kAThreads, smem, stream>>>(A);
+    kern<<<grid, kAThreads, smem, stream>>>(A);
     cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? CM_OK : set_cuda_error(e, CM_ECUDA);
 }
@@ -365,6 +370,8 @@ int launch_policy_tc_large(const cm_policy_desc *desc, const cm_policy_io *io, c
     A.attention = io->attention;
     A.scr_e = scr_e; A.scr_q = scr_q; A.scr_hw = scr_hw;
     A.n_envs = io->n_envs;
+    A.envs_per_policy = io->n_policies > 1 ? io->envs_per_policy : io->n_envs;
+    A.weights_stride = io->n_policies > 1 ? io->weights_stride : 0;       // 0: one policy (the kMulti = false kernels)
     const int KT = (n + 31) / 32, RT = attn_choose_rt(n, KT);      // keys per lane, query rows per group
     switch (KT) {
     case 3: rc = launch_attn_k<3>(RT, A, stream); break;

@@ -25,6 +25,8 @@
 #include <math.h>
 #include <stdint.h>
 
+#include <type_traits>
+
 #include "commarl_b200.h"
 #include "common.cuh"
 #include "policy_layout.cuh"
@@ -45,6 +47,19 @@ struct AttnMmaArgs {
     float *scr_hw;
     int64_t n_envs;
 };
+// several policies (the kMulti kernels): env b reads the blob at weights + (b / envs_per_policy) * weights_stride.  A struct of its
+// own, so that the one-policy kernels keep their parameter block
+struct AttnMmaSetArgs : AttnMmaArgs {
+    int64_t envs_per_policy, weights_stride;
+};
+template <bool kMulti>
+using AttnMmaArgsOf = typename std::conditional<kMulti, AttnMmaSetArgs, AttnMmaArgs>::type;
+template <bool kMulti>
+__device__ __forceinline__ int64_t blob_offset(const AttnMmaArgsOf<kMulti> &A, int64_t env)
+{
+    if constexpr (kMulti) return (env / A.envs_per_policy) * A.weights_stride;
+    else return 0;
+}
 
 __device__ __forceinline__ void mma16816(float (&c)[4], const uint32_t (&a)[4], uint32_t b0, uint32_t b1)
 {
@@ -248,8 +263,8 @@ __device__ __forceinline__ void attn_record_block(float *att0, float *att1, bool
 // far below one once the masks remove the keys that carry the attention mass, and their fp16 hi / lo split would lose its
 // relative precision (or flush to zero) before the division by their small sum.  The unmasked softmax itself (agent_infos['attention_weights']) is written, when asked for, by a second
 // walk over the blocks with the final m and z.
-template <int NS, int WARPS>
-__global__ void __launch_bounds__(WARPS * 32, 1) policy_attn_mma_kernel(const AttnMmaArgs A)
+template <int NS, int WARPS, bool kMulti>
+__global__ void __launch_bounds__(WARPS * 32, 1) policy_attn_mma_kernel(const AttnMmaArgsOf<kMulti> A)
 {
     constexpr int NK = 16 * NS, NT = 2 * NS, NFULL = NT / 8, TAIL = NT % 8, HWP = NK + 8, THREADS = WARPS * 32;   // key blocks of 8 tiles + a tail
     extern __shared__ __align__(16) unsigned char smraw[];
@@ -271,6 +286,7 @@ __global__ void __launch_bounds__(WARPS * 32, 1) policy_attn_mma_kernel(const At
 
     for (int64_t env = blockIdx.x; env < A.n_envs; env += gridDim.x) {
         const size_t r_env = (size_t)env * n;
+        const int64_t wofs = blob_offset<kMulti>(A, env);                                  // this env's policy blob
         __syncthreads();                                       // the previous env's operands are dead
         // ---- keys: E rows -> fp16 hi / lo ----
         // (unconditional loads from a clamped row, zeroed afterwards: predicated loads are not batched by the compiler)
@@ -303,7 +319,7 @@ __global__ void __launch_bounds__(WARPS * 32, 1) policy_attn_mma_kernel(const At
             }
             // ---- Wg_{l+1} (k-major [k][c] in the blob) -> transposed fp16 hi / lo [c][k] ----
             if (l + 1 < L) {
-                const float *wg = A.weights + o.gcn_w + (size_t)(l + 1) * kE * kE;
+                const float *wg = A.weights + wofs + o.gcn_w + (size_t)(l + 1) * kE * kE;
 #pragma unroll 4
                 for (int e = tid; e < kE * kE; e += THREADS) {
                     const int k = e >> 6, c = e & 63;
@@ -314,7 +330,7 @@ __global__ void __launch_bounds__(WARPS * 32, 1) policy_attn_mma_kernel(const At
                 }
             }
             __syncthreads();
-            const float *bias = A.weights + o.gcn_b + l * kE;
+            const float *bias = A.weights + wofs + o.gcn_b + l * kE;
             for (int strip = warp; strip < n_strips; strip += WARPS) {
                 const int i0 = strip << 4;                     // first query row of the strip; this lane owns rows i0+g, i0+g+8
                 __syncwarp();
@@ -445,8 +461,8 @@ __global__ void __launch_bounds__(WARPS * 32, 1) policy_attn_mma_kernel(const At
     }
 }
 
-template <int NS>
-static int launch_attn_mma_t(const AttnMmaArgs &A, cudaStream_t stream)
+template <int NS, bool kMulti>
+static int launch_attn_mma_t(const AttnMmaArgsOf<kMulti> &A, cudaStream_t stream)
 {
     constexpr int NK = 16 * NS;
     constexpr size_t base = (size_t)(2 * NK * kEhPitch + 2 * 64 * (NK + 8) + 2 * 64 * kWgPitch) * sizeof(__half);
@@ -459,23 +475,43 @@ static int launch_attn_mma_t(const AttnMmaArgs &A, cudaStream_t stream)
     if (cache.dev != dev) {
         int sms = 0, ctas = 0;
         if (cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev) != cudaSuccess) return set_cuda_error(cudaGetLastError(), CM_ECUDA);
-        cudaError_t e = cudaFuncSetAttribute(policy_attn_mma_kernel<NS, WARPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        cudaError_t e = cudaFuncSetAttribute(policy_attn_mma_kernel<NS, WARPS, kMulti>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return set_cuda_error(e, CM_ECUDA);
-        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas, policy_attn_mma_kernel<NS, WARPS>, WARPS * 32, smem) != cudaSuccess)
+        if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&ctas, policy_attn_mma_kernel<NS, WARPS, kMulti>, WARPS * 32, smem) != cudaSuccess)
             return set_cuda_error(cudaGetLastError(), CM_ECUDA);
         cache.dev = dev;
         cache.slots = sms * (ctas < 1 ? 1 : ctas);
     }
     const int grid = (int)(A.n_envs < cache.slots ? A.n_envs : cache.slots);
-    policy_attn_mma_kernel<NS, WARPS><<<grid, WARPS * 32, smem, stream>>>(A);
+    policy_attn_mma_kernel<NS, WARPS, kMulti><<<grid, WARPS * 32, smem, stream>>>(A);
     const cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? CM_OK : set_cuda_error(e, CM_ECUDA);
+}
+
+template <bool kMulti>
+static int launch_attn_mma_n(int n, const AttnMmaArgsOf<kMulti> &A, cudaStream_t stream)
+{
+    switch ((n + 15) / 16) {
+    case 5: return launch_attn_mma_t<5, kMulti>(A, stream);
+    case 6: return launch_attn_mma_t<6, kMulti>(A, stream);
+    case 7: return launch_attn_mma_t<7, kMulti>(A, stream);
+    case 8: return launch_attn_mma_t<8, kMulti>(A, stream);
+    case 9: return launch_attn_mma_t<9, kMulti>(A, stream);
+    case 10: return launch_attn_mma_t<10, kMulti>(A, stream);
+    case 11: return launch_attn_mma_t<11, kMulti>(A, stream);
+    case 12: return launch_attn_mma_t<12, kMulti>(A, stream);
+    case 13: return launch_attn_mma_t<13, kMulti>(A, stream);
+    case 14: return launch_attn_mma_t<14, kMulti>(A, stream);
+    case 15: return launch_attn_mma_t<15, kMulti>(A, stream);
+    case 16: return launch_attn_mma_t<16, kMulti>(A, stream);
+    }
+    return CM_EUNSUPPORTED;
 }
 
 int launch_policy_attn_mma(const cm_policy_desc *desc, const cm_policy_io *io, const float *scr_e, float *scr_q, float *scr_hw,
                            cudaStream_t stream)
 {
-    AttnMmaArgs A;
+    AttnMmaSetArgs A;
     A.d = *desc;
     A.weights = io->weights;
     A.adj_bits = io->adj_bits;
@@ -483,21 +519,10 @@ int launch_policy_attn_mma(const cm_policy_desc *desc, const cm_policy_io *io, c
     A.attention = io->attention;
     A.scr_e = scr_e; A.scr_q = scr_q; A.scr_hw = scr_hw;
     A.n_envs = io->n_envs;
-    switch ((desc->n_agents + 15) / 16) {
-    case 5: return launch_attn_mma_t<5>(A, stream);
-    case 6: return launch_attn_mma_t<6>(A, stream);
-    case 7: return launch_attn_mma_t<7>(A, stream);
-    case 8: return launch_attn_mma_t<8>(A, stream);
-    case 9: return launch_attn_mma_t<9>(A, stream);
-    case 10: return launch_attn_mma_t<10>(A, stream);
-    case 11: return launch_attn_mma_t<11>(A, stream);
-    case 12: return launch_attn_mma_t<12>(A, stream);
-    case 13: return launch_attn_mma_t<13>(A, stream);
-    case 14: return launch_attn_mma_t<14>(A, stream);
-    case 15: return launch_attn_mma_t<15>(A, stream);
-    case 16: return launch_attn_mma_t<16>(A, stream);
-    }
-    return CM_EUNSUPPORTED;
+    if (io->n_policies <= 1) return launch_attn_mma_n<false>(desc->n_agents, A, stream);
+    A.envs_per_policy = io->envs_per_policy;
+    A.weights_stride = io->weights_stride;
+    return launch_attn_mma_n<true>(desc->n_agents, A, stream);
 }
 
 }  // namespace cm

@@ -42,6 +42,9 @@ struct CentArgs {
     cm_policy_io io;
     int K, NO, relu;
     CentBlob o;
+    // several policies (MULTI): CTA t runs env tile t % tiles_per_policy of env block t / tiles_per_policy with that block's
+    // blob, so the tiles are counted per block and never mix two policies
+    int64_t tiles_per_policy, envs_per_policy, weights_stride;
 };
 
 // tanh(x) = 1 - 2 / (2^(2 log2(e) x) + 1) through ex2.approx / rcp.approx (|error| ~3e-7, saturates correctly): the formulation
@@ -116,7 +119,7 @@ __device__ __forceinline__ void cent_hidden(const float *__restrict__ in, int ld
     }
 }
 
-template <bool RELU, bool H1G>
+template <bool RELU, bool H1G, bool MULTI>
 __global__ void __launch_bounds__(kCThreads, 2) policy_cent_kernel(const CentArgs A)
 {
     extern __shared__ __align__(16) float smem[];
@@ -130,8 +133,14 @@ __global__ void __launch_bounds__(kCThreads, 2) policy_cent_kernel(const CentArg
     const CentBlob &o = A.o;
     const int tid = threadIdx.x, ty = tid >> 4, tx = tid & 15, lane = tid & 31, warp = tid >> 5;
     const int K = A.K, n = A.d.n_agents;
-    const int64_t row0 = (int64_t)blockIdx.x * kCRows;
-    const int rows = (int)min((int64_t)kCRows, io.n_envs - row0);
+    int64_t row0 = (int64_t)blockIdx.x * kCRows;
+    int rows = (int)min((int64_t)kCRows, io.n_envs - row0);
+    if constexpr (MULTI) {
+        const int64_t pol = (int64_t)blockIdx.x / A.tiles_per_policy, e0 = ((int64_t)blockIdx.x - pol * A.tiles_per_policy) * kCRows;
+        wts += pol * A.weights_stride;
+        row0 = pol * A.envs_per_policy + e0;
+        rows = (int)min((int64_t)kCRows, A.envs_per_policy - e0);
+    }
 
     // ---- layer 1: h1 = act(obs W1 + b1), K streamed — or the rows the tensor-core kernel left in the workspace ----
     if (H1G) {
@@ -257,6 +266,7 @@ struct CentL1Args {
     int *error_flag;
     int64_t n_envs;
     int K, n_panels;
+    int64_t tiles_per_policy, envs_per_policy, weights_stride, tc_weights_stride;   // as in CentArgs; tc stride in halves
 };
 
 // W1 [K][128] fp32 -> per K panel of kL1KP = 32 the stacked [W1_hi ; W1_lo] (256 rows x 32 k) in the canonical K-major core-matrix layout
@@ -293,7 +303,7 @@ __device__ __forceinline__ void mbar_arrive(uint64_t *bar)
 }
 
 // VEC: K is a multiple of 4 and the observation block is 16-byte aligned — 16-byte copies (a chunk is then either whole or absent)
-template <bool RELU, bool VEC>
+template <bool RELU, bool VEC, bool MULTI>
 __global__ void __launch_bounds__(kL1Threads, 1) policy_cent_l1_tc_kernel(const CentL1Args A)
 {
     using namespace tc;
@@ -307,8 +317,17 @@ __global__ void __launch_bounds__(kL1Threads, 1) policy_cent_l1_tc_kernel(const 
     uint32_t *tmem_s = reinterpret_cast<uint32_t *>(done_bar + 1);
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int K = A.K, NP = A.n_panels;
-    const int64_t row0 = (int64_t)blockIdx.x * kL1Rows;
-    const int rows = (int)min((int64_t)kL1Rows, A.n_envs - row0);
+    int64_t row0 = (int64_t)blockIdx.x * kL1Rows;
+    int rows = (int)min((int64_t)kL1Rows, A.n_envs - row0);
+    const __half *w1tc = A.w1tc;
+    const float *b1 = A.b1;
+    if constexpr (MULTI) {                                                           // this tile's policy: W1 panels and b1
+        const int64_t pol = (int64_t)blockIdx.x / A.tiles_per_policy, e0 = ((int64_t)blockIdx.x - pol * A.tiles_per_policy) * kL1Rows;
+        row0 = pol * A.envs_per_policy + e0;
+        rows = (int)min((int64_t)kL1Rows, A.envs_per_policy - e0);
+        w1tc += pol * A.tc_weights_stride;
+        b1 += pol * A.weights_stride;
+    }
     constexpr int kIssuer = kL1Teams * kL1Producers / 32, kLoader = kIssuer + 1;     // warps 16, 17
     const int team = warp >> 3, ptid = tid & (kL1Producers - 1);                     // producer team (panels team, team + 2, ...) and index inside it
 
@@ -334,7 +353,7 @@ __global__ void __launch_bounds__(kL1Threads, 1) policy_cent_l1_tc_kernel(const 
                 const int sq = q % kL1BStages, uq = q / kL1BStages;
                 if (uq > 0) ok = mbar_wait(&empty_b[sq], (uint32_t)(uq - 1) & 1u) && ok;
                 mbar_expect_tx(&full_b[sq], kL1BBytes);
-                bulk_g2s(bbase + (size_t)sq * kL1BBytes, A.w1tc + (size_t)q * kL1PanelHalves, kL1BBytes, &full_b[sq]);
+                bulk_g2s(bbase + (size_t)sq * kL1BBytes, w1tc + (size_t)q * kL1PanelHalves, kL1BBytes, &full_b[sq]);
             }
         }
         __syncwarp();
@@ -471,8 +490,8 @@ __global__ void __launch_bounds__(kL1Threads, 1) policy_cent_l1_tc_kernel(const 
             tmem_ld8(lane_addr + (uint32_t)col, v);
             tmem_ld8(lane_addr + (uint32_t)(kC1 + col), w);
             tmem_ld_wait();
-            const float4 b0 = __ldg(reinterpret_cast<const float4 *>(A.b1 + col)), b1 = __ldg(reinterpret_cast<const float4 *>(A.b1 + col + 4));
-            const float bb[8] = {b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, b1.z, b1.w};
+            const float4 bv0 = __ldg(reinterpret_cast<const float4 *>(b1 + col)), bv1 = __ldg(reinterpret_cast<const float4 *>(b1 + col + 4));
+            const float bb[8] = {bv0.x, bv0.y, bv0.z, bv0.w, bv1.x, bv1.y, bv1.z, bv1.w};
 #pragma unroll
             for (int i = 0; i < 8; ++i) v[i] = cent_act<RELU, true>(fmaf(w[i], 1.0f / 4096.0f, v[i]) + bb[i]);
             if (row < rows) {
@@ -513,8 +532,13 @@ int launch_policy_cent(const cm_policy_desc *desc, const cm_policy_io *io, cudaS
     A.NO = desc->n_agents * CM_ACTIONS;
     A.relu = desc->flags & CM_POLICY_FLAG_RELU;
     A.o = cent_blob_layout(desc->n_agents, desc->obs_dim);
+    const bool multi = io->n_policies > 1;
+    const int64_t epp = multi ? io->envs_per_policy : io->n_envs, n_pol = multi ? io->n_policies : 1;
+    A.envs_per_policy = epp;
+    A.tiles_per_policy = (epp + kCRows - 1) / kCRows;
+    A.weights_stride = multi ? io->weights_stride : 0;
     const size_t smem = kCentSmemFloats * sizeof(float);
-    static thread_local struct { int dev; bool set[8]; } cache = {-1, {false, false, false, false, false, false, false, false}};
+    static thread_local struct { int dev; bool set[16]; } cache = {-1, {}};
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess) return set_cuda_error(cudaGetLastError(), CM_ENODEVICE);
     if (cache.dev != dev) { cache.dev = dev; for (bool &b : cache.set) b = false; }
@@ -529,29 +553,30 @@ int launch_policy_cent(const cm_policy_desc *desc, const cm_policy_io *io, cudaS
         L.n_envs = io->n_envs;
         L.K = A.K;
         L.n_panels = (A.K + kL1KP - 1) / kL1KP;
-        const unsigned grid1 = (unsigned)((io->n_envs + kL1Rows - 1) / kL1Rows);
+        L.envs_per_policy = epp;
+        L.tiles_per_policy = (epp + kL1Rows - 1) / kL1Rows;
+        L.weights_stride = A.weights_stride;
+        L.tc_weights_stride = multi ? 2 * io->tc_weights_stride : 0;
+        const unsigned grid1 = (unsigned)(n_pol * L.tiles_per_policy);
         const bool vec = (A.K & 3) == 0 && (reinterpret_cast<uintptr_t>(io->obs) & 15) == 0;
-        void (*k1)(const CentL1Args) = A.relu ? (vec ? policy_cent_l1_tc_kernel<true, true> : policy_cent_l1_tc_kernel<true, false>)
-                                              : (vec ? policy_cent_l1_tc_kernel<false, true> : policy_cent_l1_tc_kernel<false, false>);
-        if ((rc = cent_set_smem(k1, kL1SmemBytes, cache.set[4 + 2 * (A.relu ? 1 : 0) + (vec ? 1 : 0)]))) return rc;
+        void (*k1)(const CentL1Args) =
+            multi ? (A.relu ? (vec ? policy_cent_l1_tc_kernel<true, true, true> : policy_cent_l1_tc_kernel<true, false, true>)
+                            : (vec ? policy_cent_l1_tc_kernel<false, true, true> : policy_cent_l1_tc_kernel<false, false, true>))
+                  : (A.relu ? (vec ? policy_cent_l1_tc_kernel<true, true, false> : policy_cent_l1_tc_kernel<true, false, false>)
+                            : (vec ? policy_cent_l1_tc_kernel<false, true, false> : policy_cent_l1_tc_kernel<false, false, false>));
+        if ((rc = cent_set_smem(k1, kL1SmemBytes, cache.set[8 * multi + 4 + 2 * (A.relu ? 1 : 0) + (vec ? 1 : 0)]))) return rc;
         k1<<<grid1, kL1Threads, kL1SmemBytes, stream>>>(L);
         const cudaError_t e1 = cudaGetLastError();
         if (e1 != cudaSuccess) return set_cuda_error(e1, CM_ECUDA);
     }
-    const unsigned grid = (unsigned)((io->n_envs + kCRows - 1) / kCRows);
-    if (A.relu && tcl1) {
-        if ((rc = cent_set_smem(policy_cent_kernel<true, true>, smem, cache.set[0]))) return rc;
-        policy_cent_kernel<true, true><<<grid, kCThreads, smem, stream>>>(A);
-    } else if (A.relu) {
-        if ((rc = cent_set_smem(policy_cent_kernel<true, false>, smem, cache.set[1]))) return rc;
-        policy_cent_kernel<true, false><<<grid, kCThreads, smem, stream>>>(A);
-    } else if (tcl1) {
-        if ((rc = cent_set_smem(policy_cent_kernel<false, true>, smem, cache.set[2]))) return rc;
-        policy_cent_kernel<false, true><<<grid, kCThreads, smem, stream>>>(A);
-    } else {
-        if ((rc = cent_set_smem(policy_cent_kernel<false, false>, smem, cache.set[3]))) return rc;
-        policy_cent_kernel<false, false><<<grid, kCThreads, smem, stream>>>(A);
-    }
+    const unsigned grid = (unsigned)(n_pol * A.tiles_per_policy);
+    void (*k2)(const CentArgs) =
+        multi ? (A.relu ? (tcl1 ? policy_cent_kernel<true, true, true> : policy_cent_kernel<true, false, true>)
+                        : (tcl1 ? policy_cent_kernel<false, true, true> : policy_cent_kernel<false, false, true>))
+              : (A.relu ? (tcl1 ? policy_cent_kernel<true, true, false> : policy_cent_kernel<true, false, false>)
+                        : (tcl1 ? policy_cent_kernel<false, true, false> : policy_cent_kernel<false, false, false>));
+    if ((rc = cent_set_smem(k2, smem, cache.set[8 * multi + 2 * (A.relu ? 0 : 1) + (tcl1 ? 0 : 1)]))) return rc;
+    k2<<<grid, kCThreads, smem, stream>>>(A);
     const cudaError_t e = cudaGetLastError();
     return e == cudaSuccess ? CM_OK : set_cuda_error(e, CM_ECUDA);
 }

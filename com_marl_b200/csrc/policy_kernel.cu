@@ -119,12 +119,14 @@ __device__ __forceinline__ void store_rowmajor(float *__restrict__ out, const fl
 // categorical head on X^T (k-major, 64 rows) + softmax / availability mask / sampling for `rows` valid rows.
 // Row r of the tile is agent `il` of env `env` (global row g):  n_div > 0: env = env_base + r / n_div,
 // il = r % n_div (tile of whole envs);  n_div == 0: env = env_base, il = il_base + r (chunk of one env).
-__device__ void head_and_sample(const PolicyArgs &A, const Blob &o, const float *XT, float *bufA, float *bufB,
+// (kMulti: the weights of the tile's policy are `wblk`; one policy: io.weights)
+template <bool kMulti>
+__device__ void head_and_sample(const PolicyArgs &A, const Blob &o, const float *wblk, const float *XT, float *bufA, float *bufB,
                                 float *logit_s, int rows, int64_t g0, int64_t env_base, int il_base, int n_div)
 {
     const cm_policy_desc &d = A.d;
     const cm_policy_io &io = A.io;
-    const float *__restrict__ wts = io.weights;
+    const float *__restrict__ wts = kMulti ? wblk : io.weights;
     const int tid = threadIdx.x;
     {
         float acc[4][8];
@@ -166,6 +168,9 @@ __device__ void head_and_sample(const PolicyArgs &A, const Blob &o, const float 
 }
 
 // ------------------------------------------------------------------------------------------------
+// kMulti: several policies in one launch — the tiles are counted per env block of io.envs_per_policy envs (a block may end
+// in a partial tile) and a tile reads the blob of its block's policy
+template <bool kMulti>
 __global__ void __launch_bounds__(kThreads, 2) policy_small_kernel(const PolicyArgs A)
 {
     extern __shared__ __align__(16) float sm[];
@@ -181,8 +186,15 @@ __global__ void __launch_bounds__(kThreads, 2) policy_small_kernel(const PolicyA
     const int tid = threadIdx.x;
 
     for (int64_t tile = blockIdx.x; tile < A.n_tiles; tile += gridDim.x) {
-        const int64_t env0 = tile * A.envs_per_tile;
-        const int envs = (int)min((int64_t)A.envs_per_tile, io.n_envs - env0);
+        int64_t env0 = tile * A.envs_per_tile;
+        int envs = (int)min((int64_t)A.envs_per_tile, io.n_envs - env0);
+        if constexpr (kMulti) {
+            const int64_t tpp = (io.envs_per_policy + A.envs_per_tile - 1) / A.envs_per_tile;    // tiles per block
+            const int64_t p = tile / tpp, e0 = (tile - p * tpp) * A.envs_per_tile;
+            wts = io.weights + p * io.weights_stride;
+            env0 = p * io.envs_per_policy + e0;
+            envs = (int)min((int64_t)A.envs_per_tile, io.envs_per_policy - e0);
+        }
         const int rows = envs * n;                 // valid rows of this tile
         const int64_t row0 = env0 * n;             // first global agent row
         __syncthreads();
@@ -307,7 +319,7 @@ __global__ void __launch_bounds__(kThreads, 2) policy_small_kernel(const PolicyA
             __syncthreads();
         }
         // ---- 8..12. categorical head, softmax, mask, sampling ----
-        head_and_sample(A, o, HT, bufA, bufB, logit_s, rows, row0, env0, 0, n);
+        head_and_sample<kMulti>(A, o, wts, HT, bufA, bufB, logit_s, rows, row0, env0, 0, n);
     }
 }
 
@@ -329,6 +341,7 @@ __device__ __forceinline__ void load_chunk_kmajor(float *dstT, const float *src,
     }
 }
 
+template <bool kMulti>
 __global__ void __launch_bounds__(kThreads, 2) policy_large_kernel(const PolicyArgs A, int np, size_t ws_floats)
 {
     extern __shared__ __align__(16) float sm[];
@@ -351,6 +364,7 @@ __global__ void __launch_bounds__(kThreads, 2) policy_large_kernel(const PolicyA
     float *QT = bufA, *AT = bufA + 64 * kPitch, *ST = bufB, *HT = bufB + 64 * kPitch;
 
     for (int64_t b = blockIdx.x; b < io.n_envs; b += gridDim.x) {
+        if constexpr (kMulti) wts = io.weights + (b / io.envs_per_policy) * io.weights_stride;
         __syncthreads();
         // ---------------- phase 1: encoder for every chunk; E^T and H_0 Wg_0 -> scratch ----------------
         for (int c = 0; c < nc; ++c) {
@@ -515,7 +529,7 @@ __global__ void __launch_bounds__(kThreads, 2) policy_large_kernel(const PolicyA
                         }
                         __syncthreads();
                     }
-                    head_and_sample(A, o, HT, bufA, bufB, logit_s, vq, b * n + q0, b, q0, 0);
+                    head_and_sample<kMulti>(A, o, wts, HT, bufA, bufB, logit_s, vq, b * n + q0, b, q0, 0);
                 }
                 __syncthreads();
             }
@@ -583,6 +597,18 @@ extern "C" int cm_policy_forward(const cm_policy_desc *desc, const cm_policy_io 
     if (io->n_envs < 0) return CM_EINVAL;
     if (io->n_envs == 0) return CM_OK;
     if (desc->kind != CM_POLICY_COMM && desc->kind != CM_POLICY_DEC && desc->kind != CM_POLICY_CENT) return CM_EINVAL;
+    if (io->n_policies < 0) return CM_EINVAL;
+    const bool multi = io->n_policies > 1;
+    if (multi) {                   // several policies: equal env blocks, strides that hold a blob and keep 16-byte alignment
+        const bool cent = desc->kind == CM_POLICY_CENT;
+        const size_t blob = cent ? cm_policy_cent_blob_floats(desc->n_agents, desc->obs_dim) : cm_policy_blob_floats(desc->obs_dim, desc->n_layers);
+        if (io->envs_per_policy < 1 || io->n_envs / io->n_policies != io->envs_per_policy || io->n_envs % io->n_policies != 0) return CM_EINVAL;
+        if (io->weights_stride < (int64_t)blob || (io->weights_stride & 3) != 0) return CM_EINVAL;
+        if (desc->math == 1 || desc->math == 2) {
+            const size_t tcb = cent ? cm_policy_cent_tc_blob_floats(desc->n_agents, desc->obs_dim) : cm_policy_tc_blob_floats(desc->obs_dim, desc->n_layers);
+            if (io->tc_weights_stride < (int64_t)tcb || (io->tc_weights_stride & 3) != 0) return CM_EINVAL;
+        }
+    }
     if (desc->kind == CM_POLICY_CENT) return launch_policy_cent(desc, io, (cudaStream_t)stream);
     if (desc->math == 1 || desc->math == 2) return launch_policy_tc(desc, io, (cudaStream_t)stream);
     if (desc->kind == CM_POLICY_DEC) return CM_EUNSUPPORTED;       // Obs-DP runs on the tensor-core kernel only
@@ -594,19 +620,22 @@ extern "C" int cm_policy_forward(const cm_policy_desc *desc, const cm_policy_io 
     if (desc->n_agents <= kTile) {
         A.envs_per_tile = kTile / desc->n_agents;
         A.n_tiles = (io->n_envs + A.envs_per_tile - 1) / A.envs_per_tile;
+        if (multi) A.n_tiles = io->n_policies * ((io->envs_per_policy + A.envs_per_tile - 1) / A.envs_per_tile);
         const size_t smem = small_smem_bytes();
-        static thread_local LaunchCache cache = {-1, 0, 0};
-        int rc = launch_geometry(policy_small_kernel, smem, cache);
+        static thread_local LaunchCache cache[2] = {{-1, 0, 0}, {-1, 0, 0}};
+        int rc = multi ? launch_geometry(policy_small_kernel<true>, smem, cache[1]) : launch_geometry(policy_small_kernel<false>, smem, cache[0]);
         if (rc) return rc;
-        const int64_t cap = (int64_t)cache.sms * cache.ctas_per_sm;   // persistent: a whole number of CTAs per SM
+        const int64_t cap = (int64_t)cache[multi].sms * cache[multi].ctas_per_sm;   // persistent: a whole number of CTAs per SM
         const int grid = (int)(A.n_tiles < cap ? A.n_tiles : cap);
-        policy_small_kernel<<<grid, kThreads, smem, (cudaStream_t)stream>>>(A);
+        if (multi) policy_small_kernel<true><<<grid, kThreads, smem, (cudaStream_t)stream>>>(A);
+        else policy_small_kernel<false><<<grid, kThreads, smem, (cudaStream_t)stream>>>(A);
     } else {
         A.envs_per_tile = 0;
         A.n_tiles = io->n_envs;
         const size_t smem = large_smem_bytes();
-        static thread_local LaunchCache cache = {-1, 0, 0};
-        int rc = launch_geometry(policy_large_kernel, smem, cache);
+        static thread_local LaunchCache caches[2] = {{-1, 0, 0}, {-1, 0, 0}};
+        LaunchCache &cache = caches[multi];
+        int rc = multi ? launch_geometry(policy_large_kernel<true>, smem, cache) : launch_geometry(policy_large_kernel<false>, smem, cache);
         if (rc) return rc;
         const size_t ws = large_ws_floats(desc->n_agents);
         if (!io->workspace || io->workspace_bytes < ws * sizeof(float)) return CM_EINVAL;
@@ -614,7 +643,8 @@ extern "C" int cm_policy_forward(const cm_policy_desc *desc, const cm_policy_io 
         const int64_t fit = (int64_t)(io->workspace_bytes / (ws * sizeof(float)));
         if (fit < cap) cap = fit;
         const int grid = (int)(io->n_envs < cap ? io->n_envs : cap);
-        policy_large_kernel<<<grid, kThreads, smem, (cudaStream_t)stream>>>(A, round_up_tile(desc->n_agents), ws);
+        if (multi) policy_large_kernel<true><<<grid, kThreads, smem, (cudaStream_t)stream>>>(A, round_up_tile(desc->n_agents), ws);
+        else policy_large_kernel<false><<<grid, kThreads, smem, (cudaStream_t)stream>>>(A, round_up_tile(desc->n_agents), ws);
     }
     e = cudaGetLastError();
     if (e != cudaSuccess) return set_cuda_error(e, CM_ECUDA);

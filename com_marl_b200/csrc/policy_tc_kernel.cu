@@ -67,6 +67,7 @@ struct TcArgs {
     int mode;                    // kTcModeComm / Dec / Enc / Head
     int in_dim;                  // width of the input rows (obs_dim; 64 in head mode: the rows are X = E + H_L)
     float *scr_e, *scr_q, *scr_hw;   // encoder mode: row-major [rows][64] outputs E, Q = E Wq, H_0 Wg_0 (large-team pipeline)
+    int tiles_per_policy;        // several policies in one launch: tiles of each env block
 };
 
 // fp16 split of one value: hi = fp16(x), lo = fp16((x - hi) * 4096)
@@ -479,7 +480,12 @@ struct MmaOp { uint32_t dcol, acc, abuf; int lo_from; };   // accumulator block,
 // of 17 .. 64 agents, env slots of 32 / 64 rows) and the kernel carries none of the CUDA-core attention loops.
 // kMode: kTcModeComm / Dec / Enc / Head as a template parameter, so that the Comm-DP kernel carries none of the other modes'
 // code (the kernel is instruction-fetch sensitive: its SASS is several times the instruction cache).
-template <int kVec, int kMode>
+// kMulti: several policies in one launch (io.n_policies > 1).  Tiles are counted per env block (A.tiles_per_policy each, the
+// last one of a block may be partial), so a tile belongs to ONE policy: policy(t) = t / tiles_per_policy.  The weight stream
+// prefetches across tile boundaries, so every block it requests is taken from the policy of the tile that will consume it;
+// the bias table is reloaded when the CTA's next tile belongs to another policy, after the CTA barrier that ends the
+// previous tile's last read of it.  A separate instantiation, so that the one-policy kernels keep their code.
+template <int kVec, int kMode, bool kMulti = false>
 __global__ void __launch_bounds__(kTcThreads, 2) policy_tc_kernel(const TcArgs A)
 {
     extern __shared__ __align__(1024) unsigned char smem[];
@@ -542,7 +548,13 @@ __global__ void __launch_bounds__(kTcThreads, 2) policy_tc_kernel(const TcArgs A
                     if (CM_TC_DEBUG & 8) { asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(&bars[slot])) : "memory"); }
                     else {
                         mbar_expect_tx(&bars[slot], bytes);
-                        bulk_g2s(WB + slot * (uint32_t)kSlotBytes, tcw + st.w_off, bytes, &bars[slot]);
+                        if constexpr (kMulti) {      // the policy of the tile this block belongs to: the CTA's (issued / seq_len)-th tile
+                            const int tl = (int)blockIdx.x + (int)(issued / (uint32_t)P.seq_len) * (int)gridDim.x;
+                            const __half *pw = tcw + (size_t)(tl / A.tiles_per_policy) * (size_t)io.tc_weights_stride * 2u;
+                            bulk_g2s(WB + slot * (uint32_t)kSlotBytes, pw + st.w_off, bytes, &bars[slot]);
+                        } else {
+                            bulk_g2s(WB + slot * (uint32_t)kSlotBytes, tcw + st.w_off, bytes, &bars[slot]);
+                        }
                     }
                 }
                 __syncwarp();
@@ -695,8 +707,14 @@ __global__ void __launch_bounds__(kTcThreads, 2) policy_tc_kernel(const TcArgs A
     const bool dec = mode != kTcModeComm;            // every mode but Comm-DP treats the agent rows independently
     const int total_rows = n_envs * n;
     auto tile_rows = [&](int tl, int &r0, int &nr) {
-        if (dec) { r0 = tl * kTcRows; nr = min(kTcRows, total_rows - r0); }
-        else { const int e0 = tl * A.envs_per_tile; r0 = e0 * n; nr = min(A.envs_per_tile, n_envs - e0) * n; }
+        if constexpr (kMulti) {
+            const int p = tl / A.tiles_per_policy, lt = tl - p * A.tiles_per_policy, epp = (int)io.envs_per_policy;
+            if (dec) { const int pr = epp * n; r0 = p * pr + lt * kTcRows; nr = min(kTcRows, pr - lt * kTcRows); }
+            else { const int e0 = lt * A.envs_per_tile; r0 = (p * epp + e0) * n; nr = min(A.envs_per_tile, epp - e0) * n; }
+        } else {
+            if (dec) { r0 = tl * kTcRows; nr = min(kTcRows, total_rows - r0); }
+            else { const int e0 = tl * A.envs_per_tile; r0 = e0 * n; nr = min(A.envs_per_tile, n_envs - e0) * n; }
+        }
     };
     // packed observations (io.obs_bits): a row is 6 words — 3 of window bits, 3 scalar columns as float bits — staged like 6 floats
     const bool packed = io.obs_bits != nullptr && kMode != kTcModeHead;
@@ -727,17 +745,26 @@ __global__ void __launch_bounds__(kTcThreads, 2) policy_tc_kernel(const TcArgs A
     if ((int)blockIdx.x < n_tiles) stage_obs((int)blockIdx.x);
     // bias table (and the last layer's weights) — after the first weight stages and the observations have been requested,
     // so that the three global round trips of the prologue overlap
-    for (int i = tid; i < kBiasFloats; i += kTcThreads) {
-        float v = 0.0f;
-        if (i < kBEnc2) v = wts[o.enc_b1 + i];
-        else if (i < kBGcn) v = wts[o.enc_b2 + i - kBEnc2];
-        else if (i < kBH1) { if (i - kBGcn < L * 64) v = wts[o.gcn_b + i - kBGcn]; }
-        else if (i < kBH2) v = wts[o.head_b1 + i - kBH1];
-        else if (i < kBH3) v = wts[o.head_b2 + i - kBH2];
-        else if (i < kBH4) v = wts[o.head_b3 + i - kBH3];
-        else if (i < kBH4 + CM_ACTIONS) v = wts[o.head_b4 + i - kBH4];
-        else if (i >= kW4) v = wts[o.head_w4 + i - kW4];
-        bias_s[i] = i < kBH4 ? v * kTanhScale : v;        // every bias below kBH4 feeds a tanh (see tanh_scaled)
+    auto load_bias = [&](const float *__restrict__ w) {
+        for (int i = tid; i < kBiasFloats; i += kTcThreads) {
+            float v = 0.0f;
+            if (i < kBEnc2) v = w[o.enc_b1 + i];
+            else if (i < kBGcn) v = w[o.enc_b2 + i - kBEnc2];
+            else if (i < kBH1) { if (i - kBGcn < L * 64) v = w[o.gcn_b + i - kBGcn]; }
+            else if (i < kBH2) v = w[o.head_b1 + i - kBH1];
+            else if (i < kBH3) v = w[o.head_b2 + i - kBH2];
+            else if (i < kBH4) v = w[o.head_b3 + i - kBH3];
+            else if (i < kBH4 + CM_ACTIONS) v = w[o.head_b4 + i - kBH4];
+            else if (i >= kW4) v = w[o.head_w4 + i - kW4];
+            bias_s[i] = i < kBH4 ? v * kTanhScale : v;        // every bias below kBH4 feeds a tanh (see tanh_scaled)
+        }
+    };
+    int bias_policy = 0;                                 // policy whose biases bias_s holds
+    if constexpr (kMulti) {
+        bias_policy = (int)blockIdx.x / A.tiles_per_policy;
+        load_bias(wts + (size_t)bias_policy * (size_t)io.weights_stride);
+    } else {
+        load_bias(wts);
     }
     __syncthreads();
 
@@ -763,6 +790,12 @@ __global__ void __launch_bounds__(kTcThreads, 2) policy_tc_kernel(const TcArgs A
         CM_TP(18);
         asm volatile("cp.async.wait_group 0;" ::: "memory");
         __syncthreads();                                   // the staged observations of this tile are visible
+        if constexpr (kMulti) {
+            // every thread is past the previous tile's last read of the bias table; the first product phase below (a CTA
+            // barrier) orders these writes before the first epilogue that reads them
+            const int p = tile / A.tiles_per_policy;
+            if (p != bias_policy) { bias_policy = p; load_bias(wts + (size_t)p * (size_t)io.weights_stride); }
+        }
         CM_TP(19);
         {
             const float *src = obs_src + (size_t)row0 * Dst;
@@ -1307,16 +1340,30 @@ static int launch_tc_mode(const cm_policy_desc *desc, const cm_policy_io *io, in
     A.slot = rows_mode ? 0 : (attn_tc ? (desc->n_agents <= 32 ? 32 : 64) : desc->n_agents);
     A.envs_per_tile = rows_mode ? 0 : kTcRows / A.slot;
     A.n_tiles = rows_mode ? (io->n_envs * desc->n_agents + kTcRows - 1) / kTcRows : (io->n_envs + A.envs_per_tile - 1) / A.envs_per_tile;
+    const bool multi = io->n_policies > 1;
+    A.tiles_per_policy = (int)A.n_tiles;
+    if (multi) {            // tiles counted per env block: no tile holds rows of two policies
+        A.tiles_per_policy = (int)(rows_mode ? (io->envs_per_policy * desc->n_agents + kTcRows - 1) / kTcRows
+                                             : (io->envs_per_policy + A.envs_per_tile - 1) / A.envs_per_tile);
+        A.n_tiles = (int64_t)io->n_policies * A.tiles_per_policy;
+    }
     const size_t smem = tc_smem_bytes();
     const int vec = rows_mode ? 1 : (attn_tc ? 0 : ((desc->n_agents & 3) == 0 ? 4 : ((desc->n_agents & 1) == 0 ? 2 : 1)));
     void (*kernel)(const TcArgs) =
-        mode == kTcModeDec ? policy_tc_kernel<1, kTcModeDec>
-        : mode == kTcModeEnc ? policy_tc_kernel<1, kTcModeEnc>
-        : mode == kTcModeHead ? policy_tc_kernel<1, kTcModeHead>
-        : vec == 0 ? policy_tc_kernel<0, kTcModeComm>
-        : vec == 4 ? policy_tc_kernel<4, kTcModeComm> : (vec == 2 ? policy_tc_kernel<2, kTcModeComm> : policy_tc_kernel<1, kTcModeComm>);
-    static thread_local struct { int dev; int sms; } cache[7] = {{-1, 0}, {-1, 0}, {-1, 0}, {-1, 0}, {-1, 0}, {-1, 0}, {-1, 0}};
-    auto &cc = cache[mode == kTcModeComm ? (vec == 0 ? 6 : (vec >> 1)) : 2 + mode];
+        !multi ? (mode == kTcModeDec ? policy_tc_kernel<1, kTcModeDec>
+                  : mode == kTcModeEnc ? policy_tc_kernel<1, kTcModeEnc>
+                  : mode == kTcModeHead ? policy_tc_kernel<1, kTcModeHead>
+                  : vec == 0 ? policy_tc_kernel<0, kTcModeComm>
+                  : vec == 4 ? policy_tc_kernel<4, kTcModeComm> : (vec == 2 ? policy_tc_kernel<2, kTcModeComm> : policy_tc_kernel<1, kTcModeComm>))
+               : (mode == kTcModeDec ? policy_tc_kernel<1, kTcModeDec, true>
+                  : mode == kTcModeEnc ? policy_tc_kernel<1, kTcModeEnc, true>
+                  : mode == kTcModeHead ? policy_tc_kernel<1, kTcModeHead, true>
+                  : vec == 0 ? policy_tc_kernel<0, kTcModeComm, true>
+                  : vec == 4 ? policy_tc_kernel<4, kTcModeComm, true>
+                  : (vec == 2 ? policy_tc_kernel<2, kTcModeComm, true> : policy_tc_kernel<1, kTcModeComm, true>));
+    static thread_local struct { int dev; int sms; } cache[2][7] = {{{-1, 0}, {-1, 0}, {-1, 0}, {-1, 0}, {-1, 0}, {-1, 0}, {-1, 0}},
+                                                                    {{-1, 0}, {-1, 0}, {-1, 0}, {-1, 0}, {-1, 0}, {-1, 0}, {-1, 0}}};
+    auto &cc = cache[multi][mode == kTcModeComm ? (vec == 0 ? 6 : (vec >> 1)) : 2 + mode];
     int dev = 0;
     if (cudaGetDevice(&dev) != cudaSuccess) return set_cuda_error(cudaGetLastError(), CM_ENODEVICE);
     if (cc.dev != dev) {

@@ -32,8 +32,11 @@ def unpack_positions(packed) -> np.ndarray:
     return np.stack([packed & 0xFF, packed >> 8], axis=-1).astype(np.int8)
 
 
-def check_conditions(spec: ScenarioSpec, conditions, n_envs: int):
+def check_conditions(spec: ScenarioSpec, conditions, n_envs: int, policy_blocks: int = 1):
     """-> the validated list of channel conditions of a BatchedEnv (None when there are none); raises ValueError"""
+    if int(policy_blocks) < 1 or int(n_envs) % int(policy_blocks):
+        raise ValueError(f"n_envs = {n_envs} does not split into {policy_blocks} equal policy blocks")
+    n_envs = int(n_envs) // int(policy_blocks)
     if conditions is None:
         return None
     conditions = list(conditions)
@@ -52,16 +55,19 @@ class BatchedEnv:
     """B environment instances of one scenario on one GPU."""
 
     def __init__(self, spec: ScenarioSpec, n_envs: int, device="cuda", env_id0: int = 0, auto_reset: bool = True,
-                 conditions=None):
+                 conditions=None, policy_blocks: int = 1):
         """``conditions``: optional list of specs that differ from ``spec`` in the channel fields only
         (ScenarioSpec.CHANNEL_FIELDS, e.g. ``spec.with_channel(pl=..., rcom=...)``).  The envs are then split into equal
         contiguous blocks in list order and block k communicates under ``conditions[k]`` (``spec``'s own channel is not
-        used); ``cond_idx`` [B] holds each env's condition.  Everything else — and the global env ids — stays as without."""
+        used); ``cond_idx`` [B] holds each env's condition.  Everything else — and the global env ids — stays as without.
+        ``policy_blocks``: the envs are that many equal blocks (one per policy of a PolicySet), each split into the conditions
+        in the same way (env order policy, condition, episode)."""
         N.lib()  # fail loudly if the CUDA library is missing; there is no CPU path
         if not torch.cuda.is_available():
             raise RuntimeError("com_marl_b200 needs a CUDA device: the rollout engine has no CPU fallback")
         spec.validate()
-        self.conditions = check_conditions(spec, conditions, n_envs)
+        self.conditions = check_conditions(spec, conditions, n_envs, policy_blocks)
+        self.policy_blocks = int(policy_blocks)
         self.spec, self.B, self.auto_reset = spec, int(n_envs), bool(auto_reset)
         self.device = torch.device(device)
         self.env_id0 = int(env_id0)
@@ -99,7 +105,8 @@ class BatchedEnv:
             K = len(self.conditions)
             self._conds_host = (N.ChannelCond * K)(*[c.channel_cond() for c in self.conditions])
             self._conds = torch.frombuffer(bytearray(bytes(self._conds_host)), dtype=torch.uint8).to(dev)
-            self.cond_idx = torch.arange(K, dtype=torch.uint8, device=dev).repeat_interleave(B // K)
+            P = self.policy_blocks
+            self.cond_idx = torch.arange(K, dtype=torch.uint8, device=dev).repeat_interleave(B // (K * P)).repeat(P)
         self.desc = self._desc()
         self.state = N.EnvState()
         self.state.n_envs = B

@@ -15,6 +15,7 @@ from typing import Dict, List, Tuple
 import numpy as np
 import torch
 
+from .policy import PolicySet
 from .rollout import RolloutEngine
 
 VECTORS = ["reward", "capture_cnt", "step_cnt", "move_cnt", "penalty_cnt", "nodeDeg", "variable", "vars2"]
@@ -59,6 +60,21 @@ def eval_sweep(env, policy, conditions, n_eval_episodes=100, max_env_steps=200, 
     return _evaluate(spec, conds, policy, int(n_eval_episodes), max_env_steps, eval_greedy, groups, chunk, return_trajectory, 0)
 
 
+def eval_policies(env, policies, conditions=None, n_eval_episodes=100, max_env_steps=200, eval_greedy=True, seed=1,
+                  groups: int = 4, chunk: int = 50, return_trajectory: bool = False):
+    """``eval_model`` / ``eval_sweep`` of many policies of one class and architecture (every checkpoint of a run, the seeds
+    of a configuration) in ONE engine, one policy launch per step for all of them.  ``policies``: a list or a PolicySet.
+    With C conditions (C = 1 and ``env``'s own channel when ``conditions`` is None) policy i under condition k plays its
+    ``n_eval_episodes`` episodes in the envs with global ids ``(i C + k) n_eval_episodes ...``, so ``results[i][k]`` equals
+    ``eval_model(conditions[k], policies[i], ..., env_id0=(i C + k) n_eval_episodes)``."""
+    pset = policies if isinstance(policies, PolicySet) else PolicySet(policies)
+    spec = _eval_spec(getattr(env, "spec_b200", env), seed)
+    conds = [_eval_spec(c, seed) for c in conditions] if conditions is not None else None
+    res = _evaluate(spec, conds, pset, int(n_eval_episodes), max_env_steps, eval_greedy, groups, chunk, return_trajectory, 0)
+    C = len(conds) if conds else 1
+    return [res[i * C:(i + 1) * C] for i in range(len(pset))]
+
+
 def _eval_spec(spec, seed):
     spec = copy.copy(spec)
     spec.seed = int(seed)
@@ -67,9 +83,9 @@ def _eval_spec(spec, seed):
 
 
 def _evaluate(spec, conditions, policy, E, max_env_steps, eval_greedy, groups, chunk, return_trajectory, env_id0):
-    """the eval loop of eval_model / eval_sweep: E episodes per condition (one condition: ``spec``'s own channel) in one
-    RolloutEngine; -> one eval_model result per condition"""
-    conds = conditions or [spec]
+    """the eval loop of eval_model / eval_sweep / eval_policies: E episodes per (policy, condition) (one condition: ``spec``'s own
+    channel) in one RolloutEngine; -> one eval_model result per (policy, condition), policy-major"""
+    conds = (conditions or [spec]) * (len(policy) if isinstance(policy, PolicySet) else 1)
     B = E * len(conds)
     K = max(1, min(int(chunk), int(max_env_steps)))
     eng = RolloutEngine(spec, policy, B, device=policy.device, env_id0=env_id0, ring=K, greedy=bool(eval_greedy),

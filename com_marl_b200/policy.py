@@ -731,3 +731,145 @@ class CentralizedCategoricalMLPPolicy(nn.Module):
     @property
     def recurrent(self):
         return False
+
+
+class PolicySet:
+    """P policies of ONE class and architecture run by one ``cm_policy_forward`` launch per call — for evaluation (every
+    checkpoint of a run, the seeds of a configuration).  The envs of a call are P equal contiguous blocks, block i runs
+    ``policies[i]`` (one policy may fill several blocks).  The set owns one stacked fp32 buffer (and one stacked tensor-core
+    buffer) with a row per block; ``refresh_weights`` (same signature and ``force`` semantics as the policies') copies a
+    member's blobs into its rows when the member's parameters changed — in place, so a captured rollout graph over the set sees
+    the update, and no other row changes.  The members' own blobs stay where they are: graphs captured on a member keep
+    following it.  Equal architecture means the same class, team size, observation width, layers, residual, attention type,
+    layer widths, kernel math and nonlinearity; anything else raises ValueError."""
+
+    def __init__(self, policies):
+        self.policies = list(policies)
+        if not self.policies:
+            raise ValueError("a PolicySet needs at least one policy")
+        keys = [self._arch(p) for p in self.policies]
+        for i, k in enumerate(keys[1:], 1):
+            if k != keys[0]:
+                raise ValueError(f"policies[{i}] differs in architecture from policies[0]: one launch runs one kernel")
+        p0 = self.policies[0]
+        self.device, self._kind, self.seed = p0.device, p0._kind, p0.seed
+        P = len(self.policies)
+        self._n_blob = p0.weight_blob().numel()
+        self._stride = (self._n_blob + 3) // 4 * 4                # the bulk copies need 16-byte aligned rows
+        self._blobs = torch.zeros((P, self._stride), dtype=torch.float32, device=self.device)
+        self._tc_blobs, self._tc_stride, self._n_tc = None, 0, 0
+        if p0.uses_tensor_cores():
+            self._n_tc = p0.tc_weight_blob().numel()
+            self._tc_stride = (self._n_tc + 3) // 4 * 4
+            self._tc_blobs = torch.zeros((P, self._tc_stride), dtype=torch.float32, device=self.device)
+        self._row_sig = [None] * P                 # member blob signature each row was copied at (None: copy pending)
+        self.refresh_weights()
+
+    @staticmethod
+    def _arch(p):
+        shapes = tuple((k, tuple(v.shape)) for k, v in p.state_dict().items())
+        math = ("tc_fp32attn" if p.math == "tc_fp32attn" else "tc") if p.uses_tensor_cores() else "fp32"   # 'auto' = its kernel
+        return (type(p), p._n_agents, p._dec_obs_dim, getattr(p, "n_gcn_layers", 0), getattr(p, "residual", False), math,
+                getattr(p, "_relu", False), shapes)
+
+    def __len__(self):
+        return len(self.policies)
+
+    def uses_tensor_cores(self):
+        return self.policies[0].uses_tensor_cores()
+
+    def _sync_row(self, i):
+        """bring row i up to date with member i (its blobs refreshed first); one device copy per blob when it changed"""
+        p = self.policies[i]
+        if self._tc_blobs is not None:
+            p.tc_weight_blob()                     # (refreshes the fp32 blob as well)
+        else:
+            p.weight_blob()
+        if self._row_sig[i] != p._blob_sig:
+            self._blobs[i, :self._n_blob].copy_(p._blob)
+            if self._tc_blobs is not None:
+                self._tc_blobs[i, :self._n_tc].copy_(p._tc_blob)
+            self._row_sig[i] = p._blob_sig
+
+    def refresh_weights(self, force=False):
+        """the rows of every member whose parameters changed since the last refresh (``force``: every row, and every member's
+        own blobs rebuilt — after a write through ``p.data``, see CommCategoricalMLPPolicy.refresh_weights)"""
+        if force:
+            for p in self.policies:
+                p.refresh_weights(force=True)
+            self._row_sig = [None] * len(self.policies)
+        for i in range(len(self.policies)):
+            self._sync_row(i)
+
+    def check_errors(self):
+        for p in self.policies:
+            p.check_errors()
+
+    @staticmethod
+    def segments(B, envs_per_policy, first_env=0):
+        """[(s0, s1, first block, whole blocks)] of a call over envs first_env .. first_env + B of a policy-major batch: runs of
+        >= 2 whole blocks are one multi-policy launch (whole blocks > 0), a block the range cuts or a single block is one
+        single-policy launch of its member (whole blocks = 0)"""
+        Ep, out, s0 = int(envs_per_policy), [], 0
+        while s0 < B:
+            i, off = divmod(first_env + s0, Ep)
+            if off == 0 and B - s0 >= 2 * Ep:
+                s1 = s0 + (B - s0) // Ep * Ep
+                out.append((s0, s1, i, (s1 - s0) // Ep))
+            else:
+                s1 = min(B, s0 + Ep - off)
+                out.append((s0, s1, i, 0))
+            s0 = s1
+        return out
+
+    def act_device(self, obs, adj_bits=None, chan_bits=None, avail_bits=None, sample_u=None, tick=None, episode=None,
+                   greedy=False, probs=None, logits=None, attention=None, actions=None, env_id0=0, ws_slot=0, obs_bits=None,
+                   obs_nbits=0, envs_per_policy=None, first_env=0):
+        """``act_device`` of the members over policy-major envs.  By default the B envs of the call are P blocks of B / P;
+        a call over a slice of a larger batch (a rollout group) gives ``envs_per_policy`` of the batch and ``first_env``,
+        the slice's first env in it.  Runs of whole blocks are one multi-policy launch; a block the slice cuts runs as a
+        single-policy launch of its member (PolicySet.segments).  Returns the number of cm_policy_forward calls made."""
+        P, B = len(self.policies), obs.shape[0]
+        Ep = B // P if envs_per_policy is None else int(envs_per_policy)
+        if envs_per_policy is None and B != P * Ep:
+            raise ValueError(f"{B} envs do not split into {P} equal policy blocks")
+        args = dict(obs=obs, adj_bits=adj_bits, chan_bits=chan_bits, avail_bits=avail_bits, sample_u=sample_u, tick=tick,
+                    episode=episode, probs=probs, logits=logits, attention=attention, actions=actions, obs_bits=obs_bits)
+        segs = self.segments(B, Ep, first_env)
+        for s0, s1, i, whole in segs:
+            seg = {k: (v[s0:s1] if v is not None else None) for k, v in args.items()}
+            if whole:
+                self._launch(seg, greedy, env_id0 + s0, ws_slot, obs_nbits, whole, Ep, i)
+            else:
+                self._member_call(self.policies[i], seg, greedy, env_id0 + s0, ws_slot, obs_nbits)
+        return len(segs)
+
+    def _member_call(self, p, seg, greedy, env_id0, ws_slot, obs_nbits):
+        kw = dict(avail_bits=seg["avail_bits"], sample_u=seg["sample_u"], tick=seg["tick"], episode=seg["episode"], greedy=greedy,
+                  probs=seg["probs"], logits=seg["logits"], actions=seg["actions"], env_id0=env_id0)
+        if self._kind == N.POLICY_COMM:
+            p.act_device(seg["obs"], adj_bits=seg["adj_bits"], chan_bits=seg["chan_bits"], attention=seg["attention"],
+                         ws_slot=ws_slot, obs_bits=seg["obs_bits"], obs_nbits=obs_nbits, **kw)
+        elif self._kind == N.POLICY_DEC:
+            p.act_device(seg["obs"], obs_bits=seg["obs_bits"], obs_nbits=obs_nbits, **kw)
+        else:
+            p.act_device(seg["obs"], **kw)
+
+    def _launch(self, seg, greedy, env_id0, ws_slot, obs_nbits, n_blocks, Ep, first_policy):
+        """one cm_policy_forward over n_blocks whole blocks of Ep envs, policies first_policy ..."""
+        p0 = self.policies[first_policy]
+        comm = self._kind == N.POLICY_COMM
+        desc, io = p0._call_structs(seg["obs"], seg["adj_bits"] if comm else None, seg["chan_bits"] if comm else None,
+                                    seg["avail_bits"], seg["sample_u"], seg["tick"], seg["episode"], greedy, seg["probs"],
+                                    seg["logits"], seg["attention"] if comm else None, seg["actions"], env_id0, ws_slot)
+        for i in range(first_policy, first_policy + n_blocks):
+            self._sync_row(i)
+        io.weights = N.ptr(self._blobs[first_policy])
+        if self._tc_blobs is not None:
+            io.tc_weights = N.ptr(self._tc_blobs[first_policy])
+        io.n_policies, io.envs_per_policy = n_blocks, Ep
+        io.weights_stride, io.tc_weights_stride = self._stride, self._tc_stride
+        if seg["obs_bits"] is not None and self._kind != N.POLICY_CENT and self.uses_tensor_cores():
+            io.obs_bits, io.obs_nbits = N.ptr(seg["obs_bits"]), int(obs_nbits)
+        with torch.cuda.device(self.device):
+            N.check("cm_policy_forward", N.lib().cm_policy_forward(C.byref(desc), C.byref(io), N.stream_ptr()))

@@ -14,7 +14,7 @@ import numpy as np
 import torch
 
 from .envs import BatchedEnv
-from .policy import CommCategoricalMLPPolicy
+from .policy import CommCategoricalMLPPolicy, PolicySet
 from .scenario import ScenarioSpec
 from .spaces import Box, Discrete, EnvSpec
 
@@ -41,10 +41,17 @@ class RolloutEngine:
     def __init__(self, spec: ScenarioSpec, policy: CommCategoricalMLPPolicy, n_envs: int, device="cuda", env_id0: int = 0,
                  ring: int = 8, record_attention: bool = False, greedy: bool = False, use_graph: bool = True,
                  groups: int = 1, auto_reset: bool = True, conditions=None):
-        """``conditions``: per-env channel conditions of the envs (BatchedEnv); the env groups may cut through them."""
+        """``conditions``: per-env channel conditions of the envs (BatchedEnv); the env groups may cut through them.
+        ``policy``: one policy, or a PolicySet of P policies: the envs are then P equal blocks in policy-major order (block i runs
+        policy i and, with ``conditions``, is itself split into the conditions); the env groups may cut through the blocks."""
         self.spec, self.policy, self.B = spec, policy, int(n_envs)
         self.device = torch.device(device)
-        self.env = BatchedEnv(spec, n_envs, device=device, env_id0=env_id0, auto_reset=auto_reset, conditions=conditions)
+        self._set = isinstance(policy, PolicySet)
+        P = len(policy) if self._set else 1
+        if self.B % P:
+            raise ValueError(f"n_envs = {n_envs} does not split into {P} equal policy blocks")
+        self.env = BatchedEnv(spec, n_envs, device=device, env_id0=env_id0, auto_reset=auto_reset, conditions=conditions,
+                              policy_blocks=P)
         # Env groups: the envs are independent, so G contiguous groups form G independent policy -> step -> policy ...
         # chains.  Each chain runs on its own stream (forked / joined inside the captured graph): there is no device-wide
         # barrier between a step of one group and the next step of another, so partially filled waves of one launch
@@ -82,6 +89,8 @@ class RolloutEngine:
         self._warm = False
         self.steps_done = 0
         self.kernel_launches = 0
+        # policy calls per iteration of each group: one, or the PolicySet segments of the group's envs
+        self._pol_calls = [len(PolicySet.segments(b1 - b0, self.B // P, b0)) if self._set else 1 for b0, b1 in self._ranges]
 
     # ---- single iteration --------------------------------------------------------------------------
     def _iteration(self, k: int, g: int = None):
@@ -93,6 +102,8 @@ class RolloutEngine:
         t, e = self.traj, self._envs[g]
         b0, b1 = self._ranges[g]
         pk = dict(obs_bits=t["obs_bits"][k, b0:b1], obs_nbits=e.obs_nbits) if self._packed else {}
+        if self._set:
+            pk.update(envs_per_policy=self.B // len(self.policy), first_env=b0)
         self.policy.act_device(t["obs"][k, b0:b1], adj_bits=t["adj_bits"][k, b0:b1], chan_bits=t["chan_bits"][k, b0:b1], tick=e.tick, episode=e.episode,
                                greedy=self.greedy, probs=t["probs"][k, b0:b1], actions=t["actions"][k, b0:b1],
                                attention=t["attention"][k, b0:b1] if "attention" in t else None, env_id0=e.env_id0, ws_slot=g, **pk)
@@ -103,7 +114,7 @@ class RolloutEngine:
         if self._packed:
             out["obs_bits"] = t["obs_bits"][k + 1, b0:b1]
         e.step(t["actions"][k, b0:b1], out=out)
-        self.kernel_launches += 2
+        self.kernel_launches += 1 + self._pol_calls[g]
 
     def _carry(self):
         """slot K (state after the last step of a chunk) becomes slot 0 of the next chunk"""
@@ -160,7 +171,7 @@ class RolloutEngine:
             if self._graph is None:
                 self._capture()
             self._graph.replay()
-            self.kernel_launches += 2 * self.K * len(self._ranges)
+            self.kernel_launches += self.K * (len(self._ranges) + sum(self._pol_calls))
         else:
             self._chunk_eager()
             self._warm = True

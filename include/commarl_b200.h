@@ -46,8 +46,9 @@
 extern "C" {
 #endif
 
-#define CM_ABI_VERSION 5   /* 2: host_arena / obs_bits members, cm_rollout_step_host; 3: cm_ppo_net; 4: CENT kinds of cm_ppo_net,
-                              cm_net_desc.flags; 5: cm_channel_cond, per-env channel conditions (cm_env_desc.conds ...) */
+#define CM_ABI_VERSION 6   /* 2: host_arena / obs_bits members, cm_rollout_step_host; 3: cm_ppo_net; 4: CENT kinds of cm_ppo_net,
+                              cm_net_desc.flags; 5: cm_channel_cond, per-env channel conditions (cm_env_desc.conds ...);
+                              6: several policies in one cm_policy_forward (cm_policy_io.n_policies ...) */
 #define CM_MAX_AGENTS 256   /* n, p */
 #define CM_MAX_GRID 64      /* grid side incl. Coverage's wall border */
 #define CM_MAX_LAYERS 4     /* n_gcn_layers */
@@ -229,6 +230,16 @@ typedef struct cm_policy_io {
                                   4 D, the 0/1 columns need no low-order operand — and `obs` may be NULL; results are bit-identical */
     int32_t obs_nbits;         /* number of leading 0/1 columns in obs_bits (D - 3 / D - 2) */
     int32_t host_arena;        /* `host` struct of the *_host calls only; see cm_step_io.host_arena */
+    /* Several policies of one kind and architecture in one launch (ABI 6; 0 or 1 = one policy, the members below are not read).
+     * The envs are cut into n_policies contiguous blocks of envs_per_policy envs; env b runs the policy whose fp32 blob starts at
+     * weights + (b / envs_per_policy) * weights_stride and whose cm_policy_tc_prepare blob (one prepare call per policy, at its
+     * offset) starts at tc_weights + (b / envs_per_policy) * tc_weights_stride.  Every kernel counts its tiles per block, so no
+     * tile holds rows of two policies.  Needs n_envs == n_policies * envs_per_policy, and each stride at least its blob's length
+     * and a multiple of 4 floats (16-byte bulk copies); else CM_EINVAL.  The *_host calls return CM_EUNSUPPORTED. */
+    int32_t n_policies;
+    int64_t envs_per_policy;
+    int64_t weights_stride;    /* floats */
+    int64_t tc_weights_stride; /* floats; math = 0 paths do not read it */
 } cm_policy_io;
 
 int cm_abi_version(void);
