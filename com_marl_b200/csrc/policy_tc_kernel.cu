@@ -76,30 +76,74 @@ __device__ __forceinline__ void split16(float x, __half &hi, __half &lo)
     hi = __float2half_rn(x);
     lo = __float2half_rn((x - __half2float(hi)) * 4096.0f);
 }
-// the same for two values at once: ONE packed conversion per pair (the scalar form costs a conversion and a byte permute
+// c_i + a_i b for the two fp16 halves a_0, a_1 of a2 in fp32: fma.rn.f32.f16, ONE instruction per value (SASS FHFMA) where
+// the remainder x - hi otherwise takes a half -> float conversion and a subtraction.  The product of two fp16 values is exact
+// in fp32, so x - hi (exact in fp32) comes out exactly.
+static constexpr uint16_t kHalfM1 = 0xBC00u, kHalf4096 = 0x6C00u, kHalfM4096 = 0xEC00u;    // -1, 4096, -4096 as fp16
+__device__ __forceinline__ void fma_f32_f16x2(uint32_t a2, uint16_t b, float c0, float c1, float &d0, float &d1)
+{
+    asm("{.reg .f16 a0, a1;\n\tmov.b32 {a0, a1}, %2;\n\tfma.rn.f32.f16 %0, a0, %5, %3;\n\tfma.rn.f32.f16 %1, a1, %5, %4;\n\t}"
+        : "=f"(d0), "=f"(d1) : "r"(a2), "f"(c0), "f"(c1), "h"(b));
+}
+__device__ __forceinline__ uint32_t pack_half2(float x0, float x1)
+{
+    const __half2 h = __floats2half2_rn(x0, x1);
+    return *reinterpret_cast<const uint32_t *>(&h);
+}
+// split16 for two values at once: ONE packed conversion per pair (the scalar form costs a conversion and a byte permute
 // per value — the conversions of the activations are the largest instruction class of the epilogues)
 __device__ __forceinline__ void split16x2(float x0, float x1, uint32_t &hi, uint32_t &lo)
 {
-    const __half2 h = __floats2half2_rn(x0, x1);
-    const float2 hf = __half22float2(h);
-    const __half2 l = __floats2half2_rn((x0 - hf.x) * 4096.0f, (x1 - hf.y) * 4096.0f);
-    hi = *reinterpret_cast<const uint32_t *>(&h);
-    lo = *reinterpret_cast<const uint32_t *>(&l);
+    float d0, d1;
+    hi = pack_half2(x0, x1);
+    fma_f32_f16x2(hi, kHalfM1, x0, x1, d0, d1);                      // x - hi
+    lo = pack_half2(d0 * 4096.0f, d1 * 4096.0f);
+}
+// The same split of x = x' 2^-12 from the PRE-SCALED x' = 4096 x that the tanh epilogues emit (|x| <= 2): h' = fp16(x') is
+// 4096 fp16(x) and 2^-12 h' = fp16(x) exactly wherever fp16(x) is normal; lo = fp16(x' - 4096 hi) with the remainder exact,
+// so the operand is the one split16x2 makes, in 5 instructions per pair instead of 6.  (Below 2^-14, where fp16(x) is
+// subnormal, hi may round differently from fp16(x) at a tie; lo is taken against the hi actually stored, so hi + 2^-12 lo
+// still represents x to the same precision.)
+__device__ __forceinline__ void split16x2_pre(float x0, float x1, uint32_t &hi, uint32_t &lo)
+{
+    float d0, d1;
+    asm("mul.rn.f16x2 %0, %1, %2;" : "=r"(hi) : "r"(pack_half2(x0, x1)), "r"(0x0C000C00u));   // * 2^-12
+    fma_f32_f16x2(hi, kHalfM4096, x0, x1, d0, d1);                   // x' - 4096 hi = 4096 (x - hi)
+    lo = pack_half2(d0, d1);
+}
+static constexpr float kActScale = 4096.0f;                          // x' = kActScale x: the form split16x2_pre takes
+// back from 8 columns of an A operand (hi, lo) to the pre-scaled x' = 4096 hi + lo
+__device__ __forceinline__ void unpack_act_pre(const uint4 &hq, const uint4 &lq, float *x)
+{
+    const uint32_t *hw = &hq.x;
+    const __half2 *ll = reinterpret_cast<const __half2 *>(&lq);
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+        const float2 lf = __half22float2(ll[i]);
+        fma_f32_f16x2(hw[i], kHalf4096, lf.x, lf.y, x[2 * i], x[2 * i + 1]);
+    }
 }
 
 // write CW (8 or 16) consecutive columns, starting at local column c0 (a multiple of 8) of a Kp-wide panel, of row `row`
-// as the next A operand: hi block, then the lo block 128 * Kp halves further
-template <int CW>
+// as the next A operand: hi block, then the lo block 128 * Kp halves further.  kPre: v holds kActScale x (split16x2_pre)
+template <int CW, bool kPre = false>
 __device__ __forceinline__ void write_act(unsigned char *act, int Kp, int row, int c0, const float (&v)[CW])
 {
     const uint32_t lo_off = (uint32_t)kTcRows * Kp * 2;
 #pragma unroll
     for (int g = 0; g < CW; g += 8) {
         uint4 h, l;
-        split16x2(v[g + 0], v[g + 1], h.x, l.x);
-        split16x2(v[g + 2], v[g + 3], h.y, l.y);
-        split16x2(v[g + 4], v[g + 5], h.z, l.z);
-        split16x2(v[g + 6], v[g + 7], h.w, l.w);
+        if constexpr (kPre) {
+            split16x2_pre(v[g + 0], v[g + 1], h.x, l.x);
+            split16x2_pre(v[g + 2], v[g + 3], h.y, l.y);
+            split16x2_pre(v[g + 4], v[g + 5], h.z, l.z);
+            split16x2_pre(v[g + 6], v[g + 7], h.w, l.w);
+        } else {
+            split16x2(v[g + 0], v[g + 1], h.x, l.x);
+            split16x2(v[g + 2], v[g + 3], h.y, l.y);
+            split16x2(v[g + 4], v[g + 5], h.z, l.z);
+            split16x2(v[g + 6], v[g + 7], h.w, l.w);
+        }
         const uint32_t off = canon_off16(row, c0 + g, Kp);
         *reinterpret_cast<uint4 *>(act + off) = h;
         *reinterpret_cast<uint4 *>(act + lo_off + off) = l;
@@ -112,11 +156,10 @@ __device__ __forceinline__ void write_act(unsigned char *act, int Kp, int row, i
 static constexpr float kVScale = 64.0f, kPScale = 1024.0f, kPVUnscale = 1.0f / 65536.0f;
 __device__ __forceinline__ void split_unscaled_x2(float x0, float x1, uint32_t &hi, uint32_t &lo)
 {
-    const __half2 h = __floats2half2_rn(x0, x1);
-    const float2 hf = __half22float2(h);
-    const __half2 l = __floats2half2_rn(x0 - hf.x, x1 - hf.y);
-    hi = *reinterpret_cast<const uint32_t *>(&h);
-    lo = *reinterpret_cast<const uint32_t *>(&l);
+    float d0, d1;
+    hi = pack_half2(x0, x1);
+    fma_f32_f16x2(hi, kHalfM1, x0, x1, d0, d1);
+    lo = pack_half2(d0, d1);
 }
 template <int CW>
 __device__ __forceinline__ void write_unscaled(unsigned char *buf, int Kp, uint32_t lo_off, int row, int c0, const float (&v)[CW], float scale)
@@ -140,12 +183,13 @@ __device__ __forceinline__ void write_unscaled(unsigned char *buf, int Kp, uint3
 // and the shared-memory bias table holds 2 log2(e) * bias.  Saturates correctly: 2^a = inf -> 1, 2^a = 0 -> -1.
 static constexpr float kTanhScale = 2.8853900817779268f;            // 2 log2(e)
 static constexpr float kTanhScaleLo = 2.8853900817779268f / 4096.0f;
-__device__ __forceinline__ float tanh_scaled(float a)
+// `out` (a power of two) scales the result for free in the last FMA: out = kActScale gives the pre-scaled form of write_act
+__device__ __forceinline__ float tanh_scaled(float a, float out = 1.0f)
 {
     float e, r;
     asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(e) : "f"(a));
     asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(e + 1.0f));
-    return fmaf(-2.0f, r, 1.0f);
+    return fmaf(-2.0f * out, r, out);
 }
 // Four tanh's with ONE reciprocal: 1/A = B C D / (A B C D) ...  The special-function unit (16 lanes per clock per SM) is what
 // bounds the dense epilogues locally — two MUFU per tanh occupy it for ~60 % of an epilogue — so the four reciprocals of a
@@ -154,10 +198,10 @@ __device__ __forceinline__ float tanh_scaled(float a)
 #ifndef CM_TANH_SHARED_RCP
 #define CM_TANH_SHARED_RCP 1
 #endif
-__device__ __forceinline__ void tanh4_scaled(float &a0, float &a1, float &a2, float &a3)
+__device__ __forceinline__ void tanh4_scaled(float &a0, float &a1, float &a2, float &a3, float out = 1.0f)
 {
 #if !CM_TANH_SHARED_RCP
-    a0 = tanh_scaled(a0); a1 = tanh_scaled(a1); a2 = tanh_scaled(a2); a3 = tanh_scaled(a3);
+    a0 = tanh_scaled(a0, out); a1 = tanh_scaled(a1, out); a2 = tanh_scaled(a2, out); a3 = tanh_scaled(a3, out);
     return;
 #endif
     float e0, e1, e2, e3, r;
@@ -169,19 +213,19 @@ __device__ __forceinline__ void tanh4_scaled(float &a0, float &a1, float &a2, fl
     const float ab = A * B, cd = C * D;
     asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(ab * cd));
     const float rab = r * ab, rcd = r * cd;          // 1 / (C D), 1 / (A B)
-    a0 = fmaf(-2.0f, rcd * B, 1.0f);
-    a1 = fmaf(-2.0f, rcd * A, 1.0f);
-    a2 = fmaf(-2.0f, rab * D, 1.0f);
-    a3 = fmaf(-2.0f, rab * C, 1.0f);
+    a0 = fmaf(-2.0f * out, rcd * B, out);
+    a1 = fmaf(-2.0f * out, rcd * A, out);
+    a2 = fmaf(-2.0f * out, rab * D, out);
+    a3 = fmaf(-2.0f * out, rab * C, out);
 }
-// tanh(acc0 + 2^-12 acc1 + bias) for 4 consecutive columns, bias4 = 2 log2(e) * bias from the shared-memory table
-__device__ __forceinline__ void tanh4(float *v, const float *w, const float4 b4)
+// out * tanh(acc0 + 2^-12 acc1 + bias) for 4 consecutive columns, bias4 = 2 log2(e) * bias from the shared-memory table
+__device__ __forceinline__ void tanh4(float *v, const float *w, const float4 b4, float out = 1.0f)
 {
     v[0] = fmaf(v[0], kTanhScale, fmaf(w[0], kTanhScaleLo, b4.x));
     v[1] = fmaf(v[1], kTanhScale, fmaf(w[1], kTanhScaleLo, b4.y));
     v[2] = fmaf(v[2], kTanhScale, fmaf(w[2], kTanhScaleLo, b4.z));
     v[3] = fmaf(v[3], kTanhScale, fmaf(w[3], kTanhScaleLo, b4.w));
-    tanh4_scaled(v[0], v[1], v[2], v[3]);
+    tanh4_scaled(v[0], v[1], v[2], v[3], out);
 }
 
 // one converged warp: D[:, 0:N] (+)= A_hi B_hi^T, D[:, N:2N] (+)= A_hi B_lo^T + A_lo B_hi^T.  All lanes run the code
@@ -673,8 +717,8 @@ __global__ void __launch_bounds__(kTcThreads, 2) policy_tc_kernel(const TcArgs A
         ld_acc_raw<16>(lane_addr + blk, 64, 16 * sub, v, w);
         const float4 *bp = reinterpret_cast<const float4 *>(bias_s + bias0 + 16 * sub);
 #pragma unroll
-        for (int q = 0; q < 4; ++q) tanh4(v + 4 * q, w + 4 * q, bp[q]);
-        write_act<16>(dst, 64, row, 16 * sub, v);
+        for (int q = 0; q < 4; ++q) tanh4(v + 4 * q, w + 4 * q, bp[q], kActScale);
+        write_act<16, true>(dst, 64, row, 16 * sub, v);
     };
     // neighbour mask of this row for layer l (dist_adj & channels[l], comm_base_net.py:101)
     uint32_t m0 = 0u, m1 = 0u;
@@ -867,11 +911,14 @@ __global__ void __launch_bounds__(kTcThreads, 2) policy_tc_kernel(const TcArgs A
         run_mma(2, MmaOp{kR0, 0u, 0u}, MmaOp{kR0, 1u, 1u});
         // ---------------- E = tanh(. + b2): keys (k-major fp32) + A operand; Q -> R0, H_0 Wg_0 -> R1 ----------------
         {
+            // E is also wanted unscaled as fp32 (the CUDA-core attention's keys, the large-team pipeline's rows): those
+            // instantiations split it from the unscaled value
+            constexpr bool e_pre = !((kMode == kTcModeComm && !kAttnTc) || kMode == kTcModeEnc);
             float v[16], w[16];
             ld_acc_raw<16>(lane_addr + kR0, 64, 16 * sub, v, w);
             const float4 *bp = reinterpret_cast<const float4 *>(bias_s + kBEnc2 + 16 * sub);
 #pragma unroll
-            for (int q = 0; q < 4; ++q) tanh4(v + 4 * q, w + 4 * q, bp[q]);
+            for (int q = 0; q < 4; ++q) tanh4(v + 4 * q, w + 4 * q, bp[q], e_pre ? kActScale : 1.0f);
             if (!dec && !kAttnTc) {
 #pragma unroll
                 for (int c = 0; c < 16; ++c) KV[(16 * sub + c) * kTPitch + row] = v[c];
@@ -881,7 +928,7 @@ __global__ void __launch_bounds__(kTcThreads, 2) policy_tc_kernel(const TcArgs A
                 for (int c = 0; c < 16; c += 4)
                     *reinterpret_cast<float4 *>(A.scr_e + (size_t)g * kE + 16 * sub + c) = make_float4(v[c], v[c + 1], v[c + 2], v[c + 3]);
             }
-            write_act<16>(ACT, 64, row, 16 * sub, v);
+            write_act<16, e_pre>(ACT, 64, row, 16 * sub, v);
         }
         }   // mode != head
         uint32_t tk = 0u, ep = 0u;                                                // sampling keys: latency hidden by the head
@@ -937,13 +984,7 @@ __global__ void __launch_bounds__(kTcThreads, 2) policy_tc_kernel(const TcArgs A
                     const uint32_t off = canon_off16(row, 16 * sub + g8, 64);
                     const uint4 hq = *reinterpret_cast<const uint4 *>(ACT + off);
                     const uint4 lq = *reinterpret_cast<const uint4 *>(ACT + v_lo + off);
-                    const __half2 *hh = reinterpret_cast<const __half2 *>(&hq), *ll = reinterpret_cast<const __half2 *>(&lq);
-#pragma unroll
-                    for (int i = 0; i < 4; ++i) {
-                        const float2 hf = __half22float2(hh[i]), lf = __half22float2(ll[i]);
-                        ev[g8 + 2 * i] = fmaf(lf.x, 1.0f / 4096.0f, hf.x);
-                        ev[g8 + 2 * i + 1] = fmaf(lf.y, 1.0f / 4096.0f, hf.y);
-                    }
+                    unpack_act_pre(hq, lq, ev + g8);
                 }
                 tmem_st<8>(lane_addr + kColE + (uint32_t)(16 * sub), ev);
                 tmem_st<8>(lane_addr + kColE + (uint32_t)(16 * sub + 8), ev + 8);
@@ -988,21 +1029,23 @@ __global__ void __launch_bounds__(kTcThreads, 2) policy_tc_kernel(const TcArgs A
             const float den = ((red[row] + red[kTPitch + row]) + red[2 * kTPitch + row]) + red[3 * kTPitch + row];
             CM_TP(3 + 4 * l);
             {   // out^T (tensor memory: lane = column c, columns = tile rows) -> T[row][64] fp32, the 16-byte chunk index
-                // XOR-swizzled by (row & 7): a lane stores its 8 consecutive rows as scalars (the 16 lanes of a store hit 16
-                // different banks), a thread reads its 16 columns back as four 128-bit loads (8 lanes = 8 different chunks);
-                // row & 7 == j is a compile-time constant on the store side
-                const int c = 16 * quad + (lane & 15);
-                float *Tw = KV + (32 * sub) * 64 + (c & 3);
-                const int cq = c >> 2;
+                // XOR-swizzled by t_key(row): the warp reads its 32 tile rows in ONE load, the half-warp h taking rows
+                // 32 sub + 16 h + k (k = 0 .. 15) of the 16 columns c of its quadrant, and stores them as scalars.  The key
+                // (row & 7) ^ 4 (row / 16 % 2) keeps such a store conflict-free (the 16 lanes of a half-warp hit 16 banks, the
+                // other half the other 16), a thread reads its 16 columns back as four 128-bit loads (8 lanes = 8 chunks).
+                // t_key(row) = (k & 7) ^ 4 h is a compile-time constant per store up to the half-warp term.
+                const int c = 16 * quad + (lane & 15), h = lane >> 4;
+                float o[16];
+                tmem_ld16x32(lane_addr + kR1 + (uint32_t)(32 * sub), o);
+                // word index of (row 32 sub + 16 h, chunk (c / 4) ^ 4 h); the chunk occupies bits 2..5 alone, so the swizzle of
+                // row + j (j < 8) is an XOR of j << 2
+                const int t0 = (32 * sub + 16 * h) * 64 + ((((c >> 2) ^ (h << 2))) << 2) + (c & 3);
+                tmem_ld_wait();
 #pragma unroll
-                for (int i = 0; i < 4; ++i) {
-                    float v8[8];
-                    tmem_ld8(lane_addr + kR1 + (uint32_t)(32 * sub + 8 * i), v8);
-                    tmem_ld_wait();
-                    if (lane < 16) {
-#pragma unroll
-                        for (int j = 0; j < 8; ++j) Tw[(8 * i + j) * 64 + ((cq ^ j) << 2)] = v8[j];
-                    }
+                for (int j = 0; j < 8; ++j) {
+                    float *tj = KV + (t0 ^ (j << 2));
+                    tj[j * 64] = o[j];
+                    tj[(8 + j) * 64] = o[8 + j];
                 }
                 fence_before_thread_sync();
                 __syncthreads();
@@ -1017,14 +1060,14 @@ __global__ void __launch_bounds__(kTcThreads, 2) policy_tc_kernel(const TcArgs A
 #pragma unroll
             for (int q = 0; q < 4; ++q) {
                 const float4 b4 = bp[q];
-                const float4 t4 = Tr[(4 * sub + q) ^ (row & 7)];
+                const float4 t4 = Tr[(4 * sub + q) ^ ((row & 7) ^ ((row >> 2) & 4))];   // t_key(row)
                 v[4 * q + 0] = fmaf(t4.x, inv, b4.x);
                 v[4 * q + 1] = fmaf(t4.y, inv, b4.y);
                 v[4 * q + 2] = fmaf(t4.z, inv, b4.z);
                 v[4 * q + 3] = fmaf(t4.w, inv, b4.w);
-                tanh4_scaled(v[4 * q + 0], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]);
+                tanh4_scaled(v[4 * q + 0], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3], kActScale);
             }
-            if (d.residual && l + 1 == L) {               // X = E + H_L (comm_base_net.py:105-106)
+            if (d.residual && l + 1 == L) {               // X = E + H_L (comm_base_net.py:105-106), both pre-scaled
                 float ev[16];
                 tmem_ld8(lane_addr + kColE + (uint32_t)(16 * sub), *reinterpret_cast<float(*)[8]>(ev));
                 tmem_ld8(lane_addr + kColE + (uint32_t)(16 * sub + 8), *reinterpret_cast<float(*)[8]>(ev + 8));
@@ -1032,7 +1075,7 @@ __global__ void __launch_bounds__(kTcThreads, 2) policy_tc_kernel(const TcArgs A
 #pragma unroll
                 for (int c = 0; c < 16; ++c) v[c] += ev[c];
             }
-            write_act<16>(ACT, 64, row, 16 * sub, v);
+            write_act<16, true>(ACT, 64, row, 16 * sub, v);
             CM_TP(4 + 4 * l);
             if (l + 1 < L) {
                 load_mask(env, il, l + 1, valid);
@@ -1135,9 +1178,9 @@ __global__ void __launch_bounds__(kTcThreads, 2) policy_tc_kernel(const TcArgs A
                 v[4 * q + 1] = fmaf(acc[4 * q + 1], inv, b4.y);
                 v[4 * q + 2] = fmaf(acc[4 * q + 2], inv, b4.z);
                 v[4 * q + 3] = fmaf(acc[4 * q + 3], inv, b4.w);
-                tanh4_scaled(v[4 * q + 0], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3]);
+                tanh4_scaled(v[4 * q + 0], v[4 * q + 1], v[4 * q + 2], v[4 * q + 3], kActScale);
             }
-            if (d.residual) {                             // X = E + H_L (comm_base_net.py:105-106)
+            if (d.residual) {                             // X = E + H_L (comm_base_net.py:105-106), both pre-scaled
                 // E is still in the A operand buffer (this thread wrote these 16 columns itself) until the first layer's
                 // output replaces it; with more than one layer it is parked in tensor memory meanwhile
                 if (l == 0) {
@@ -1147,13 +1190,7 @@ __global__ void __launch_bounds__(kTcThreads, 2) policy_tc_kernel(const TcArgs A
                         const uint32_t off = canon_off16(row, 16 * sub + g8, 64);
                         const uint4 hq = *reinterpret_cast<const uint4 *>(ACT + off);
                         const uint4 lq = *reinterpret_cast<const uint4 *>(ACT + (uint32_t)kTcRows * 64 * 2 + off);
-                        const __half2 *hh = reinterpret_cast<const __half2 *>(&hq), *ll = reinterpret_cast<const __half2 *>(&lq);
-#pragma unroll
-                        for (int i = 0; i < 4; ++i) {
-                            const float2 hf = __half22float2(hh[i]), lf = __half22float2(ll[i]);
-                            ev[g8 + 2 * i] = fmaf(lf.x, 1.0f / 4096.0f, hf.x);
-                            ev[g8 + 2 * i + 1] = fmaf(lf.y, 1.0f / 4096.0f, hf.y);
-                        }
+                        unpack_act_pre(hq, lq, ev + g8);
                     }
                     if (L == 1) {
 #pragma unroll
@@ -1172,7 +1209,7 @@ __global__ void __launch_bounds__(kTcThreads, 2) policy_tc_kernel(const TcArgs A
                     for (int c = 0; c < 16; ++c) v[c] += ev[c];
                 }
             }
-            write_act<16>(ACT, 64, row, 16 * sub, v);
+            write_act<16, true>(ACT, 64, row, 16 * sub, v);
             CM_TP(4 + 4 * l);
             if (l + 1 < L) {
                 load_mask(env, il, l + 1, valid);

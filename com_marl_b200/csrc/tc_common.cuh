@@ -224,6 +224,19 @@ __device__ __forceinline__ void tmem_ld8(uint32_t taddr, float (&v)[8])
 #pragma unroll
     for (int i = 0; i < 8; ++i) v[i] = __uint_as_float(r[i]);
 }
+// TMEM -> registers for an M = 64 accumulator, whose rows sit in lanes 0..15 of each lane quadrant: the 16 lanes from `taddr`
+// (the lane field of taddr selects them) x 32 consecutive columns, split between the two half-warps so that every thread
+// carries data — thread t holds lane t % 16, columns col + 16 (t / 16) .. + 15 (shape 16x32bx2, half split offset 16)
+__device__ __forceinline__ void tmem_ld16x32(uint32_t taddr, float (&v)[16])
+{
+    uint32_t r[16];
+    asm volatile("tcgen05.ld.sync.aligned.16x32bx2.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16], 16;"
+                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
+                   "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
+                 : "r"(taddr));
+#pragma unroll
+    for (int i = 0; i < 16; ++i) v[i] = __uint_as_float(r[i]);
+}
 __device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 
 // registers -> TMEM: this warp's 32 lanes x NC (1, 2, 4 or 8) consecutive fp32 columns starting at column `col`.
