@@ -16,14 +16,14 @@ CH_FC, CH_FL, CH_IID, CH_GE = 0, 1, 2, 3
 POLICY_COMM, POLICY_DEC, POLICY_CENT = 0, 1, 2
 POLICY_FLAG_RELU = 1
 MAX_AGENTS, MAX_GRID, MAX_LAYERS = 256, 64, 4
-ABI_VERSION = 6
+ABI_VERSION = 7
 MAX_CONDS = 256
 
 EXPORTS = ("cm_abi_version", "cm_strerror", "cm_last_cuda_error", "cm_device_count", "cm_env_reset", "cm_env_step",
            "cm_comm_update", "cm_policy_forward", "cm_policy_blob_floats", "cm_policy_cent_blob_floats", "cm_policy_cent_tc_blob_floats", "cm_policy_cent_workspace_bytes", "cm_policy_workspace_bytes", "cm_policy_tc_blob_floats", "cm_policy_tc_prepare", "cm_mask_pack",
            "cm_mask_unpack", "cm_policy_forward_host", "cm_env_step_host", "cm_env_reset_host", "cm_rollout_step_host", "cm_ppo_advantages",
            "cm_adam_step", "cm_adam_step_dev", "cm_critic_blob_floats", "cm_baseline_mlp_blob_floats", "cm_ppo_net_workspace_floats",
-           "cm_ppo_net")
+           "cm_ppo_net", "cm_adam_step_set")
 NET_POLICY, NET_CRITIC, NET_POLICY_DEC, NET_POLICY_CENT, NET_BASELINE_MLP = 0, 1, 2, 3, 4
 NET_FLAG_RELU = 1
 
@@ -85,7 +85,14 @@ class NetIO(C.Structure):
                                           "valid", "returns")] + \
                [("inv_count", C.c_float)] + \
                [(k, C.c_void_p) for k in ("ll", "entropy", "probs", "values", "loss", "workspace")] + \
-               [("workspace_floats", C.c_size_t)]
+               [("workspace_floats", C.c_size_t)] + \
+               [("n_policies", C.c_int32), ("steps_per_policy", C.c_int64), ("weights_stride", C.c_int64), ("grad_stride", C.c_int64),
+                ("inv_counts", C.c_void_p)]
+
+
+def net_set_workspace_extra(n_policies):
+    """floats a cm_ppo_net call over a set of n_policies networks needs beyond cm_ppo_net_workspace_floats (per-member loss sums)"""
+    return ((2 * max(int(n_policies), 1) + 3) & ~3) - 4
 
 
 class NativeError(RuntimeError):
@@ -151,6 +158,9 @@ def lib():
     L.cm_ppo_net_workspace_floats.argtypes = [C.POINTER(NetDesc), C.c_int64, C.c_int32]
     L.cm_ppo_net.restype = C.c_int
     L.cm_ppo_net.argtypes = [C.POINTER(NetDesc), C.POINTER(NetIO), C.c_void_p]
+    L.cm_adam_step_set.restype = C.c_int
+    L.cm_adam_step_set.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int64, C.c_int64, C.c_float,
+                                   C.c_float, C.c_float, C.c_float, C.POINTER(C.c_int32), C.c_void_p, C.c_void_p]
     for fn in ("cm_env_reset", "cm_env_step", "cm_comm_update", "cm_policy_forward", "cm_mask_pack", "cm_mask_unpack",
                "cm_policy_forward_host", "cm_env_step_host", "cm_env_reset_host", "cm_rollout_step_host", "cm_ppo_advantages", "cm_adam_step"):
         getattr(L, fn).restype = C.c_int

@@ -87,6 +87,31 @@ __global__ void adam_step_kernel(float *__restrict__ p, const float *__restrict_
     }
 }
 
+// The same step over members of a set, member = blockIdx.y + the launch's first member; one that is not stepped has step_size 0 and
+// is skipped whole (a zero-gradient step would still move its parameters through the moments)
+static constexpr int kAdamSetMax = 256;                      // members per launch (their coefficients travel as kernel parameters)
+struct AdamSetCoef { float step_size[kAdamSetMax], inv_sqrt_bc2[kAdamSetMax]; };
+__global__ void adam_step_set_kernel(float *__restrict__ p, const float *__restrict__ g, float *__restrict__ m, float *__restrict__ v,
+                                     int64_t n, int64_t stride, float beta1, float beta2, float eps, const AdamSetCoef c,
+                                     const float *__restrict__ grad_scale_dev)
+{
+    const int k = blockIdx.y;
+    const float step_size = c.step_size[k], inv_sqrt_bc2 = c.inv_sqrt_bc2[k];
+    if (step_size == 0.0f) return;
+    const float grad_scale = grad_scale_dev[k];
+    const int64_t o = (int64_t)k * stride;
+    p += o; g += o; m += o; v += o;
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+        const float gi = g[i] * grad_scale;
+        const float mi = beta1 * m[i] + (1.0f - beta1) * gi;
+        const float vi = beta2 * v[i] + (1.0f - beta2) * gi * gi;
+        m[i] = mi;
+        v[i] = vi;
+        const float denom = sqrtf(vi) * inv_sqrt_bc2 + eps;
+        p[i] = p[i] - step_size * (mi / denom);
+    }
+}
+
 }  // namespace cm
 
 extern "C" int cm_ppo_advantages(const double *rewards, const float *baselines, const int32_t *valids, int64_t n_paths, int32_t T,
@@ -138,4 +163,39 @@ extern "C" int cm_adam_step_dev(float *params, const float *grads, float *exp_av
 {
     if (!grad_scale_dev) return CM_EINVAL;
     return adam_step_impl(params, grads, exp_avg, exp_avg_sq, n, lr, beta1, beta2, eps, step, 1.0f, grad_scale_dev, stream);
+}
+
+extern "C" int cm_adam_step_set(float *params, const float *grads, float *exp_avg, float *exp_avg_sq, int32_t n_policies, int64_t n,
+                                int64_t stride, float lr, float beta1, float beta2, float eps, const int32_t *steps, const float *grad_scale_dev,
+                                cm_stream_t stream)
+{
+    using namespace cm;
+    if (!params || !grads || !exp_avg || !exp_avg_sq || !steps || !grad_scale_dev || n_policies < 0 || n < 0 || stride < n) return CM_EINVAL;
+    for (int32_t k = 0; k < n_policies; ++k)
+        if (steps[k] < 0) return CM_EINVAL;
+    if (n == 0) return CM_OK;
+    for (int32_t k0 = 0; k0 < n_policies; k0 += kAdamSetMax) {
+        const int cnt = n_policies - k0 < kAdamSetMax ? n_policies - k0 : kAdamSetMax;
+        AdamSetCoef c;
+        bool any = false;
+        for (int k = 0; k < cnt; ++k) {
+            const int32_t step = steps[k0 + k];
+            c.step_size[k] = c.inv_sqrt_bc2[k] = 0.0f;
+            if (step == 0) continue;
+            const double bc1 = 1.0 - pow((double)beta1, (double)step), bc2 = 1.0 - pow((double)beta2, (double)step);
+            c.step_size[k] = (float)((double)lr / bc1);
+            c.inv_sqrt_bc2[k] = (float)(1.0 / sqrt(bc2));
+            if (c.step_size[k] == 0.0f) return CM_EINVAL;              // (lr = 0 would read as "not stepped")
+            any = true;
+        }
+        if (!any) continue;
+        const int64_t want = (n + 255) / 256, cap = (148 * 8 + cnt - 1) / cnt;
+        const dim3 grid((unsigned)(want < cap ? want : cap), (unsigned)cnt);
+        const int64_t o = (int64_t)k0 * stride;
+        adam_step_set_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(params + o, grads + o, exp_avg + o, exp_avg_sq + o, n, stride, beta1,
+                                                                     beta2, eps, c, grad_scale_dev + k0);
+        const cudaError_t e = cudaGetLastError();
+        if (e != cudaSuccess) return set_cuda_error(e, CM_ECUDA);
+    }
+    return CM_OK;
 }

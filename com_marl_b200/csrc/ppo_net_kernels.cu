@@ -35,6 +35,16 @@ static constexpr int kNP = 68;          // pitch (floats) of a [row][64] array i
 static constexpr int kRows = 256;       // most rows (agents) of the envs a CTA of the per-env kernels owns at a time
 static constexpr int kNetThreads = 256; // head kernels: one thread per row
 
+// Sets of networks (cm_net_io.n_policies > 1): one launch runs gridDim.y members side by side, member m = blockIdx.y.  Each kernel
+// moves its row pointers by m times one member's rows and its weight / gradient pointers by m times the blob strides, so no tile or
+// env block holds rows of two members, and the partial sums a persistent CTA keeps over its tiles belong to one member.  With one
+// network gridDim.y = 1 and every offset is 0.
+template <typename T>
+__device__ __forceinline__ T *mem_off(T *p, int64_t per_member)
+{
+    return p ? p + (int64_t)blockIdx.y * per_member : p;
+}
+
 // ------------------------------------------------------------------------------------------------------------------
 // dense layers
 // ------------------------------------------------------------------------------------------------------------------
@@ -43,9 +53,11 @@ static constexpr int kNetThreads = 256; // head kernels: one thread per row
 // (the observation rows, D floats) take the synchronous load.  ACT: 0 none, 1 tanh, 2 relu.
 template <int N, int ACT, int ASYNC>
 __global__ void __launch_bounds__(256) net_dense_fwd_kernel(const float *__restrict__ X, int ldx, const float *__restrict__ W,
-                                                            const float *__restrict__ bias, float *__restrict__ Y, int ldy, int64_t R, int K)
+                                                            const float *__restrict__ bias, float *__restrict__ Y, int ldy, int64_t R, int K,
+                                                            int64_t wstr)
 {
     constexpr int TX = N >= 64 ? 16 : N / 4, TY = 256 / TX, RI = 128 / TY, CJ = N / (4 * TX);
+    X = mem_off(X, R * ldx); W = mem_off(W, wstr); bias = mem_off(bias, wstr); Y = mem_off(Y, R * ldy);
     extern __shared__ float4 smem4[];
     float *sm = reinterpret_cast<float *>(smem4);
     const int K4 = (K + 3) & ~3, KP = K4 + 4;
@@ -149,9 +161,12 @@ __global__ void __launch_bounds__(256) net_dense_fwd_kernel(const float *__restr
 template <int N, int KMAX, int ROWS, int ASYNC, int XRELU = 0>
 __global__ void __launch_bounds__(512) net_dense_bwd_kernel(const float *__restrict__ dZ, const float *__restrict__ X, int ldx,
                                                             const float *__restrict__ W, float *__restrict__ dX, int lddx, int accumulate,
-                                                            int xact, float *__restrict__ dW, float *__restrict__ db, int64_t R, int K)
+                                                            int xact, float *__restrict__ dW, float *__restrict__ db, int64_t R, int K,
+                                                            int64_t wstr, int64_t gstr)
 {
     constexpr int NP = N + 4, KP = KMAX + 4;
+    dZ = mem_off(dZ, R * N); X = mem_off(X, R * ldx); W = mem_off(W, wstr); dX = mem_off(dX, R * lddx);
+    dW = mem_off(dW, gstr); db = mem_off(db, gstr);
     constexpr int RI = ROWS / 16;                                          // dX warps: rows ty + 16 i, k = kx + 16 j
     constexpr int KJ = KMAX / 16;
     constexpr int NX = N >= 64 ? 16 : N / 4, NJ = N / (4 * NX), KY = 256 / NX;   // dW warps: n = 4 nx + 64 j, k = 4 ky + 4 KY i
@@ -477,6 +492,7 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? (KT <= 2 ? 3 : 2) : 
 {
     extern __shared__ float4 smem4[];
     float *Es = reinterpret_cast<float *>(smem4), *Qs = Es + cap * kNP;
+    Q = mem_off(Q, S * n * 64); E = mem_off(E, S * n * 64); M = mem_off(M, S * n * n);
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     const int ns = (n + 7) >> 3;
     const int64_t nblk = (S + G - 1) / G;
@@ -516,7 +532,7 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? (KT <= 2 ? 3 : 2) : 
                                                                   const uint32_t *__restrict__ chan, int L, int l,
                                                                   const float *__restrict__ V, const float *__restrict__ bias,
                                                                   float *__restrict__ H, const float *__restrict__ res_in,
-                                                                  float *__restrict__ Xout, int n, int G, int cap, int64_t S)
+                                                                  float *__restrict__ Xout, int n, int G, int cap, int64_t S, int64_t wstr)
 {
     extern __shared__ float4 smem4[];
     constexpr int CP = KT * 32 + 4;
@@ -524,6 +540,8 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? (KT <= 2 ? 3 : 2) : 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     float *Cs = Call + warp * 8 * CP;
     const int ns = (n + 7) >> 3, W = (n + 31) >> 5;
+    M = mem_off(M, S * n * n); adj = mem_off(adj, S * n * W); chan = mem_off(chan, S * L * n * W); V = mem_off(V, S * n * 64);
+    bias = mem_off(bias, wstr); H = mem_off(H, S * n * 64); res_in = mem_off(res_in, S * n * 64); Xout = mem_off(Xout, S * n * 64);
     const float4 bv = *reinterpret_cast<const float4 *>(bias + 4 * (lane & 15));
     const int64_t nblk = (S + G - 1) / G;
     for (int64_t blk = blockIdx.x; blk < nblk; blk += gridDim.x) {
@@ -570,7 +588,7 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? (KT <= 2 ? 3 : 2) : 
                                                                   const float *__restrict__ V, const float *__restrict__ H,
                                                                   const float *__restrict__ dH, float *__restrict__ dV,
                                                                   float *__restrict__ dM, float *__restrict__ CT,
-                                                                  float *__restrict__ db, int n, int G, int cap, int64_t S)
+                                                                  float *__restrict__ db, int n, int G, int cap, int64_t S, int64_t gstr)
 {
     extern __shared__ float4 smem4[];
     constexpr int CP = KT * 32 + 4;
@@ -578,6 +596,9 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? (KT <= 2 ? 3 : 2) : 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     float *Cs = Call + warp * 8 * CP;
     const int ns = (n + 7) >> 3, W = (n + 31) >> 5;
+    M = mem_off(M, S * n * n); adj = mem_off(adj, S * n * W); chan = mem_off(chan, S * L * n * W); V = mem_off(V, S * n * 64);
+    H = mem_off(H, S * n * 64); dH = mem_off(dH, S * n * 64); dV = mem_off(dV, S * n * 64); dM = mem_off(dM, S * n * n);
+    CT = mem_off(CT, S * n * n); db = mem_off(db, gstr);
     float bacc = 0.0f;
     const int64_t nblk = (S + G - 1) / G;
     for (int64_t blk = blockIdx.x; blk < nblk; blk += gridDim.x) {
@@ -661,6 +682,8 @@ __global__ void __launch_bounds__(THREADS, THREADS == 256 ? (KT <= 2 ? 3 : 2) : 
     extern __shared__ float4 smem4[];
     constexpr int CP = KT * 32 + 4;
     float *Es = reinterpret_cast<float *>(smem4), *Qs = Es + cap * kNP, *Call = Qs + cap * kNP;
+    M = mem_off(M, S * n * n); dM = mem_off(dM, S * n * n); E = mem_off(E, S * n * 64); Q = mem_off(Q, S * n * 64);
+    dQ = mem_off(dQ, S * n * 64); dE = mem_off(dE, S * n * 64); CT = mem_off(CT, S * n * n);
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     float *Cs = Call + warp * 8 * CP;
     const int ns = (n + 7) >> 3;
@@ -814,6 +837,7 @@ __global__ void __launch_bounds__(kSmallRows) net_small_scores_kernel(const floa
 {
     __shared__ __align__(16) float Es[kSmallRows * kNP];
     const int tid = threadIdx.x;
+    Q = mem_off(Q, S * n * 64); E = mem_off(E, S * n * 64); M = mem_off(M, S * n * n);
     const int64_t nblk = (S + G - 1) / G;
     for (int64_t blk = blockIdx.x; blk < nblk; blk += gridDim.x) {
         const EnvBlock eb = env_block(blk, G, n, S);
@@ -844,11 +868,13 @@ __global__ void __launch_bounds__(kSmallRows) net_small_agg_fwd_kernel(const flo
                                                                        const uint32_t *__restrict__ chan, int L, int l,
                                                                        const float *__restrict__ V, const float *__restrict__ bias,
                                                                        float *__restrict__ H, const float *__restrict__ res,
-                                                                       float *__restrict__ Xout, int n, int G, int64_t S)
+                                                                       float *__restrict__ Xout, int n, int G, int64_t S, int64_t wstr)
 {
     __shared__ __align__(16) float Vs[kSmallRows * kNP];
     __shared__ float bs[64];
     const int tid = threadIdx.x;
+    M = mem_off(M, S * n * n); adj = mem_off(adj, S * n); chan = mem_off(chan, S * L * n); V = mem_off(V, S * n * 64);
+    bias = mem_off(bias, wstr); H = mem_off(H, S * n * 64); res = mem_off(res, S * n * 64); Xout = mem_off(Xout, S * n * 64);
     if (tid < 64) bs[tid] = bias[tid];
     const int64_t nblk = (S + G - 1) / G;
     for (int64_t blk = blockIdx.x; blk < nblk; blk += gridDim.x) {
@@ -881,11 +907,14 @@ __global__ void __launch_bounds__(kSmallRows) net_small_agg_bwd_kernel(const flo
                                                                        const float *__restrict__ V, const float *__restrict__ H,
                                                                        const float *__restrict__ dH, float *__restrict__ dV,
                                                                        float *__restrict__ dM, float *__restrict__ db,
-                                                                       int n, int G, int64_t S)
+                                                                       int n, int G, int64_t S, int64_t gstr)
 {
     extern __shared__ float4 smem4[];
     float *Vs = reinterpret_cast<float *>(smem4), *dZs = Vs + kSmallRows * kNP, *As = dZs + kSmallRows * kNP;
     const int tid = threadIdx.x;
+    M = mem_off(M, S * n * n); adj = mem_off(adj, S * n); chan = mem_off(chan, S * L * n); V = mem_off(V, S * n * 64);
+    H = mem_off(H, S * n * 64); dH = mem_off(dH, S * n * 64); dV = mem_off(dV, S * n * 64); dM = mem_off(dM, S * n * n);
+    db = mem_off(db, gstr);
     float bacc = 0.0f;
     const int64_t nblk = (S + G - 1) / G;
     for (int64_t blk = blockIdx.x; blk < nblk; blk += gridDim.x) {
@@ -949,6 +978,8 @@ __global__ void __launch_bounds__(kSmallRows) net_small_softmax_bwd_kernel(const
     extern __shared__ float4 smem4[];
     float *Es = reinterpret_cast<float *>(smem4), *Qs = Es + kSmallRows * kNP, *Ds = Qs + kSmallRows * kNP;
     const int tid = threadIdx.x;
+    M = mem_off(M, S * n * n); dM = mem_off(dM, S * n * n); E = mem_off(E, S * n * 64); Q = mem_off(Q, S * n * 64);
+    dQ = mem_off(dQ, S * n * 64); dE = mem_off(dE, S * n * 64);
     const int64_t nblk = (S + G - 1) / G;
     for (int64_t blk = blockIdx.x; blk < nblk; blk += gridDim.x) {
         const EnvBlock eb = env_block(blk, G, n, S);
@@ -1008,8 +1039,24 @@ struct PolicyHeadArgs {
     float *dlogits;              // CENT: [S][5n] d logits for the dW4 product
     int relu;                    // CENT: act = relu instead of tanh
     int n, G;
-    int64_t S;
+    int64_t S;                   // steps of one member
+    const float *inv_counts;     // set: [members] 1 / count, replaces inv_count (NULL: inv_count)
+    int64_t wstr, gstr;          // set: weight / gradient blob strides
 };
+
+// member blockIdx.y of a set: its rows, weights, gradient targets, loss slot and 1 / count
+__device__ __forceinline__ PolicyHeadArgs policy_member(const PolicyHeadArgs &a0)
+{
+    PolicyHeadArgs a = a0;
+    const int64_t S = a.S, R = S * a.n;
+    a.g3 = mem_off(a.g3, R * 32); a.w4 = mem_off(a.w4, a.wstr); a.b4 = mem_off(a.b4, a.wstr);
+    a.avail_bits = mem_off(a.avail_bits, R); a.actions = mem_off(a.actions, R);
+    a.adv = mem_off(a.adv, S); a.old_ll = mem_off(a.old_ll, S); a.valid = mem_off(a.valid, S);
+    a.ll = mem_off(a.ll, S); a.ent = mem_off(a.ent, S); a.probs = mem_off(a.probs, R * CM_ACTIONS);
+    a.loss = mem_off(a.loss, 1); a.dg3 = mem_off(a.dg3, R * 32); a.dw4 = mem_off(a.dw4, a.gstr); a.db4 = mem_off(a.db4, a.gstr);
+    if (a.inv_counts) a.inv_count = a.inv_counts[blockIdx.y];
+    return a;
+}
 
 static constexpr float kProbEps = 1.1920928955078125e-07f;   // torch.finfo(float32).eps: probs_to_logits clamps to [eps, 1 - eps]
 
@@ -1077,7 +1124,10 @@ __device__ __forceinline__ void cta_loss_add(double *loss, float lsum, float *re
     if (threadIdx.x == 0) atomicAdd(loss, (double)*red1);
 }
 
-__global__ void net_loss_store_kernel(float *loss, const double *sum) { *loss += (float)*sum; }
+__global__ void net_loss_store_kernel(float *loss, const double *sum, int count)
+{
+    for (int i = threadIdx.x; i < count; i += blockDim.x) loss[i] += (float)sum[i];
+}
 
 // One env step s with joint log-likelihood ll and mean entropy en: outputs, the clipped surrogate added to the loss and the
 // gradients gl = d loss / d ll, ge = d loss / d (one agent's entropy)
@@ -1103,8 +1153,9 @@ __device__ __forceinline__ void head_step_objective(const PolicyHeadArgs &a, int
     }
 }
 
-__global__ void __launch_bounds__(kNetThreads) net_policy_head_kernel(const PolicyHeadArgs a)
+__global__ void __launch_bounds__(kNetThreads) net_policy_head_kernel(const PolicyHeadArgs a0)
 {
+    const PolicyHeadArgs a = policy_member(a0);
     __shared__ float w4s[32 * CM_ACTIONS + CM_ACTIONS];
     __shared__ float ll_row[kRows], ent_row[kRows], gll_env[kRows], gent_env[kRows];
     __shared__ float red[32 * CM_ACTIONS + CM_ACTIONS], lred;
@@ -1315,11 +1366,26 @@ struct CriticHeadArgs {
     float *dc1, *dw2, *db2, *dlog_std;
     int unclamped;               // 1: std = exp(log_std) without CommBaseCritic's clamp at log 1e-6 (GaussianMLPBaseline)
     int n, G;
-    int64_t S;
+    int64_t S;                   // steps of one member
+    const uint8_t *valid;        // [S] or NULL: 0 = padded step, its value is written but adds nothing to the loss or gradient
+    const float *inv_counts;     // (as PolicyHeadArgs)
+    int64_t wstr, gstr;
 };
 
-__global__ void __launch_bounds__(kNetThreads) net_critic_head_kernel(const CriticHeadArgs a)
+__device__ __forceinline__ CriticHeadArgs critic_member(const CriticHeadArgs &a0)
 {
+    CriticHeadArgs a = a0;
+    const int64_t S = a.S, R = S * a.n;
+    a.c1 = mem_off(a.c1, R * 64); a.w2 = mem_off(a.w2, a.wstr); a.b2 = mem_off(a.b2, a.wstr); a.log_std = mem_off(a.log_std, a.wstr);
+    a.returns = mem_off(a.returns, S); a.values = mem_off(a.values, S); a.valid = mem_off(a.valid, S); a.loss = mem_off(a.loss, 1);
+    a.dc1 = mem_off(a.dc1, R * 64); a.dw2 = mem_off(a.dw2, a.gstr); a.db2 = mem_off(a.db2, a.gstr); a.dlog_std = mem_off(a.dlog_std, a.gstr);
+    if (a.inv_counts) a.inv_count = a.inv_counts[blockIdx.y];
+    return a;
+}
+
+__global__ void __launch_bounds__(kNetThreads) net_critic_head_kernel(const CriticHeadArgs a0)
+{
+    const CriticHeadArgs a = critic_member(a0);
     __shared__ float w2s[64], v_row[kRows], gv_env[kRows], red[66], lred;
     const int tid = threadIdx.x, lane = tid & 31;
     const int n = a.n;
@@ -1356,7 +1422,7 @@ __global__ void __launch_bounds__(kNetThreads) net_critic_head_kernel(const Crit
             const int64_t s = eb.s0 + tid;
             if (a.values) a.values[s] = V;
             float gv = 0.0f;
-            if (a.returns) {
+            if (a.returns && (!a.valid || a.valid[s])) {
                 const float d = (a.returns[s] - V) / sd;
                 lsum += (0.5f * d * d + logf(sd) + 0.91893853320467274178f) * a.inv_count;
                 gv = -d / sd * a.inv_count;
@@ -1601,8 +1667,21 @@ static cudaError_t set_smem(Kern k, size_t bytes)
 
 static const size_t kSmemMax = 227 * 1024;
 
+// The members of a set one launch runs (gridDim.y = g) and their blob strides in floats; Grp() = one network
+struct Grp {
+    int g = 1;
+    int64_t wstr = 0, gstr = 0;
+};
+// CTAs along x when g members of `units` work units each share about `cap` CTAs (the SMs times the occupancy)
+static int grid_x(int64_t units, int64_t cap, int g)
+{
+    const int64_t c = (cap + g - 1) / g;
+    return (int)(units < c ? units : c);
+}
+
 template <int N, int ACT, int ASYNC>
-static cudaError_t dense_fwd_a(const float *X, int ldx, const float *W, const float *b, float *Y, int64_t R, int K, cudaStream_t st)
+static cudaError_t dense_fwd_a(const float *X, int ldx, const float *W, const float *b, float *Y, int64_t R, int K, cudaStream_t st,
+                               const Grp &q)
 {
     const int K4 = (K + 3) & ~3;
     const size_t smem = ((size_t)K4 * N + (ASYNC ? 2 : 1) * 128 * (size_t)(K4 + 4)) * sizeof(float) + 16;
@@ -1610,67 +1689,68 @@ static cudaError_t dense_fwd_a(const float *X, int ldx, const float *W, const fl
     int per_sm = 1;
     NET_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, net_dense_fwd_kernel<N, ACT, ASYNC>, 256, smem));
     if (per_sm < 1) per_sm = 1;
-    const int64_t tiles = (R + 127) / 128;
-    const int grid = (int)(tiles < (int64_t)sm_count() * per_sm ? tiles : (int64_t)sm_count() * per_sm);
-    net_dense_fwd_kernel<N, ACT, ASYNC><<<grid, 256, smem, st>>>(X, ldx, W, b, Y, N, R, K);
+    const dim3 grid(grid_x((R + 127) / 128, (int64_t)sm_count() * per_sm, q.g), q.g);
+    net_dense_fwd_kernel<N, ACT, ASYNC><<<grid, 256, smem, st>>>(X, ldx, W, b, Y, N, R, K, q.wstr);
     return cudaGetLastError();
 }
 static bool rows_aligned(const float *X, int ldx, int K) { return (ldx & 3) == 0 && (K & 3) == 0 && (reinterpret_cast<uintptr_t>(X) & 15) == 0; }
 
 template <int N, int ACT>
-static cudaError_t dense_fwd_t(const float *X, int ldx, const float *W, const float *b, float *Y, int64_t R, int K, cudaStream_t st)
+static cudaError_t dense_fwd_t(const float *X, int ldx, const float *W, const float *b, float *Y, int64_t R, int K, cudaStream_t st,
+                               const Grp &q)
 {
-    return rows_aligned(X, ldx, K) ? dense_fwd_a<N, ACT, 1>(X, ldx, W, b, Y, R, K, st) : dense_fwd_a<N, ACT, 0>(X, ldx, W, b, Y, R, K, st);
+    return rows_aligned(X, ldx, K) ? dense_fwd_a<N, ACT, 1>(X, ldx, W, b, Y, R, K, st, q) : dense_fwd_a<N, ACT, 0>(X, ldx, W, b, Y, R, K, st, q);
 }
 
+// R = rows of one member (q.g members side by side, X / Y rows member-major)
 static cudaError_t dense_fwd(const float *X, int ldx, const float *W, const float *b, float *Y, int64_t R, int K, int N, int act,
-                             cudaStream_t st)
+                             cudaStream_t st, const Grp &q = Grp())
 {
     if (act == 2)                            // relu: the CENT policy's 128 -> 64 and 64 -> 32 layers
-        return N == 64 ? dense_fwd_t<64, 2>(X, ldx, W, b, Y, R, K, st) : dense_fwd_t<32, 2>(X, ldx, W, b, Y, R, K, st);
-    if (N == 128) return act ? dense_fwd_t<128, 1>(X, ldx, W, b, Y, R, K, st) : dense_fwd_t<128, 0>(X, ldx, W, b, Y, R, K, st);
-    if (N == 64) return act ? dense_fwd_t<64, 1>(X, ldx, W, b, Y, R, K, st) : dense_fwd_t<64, 0>(X, ldx, W, b, Y, R, K, st);
-    return act ? dense_fwd_t<32, 1>(X, ldx, W, b, Y, R, K, st) : dense_fwd_t<32, 0>(X, ldx, W, b, Y, R, K, st);
+        return N == 64 ? dense_fwd_t<64, 2>(X, ldx, W, b, Y, R, K, st, q) : dense_fwd_t<32, 2>(X, ldx, W, b, Y, R, K, st, q);
+    if (N == 128) return act ? dense_fwd_t<128, 1>(X, ldx, W, b, Y, R, K, st, q) : dense_fwd_t<128, 0>(X, ldx, W, b, Y, R, K, st, q);
+    if (N == 64) return act ? dense_fwd_t<64, 1>(X, ldx, W, b, Y, R, K, st, q) : dense_fwd_t<64, 0>(X, ldx, W, b, Y, R, K, st, q);
+    return act ? dense_fwd_t<32, 1>(X, ldx, W, b, Y, R, K, st, q) : dense_fwd_t<32, 0>(X, ldx, W, b, Y, R, K, st, q);
 }
 
 template <int N, int KMAX, int ROWS, int ASYNC, int XRELU>
 static cudaError_t dense_bwd_a(const float *dZ, const float *X, int ldx, const float *W, float *dX, int accumulate, int xact, float *dW,
-                               float *db, int64_t R, int K, cudaStream_t st)
+                               float *db, int64_t R, int K, cudaStream_t st, const Grp &q)
 {
     const size_t smem = ((size_t)KMAX * (N + 4) + (ASYNC ? 2 : 1) * (size_t)ROWS * (N + 4 + KMAX + 4)) * sizeof(float) + 16;
     NET_TRY(set_smem(net_dense_bwd_kernel<N, KMAX, ROWS, ASYNC, XRELU>, smem));
     int per_sm = 1;
     NET_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, net_dense_bwd_kernel<N, KMAX, ROWS, ASYNC, XRELU>, 512, smem));
     if (per_sm < 1) per_sm = 1;
-    const int64_t tiles = (R + ROWS - 1) / ROWS;
-    const int grid = (int)(tiles < (int64_t)sm_count() * per_sm ? tiles : (int64_t)sm_count() * per_sm);
-    net_dense_bwd_kernel<N, KMAX, ROWS, ASYNC, XRELU><<<grid, 512, smem, st>>>(dZ, X, ldx, W, dX, K, accumulate, xact, dW, db, R, K);
+    const dim3 grid(grid_x((R + ROWS - 1) / ROWS, (int64_t)sm_count() * per_sm, q.g), q.g);
+    net_dense_bwd_kernel<N, KMAX, ROWS, ASYNC, XRELU><<<grid, 512, smem, st>>>(dZ, X, ldx, W, dX, K, accumulate, xact, dW, db, R, K,
+                                                                               q.wstr, q.gstr);
     return cudaGetLastError();
 }
 
 template <int N, int KMAX, int XRELU = 0>
 static cudaError_t dense_bwd_t(const float *dZ, const float *X, int ldx, const float *W, float *dX, int accumulate, int xact, float *dW,
-                               float *db, int64_t R, int K, cudaStream_t st)
+                               float *db, int64_t R, int K, cudaStream_t st, const Grp &q)
 {
     // two stages of 128-row tiles where they fit into shared memory, else of 64-row tiles
     constexpr bool fits = ((size_t)KMAX * (N + 4) + 2 * (size_t)128 * (N + 4 + KMAX + 4)) * sizeof(float) + 16 <= 227 * 1024;
-    if (!rows_aligned(X, ldx, K)) return dense_bwd_a<N, KMAX, 128, 0, XRELU>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st);
-    return dense_bwd_a<N, KMAX, fits ? 128 : 64, 1, XRELU>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st);
+    if (!rows_aligned(X, ldx, K)) return dense_bwd_a<N, KMAX, 128, 0, XRELU>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st, q);
+    return dense_bwd_a<N, KMAX, fits ? 128 : 64, 1, XRELU>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st, q);
 }
 
 // gradients of Y = X W + b from dZ [R][N]; dX [R][K] (lddx = K) may be NULL; xact: dX *= act'(X), 1 = tanh, 2 = relu (the CENT
 // policy's 64 -> 32 and 128 -> 64 layers, the only ones built for it)
 static cudaError_t dense_bwd(const float *dZ, const float *X, int ldx, const float *W, float *dX, int accumulate, int xact, float *dW,
-                             float *db, int64_t R, int K, int N, cudaStream_t st)
+                             float *db, int64_t R, int K, int N, cudaStream_t st, const Grp &q = Grp())
 {
-    if (xact == 2) return N == 32 ? dense_bwd_t<32, 64, 1>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st)
-                                  : dense_bwd_t<64, 128, 1>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st);
-    if (N == 128) return K <= 64 ? dense_bwd_t<128, 64>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st)
-                                 : dense_bwd_t<128, 128>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st);
-    if (N == 64) return K <= 64 ? dense_bwd_t<64, 64>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st)
-                                : dense_bwd_t<64, 128>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st);
-    return K <= 64 ? dense_bwd_t<32, 64>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st)
-                   : dense_bwd_t<32, 128>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st);
+    if (xact == 2) return N == 32 ? dense_bwd_t<32, 64, 1>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st, q)
+                                  : dense_bwd_t<64, 128, 1>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st, q);
+    if (N == 128) return K <= 64 ? dense_bwd_t<128, 64>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st, q)
+                                 : dense_bwd_t<128, 128>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st, q);
+    if (N == 64) return K <= 64 ? dense_bwd_t<64, 64>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st, q)
+                                : dense_bwd_t<64, 128>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st, q);
+    return K <= 64 ? dense_bwd_t<32, 64>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st, q)
+                   : dense_bwd_t<32, 128>(dZ, X, ldx, W, dX, accumulate, xact, dW, db, R, K, st, q);
 }
 
 // wide-K layers (CENT family)
@@ -1703,11 +1783,10 @@ static cudaError_t wide_dw_t(const float *X, int ldx, const float *dZ, float *dW
 }
 
 static int env_group(int n) { return n >= kRows ? 1 : kRows / n; }          // head kernels: one thread per row, 256 rows per CTA
-static int env_grid(int n, int64_t S, int per_sm)
+static dim3 env_grid(int n, int64_t S, int per_sm, int g = 1)
 {
     const int G = env_group(n);
-    const int64_t nblk = (S + G - 1) / G;
-    return (int)(nblk < (int64_t)sm_count() * per_sm ? nblk : (int64_t)sm_count() * per_sm);
+    return dim3(grid_x((S + G - 1) / G, (int64_t)sm_count() * per_sm, g), g);
 }
 
 // n x n kernels: a CTA owns G whole envs at a time, at most `cap` rows: 64 rows up to n = 32 (three or more CTAs per SM hide the
@@ -1724,21 +1803,21 @@ static EnvGeom env_geom(int n)
 
 struct EnvCall {
     int n, L;
-    int64_t S;
+    int64_t S;                   // steps of one member
     const uint32_t *adj, *chan;
     cudaStream_t st;
+    Grp q;
 };
 
 template <typename Kern>
-static cudaError_t env_launch_dims(Kern k, int threads, size_t smem, const EnvCall &c, int *grid)
+static cudaError_t env_launch_dims(Kern k, int threads, size_t smem, const EnvCall &c, dim3 *grid)
 {
     NET_TRY(set_smem(k, smem));
     int per_sm = 1;
     NET_TRY(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, threads, smem));
     if (per_sm < 1) per_sm = 1;
     const EnvGeom g = env_geom(c.n);
-    const int64_t nblk = (c.S + g.G - 1) / g.G;
-    *grid = (int)(nblk < (int64_t)sm_count() * per_sm ? nblk : (int64_t)sm_count() * per_sm);
+    *grid = dim3(grid_x((c.S + g.G - 1) / g.G, (int64_t)sm_count() * per_sm, c.q.g), c.q.g);
     return cudaSuccess;
 }
 static size_t cs_floats(int KT, int threads) { return (size_t)(threads / 32) * 8 * (KT * 32 + 4); }
@@ -1748,7 +1827,7 @@ static cudaError_t scores_t(const EnvCall &c, const float *Q, const float *E, fl
 {
     const EnvGeom g = env_geom(c.n);
     const size_t smem = 2 * (size_t)g.cap * kNP * sizeof(float);
-    int grid;
+    dim3 grid;
     NET_TRY(env_launch_dims(net_scores_kernel<KT, 256>, 256, smem, c, &grid));
     net_scores_kernel<KT, 256><<<grid, 256, smem, c.st>>>(Q, E, M, c.n, g.G, g.cap, c.S);
     return cudaGetLastError();
@@ -1761,13 +1840,13 @@ static cudaError_t agg_fwd_t(const EnvCall &c, int l, const float *M, const floa
     const size_t rows = (size_t)g.cap * kNP;
     const bool wide = c.n > 64 && (rows + cs_floats(KT, 512)) * sizeof(float) <= kSmemMax;      // one env per CTA: 16 warps share it
     const size_t smem = (rows + cs_floats(KT, wide ? 512 : 256)) * sizeof(float);
-    int grid;
+    dim3 grid;
     if (wide) {
         NET_TRY(env_launch_dims(net_agg_fwd_kernel<KT, 512>, 512, smem, c, &grid));
-        net_agg_fwd_kernel<KT, 512><<<grid, 512, smem, c.st>>>(M, c.adj, c.chan, c.L, l, V, bias, H, res, Xout, c.n, g.G, g.cap, c.S);
+        net_agg_fwd_kernel<KT, 512><<<grid, 512, smem, c.st>>>(M, c.adj, c.chan, c.L, l, V, bias, H, res, Xout, c.n, g.G, g.cap, c.S, c.q.wstr);
     } else {
         NET_TRY(env_launch_dims(net_agg_fwd_kernel<KT, 256>, 256, smem, c, &grid));
-        net_agg_fwd_kernel<KT, 256><<<grid, 256, smem, c.st>>>(M, c.adj, c.chan, c.L, l, V, bias, H, res, Xout, c.n, g.G, g.cap, c.S);
+        net_agg_fwd_kernel<KT, 256><<<grid, 256, smem, c.st>>>(M, c.adj, c.chan, c.L, l, V, bias, H, res, Xout, c.n, g.G, g.cap, c.S, c.q.wstr);
     }
     return cudaGetLastError();
 }
@@ -1781,13 +1860,15 @@ static cudaError_t agg_bwd_t(const EnvCall &c, int l, const float *M, const floa
     const size_t rows = 2 * (size_t)g.cap * kNP;
     const bool wide = c.n > 64 && (rows + cs_floats(KT, 512)) * sizeof(float) <= kSmemMax;
     const size_t smem = (rows + cs_floats(KT, wide ? 512 : 256)) * sizeof(float);
-    int grid;
+    dim3 grid;
     if (wide) {
         NET_TRY(env_launch_dims(net_agg_bwd_kernel<KT, 512>, 512, smem, c, &grid));
-        net_agg_bwd_kernel<KT, 512><<<grid, 512, smem, c.st>>>(M, c.adj, c.chan, c.L, l, V, H, dH, dV, dM, CT, db, c.n, g.G, g.cap, c.S);
+        net_agg_bwd_kernel<KT, 512><<<grid, 512, smem, c.st>>>(M, c.adj, c.chan, c.L, l, V, H, dH, dV, dM, CT, db, c.n, g.G, g.cap, c.S,
+                                                               c.q.gstr);
     } else {
         NET_TRY(env_launch_dims(net_agg_bwd_kernel<KT, 256>, 256, smem, c, &grid));
-        net_agg_bwd_kernel<KT, 256><<<grid, 256, smem, c.st>>>(M, c.adj, c.chan, c.L, l, V, H, dH, dV, dM, CT, db, c.n, g.G, g.cap, c.S);
+        net_agg_bwd_kernel<KT, 256><<<grid, 256, smem, c.st>>>(M, c.adj, c.chan, c.L, l, V, H, dH, dV, dM, CT, db, c.n, g.G, g.cap, c.S,
+                                                               c.q.gstr);
     }
     return cudaGetLastError();
 }
@@ -1799,7 +1880,7 @@ static cudaError_t softmax_bwd_t(const EnvCall &c, const float *M, const float *
     const size_t rows = 2 * (size_t)g.cap * kNP;
     const bool wide = c.n > 64 && (rows + cs_floats(KT, 512)) * sizeof(float) <= kSmemMax;
     const size_t smem = (rows + cs_floats(KT, wide ? 512 : 256)) * sizeof(float);
-    int grid;
+    dim3 grid;
     if (wide) {
         NET_TRY(env_launch_dims(net_softmax_bwd_kernel<KT, 512>, 512, smem, c, &grid));
         net_softmax_bwd_kernel<KT, 512><<<grid, 512, smem, c.st>>>(M, dM, c.L, dm_stride, E, Q, dQ, dE, CT, c.n, g.G, g.cap, c.S);
@@ -1821,11 +1902,10 @@ static cudaError_t softmax_bwd_t(const EnvCall &c, const float *M, const float *
     } while (0)
 
 static const size_t kSmallBwdSmem = (2 * (size_t)kSmallRows * kNP + (size_t)kSmallRows * kSmallN) * sizeof(float);
-static int small_grid(const EnvCall &c, int per_sm)
+static dim3 small_grid(const EnvCall &c, int per_sm)
 {
     const int G = kSmallRows / c.n;
-    const int64_t nblk = (c.S + G - 1) / G;
-    return (int)(nblk < (int64_t)sm_count() * per_sm ? nblk : (int64_t)sm_count() * per_sm);
+    return dim3(grid_x((c.S + G - 1) / G, (int64_t)sm_count() * per_sm, c.q.g), c.q.g);
 }
 static cudaError_t scores(const EnvCall &c, const float *Q, const float *E, float *M)
 {
@@ -1840,7 +1920,7 @@ static cudaError_t agg_fwd(const EnvCall &c, int l, const float *M, const float 
 {
     if (c.n <= kSmallN) {
         net_small_agg_fwd_kernel<<<small_grid(c, 6), kSmallRows, 0, c.st>>>(M, c.adj, c.chan, c.L, l, V, bias, H, res, Xout, c.n,
-                                                                             kSmallRows / c.n, c.S);
+                                                                             kSmallRows / c.n, c.S, c.q.wstr);
         return cudaGetLastError();
     }
     KT_DISPATCH(agg_fwd_t, c, l, M, V, bias, H, res, Xout);
@@ -1851,7 +1931,7 @@ static cudaError_t agg_bwd(const EnvCall &c, int l, const float *M, const float 
     if (c.n <= kSmallN) {
         NET_TRY(set_smem(net_small_agg_bwd_kernel, kSmallBwdSmem));
         net_small_agg_bwd_kernel<<<small_grid(c, 3), kSmallRows, kSmallBwdSmem, c.st>>>(M, c.adj, c.chan, c.L, l, V, H, dH, dV, dM, db, c.n,
-                                                                             kSmallRows / c.n, c.S);
+                                                                             kSmallRows / c.n, c.S, c.q.gstr);
         return cudaGetLastError();
     }
     KT_DISPATCH(agg_bwd_t, c, l, M, V, H, dH, dV, dM, CT, db);
@@ -1902,14 +1982,14 @@ static NetWs carve(float *p, int n, int L, int64_t steps, bool backward)
 // the shared trunk: encoder -> attention -> graph convolutions -> X
 static cudaError_t trunk_fwd(const cm_net_desc &d, const EnvCall &c, const float *wts, const Blob &o, const float *obs, const NetWs &w)
 {
-    const int64_t R = c.S * d.n_agents;
-    NET_TRY(dense_fwd(obs, d.obs_dim, wts + o.enc_w1, wts + o.enc_b1, w.h1, R, d.obs_dim, 128, 1, c.st));
-    NET_TRY(dense_fwd(w.h1, 128, wts + o.enc_w2, wts + o.enc_b2, w.E, R, 128, 64, 1, c.st));
-    NET_TRY(dense_fwd(w.E, 64, wts + o.att_w, nullptr, w.Q, R, 64, 64, 0, c.st));
+    const int64_t R = c.S * d.n_agents;                               // rows of one member
+    NET_TRY(dense_fwd(obs, d.obs_dim, wts + o.enc_w1, wts + o.enc_b1, w.h1, R, d.obs_dim, 128, 1, c.st, c.q));
+    NET_TRY(dense_fwd(w.h1, 128, wts + o.enc_w2, wts + o.enc_b2, w.E, R, 128, 64, 1, c.st, c.q));
+    NET_TRY(dense_fwd(w.E, 64, wts + o.att_w, nullptr, w.Q, R, 64, 64, 0, c.st, c.q));
     NET_TRY(scores(c, w.Q, w.E, w.M));
     for (int l = 0; l < d.n_layers; ++l) {
         const float *Hin = l == 0 ? w.E : w.H[l - 1];
-        NET_TRY(dense_fwd(Hin, 64, wts + o.gcn_w + l * kE * kE, nullptr, w.V[l], R, 64, 64, 0, c.st));
+        NET_TRY(dense_fwd(Hin, 64, wts + o.gcn_w + l * kE * kE, nullptr, w.V[l], R, 64, 64, 0, c.st, c.q));
         const bool last = l == d.n_layers - 1;
         NET_TRY(agg_fwd(c, l, w.M, w.V[l], wts + o.gcn_b + l * kE, w.H[l], (last && d.residual) ? w.E : nullptr,
                         (last && d.residual) ? w.X : nullptr));
@@ -1923,31 +2003,31 @@ static cudaError_t trunk_bwd(const cm_net_desc &d, const EnvCall &c, const float
 {
     const int64_t R = c.S * d.n_agents;
     const int L = d.n_layers;
-    const size_t S2 = (size_t)c.S * d.n_agents * d.n_agents;          // layer l's dM array starts at w.dM + l * S2 (scalar accesses only)
+    const size_t S2 = (size_t)c.q.g * c.S * d.n_agents * d.n_agents;  // layer l's dM array starts at w.dM + l * S2 (scalar accesses only)
     float *dE = w.t64b;                       // with the residual connection the gradient of X is the first term of dE
     const float *dHl = w.t64b;
     bool dE_init = d.residual != 0;
     if (!d.residual) {                        // dX is dH_L only: park it, dE starts empty
-        NET_TRY(cudaMemcpyAsync(w.t64a, w.t64b, (size_t)R * 64 * sizeof(float), cudaMemcpyDeviceToDevice, c.st));
+        NET_TRY(cudaMemcpyAsync(w.t64a, w.t64b, (size_t)c.q.g * R * 64 * sizeof(float), cudaMemcpyDeviceToDevice, c.st));
         dHl = w.t64a;
     }
     for (int l = L - 1; l >= 0; --l) {
         NET_TRY(agg_bwd(c, l, w.M, w.V[l], w.H[l], dHl, w.t64c, w.dM + (size_t)l * S2, w.CT, grad + o.gcn_b + l * kE));
         const float *Hin = l == 0 ? w.E : w.H[l - 1];
         if (l == 0) {
-            NET_TRY(dense_bwd(w.t64c, Hin, 64, wts + o.gcn_w, dE, dE_init ? 1 : 0, 0, grad + o.gcn_w, nullptr, R, 64, 64, c.st));
+            NET_TRY(dense_bwd(w.t64c, Hin, 64, wts + o.gcn_w, dE, dE_init ? 1 : 0, 0, grad + o.gcn_w, nullptr, R, 64, 64, c.st, c.q));
             dE_init = true;
         } else {
             NET_TRY(dense_bwd(w.t64c, Hin, 64, wts + o.gcn_w + l * kE * kE, w.t64a, 0, 0, grad + o.gcn_w + l * kE * kE, nullptr, R, 64, 64,
-                              c.st));
+                              c.st, c.q));
             dHl = w.t64a;
         }
     }
     NET_TRY(softmax_bwd(c, w.M, w.dM, (int64_t)S2, w.E, w.Q, w.t64c, dE, w.CT));
     // the last term of dE (through Q = E W_a); the same pass turns the sum into dZ of the embedding layer: dE (1 - E^2)
-    NET_TRY(dense_bwd(w.t64c, w.E, 64, wts + o.att_w, dE, 1, 1, grad + o.att_w, nullptr, R, 64, 64, c.st));
-    NET_TRY(dense_bwd(dE, w.h1, 128, wts + o.enc_w2, w.t128, 0, 1, grad + o.enc_w2, grad + o.enc_b2, R, 128, 64, c.st));
-    NET_TRY(dense_bwd(w.t128, obs, d.obs_dim, wts + o.enc_w1, nullptr, 0, 0, grad + o.enc_w1, grad + o.enc_b1, R, d.obs_dim, 128, c.st));
+    NET_TRY(dense_bwd(w.t64c, w.E, 64, wts + o.att_w, dE, 1, 1, grad + o.att_w, nullptr, R, 64, 64, c.st, c.q));
+    NET_TRY(dense_bwd(dE, w.h1, 128, wts + o.enc_w2, w.t128, 0, 1, grad + o.enc_w2, grad + o.enc_b2, R, 128, 64, c.st, c.q));
+    NET_TRY(dense_bwd(w.t128, obs, d.obs_dim, wts + o.enc_w1, nullptr, 0, 0, grad + o.enc_w1, grad + o.enc_b1, R, d.obs_dim, 128, c.st, c.q));
     return cudaSuccess;
 }
 
@@ -2031,34 +2111,47 @@ static cudaError_t run_chunk_cent(const cm_net_desc &d, const cm_net_io &io, int
     return wide_dw_t<128, 0>(obs, K, dz1, g + o.w1, g + o.b1, R, K, st);
 }
 
-static cudaError_t run_chunk(const cm_net_desc &d, const cm_net_io &io, int64_t s0, int64_t steps, float *wsp, double *lacc, cudaStream_t st)
+// One launch sequence over steps [s0, s0 + steps) of members m0 .. m0 + g - 1 of a set, s0 = m0 * P + off (P = steps per member;
+// one network: m0 = 0, ng = 1).  ng > 1 only for whole members (off = 0, steps = P), so that the inputs and the workspace both hold
+// the ng members' rows `steps` steps apart.
+static cudaError_t run_chunk(const cm_net_desc &d, const cm_net_io &io, int64_t P, int m0, int ng, int64_t off, int64_t steps, float *wsp,
+                             double *lacc, cudaStream_t st)
 {
+    const int64_t s0 = m0 * P + off;
     if (cent_kind(d.kind)) return run_chunk_cent(d, io, s0, steps, wsp, lacc, st);
     const int n = d.n_agents, D = d.obs_dim, L = d.n_layers, W = (n + 31) / 32;
     const bool backward = io.grad != nullptr;
-    const NetWs w = carve(wsp, n, L, steps, backward);
+    const bool set = io.n_policies > 1;
+    const NetWs w = carve(wsp, n, L, ng * steps, backward);
     const int64_t R = steps * n, r0 = s0 * n;
     EnvCall c;
     c.n = n; c.L = L; c.S = steps; c.st = st;
     c.adj = io.adj_bits ? io.adj_bits + r0 * W : nullptr;
     c.chan = io.chan_bits ? io.chan_bits + s0 * L * n * W : nullptr;
+    c.q.g = ng;
+    c.q.wstr = set ? io.weights_stride : 0;
+    c.q.gstr = set ? io.grad_stride : 0;
+    const Grp &q = c.q;
     const float *obs = io.obs + r0 * D;
-    const float *wts = io.weights;
+    const float *wts = io.weights + m0 * q.wstr;
+    float *grad = io.grad ? io.grad + m0 * q.gstr : nullptr;
+    const float *inv_counts = set ? io.inv_counts + m0 : nullptr;
+    if (lacc) lacc += m0;
     const int G = env_group(n);
     if (d.kind == CM_NET_POLICY || d.kind == CM_NET_POLICY_DEC) {
         const bool dec = d.kind == CM_NET_POLICY_DEC;        // Obs-DP: encoder D -> 128 -> 64 and head 64 -> 32 -> 5 per agent row, no communication
         const Blob o = blob_layout(D, L);
         const float *Xin = nullptr;
         if (dec) {
-            NET_TRY(dense_fwd(obs, D, wts + o.enc_w1, wts + o.enc_b1, w.h1, R, D, 128, 1, st));
-            NET_TRY(dense_fwd(w.h1, 128, wts + o.enc_w2, wts + o.enc_b2, w.E, R, 128, 64, 1, st));
-            NET_TRY(dense_fwd(w.E, 64, wts + o.head_w3, wts + o.head_b3, w.g3, R, 64, 32, 1, st));
+            NET_TRY(dense_fwd(obs, D, wts + o.enc_w1, wts + o.enc_b1, w.h1, R, D, 128, 1, st, q));
+            NET_TRY(dense_fwd(w.h1, 128, wts + o.enc_w2, wts + o.enc_b2, w.E, R, 128, 64, 1, st, q));
+            NET_TRY(dense_fwd(w.E, 64, wts + o.head_w3, wts + o.head_b3, w.g3, R, 64, 32, 1, st, q));
         } else {
             NET_TRY(trunk_fwd(d, c, wts, o, obs, w));
             Xin = d.residual ? w.X : w.H[L - 1];
-            NET_TRY(dense_fwd(Xin, 64, wts + o.head_w1, wts + o.head_b1, w.g1, R, 64, 128, 1, st));
-            NET_TRY(dense_fwd(w.g1, 128, wts + o.head_w2, wts + o.head_b2, w.g2, R, 128, 64, 1, st));
-            NET_TRY(dense_fwd(w.g2, 64, wts + o.head_w3, wts + o.head_b3, w.g3, R, 64, 32, 1, st));
+            NET_TRY(dense_fwd(Xin, 64, wts + o.head_w1, wts + o.head_b1, w.g1, R, 64, 128, 1, st, q));
+            NET_TRY(dense_fwd(w.g1, 128, wts + o.head_w2, wts + o.head_b2, w.g2, R, 128, 64, 1, st, q));
+            NET_TRY(dense_fwd(w.g2, 64, wts + o.head_w3, wts + o.head_b3, w.g3, R, 64, 32, 1, st, q));
         }
         PolicyHeadArgs a = {};
         a.g3 = w.g3; a.w4 = wts + o.head_w4; a.b4 = wts + o.head_b4;
@@ -2073,27 +2166,28 @@ static cudaError_t run_chunk(const cm_net_desc &d, const cm_net_io &io, int64_t 
         a.probs = io.probs ? io.probs + r0 * CM_ACTIONS : nullptr;
         a.loss = lacc;
         a.n = n; a.G = G; a.S = steps;
-        if (backward) { a.dg3 = w.t32; a.dw4 = io.grad + o.head_w4; a.db4 = io.grad + o.head_b4; }
-        net_policy_head_kernel<<<env_grid(n, steps, 4), kNetThreads, 0, st>>>(a);
+        a.inv_counts = inv_counts; a.wstr = q.wstr; a.gstr = q.gstr;
+        if (backward) { a.dg3 = w.t32; a.dw4 = grad + o.head_w4; a.db4 = grad + o.head_b4; }
+        net_policy_head_kernel<<<env_grid(n, steps, 4, ng), kNetThreads, 0, st>>>(a);
         NET_TRY(cudaGetLastError());
         if (!backward) return cudaSuccess;
-        float *g = io.grad;
+        float *g = grad;
         if (dec) {
-            NET_TRY(dense_bwd(w.t32, w.E, 64, wts + o.head_w3, w.t64b, 0, 1, g + o.head_w3, g + o.head_b3, R, 64, 32, st));
-            NET_TRY(dense_bwd(w.t64b, w.h1, 128, wts + o.enc_w2, w.t128, 0, 1, g + o.enc_w2, g + o.enc_b2, R, 128, 64, st));
-            return dense_bwd(w.t128, obs, D, wts + o.enc_w1, nullptr, 0, 0, g + o.enc_w1, g + o.enc_b1, R, D, 128, st);
+            NET_TRY(dense_bwd(w.t32, w.E, 64, wts + o.head_w3, w.t64b, 0, 1, g + o.head_w3, g + o.head_b3, R, 64, 32, st, q));
+            NET_TRY(dense_bwd(w.t64b, w.h1, 128, wts + o.enc_w2, w.t128, 0, 1, g + o.enc_w2, g + o.enc_b2, R, 128, 64, st, q));
+            return dense_bwd(w.t128, obs, D, wts + o.enc_w1, nullptr, 0, 0, g + o.enc_w1, g + o.enc_b1, R, D, 128, st, q);
         }
         // (the head kernel hands over dZ of the last hidden layer; every layer's dX pass applies the tanh derivative of the one below)
-        NET_TRY(dense_bwd(w.t32, w.g2, 64, wts + o.head_w3, w.t64a, 0, 1, g + o.head_w3, g + o.head_b3, R, 64, 32, st));
-        NET_TRY(dense_bwd(w.t64a, w.g1, 128, wts + o.head_w2, w.t128, 0, 1, g + o.head_w2, g + o.head_b2, R, 128, 64, st));
-        NET_TRY(dense_bwd(w.t128, Xin, 64, wts + o.head_w1, w.t64b, 0, 0, g + o.head_w1, g + o.head_b1, R, 64, 128, st));
+        NET_TRY(dense_bwd(w.t32, w.g2, 64, wts + o.head_w3, w.t64a, 0, 1, g + o.head_w3, g + o.head_b3, R, 64, 32, st, q));
+        NET_TRY(dense_bwd(w.t64a, w.g1, 128, wts + o.head_w2, w.t128, 0, 1, g + o.head_w2, g + o.head_b2, R, 128, 64, st, q));
+        NET_TRY(dense_bwd(w.t128, Xin, 64, wts + o.head_w1, w.t64b, 0, 0, g + o.head_w1, g + o.head_b1, R, 64, 128, st, q));
         return trunk_bwd(d, c, wts, g, o, obs, w);
     }
     const CriticBlob cb = critic_blob_layout(D, L);
     const Blob o = trunk_of(cb);
     NET_TRY(trunk_fwd(d, c, wts, o, obs, w));
     const float *Xin = d.residual ? w.X : w.H[L - 1];
-    NET_TRY(dense_fwd(Xin, 64, wts + cb.dec_w1, wts + cb.dec_b1, w.g2, R, 64, 64, 1, st));
+    NET_TRY(dense_fwd(Xin, 64, wts + cb.dec_w1, wts + cb.dec_b1, w.g2, R, 64, 64, 1, st, q));
     CriticHeadArgs a = {};
     a.c1 = w.g2; a.w2 = wts + cb.dec_w2; a.b2 = wts + cb.dec_b2; a.log_std = wts + cb.log_std;
     a.returns = io.returns ? io.returns + s0 : nullptr;
@@ -2101,12 +2195,14 @@ static cudaError_t run_chunk(const cm_net_desc &d, const cm_net_io &io, int64_t 
     a.values = io.values ? io.values + s0 : nullptr;
     a.loss = lacc;
     a.n = n; a.G = G; a.S = steps;
-    if (backward) { a.dc1 = w.t64a; a.dw2 = io.grad + cb.dec_w2; a.db2 = io.grad + cb.dec_b2; a.dlog_std = io.grad + cb.log_std; }
-    net_critic_head_kernel<<<env_grid(n, steps, 4), kNetThreads, 0, st>>>(a);
+    a.valid = io.valid ? io.valid + s0 : nullptr;
+    a.inv_counts = inv_counts; a.wstr = q.wstr; a.gstr = q.gstr;
+    if (backward) { a.dc1 = w.t64a; a.dw2 = grad + cb.dec_w2; a.db2 = grad + cb.dec_b2; a.dlog_std = grad + cb.log_std; }
+    net_critic_head_kernel<<<env_grid(n, steps, 4, ng), kNetThreads, 0, st>>>(a);
     NET_TRY(cudaGetLastError());
     if (!backward) return cudaSuccess;
-    NET_TRY(dense_bwd(w.t64a, Xin, 64, wts + cb.dec_w1, w.t64b, 0, 0, io.grad + cb.dec_w1, io.grad + cb.dec_b1, R, 64, 64, st));
-    return trunk_bwd(d, c, wts, io.grad, o, obs, w);
+    NET_TRY(dense_bwd(w.t64a, Xin, 64, wts + cb.dec_w1, w.t64b, 0, 0, grad + cb.dec_w1, grad + cb.dec_b1, R, 64, 64, st, q));
+    return trunk_bwd(d, c, wts, grad, o, obs, w);
 }
 
 }  // namespace cm
@@ -2136,26 +2232,44 @@ extern "C" int cm_ppo_net(const cm_net_desc *desc, const cm_net_io *io, cm_strea
     if (d.n_agents < 1 || d.n_agents > CM_MAX_AGENTS || d.obs_dim < 1 || d.obs_dim > 128 ||
         (!cent_kind(d.kind) && (d.n_layers < 1 || d.n_layers > CM_MAX_LAYERS)))
         return CM_EUNSUPPORTED;
+    if (io->n_policies > 1 && cent_kind(d.kind)) return CM_EUNSUPPORTED;      // (sets: the Comm-DP / Obs-DP kinds only)
     const bool value_net = d.kind == CM_NET_CRITIC || d.kind == CM_NET_BASELINE_MLP;
     if (io->grad && !value_net && (!io->actions || !io->adv)) return CM_EINVAL;
     if (io->grad && value_net && !io->returns) return CM_EINVAL;
     if (io->n_steps == 0) return CM_OK;
     if (cm_device_count() <= 0) return CM_ENODEVICE;
     const bool backward = io->grad != nullptr;
+    const bool set = io->n_policies > 1;
+    const int np = set ? io->n_policies : 1;
+    const int64_t P = set ? io->steps_per_policy : io->n_steps;       // steps per member
+    if (set) {
+        const int64_t blob = d.kind == CM_NET_CRITIC ? critic_blob_layout(d.obs_dim, d.n_layers).total
+                                                     : blob_layout(d.obs_dim, d.n_layers).total;
+        if (io->n_policies > 65535 || P < 1 || io->n_steps != (int64_t)np * P || io->weights_stride < blob || (io->weights_stride & 3) ||
+            (backward && (io->grad_stride < blob || (io->grad_stride & 3))))
+            return CM_EINVAL;
+        if (!io->inv_counts && (io->loss || backward)) return CM_EINVAL;
+    }
     const size_t per_step = ws_floats_per_step(d, backward);
-    if (io->workspace_floats < per_step + kWsSlack) return CM_EINVAL;
-    const int64_t chunk = (int64_t)((io->workspace_floats - kWsSlack) / per_step);
+    const size_t lacc_floats = ((size_t)2 * np + 3) & ~(size_t)3;     // one float64 loss sum per member, 16-byte aligned
+    if (io->workspace_floats < per_step + kWsSlack + lacc_floats - 4) return CM_EINVAL;
+    const int64_t chunk = (int64_t)((io->workspace_floats - kWsSlack - (lacc_floats - 4)) / per_step);
     float *wsp = reinterpret_cast<float *>((reinterpret_cast<uintptr_t>(io->workspace) + 15) & ~(uintptr_t)15);
-    double *lacc = io->loss ? reinterpret_cast<double *>(wsp) : nullptr;      // the loss sum of every chunk (16-byte aligned)
-    wsp += 4;
+    double *lacc = io->loss ? reinterpret_cast<double *>(wsp) : nullptr;      // the loss sums of every chunk (16-byte aligned)
+    wsp += lacc_floats;
     const cudaStream_t st = (cudaStream_t)stream;
-    cudaError_t e = lacc ? cudaMemsetAsync(lacc, 0, sizeof(double), st) : cudaSuccess;
-    for (int64_t s0 = 0; e == cudaSuccess && s0 < io->n_steps; s0 += chunk) {
-        int64_t steps = io->n_steps - s0 < chunk ? io->n_steps - s0 : chunk;
-        e = run_chunk(d, *io, s0, steps, wsp, lacc, st);
+    cudaError_t e = lacc ? cudaMemsetAsync(lacc, 0, np * sizeof(double), st) : cudaSuccess;
+    if (chunk >= P) {                    // whole members per chunk, side by side in one launch sequence
+        const int per = (int)(chunk / P < np ? chunk / P : np);
+        for (int m0 = 0; e == cudaSuccess && m0 < np; m0 += per)
+            e = run_chunk(d, *io, P, m0, per < np - m0 ? per : np - m0, 0, P, wsp, lacc, st);
+    } else {                             // a member longer than a chunk: its own chunks, one after the other
+        for (int m = 0; m < np; ++m)
+            for (int64_t off = 0; e == cudaSuccess && off < P; off += chunk)
+                e = run_chunk(d, *io, P, m, 1, off, P - off < chunk ? P - off : chunk, wsp, lacc, st);
     }
     if (e == cudaSuccess && lacc) {
-        net_loss_store_kernel<<<1, 1, 0, st>>>(io->loss, lacc);
+        net_loss_store_kernel<<<1, 64, 0, st>>>(io->loss, lacc, np);
         e = cudaGetLastError();
     }
     return e == cudaSuccess ? CM_OK : set_cuda_error(e, CM_ECUDA);

@@ -32,7 +32,7 @@ def unpack_positions(packed) -> np.ndarray:
     return np.stack([packed & 0xFF, packed >> 8], axis=-1).astype(np.int8)
 
 
-def check_conditions(spec: ScenarioSpec, conditions, n_envs: int, policy_blocks: int = 1):
+def check_conditions(spec: ScenarioSpec, conditions, n_envs: int, policy_blocks: int = 1, block_conditions: bool = False):
     """-> the validated list of channel conditions of a BatchedEnv (None when there are none); raises ValueError"""
     if int(policy_blocks) < 1 or int(n_envs) % int(policy_blocks):
         raise ValueError(f"n_envs = {n_envs} does not split into {policy_blocks} equal policy blocks")
@@ -40,6 +40,10 @@ def check_conditions(spec: ScenarioSpec, conditions, n_envs: int, policy_blocks:
     if conditions is None:
         return None
     conditions = list(conditions)
+    if block_conditions:
+        if len(conditions) != int(policy_blocks):
+            raise ValueError(f"block_conditions needs one condition per policy block: {len(conditions)} for {policy_blocks}")
+        n_envs = len(conditions)                 # (every block is whole under its condition)
     if not 1 <= len(conditions) <= N.MAX_CONDS:
         raise ValueError(f"between 1 and {N.MAX_CONDS} channel conditions are supported, got {len(conditions)}")
     if int(n_envs) % len(conditions):
@@ -55,18 +59,19 @@ class BatchedEnv:
     """B environment instances of one scenario on one GPU."""
 
     def __init__(self, spec: ScenarioSpec, n_envs: int, device="cuda", env_id0: int = 0, auto_reset: bool = True,
-                 conditions=None, policy_blocks: int = 1):
+                 conditions=None, policy_blocks: int = 1, block_conditions: bool = False):
         """``conditions``: optional list of specs that differ from ``spec`` in the channel fields only
         (ScenarioSpec.CHANNEL_FIELDS, e.g. ``spec.with_channel(pl=..., rcom=...)``).  The envs are then split into equal
         contiguous blocks in list order and block k communicates under ``conditions[k]`` (``spec``'s own channel is not
         used); ``cond_idx`` [B] holds each env's condition.  Everything else — and the global env ids — stays as without.
         ``policy_blocks``: the envs are that many equal blocks (one per policy of a PolicySet), each split into the conditions
-        in the same way (env order policy, condition, episode)."""
+        in the same way (env order policy, condition, episode).  ``block_conditions``: instead, one condition per policy block —
+        block i communicates under ``conditions[i]`` (the members of a set trained each under its own channel)."""
         N.lib()  # fail loudly if the CUDA library is missing; there is no CPU path
         if not torch.cuda.is_available():
             raise RuntimeError("com_marl_b200 needs a CUDA device: the rollout engine has no CPU fallback")
         spec.validate()
-        self.conditions = check_conditions(spec, conditions, n_envs, policy_blocks)
+        self.conditions = check_conditions(spec, conditions, n_envs, policy_blocks, block_conditions)
         self.policy_blocks = int(policy_blocks)
         self.spec, self.B, self.auto_reset = spec, int(n_envs), bool(auto_reset)
         self.device = torch.device(device)
@@ -106,7 +111,10 @@ class BatchedEnv:
             self._conds_host = (N.ChannelCond * K)(*[c.channel_cond() for c in self.conditions])
             self._conds = torch.frombuffer(bytearray(bytes(self._conds_host)), dtype=torch.uint8).to(dev)
             P = self.policy_blocks
-            self.cond_idx = torch.arange(K, dtype=torch.uint8, device=dev).repeat_interleave(B // (K * P)).repeat(P)
+            if block_conditions:
+                self.cond_idx = torch.arange(K, dtype=torch.uint8, device=dev).repeat_interleave(B // K)
+            else:
+                self.cond_idx = torch.arange(K, dtype=torch.uint8, device=dev).repeat_interleave(B // (K * P)).repeat(P)
         self.desc = self._desc()
         self.state = N.EnvState()
         self.state.n_envs = B

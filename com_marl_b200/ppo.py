@@ -562,3 +562,238 @@ class DevicePPO:
         tolist = lambda xs: [float(x) for x in torch.cat([x.reshape(1) for x in xs]).cpu()] if xs else []  # noqa: E731
         return dict(loss_before=float(loss_before), loss_after=float(after["loss"]), kl=kl, entropy=entropy, losses=tolist(losses),
                     baseline_losses=tolist(bl_losses), grad_norms=tolist(gnorms), n_paths=P)
+
+
+class DevicePPOSet:
+    """K independent ``DevicePPO`` updates of one architecture and one set of hyper-parameters run side by side: every optimizer
+    step is ONE ``cm_ppo_net`` call per network over all members (``cm_net_io.n_policies``) and ONE ``cm_adam_step_set`` per
+    network, instead of K of each.  Member i computes what a standalone ``DevicePPO(policies[i], critics[i], fused=True)``
+    computes; only the order of fp32 atomic sums differs.
+
+    Storage: one ``[K][n]`` flat bucket per network (parameters, gradient, both moments); member i's parameters are views of row
+    i, and ``members[i]`` — the member's own ``DevicePPO`` — works on those rows, so its ``process_samples`` /
+    ``batch_from_trajectory`` build the member's batch.  Kernel-only: Comm-DP and Obs-DP policies with a ``CommBaseCritic`` on a
+    GPU; CENT and multi-rank sets raise."""
+
+    def __init__(self, policies, critics, **ppo_args):
+        from .policy import PolicySet
+        from .ppo_fused import FusedCommNets, _SetBlobMap
+        policies, critics = list(policies), list(critics)
+        if not policies or len(policies) != len(critics):
+            raise ValueError("a DevicePPOSet needs one critic per policy")
+        if _world(ppo_args.get("process_group")) > 1:
+            raise NotImplementedError("DevicePPOSet runs on one rank: sets across ranks are not built")
+        for p, c in zip(policies, critics):
+            if p.device.type != "cuda" or not (FusedCommNets.supports(p, c) and getattr(c, "_fusable", False)):
+                raise NotImplementedError("DevicePPOSet runs the update kernels of the Comm-DP / Obs-DP families only "
+                                          "(CommCategoricalMLPPolicy or DecCategoricalMLPPolicy with a CommBaseCritic, on a GPU)")
+        for i in range(1, len(policies)):
+            if PolicySet._arch(policies[i]) != PolicySet._arch(policies[0]) or \
+                    tuple((k, tuple(v.shape)) for k, v in critics[i].state_dict().items()) != \
+                    tuple((k, tuple(v.shape)) for k, v in critics[0].state_dict().items()):
+                raise ValueError(f"member {i} differs in architecture from member 0: one launch runs one network shape")
+        ppo_args = dict(ppo_args, fused=True)
+        self.members = [DevicePPO(p, c, **ppo_args) for p, c in zip(policies, critics)]
+        m0 = self.members[0]
+        self.K, self.device = len(policies), m0.device
+        self.clip_grad_norm, self.n_minibatches, self.mini_epochs = m0.clip_grad_norm, m0.n_minibatches, m0.mini_epochs
+        self.positive_adv = m0.positive_adv
+        self.opt = _SetBuckets([m.opt for m in self.members])
+        self.baseline_opt = _SetBuckets([m.baseline_opt for m in self.members])
+        F0 = m0._fused
+        self.pol = _SetBlobMap(F0.pol_map, self.opt.flat)
+        self.cri = _SetBlobMap(F0.cri_map, self.baseline_opt.flat)
+        for i, m in enumerate(self.members):          # the members' maps read and write the set's rows
+            for mp, sm, fl in ((m._fused.pol_map, self.pol, self.opt.flat), (m._fused.cri_map, self.cri, self.baseline_opt.flat)):
+                mp.flat, mp.blob, mp.grad = fl[i], sm.blob[i, :sm.nb], sm.grad[i, :sm.nb]
+        self._ws = None
+
+    # ---- one cm_ppo_net call over every member ------------------------------------------------------------------------
+    def _run_set(self, desc, smap, inp, P, backward, inv_counts, policy):
+        F = self.members[0]._fused
+        K = self.K
+        io = N.NetIO()
+        io.n_steps = K * P
+        io.weights, io.grad = N.ptr(smap.blob), (N.ptr(smap.grad) if backward else None)
+        io.obs, io.adj_bits, io.chan_bits, io.valid = N.ptr(inp["obs"]), N.ptr(inp["adj"]), N.ptr(inp["chan"]), N.ptr(inp["valid"])
+        if policy:
+            io.avail_bits, io.actions, io.adv, io.old_ll = N.ptr(inp["avail"]), N.ptr(inp["actions"]), N.ptr(inp["adv"]), N.ptr(inp["old"])
+        else:
+            io.returns = N.ptr(inp["ret"])
+        loss = torch.zeros(K, dtype=torch.float32, device=self.device)
+        io.loss = N.ptr(loss)
+        io.inv_counts, io.inv_count = N.ptr(inv_counts), float(inp["inv_host"][0])
+        io.n_policies, io.steps_per_policy, io.weights_stride, io.grad_stride = K, P, smap.stride, smap.stride
+        F._ws, ws = self._ws, None
+        try:
+            ws = F._workspace(desc, K * P, backward, extra=N.net_set_workspace_extra(K))
+        finally:
+            self._ws, F._ws = F._ws, None
+        io.workspace, io.workspace_floats = N.ptr(ws), ws.numel()
+        with torch.cuda.device(self.device):
+            N.check("cm_ppo_net", N.lib().cm_ppo_net(C.byref(desc), C.byref(io), N.stream_ptr()))
+        return loss
+
+    @staticmethod
+    def _stack(parts, P, fill, template):
+        """member rows [n_i, ...] -> [K * P, ...] padded per member with `fill` to P rows"""
+        out = torch.full((len(parts), P) + tuple(template.shape[1:]), fill, dtype=template.dtype, device=template.device)
+        for i, t in enumerate(parts):
+            if t is not None and t.shape[0]:
+                out[i, :t.shape[0]] = t
+        return out.reshape((len(parts) * P,) + tuple(template.shape[1:])).contiguous()
+
+    def _slice_inputs(self, mbs, policy):
+        """the set inputs of one optimizer step: member i's minibatch rows (or none), padded to the longest with finite valid = 0
+        steps (zero observation, all-ones bit rows, every action available, action 0, advantage 0)"""
+        key = "pol" if policy else "cri"
+        rows = [mb[key]["obs"].shape[0] if mb is not None else 0 for mb in mbs]
+        P = max(max(rows), 1)
+        t = next(mb for mb in mbs if mb is not None)
+        g = lambda k: [mb[key][k] if mb is not None else None for mb in mbs]  # noqa: E731
+        inp = dict(obs=self._stack(g("obs"), P, 0, t[key]["obs"]), adj=self._stack(g("adj"), P, -1, t[key]["adj"]),
+                   chan=self._stack(g("chan"), P, -1, t[key]["chan"]))
+        v = torch.zeros(len(mbs), P, dtype=torch.uint8, device=self.device)
+        for i, r in enumerate(rows):
+            v[i, :r] = 1
+        inp["valid"] = v.reshape(-1).contiguous()
+        if policy:
+            inp["avail"] = self._stack(g("avail"), P, 0x1F, t["pol"]["avail"])
+            inp["actions"] = self._stack(g("actions"), P, 0, t["pol"]["actions"])
+            inp["adv"] = self._stack([mb["adv"] if mb is not None else None for mb in mbs], P, 0.0, t["adv"])
+            inp["old"] = self._stack([mb["old"] if mb is not None else None for mb in mbs], P, 0.0, t["old"])
+            inv = [1.0 / max(mb["n_valid"], 1) if mb is not None else 1.0 for mb in mbs]
+        else:
+            inp["ret"] = self._stack([mb["ret"] if mb is not None else None for mb in mbs], P, 0.0, t["ret"])
+            inv = [1.0 / max(mb["n_all"], 1) if mb is not None else 1.0 for mb in mbs]
+        inp["inv_host"] = inv
+        inp["inv"] = torch.tensor(inv, dtype=torch.float32, device=self.device)
+        return inp, P
+
+    # ---- train_once ---------------------------------------------------------------------------------------------------
+    def train_once(self, batches, shuffled_ids=None):
+        """One round of every member: ``batches[i]`` is member i's padded device batch (``members[i].process_samples`` /
+        ``batch_from_trajectory``), ``shuffled_ids[i]`` its path permutation.  Returns one dict per member with the keys of
+        ``DevicePPO.train_once``."""
+        K = self.K
+        if len(batches) != K:
+            raise ValueError(f"{len(batches)} batches for {K} members")
+        shuffled_ids = [None] * K if shuffled_ids is None else list(shuffled_ids)
+        nan = torch.full((1,), float("nan"), device=self.device)
+        with torch.no_grad():
+            self.pol.refresh()
+            self.cri.refresh()
+            st = []                       # per member: flat batch, advantages, old policy, minibatches
+            for i, (m, b) in enumerate(zip(self.members, batches)):
+                F = m._fused
+                f = b.get("_flat") or F.prepare(b)
+                P = int(b["rewards"].shape[0])
+                raw_adv, ret_all = b["adv"].reshape(-1), b["returns"].reshape(-1)
+                adv_all = raw_adv - raw_adv.min() if self.positive_adv else raw_adv
+                n_valid_all = max(int(f["valids_host"].sum()), 1)
+                F._ws, self._ws = self._ws, None
+                old = F.policy_call(f, None, adv=adv_all, want_probs=True, inv_count=1.0 / n_valid_all)
+                self._ws, F._ws = F._ws, None
+                ids_all = np.random.permutation(P) if shuffled_ids[i] is None else np.asarray(shuffled_ids[i])
+                mbs = []
+                for start, stop in minibatch_plan(P, self.n_minibatches):
+                    ids = ids_all[start:stop]
+                    idx_all, idx = F.step_index(f, ids, valid_only=False), F.step_index(f, ids, valid_only=True)
+                    adv = raw_adv.index_select(0, idx)
+                    if self.positive_adv:
+                        adv = adv - raw_adv.index_select(0, idx_all).min()
+                    mbs.append(dict(cri=F.subset(f, idx_all, policy=False), ret=ret_all.index_select(0, idx_all), pol=F.subset(f, idx),
+                                    adv=adv, old=old["ll"].index_select(0, idx), n_valid=int(idx.numel()), n_all=int(idx_all.numel())))
+                st.append(dict(f=f, P=P, adv_all=adv_all, n_valid_all=n_valid_all, old=old, mbs=mbs, losses=[], bl=[], gn=[]))
+            n_slices = max(len(s["mbs"]) for s in st)
+            steps = []                    # per slice: the set inputs of both networks and which members step
+            for j in range(n_slices):
+                mbs = [s["mbs"][j] if j < len(s["mbs"]) else None for s in st]
+                steps.append((self._slice_inputs(mbs, False), self._slice_inputs(mbs, True), [mb is not None for mb in mbs]))
+            F0 = self.members[0]._fused
+            ones = torch.ones(K, dtype=torch.float32, device=self.device)
+            for _ in range(self.mini_epochs):
+                for (cri_in, Pc), (pol_in, Pp), stepped in steps:
+                    self.cri.grad.zero_()
+                    bl = self._run_set(F0.cri_desc, self.cri, cri_in, Pc, True, cri_in["inv"], policy=False)
+                    self.cri.scatter_grad(self.baseline_opt.grad)
+                    self.pol.grad.zero_()
+                    loss = self._run_set(F0.pol_desc, self.pol, pol_in, Pp, True, pol_in["inv"], policy=True)
+                    self.pol.scatter_grad(self.opt.grad)
+                    scale = ones
+                    if self.clip_grad_norm is not None:
+                        coef, norm = self.opt.clip_coefficient(self.clip_grad_norm)
+                        scale, gn = coef, norm * coef
+                    self.opt.step(stepped, scale)
+                    self.baseline_opt.step(stepped, ones)
+                    self.pol.refresh()
+                    self.cri.refresh()
+                    for i, s in enumerate(st):
+                        if stepped[i]:
+                            s["losses"].append(loss[i:i + 1])
+                            s["bl"].append(bl[i:i + 1])
+                            if self.clip_grad_norm is not None:
+                                s["gn"].append(gn[i:i + 1])
+            outs = []
+            for m, s in zip(self.members, st):
+                F = m._fused
+                F._ws, self._ws = self._ws, None
+                after = F.policy_call(s["f"], None, adv=s["adv_all"], old_ll=s["old"]["ll"], want_probs=True,
+                                      inv_count=1.0 / s["n_valid_all"])
+                self._ws, F._ws = F._ws, None
+                old_probs, new = s["old"]["probs"], after["probs"]
+                t = old_probs * (old_probs.clamp_min(1e-38).log() - new.clamp_min(1e-38).log())
+                kl = float(torch.where(old_probs > 0, t, torch.zeros_like(t)).sum(-1).mean())
+                tolist = lambda xs: [float(x) for x in torch.cat(xs).cpu()] if xs else []  # noqa: E731
+                outs.append(dict(loss_before=float(s["old"]["loss"]), loss_after=float(after["loss"]), kl=kl,
+                                 entropy=float(after["entropy"].mean()), losses=tolist(s["losses"]), baseline_losses=tolist(s["bl"]),
+                                 grad_norms=tolist(s["gn"]), n_paths=s["P"]))
+        return outs
+
+
+class _SetBuckets:
+    """The flat buckets of K ``FlatAdam``s of one layout moved into ``[K][n]`` tensors (parameters, gradient, both moments):
+    every member's parameters, gradient views and ``FlatAdam`` tensors become views of row i.  ``step`` is ONE
+    ``cm_adam_step_set`` over the members that take a step."""
+
+    def __init__(self, opts):
+        K, o0 = len(opts), opts[0]
+        n = o0.flat.numel()
+        if any(o.flat.numel() != n for o in opts):
+            raise ValueError("the members' parameter buckets differ in size")
+        self.opts = opts
+        self.flat = torch.stack([o.flat for o in opts]).contiguous()
+        self.grad = torch.zeros_like(self.flat)
+        self.exp_avg = torch.stack([o.exp_avg for o in opts]).contiguous()
+        self.exp_avg_sq = torch.stack([o.exp_avg_sq for o in opts]).contiguous()
+        for i, o in enumerate(opts):
+            o.flat, o.grad, o.exp_avg, o.exp_avg_sq = self.flat[i], self.grad[i], self.exp_avg[i], self.exp_avg_sq[i]
+            k0 = 0
+            for p in o.params:
+                k = p.numel()
+                p.data = self.flat[i, k0:k0 + k].view_as(p)
+                p.grad = self.grad[i, k0:k0 + k].view_as(p)
+                k0 += k
+        self.lr, self.betas, self.eps = o0.lr, o0.betas, o0.eps
+
+    def clip_coefficient(self, max_norm):
+        """per member: min(1, max_norm / (||g_i|| + 1e-6)) and ||g_i|| as [K] device tensors"""
+        norm = self.grad.norm(2, dim=1)
+        return torch.clamp(max_norm / (norm + 1e-6), max=1.0), norm
+
+    def step(self, stepped, grad_scale):
+        """one Adam step of every member i with stepped[i] (its own step count), gradient scaled by grad_scale[i] (a [K] float32
+        device tensor); the other members stay bit for bit as they are"""
+        K, n = self.flat.shape
+        for o, s in zip(self.opts, stepped):
+            o.steps += int(bool(s))
+        steps = (C.c_int32 * K)(*[o.steps if s else 0 for o, s in zip(self.opts, stepped)])
+        self._scale = grad_scale.detach().to(torch.float32).reshape(K).contiguous()      # (kept alive until the next step)
+        with torch.cuda.device(self.flat.device):
+            N.check("cm_adam_step_set", N.lib().cm_adam_step_set(N.ptr(self.flat), N.ptr(self.grad), N.ptr(self.exp_avg),
+                                                                 N.ptr(self.exp_avg_sq), K, n, n, self.lr, self.betas[0], self.betas[1],
+                                                                 self.eps, steps, N.ptr(self._scale), N.stream_ptr()))
+        for o, s in zip(self.opts, stepped):
+            if s:
+                for p in o.params:
+                    torch.autograd.graph.increment_version(p)

@@ -109,9 +109,9 @@ class _FusedNets:
         return g
 
     # ---- one call ------------------------------------------------------------------------------------------------
-    def _workspace(self, desc, steps, backward):
+    def _workspace(self, desc, steps, backward, extra=0):
         chunk = min(max(int(steps), 1), self.chunk_steps)
-        need = N.lib().cm_ppo_net_workspace_floats(C.byref(desc), chunk, int(backward))
+        need = N.lib().cm_ppo_net_workspace_floats(C.byref(desc), chunk, int(backward)) + extra
         if self._ws is None or self._ws.numel() < need:
             self._ws = None
             self._ws = torch.empty(need, dtype=torch.float32, device=self.device)
@@ -250,3 +250,33 @@ class FusedCentNets(_FusedNets):
     def prepare(self, b):
         """flat (step-major) views of a padded [P, T, ...] batch, availability as bits (no masks)"""
         return self._prepare_common(b)
+
+
+class _SetBlobMap:
+    """K members' flat parameter rows ``flat [K][n]`` <-> K kernel blobs ``blob [K][stride]`` (stride = blob length rounded up to
+    4 floats, the row alignment cm_ppo_net asks of a set): the gather / inverse maps of ONE member (``_BlobMap``) with a row
+    offset per member, so that each direction is one index_select for all members.  Member i's single-network blob and
+    gradient are ``blob[i, :nb]`` / ``grad[i, :nb]``."""
+
+    def __init__(self, one, flat):
+        K, n = flat.shape
+        dev = flat.device
+        self.nb = nb = one.const.numel()
+        self.stride = stride = (nb + 3) // 4 * 4
+        pad = lambda t: torch.cat([t, torch.zeros(stride - nb, dtype=t.dtype, device=dev)])  # noqa: E731
+        rows = torch.arange(K, device=dev, dtype=torch.int64)[:, None]
+        self.const, self.mask = pad(one.const)[None, :].contiguous(), pad(one.mask)[None, :].contiguous()
+        self.gather = (pad(one.gather)[None, :] + rows * n).reshape(-1)
+        self.inverse = (one.inverse[None, :] + rows * stride).reshape(-1)
+        self.flat = flat
+        self.blob = torch.zeros((K, stride), dtype=torch.float32, device=dev)
+        self.grad = torch.zeros((K, stride), dtype=torch.float32, device=dev)
+
+    def refresh(self):
+        torch.index_select(self.flat.reshape(-1), 0, self.gather, out=self.blob.view(-1))
+        self.blob.mul_(self.mask).add_(self.const)
+        return self.blob
+
+    def scatter_grad(self, flat_grad):
+        """the gradient blobs -> flat_grad [K][n] (contiguous)"""
+        torch.index_select(self.grad.view(-1), 0, self.inverse, out=flat_grad.view(-1))

@@ -40,10 +40,11 @@ def make_policy(spec: ScenarioSpec, device="cuda", seed: Optional[int] = None, t
 class RolloutEngine:
     def __init__(self, spec: ScenarioSpec, policy: CommCategoricalMLPPolicy, n_envs: int, device="cuda", env_id0: int = 0,
                  ring: int = 8, record_attention: bool = False, greedy: bool = False, use_graph: bool = True,
-                 groups: int = 1, auto_reset: bool = True, conditions=None):
+                 groups: int = 1, auto_reset: bool = True, conditions=None, block_conditions: bool = False):
         """``conditions``: per-env channel conditions of the envs (BatchedEnv); the env groups may cut through them.
         ``policy``: one policy, or a PolicySet of P policies: the envs are then P equal blocks in policy-major order (block i runs
-        policy i and, with ``conditions``, is itself split into the conditions); the env groups may cut through the blocks."""
+        policy i and, with ``conditions``, is itself split into the conditions, or with ``block_conditions`` runs under
+        ``conditions[i]`` alone); the env groups may cut through the blocks."""
         self.spec, self.policy, self.B = spec, policy, int(n_envs)
         self.device = torch.device(device)
         self._set = isinstance(policy, PolicySet)
@@ -51,7 +52,7 @@ class RolloutEngine:
         if self.B % P:
             raise ValueError(f"n_envs = {n_envs} does not split into {P} equal policy blocks")
         self.env = BatchedEnv(spec, n_envs, device=device, env_id0=env_id0, auto_reset=auto_reset, conditions=conditions,
-                              policy_blocks=P)
+                              policy_blocks=P, block_conditions=block_conditions)
         # Env groups: the envs are independent, so G contiguous groups form G independent policy -> step -> policy ...
         # chains.  Each chain runs on its own stream (forked / joined inside the captured graph): there is no device-wide
         # barrier between a step of one group and the next step of another, so partially filled waves of one launch

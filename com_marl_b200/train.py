@@ -11,7 +11,8 @@ import torch
 import torch.distributed as dist
 
 from . import distributed as D
-from .ppo import CommBaseCritic, DevicePPO, GaussianMLPBaseline
+from .policy import PolicySet
+from .ppo import CommBaseCritic, DevicePPO, DevicePPOSet, GaussianMLPBaseline
 from .rollout import RolloutEngine, make_policy
 from .spaces import Box, Discrete, EnvSpec
 
@@ -69,31 +70,107 @@ class DeviceTrainer:
         (SuccessRate, Average*Count) come from the kernels' episode accounting over every episode that finished during the
         round; return columns from the padded batch like the reference (paths that finished inside the window).
         KLBefore (KL against the policy of the previous round) and GPUMemoryMax are not reproduced."""
-        rewards, mask = batch["rewards"], batch["mask"]
-        und = (rewards * mask).sum(1)
-        es = out["episode_stats"]
-        row = dict(Iteration=self.epoch - 1, NumTrajs=int(rewards.shape[0]) * self.spec.n_agents,
-                   AverageDiscountedReturn=float(batch["returns"][:, 0].double().mean()), AverageReturn=float(und.mean()),
-                   SuccessRate=es["SuccessRate"], AverageCaptureCount=es["AverageCaptureCount"],
-                   AverageStepCount=es["AverageStepCount"], AverageMovingCount=es["AverageMovingCount"],
-                   AveragePenaltyCount=es["AveragePenaltyCount"], AverageVariable=es["AverageVariable"], AverageVar2=es["AverageVar2"],
-                   StdReturn=float(und.std(unbiased=False)), MaxReturn=float(und.max()), MinReturn=float(und.min()),
-                   LossBefore=out["loss_before"], LossAfter=out["loss_after"], dLoss=out["loss_before"] - out["loss_after"],
-                   KL=out["kl"], Entropy=out["entropy"], GradNorm=float(np.mean(out["grad_norms"])) if out["grad_norms"] else 0.0,
-                   EpochTime=out["update_ms"] * 1e-3)
-        # AveDegree: mean over paths of the per-path mean degree (:316-318); Diameter / AveTroughput are constants of the scenario
-        t = self.engine.traj
-        row["AveDegree"] = float(t["ave_deg"][:self.engine.K].double().mean()) if self.spec.rcom != 0 else float(self.spec.n_agents)
-        row["Diameter"] = float(self.spec.n_agents if self.spec.rcom == 0 else 0)
-        row["AveTroughput"] = float(self.spec.ave_trput)
-        try:
-            from dowel import tabular as dt
-            for k, v in row.items():
-                dt.record(k, v)
-        except Exception:                      # dowel is optional here
-            pass
-        return row
+        return tabular_row(self.spec, self.epoch - 1, batch, out, self.engine.traj["ave_deg"][:self.engine.K])
 
     def weights_checksum(self):
         """float64 sum of every policy + critic parameter: equal on all ranks when the gradient all-reduce works"""
         return float(sum(p.detach().double().sum() for m in (self.policy, self.critic) for p in m.parameters()))
+
+
+def tabular_row(spec, iteration, batch, out, ave_deg):
+    """DeviceTrainer.tabular's row from a padded device batch, the round's output dict (episode_stats, losses, times) and the
+    [K, envs] per-step mean degrees of the round's envs; recorded in dowel's tabular when it is installed"""
+    rewards, mask = batch["rewards"], batch["mask"]
+    und = (rewards * mask).sum(1)
+    es = out["episode_stats"]
+    row = dict(Iteration=iteration, NumTrajs=int(rewards.shape[0]) * spec.n_agents,
+               AverageDiscountedReturn=float(batch["returns"][:, 0].double().mean()), AverageReturn=float(und.mean()),
+               SuccessRate=es["SuccessRate"], AverageCaptureCount=es["AverageCaptureCount"],
+               AverageStepCount=es["AverageStepCount"], AverageMovingCount=es["AverageMovingCount"],
+               AveragePenaltyCount=es["AveragePenaltyCount"], AverageVariable=es["AverageVariable"], AverageVar2=es["AverageVar2"],
+               StdReturn=float(und.std(unbiased=False)), MaxReturn=float(und.max()), MinReturn=float(und.min()),
+               LossBefore=out["loss_before"], LossAfter=out["loss_after"], dLoss=out["loss_before"] - out["loss_after"],
+               KL=out["kl"], Entropy=out["entropy"], GradNorm=float(np.mean(out["grad_norms"])) if out["grad_norms"] else 0.0,
+               EpochTime=out["update_ms"] * 1e-3)
+    # AveDegree: mean over paths of the per-path mean degree (:316-318); Diameter / AveTroughput are constants of the scenario
+    row["AveDegree"] = float(ave_deg.double().mean()) if spec.rcom != 0 else float(spec.n_agents)
+    row["Diameter"] = float(spec.n_agents if spec.rcom == 0 else 0)
+    row["AveTroughput"] = float(spec.ave_trput)
+    try:
+        from dowel import tabular as dt
+        for k, v in row.items():
+            dt.record(k, v)
+    except Exception:                      # dowel is optional here
+        pass
+    return row
+
+
+class DeviceTrainerSet:
+    """K training runs of one scenario and architecture as ONE batched run — the seeds x channel conditions grids of the paper's
+    experiments.  Member i is ``DeviceTrainer(conditions[i] or spec, n_envs, env_id0=env_id0 + i * n_envs, seed=seeds[i],
+    kind=kind, **ppo_args)`` started from member i's initial policy and critic: global env ids i E .. (i + 1) E - 1, its own
+    channel condition, path permutation ``default_rng([seeds[i], epoch])`` and initial weights drawn under
+    ``torch_seed=seeds[i]``.  One RolloutEngine over a PolicySet rolls out all K E envs; one DevicePPOSet updates all members.
+    Comm-DP and Obs-DP ('comm', 'dec') on one rank; 'cent' and multi-rank sets raise."""
+
+    def __init__(self, spec, n_envs, seeds, conditions=None, kind="comm", device="cuda", env_id0=0, groups=1, **ppo_args):
+        if kind == "cent":
+            raise NotImplementedError("DeviceTrainerSet covers the Comm-DP and Obs-DP families: CENT sets are not built")
+        if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
+            raise NotImplementedError("DeviceTrainerSet runs on one rank: sets across ranks are not built")
+        self.seeds = [int(s) for s in seeds]
+        K = len(self.seeds)
+        if K < 1:
+            raise ValueError("a DeviceTrainerSet needs at least one seed")
+        conditions = [None] * K if conditions is None else list(conditions)
+        if len(conditions) != K:
+            raise ValueError(f"{len(conditions)} conditions for {K} members")
+        self.spec, self.device, self.E, self.K = spec, torch.device(device), int(n_envs), K
+        spec.max_path_length = spec.max_steps
+        self.specs = []
+        for c in conditions:
+            m = spec if c is None else c
+            m.max_path_length = spec.max_steps
+            self.specs.append(m)
+        n, Dobs = spec.n_agents, spec.obs_dim
+        env_spec = EnvSpec(Box(np.zeros(n * Dobs), np.ones(n * Dobs)), Discrete(5))
+        self.policies, self.critics = [], []
+        for s in self.seeds:                   # the critic right after its policy, from the same generator state
+            self.policies.append(make_policy(spec, device=self.device, kind=kind, torch_seed=s))
+            self.critics.append(CommBaseCritic(env_spec, n, n_gcn_layers=spec.n_layers, device=self.device))
+        self.algo = DevicePPOSet(self.policies, self.critics, **ppo_args)
+        self.pset = PolicySet(self.policies)
+        conds = None if all(c is None for c in conditions) else self.specs
+        self.engine = RolloutEngine(spec, self.pset, K * self.E, device=self.device, env_id0=env_id0, ring=spec.max_steps,
+                                    use_graph=True, groups=groups, conditions=conds, block_conditions=conds is not None)
+        self.epoch = 0
+
+    def member_traj(self, i):
+        """member i's env columns of the trajectory ring (views)"""
+        return {k: v[:, i * self.E:(i + 1) * self.E] for k, v in self.engine.traj.items()}
+
+    def train_epoch(self):
+        """one round of every member; returns one dict per member with the keys of DeviceTrainer.train_epoch (times: the set's)"""
+        ev = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
+        ev[0].record()
+        self.engine.reset()
+        self.engine.run_chunk()
+        ev[1].record()
+        batches = [m.batch_from_trajectory(self.member_traj(i)) for i, m in enumerate(self.algo.members)]
+        self.batches = batches                 # (the round's padded batches, kept until the next round)
+        ev[2].record()
+        perms = [np.random.default_rng([s, self.epoch]).permutation(int(b["rewards"].shape[0])) for s, b in zip(self.seeds, batches)]
+        outs = self.algo.train_once(batches, perms)
+        ev[3].record()
+        torch.cuda.synchronize(self.device)
+        self.engine.env.check_errors()
+        self.epoch += 1
+        times = dict(rollout_ms=ev[0].elapsed_time(ev[1]), batch_ms=ev[1].elapsed_time(ev[2]), update_ms=ev[2].elapsed_time(ev[3]))
+        Kr = self.engine.K
+        for i, (out, b) in enumerate(zip(outs, batches)):
+            stats = self.engine.env.stats[i * self.E:(i + 1) * self.E, 7:16].sum(dim=0).reshape(1, -1)
+            out.update(times, agent_steps=Kr * self.E * self.spec.n_agents,
+                       episode_stats=D.summarize_stats(stats, self.spec.scenario, self.spec.n_agents))
+            out["tabular"] = tabular_row(self.specs[i], self.epoch - 1, b, out,
+                                         self.engine.traj["ave_deg"][:Kr, i * self.E:(i + 1) * self.E])
+        return outs

@@ -46,9 +46,10 @@
 extern "C" {
 #endif
 
-#define CM_ABI_VERSION 6   /* 2: host_arena / obs_bits members, cm_rollout_step_host; 3: cm_ppo_net; 4: CENT kinds of cm_ppo_net,
+#define CM_ABI_VERSION 7   /* 2: host_arena / obs_bits members, cm_rollout_step_host; 3: cm_ppo_net; 4: CENT kinds of cm_ppo_net,
                               cm_net_desc.flags; 5: cm_channel_cond, per-env channel conditions (cm_env_desc.conds ...);
-                              6: several policies in one cm_policy_forward (cm_policy_io.n_policies ...) */
+                              6: several policies in one cm_policy_forward (cm_policy_io.n_policies ...);
+                              7: several networks in one cm_ppo_net (cm_net_io.n_policies ...), cm_adam_step_set */
 #define CM_MAX_AGENTS 256   /* n, p */
 #define CM_MAX_GRID 64      /* grid side incl. Coverage's wall border */
 #define CM_MAX_LAYERS 4     /* n_gcn_layers */
@@ -339,6 +340,14 @@ int cm_adam_step(float *params, const float *grads, float *exp_avg, float *exp_a
  * no host round trip between the backward pass and the optimizer step) */
 int cm_adam_step_dev(float *params, const float *grads, float *exp_avg, float *exp_avg_sq, int64_t n, float lr, float beta1,
                      float beta2, float eps, int32_t step, const float *grad_scale_dev, cm_stream_t stream);
+/* cm_adam_step_dev over a set of n_policies buckets in ONE launch: member i's n floats start at params / grads / exp_avg / exp_avg_sq
+ * + i * stride (stride >= n floats).  steps: HOST [n_policies] step numbers (read at call time; the bias corrections are formed on
+ * the host in double like cm_adam_step's); grad_scale_dev: DEVICE [n_policies] clip coefficients.  A member whose step number is 0
+ * is not stepped: its parameters and moments stay bit for bit as they are.  Every stepped member's result is bit-identical to
+ * cm_adam_step_dev on its row. */
+int cm_adam_step_set(float *params, const float *grads, float *exp_avg, float *exp_avg_sq, int32_t n_policies, int64_t n,
+                     int64_t stride, float lr, float beta1, float beta2, float eps, const int32_t *steps, const float *grad_scale_dev,
+                     cm_stream_t stream);
 
 /* ---- PPO update: hand-written forward + backward of the comm-GNN (csrc/ppo_net_kernels.cu) -----------------------------
  * cm_ppo_net runs ONE network over n_steps env steps of n agents each — the flattened (path, t) pairs of a minibatch of
@@ -394,15 +403,29 @@ typedef struct cm_net_io {
     const int64_t *actions;    /* policy: [S][n] */
     const float *adv;          /* policy: [S] advantages; NULL = no objective (forward only) */
     const float *old_ll;       /* policy: [S] log-likelihood under the frozen old policy; NULL = ratio 1 */
-    const uint8_t *valid;      /* policy: [S] 0 = padded step (no contribution), or NULL = all valid */
+    const uint8_t *valid;      /* [S] 0 = padded step (no contribution), or NULL = all valid; the critic reads it since ABI 7 */
     const float *returns;      /* critic: [S] */
     float inv_count;           /* 1 / (number of steps the mean of the loss runs over) */
     float *ll, *entropy;       /* policy outputs [S], optional */
     float *probs;              /* policy output [S][n][5], optional */
     float *values;             /* critic output [S], optional */
-    float *loss;               /* DEVICE f32[1], optional: the loss (summed in float64 over the call) is ADDED to it */
+    float *loss;               /* DEVICE f32[1] (a set: [n_policies]), optional: the loss (summed in float64 over the call) is ADDED to it */
     float *workspace;
     size_t workspace_floats;
+    /* Several networks of one kind and architecture in one call (ABI 7; 0 or 1 = one network, the members below are not read).  The
+     * n_steps steps are n_policies contiguous blocks of steps_per_policy steps; step s runs the network whose blob starts at
+     * weights + (s / steps_per_policy) * weights_stride, its gradient is ADDED at grad + (s / steps_per_policy) * grad_stride, its loss
+     * is added to loss[s / steps_per_policy] (float64 sum per member) and inv_counts[s / steps_per_policy] replaces inv_count.  Every
+     * kernel counts its tiles and env blocks per member, so no tile holds rows of two members; members of equal length are padded
+     * with valid = 0 steps holding finite data (the critic reads `valid` too: such a step writes its value and adds nothing).  Needs
+     * n_steps == n_policies * steps_per_policy, strides of at least the blob length and a multiple of 4 floats, and inv_counts when
+     * a loss or gradient is asked for; else CM_EINVAL.  The workspace needs ((2 * n_policies + 3) & ~3) - 4 floats more than
+     * cm_ppo_net_workspace_floats gives, for the per-member float64 loss sums.  CM_NET_POLICY_CENT / CM_NET_BASELINE_MLP:
+     * CM_EUNSUPPORTED. */
+    int32_t n_policies;
+    int64_t steps_per_policy;
+    int64_t weights_stride, grad_stride;   /* floats */
+    const float *inv_counts;   /* DEVICE [n_policies] */
 } cm_net_io;
 size_t cm_critic_blob_floats(int32_t obs_dim, int32_t n_layers);
 size_t cm_baseline_mlp_blob_floats(int32_t in_dim);
