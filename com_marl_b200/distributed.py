@@ -3,10 +3,12 @@
 Env instances are independent (SURVEY.md §8e), so each rank steps its own slice; the RNG streams are keyed
 by GLOBAL env id, which makes results independent of the sharding.  The only exchange is the all-gather of
 the per-rank episode-statistics vector once per obtain_samples (NCCL over NVLink on GPUs; gloo in the CPU
-tests) — a few dozen bytes, latency bound.
+tests) — a few dozen bytes, latency bound.  Grids of runs (DeviceTrainerSet, eval_policies) shard whole members the same
+way (member_range) and gather their results once per round (gather_objects).
 """
+import hashlib
 import os
-from typing import Dict, Tuple
+from typing import Dict, List, Tuple
 
 import torch
 import torch.distributed as dist
@@ -19,6 +21,49 @@ def shard_range(n_envs_total: int, rank: int, world: int) -> Tuple[int, int]:
     base, rem = divmod(int(n_envs_total), int(world))
     lo = rank * base + min(rank, rem)
     return lo, lo + base + (1 if rank < rem else 0)
+
+
+def member_range(n_members: int, rank: int, world: int) -> Tuple[int, int]:
+    """Contiguous global member ids [lo, hi) of a training or evaluation grid that `rank` owns (shard_range's rule: sizes
+    differ by at most one).  A member's random streams are keyed by its global env ids, seed and condition, so it computes
+    the same thing whichever rank runs it."""
+    return shard_range(n_members, rank, world)
+
+
+def group_rank_world(group=None) -> Tuple[int, int]:
+    """(rank, world) of this process in `group` (the default group when None); (0, 1) without torch.distributed"""
+    if not (dist.is_available() and dist.is_initialized()):
+        return 0, 1
+    return dist.get_rank(group), dist.get_world_size(group)
+
+
+def gather_objects(obj, group=None) -> List:
+    """all-gather of one picklable object per rank -> [object of rank 0, object of rank 1, ...] on every rank
+    (dist.all_gather_object; under NCCL the current device must be the rank's GPU, which init_from_env sets).  [obj]
+    without a process group or with a group of one rank."""
+    rank, world = group_rank_world(group)
+    if world == 1:
+        return [obj]
+    out = [None] * world
+    dist.all_gather_object(out, obj, group=group)
+    return out
+
+
+def rank_alone_group():
+    """A process group holding this rank alone: what a rank's own members hand to the collectives of DevicePPO (its
+    global_max / gradient all-reduce) so that they stay on this rank when a process group of several ranks exists.  Only
+    this rank takes part in creating it."""
+    return dist.new_group([dist.get_rank()], use_local_synchronization=True)
+
+
+def check_same_on_all_ranks(what: str, value, group=None) -> None:
+    """ValueError on EVERY rank when `value` (its repr, hashed) differs between the ranks of `group`: one gather of a digest,
+    so that a rank given other arguments fails together with the others instead of leaving them waiting in a collective"""
+    digest = hashlib.sha256(repr(value).encode()).hexdigest()
+    got = gather_objects(digest, group)
+    bad = [r for r, d in enumerate(got) if d != got[0]]
+    if bad:
+        raise ValueError(f"{what} differ between the ranks: rank(s) {bad} disagree with rank 0")
 
 
 def init_from_env(backend: str = None) -> Tuple[int, int, int]:

@@ -15,6 +15,7 @@ from typing import Dict, List, Tuple
 import numpy as np
 import torch
 
+from . import distributed as D
 from .policy import PolicySet
 from .rollout import RolloutEngine
 
@@ -61,18 +62,39 @@ def eval_sweep(env, policy, conditions, n_eval_episodes=100, max_env_steps=200, 
 
 
 def eval_policies(env, policies, conditions=None, n_eval_episodes=100, max_env_steps=200, eval_greedy=True, seed=1,
-                  groups: int = 4, chunk: int = 50, return_trajectory: bool = False):
+                  groups: int = 4, chunk: int = 50, return_trajectory: bool = False, group=None):
     """``eval_model`` / ``eval_sweep`` of many policies of one class and architecture (every checkpoint of a run, the seeds
     of a configuration) in ONE engine, one policy launch per step for all of them.  ``policies``: a list or a PolicySet.
     With C conditions (C = 1 and ``env``'s own channel when ``conditions`` is None) policy i under condition k plays its
     ``n_eval_episodes`` episodes in the envs with global ids ``(i C + k) n_eval_episodes ...``, so ``results[i][k]`` equals
-    ``eval_model(conditions[k], policies[i], ..., env_id0=(i C + k) n_eval_episodes)``."""
-    pset = policies if isinstance(policies, PolicySet) else PolicySet(policies)
+    ``eval_model(conditions[k], policies[i], ..., env_id0=(i C + k) n_eval_episodes)``.
+
+    Across ranks (``group``, by default torch.distributed's default group when it is initialized): every rank passes all K
+    policies and evaluates policies ``distributed.member_range(K, rank, world)`` in one engine of its own (the others are not
+    touched); the ranks exchange the recorded per-step columns once, and every rank returns all K results, equal bit for bit
+    to the single-rank call."""
+    pols = policies.policies if isinstance(policies, PolicySet) else list(policies)
     spec = _eval_spec(getattr(env, "spec_b200", env), seed)
     conds = [_eval_spec(c, seed) for c in conditions] if conditions is not None else None
-    res = _evaluate(spec, conds, pset, int(n_eval_episodes), max_env_steps, eval_greedy, groups, chunk, return_trajectory, 0)
     C = len(conds) if conds else 1
-    return [res[i * C:(i + 1) * C] for i in range(len(pset))]
+    rank, world = D.group_rank_world(group)
+    if world == 1:
+        pset = policies if isinstance(policies, PolicySet) else PolicySet(pols)
+        res = _evaluate(spec, conds, pset, int(n_eval_episodes), max_env_steps, eval_greedy, groups, chunk, return_trajectory, 0)
+        return [res[i * C:(i + 1) * C] for i in range(len(pset))]
+    E = int(n_eval_episodes)
+    lo, hi = D.member_range(len(pols), rank, world)
+    mine = None                                        # (columns, lengths) of this rank's hi - lo policies x C conditions
+    if hi > lo:
+        mine = _record(spec, conds, PolicySet(pols[lo:hi]), E, max_env_steps, eval_greedy, groups, chunk, return_trajectory,
+                       lo * C * E, longest=lambda steps: _longest(steps, group))
+    else:                                              # no policy here: still takes part in the step count's gather
+        _longest(0, group)
+    parts = [p for p in D.gather_objects(mine, group) if p is not None]
+    cat = {k: np.concatenate([p[0][k] for p in parts], axis=1) for k in parts[0][0]}
+    length = np.concatenate([p[1] for p in parts])
+    res = _columns_results(conds or [spec], len(pols), cat, length, E, return_trajectory)
+    return [res[i * C:(i + 1) * C] for i in range(len(pols))]
 
 
 def _eval_spec(spec, seed):
@@ -85,6 +107,15 @@ def _eval_spec(spec, seed):
 def _evaluate(spec, conditions, policy, E, max_env_steps, eval_greedy, groups, chunk, return_trajectory, env_id0):
     """the eval loop of eval_model / eval_sweep / eval_policies: E episodes per (policy, condition) (one condition: ``spec``'s own
     channel) in one RolloutEngine; -> one eval_model result per (policy, condition), policy-major"""
+    cat, length = _record(spec, conditions, policy, E, max_env_steps, eval_greedy, groups, chunk, return_trajectory, env_id0)
+    return _columns_results(conditions or [spec], len(policy) if isinstance(policy, PolicySet) else 1, cat, length, E,
+                            return_trajectory)
+
+
+def _record(spec, conditions, policy, E, max_env_steps, eval_greedy, groups, chunk, return_trajectory, env_id0, longest=None):
+    """run the eval loop -> (recorded per-step columns {key: [steps, envs, ...]}, episode lengths [envs]).  ``longest`` (a
+    rank's share of eval_policies across ranks: this rank's step count -> the largest of the ranks') makes the loop run on to
+    the step count of the rank that ran longest, so that the recorded columns have the rows of the single-rank loop"""
     conds = (conditions or [spec]) * (len(policy) if isinstance(policy, PolicySet) else 1)
     B = E * len(conds)
     K = max(1, min(int(chunk), int(max_env_steps)))
@@ -94,7 +125,8 @@ def _evaluate(spec, conditions, policy, E, max_env_steps, eval_greedy, groups, c
     length = np.zeros(B, dtype=np.int64)              # 0 = still running
     keep = {k: [] for k in ("reward", "done", "counts", "ave_deg", "success", "actions")}
     steps = 0
-    while steps < max_env_steps and (length == 0).any():
+
+    def record_chunk(steps):
         eng.run_chunk()
         t = eng.traj
         m = min(K, max_env_steps - steps)
@@ -110,11 +142,28 @@ def _evaluate(spec, conditions, policy, E, max_env_steps, eval_greedy, groups, c
             hit = np.nonzero(d[:, b])[0]
             if hit.size:
                 length[b] = steps + int(hit[0]) + 1
-        steps += m
+        return steps + m
+
+    while steps < max_env_steps and (length == 0).any():
+        steps = record_chunk(steps)
+    if longest is not None:                            # this rank's envs are done (or cut): on to the longest rank's count
+        until = longest(steps)
+        while steps < until:
+            steps = record_chunk(steps)
     eng.env.check_errors()
     policy.check_errors()
     length[length == 0] = steps                          # cut by max_env_steps (eval_pp.py:71)
-    cat = {k: np.concatenate(v) for k, v in keep.items() if v}
+    return {k: np.concatenate(v) for k, v in keep.items() if v}, length
+
+
+def _longest(steps, group):
+    """the largest step count of the ranks' eval loops"""
+    return max(D.gather_objects(int(steps), group))
+
+
+def _columns_results(conds, n_policies, cat, length, E, return_trajectory):
+    """one eval_model result per (policy, condition), policy-major, from the recorded columns of all their envs"""
+    conds = list(conds) * n_policies
     return [_results(c, {k: v[:, i * E:(i + 1) * E] for k, v in cat.items()}, length[i * E:(i + 1) * E], return_trajectory)
             for i, c in enumerate(conds)]
 

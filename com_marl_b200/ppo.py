@@ -696,7 +696,7 @@ class DevicePPOSet:
                 self._ws, F._ws = F._ws, None
                 ids_all = np.random.permutation(P) if shuffled_ids[i] is None else np.asarray(shuffled_ids[i])
                 mbs = []
-                for start, stop in minibatch_plan(P, self.n_minibatches):
+                for start, stop in minibatch_plan(P, self.n_minibatches, group=m.group):   # (a member's group: its rank alone)
                     ids = ids_all[start:stop]
                     idx_all, idx = F.step_index(f, ids, valid_only=False), F.step_index(f, ids, valid_only=True)
                     adv = raw_adv.index_select(0, idx)

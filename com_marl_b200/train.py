@@ -5,10 +5,10 @@ every env into its device trajectory ring, ``DevicePPO.batch_from_trajectory`` p
 updates policy and critic.  One process per GPU; every rank rolls out its own slice of the global env ids and the flat
 gradient buckets are all-reduced inside the update (NCCL), so all ranks hold identical weights after every step."""
 import time
+from dataclasses import fields
 
 import numpy as np
 import torch
-import torch.distributed as dist
 
 from . import distributed as D
 from .policy import PolicySet
@@ -77,9 +77,9 @@ class DeviceTrainer:
         return float(sum(p.detach().double().sum() for m in (self.policy, self.critic) for p in m.parameters()))
 
 
-def tabular_row(spec, iteration, batch, out, ave_deg):
+def tabular_row(spec, iteration, batch, out, ave_deg, record=True):
     """DeviceTrainer.tabular's row from a padded device batch, the round's output dict (episode_stats, losses, times) and the
-    [K, envs] per-step mean degrees of the round's envs; recorded in dowel's tabular when it is installed"""
+    [K, envs] per-step mean degrees of the round's envs; recorded in dowel's tabular when it is installed and ``record``"""
     rewards, mask = batch["rewards"], batch["mask"]
     und = (rewards * mask).sum(1)
     es = out["episode_stats"]
@@ -96,13 +96,39 @@ def tabular_row(spec, iteration, batch, out, ave_deg):
     row["AveDegree"] = float(ave_deg.double().mean()) if spec.rcom != 0 else float(spec.n_agents)
     row["Diameter"] = float(spec.n_agents if spec.rcom == 0 else 0)
     row["AveTroughput"] = float(spec.ave_trput)
+    if record:
+        record_tabular(row)
+    return row
+
+
+def record_tabular(row):
+    """a tabular row into dowel's tabular, when dowel is installed"""
     try:
         from dowel import tabular as dt
         for k, v in row.items():
             dt.record(k, v)
     except Exception:                      # dowel is optional here
         pass
-    return row
+
+
+class _Owned(list):
+    """the per-member objects of the members a rank owns (DeviceTrainerSet across ranks), indexed by GLOBAL member id;
+    iteration yields them in member order.  A member another rank owns raises KeyError."""
+
+    def __init__(self, items, members):
+        super().__init__(items)
+        self.members = members
+
+    def __getitem__(self, i):
+        if isinstance(i, slice) or i not in self.members:
+            raise KeyError(f"member {i!r}: this rank owns members {self.members.start} .. {self.members.stop - 1}")
+        return list.__getitem__(self, i - self.members.start)
+
+
+def _spec_key(spec):
+    """what identifies a scenario / channel condition (every field but the ones DeviceTrainerSet sets and the derived map)"""
+    return None if spec is None else tuple((f.name, getattr(spec, f.name)) for f in fields(spec)
+                                           if f.name not in ("max_path_length", "wall"))
 
 
 class DeviceTrainerSet:
@@ -110,22 +136,43 @@ class DeviceTrainerSet:
     experiments.  Member i is ``DeviceTrainer(conditions[i] or spec, n_envs, env_id0=env_id0 + i * n_envs, seed=seeds[i],
     kind=kind, **ppo_args)`` started from member i's initial policy and critic: global env ids i E .. (i + 1) E - 1, its own
     channel condition, path permutation ``default_rng([seeds[i], epoch])`` and initial weights drawn under
-    ``torch_seed=seeds[i]``.  One RolloutEngine over a PolicySet rolls out all K E envs; one DevicePPOSet updates all members.
-    Comm-DP and Obs-DP ('comm', 'dec') on one rank; 'cent' and multi-rank sets raise."""
+    ``torch_seed=seeds[i]``.  One RolloutEngine over a PolicySet rolls out the envs of the members; one DevicePPOSet updates
+    them.  Comm-DP and Obs-DP ('comm', 'dec'); 'cent' raises.
 
-    def __init__(self, spec, n_envs, seeds, conditions=None, kind="comm", device="cuda", env_id0=0, groups=1, **ppo_args):
+    Across ranks (``group``, by default torch.distributed's default group when it is initialized): every rank is given the
+    same seeds and conditions and runs the members ``distributed.member_range(K, rank, world)`` — ``members`` — with their
+    own engine and update; nothing is exchanged on the data path, since a member computes the same thing on any rank.
+    ``train_epoch`` gathers the K result dicts to every rank, ``policy_state_dicts`` the K trained policies.  ``policies``,
+    ``critics``, ``batches`` and ``member_traj`` hold this rank's members, indexed by global member id (on one rank: plain
+    lists of all K)."""
+
+    def __init__(self, spec, n_envs, seeds, conditions=None, kind="comm", device="cuda", env_id0=0, groups=1, group=None,
+                 **ppo_args):
+        self.group = group
+        self.rank, self.world = D.group_rank_world(group)
+        data_parallel = ppo_args.get("process_group") is not None
+        if self.world > 1:                     # first, so that every later error is raised by every rank alike
+            conds = None if conditions is None else [_spec_key(c) for c in conditions]
+            ppo = sorted((k, v) for k, v in ppo_args.items() if k != "process_group")    # (a group handle: only whether given)
+            D.check_same_on_all_ranks("DeviceTrainerSet arguments (seeds, conditions, n_envs, kind, env_id0, spec, PPO arguments)",
+                                      ([int(s) for s in seeds], conds, int(n_envs), kind, int(env_id0), _spec_key(spec), ppo,
+                                       data_parallel), group)
         if kind == "cent":
             raise NotImplementedError("DeviceTrainerSet covers the Comm-DP and Obs-DP families: CENT sets are not built")
-        if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
-            raise NotImplementedError("DeviceTrainerSet runs on one rank: sets across ranks are not built")
+        if self.world > 1 and data_parallel:
+            raise NotImplementedError("a DeviceTrainerSet member runs on one rank: members data-parallel over ranks are not built")
         self.seeds = [int(s) for s in seeds]
         K = len(self.seeds)
         if K < 1:
             raise ValueError("a DeviceTrainerSet needs at least one seed")
+        if K < self.world:
+            raise ValueError(f"{K} members over {self.world} ranks: every rank needs at least one member")
         conditions = [None] * K if conditions is None else list(conditions)
         if len(conditions) != K:
             raise ValueError(f"{len(conditions)} conditions for {K} members")
         self.spec, self.device, self.E, self.K = spec, torch.device(device), int(n_envs), K
+        lo, hi = D.member_range(K, self.rank, self.world)
+        self.members = range(lo, hi)
         spec.max_path_length = spec.max_steps
         self.specs = []
         for c in conditions:
@@ -134,32 +181,51 @@ class DeviceTrainerSet:
             self.specs.append(m)
         n, Dobs = spec.n_agents, spec.obs_dim
         env_spec = EnvSpec(Box(np.zeros(n * Dobs), np.ones(n * Dobs)), Discrete(5))
-        self.policies, self.critics = [], []
-        for s in self.seeds:                   # the critic right after its policy, from the same generator state
-            self.policies.append(make_policy(spec, device=self.device, kind=kind, torch_seed=s))
-            self.critics.append(CommBaseCritic(env_spec, n, n_gcn_layers=spec.n_layers, device=self.device))
-        self.algo = DevicePPOSet(self.policies, self.critics, **ppo_args)
-        self.pset = PolicySet(self.policies)
-        conds = None if all(c is None for c in conditions) else self.specs
-        self.engine = RolloutEngine(spec, self.pset, K * self.E, device=self.device, env_id0=env_id0, ring=spec.max_steps,
-                                    use_graph=True, groups=groups, conditions=conds, block_conditions=conds is not None)
+        policies, critics = [], []
+        for s in self.seeds[lo:hi]:            # the critic right after its policy, from the same generator state
+            policies.append(make_policy(spec, device=self.device, kind=kind, torch_seed=s))
+            critics.append(CommBaseCritic(env_spec, n, n_gcn_layers=spec.n_layers, device=self.device))
+        self.policies, self.critics = self._owned(policies), self._owned(critics)
+        if D.group_rank_world()[1] > 1 and not data_parallel:
+            # a job of several ranks (whether or not this set spans them): the members' own collectives (padded lengths,
+            # minibatch plan) stay on this rank
+            ppo_args = dict(ppo_args, process_group=D.rank_alone_group())
+        self.algo = DevicePPOSet(policies, critics, **ppo_args)
+        self.pset = PolicySet(policies)
+        conds = None if all(c is None for c in conditions[lo:hi]) else self.specs[lo:hi]
+        self.engine = RolloutEngine(spec, self.pset, (hi - lo) * self.E, device=self.device, env_id0=env_id0 + lo * self.E,
+                                    ring=spec.max_steps, use_graph=True, groups=groups, conditions=conds,
+                                    block_conditions=conds is not None)
         self.epoch = 0
 
+    def _owned(self, items):
+        return list(items) if self.world == 1 else _Owned(items, self.members)
+
+    def _column(self, i):
+        """first env column of member i in this rank's engine"""
+        if i not in self.members:
+            raise KeyError(f"member {i!r}: this rank owns members {self.members.start} .. {self.members.stop - 1}")
+        return (i - self.members.start) * self.E
+
     def member_traj(self, i):
-        """member i's env columns of the trajectory ring (views)"""
-        return {k: v[:, i * self.E:(i + 1) * self.E] for k, v in self.engine.traj.items()}
+        """member i's env columns of the trajectory ring (views); i is a global member id this rank owns"""
+        b = self._column(i)
+        return {k: v[:, b:b + self.E] for k, v in self.engine.traj.items()}
 
     def train_epoch(self):
-        """one round of every member; returns one dict per member with the keys of DeviceTrainer.train_epoch (times: the set's)"""
+        """one round of every member; returns one dict per member, all K in member order on every rank, with the keys of
+        DeviceTrainer.train_epoch (times: those of the set on the rank that ran the member) and ``rank``.  The members' tabular
+        rows are recorded in dowel on rank 0."""
         ev = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
         ev[0].record()
         self.engine.reset()
         self.engine.run_chunk()
         ev[1].record()
-        batches = [m.batch_from_trajectory(self.member_traj(i)) for i, m in enumerate(self.algo.members)]
-        self.batches = batches                 # (the round's padded batches, kept until the next round)
+        batches = [m.batch_from_trajectory(self.member_traj(i)) for i, m in zip(self.members, self.algo.members)]
+        self.batches = self._owned(batches)    # (the round's padded batches, kept until the next round)
         ev[2].record()
-        perms = [np.random.default_rng([s, self.epoch]).permutation(int(b["rewards"].shape[0])) for s, b in zip(self.seeds, batches)]
+        perms = [np.random.default_rng([self.seeds[i], self.epoch]).permutation(int(b["rewards"].shape[0]))
+                 for i, b in zip(self.members, batches)]
         outs = self.algo.train_once(batches, perms)
         ev[3].record()
         torch.cuda.synchronize(self.device)
@@ -167,10 +233,22 @@ class DeviceTrainerSet:
         self.epoch += 1
         times = dict(rollout_ms=ev[0].elapsed_time(ev[1]), batch_ms=ev[1].elapsed_time(ev[2]), update_ms=ev[2].elapsed_time(ev[3]))
         Kr = self.engine.K
-        for i, (out, b) in enumerate(zip(outs, batches)):
-            stats = self.engine.env.stats[i * self.E:(i + 1) * self.E, 7:16].sum(dim=0).reshape(1, -1)
-            out.update(times, agent_steps=Kr * self.E * self.spec.n_agents,
+        for i, out, b in zip(self.members, outs, batches):
+            b0 = self._column(i)
+            stats = self.engine.env.stats[b0:b0 + self.E, 7:16].sum(dim=0).reshape(1, -1)
+            out.update(times, agent_steps=Kr * self.E * self.spec.n_agents, rank=self.rank,
                        episode_stats=D.summarize_stats(stats, self.spec.scenario, self.spec.n_agents))
-            out["tabular"] = tabular_row(self.specs[i], self.epoch - 1, b, out,
-                                         self.engine.traj["ave_deg"][:Kr, i * self.E:(i + 1) * self.E])
+            out["tabular"] = tabular_row(self.specs[i], self.epoch - 1, b, out, self.engine.traj["ave_deg"][:Kr, b0:b0 + self.E],
+                                         record=False)
+        if self.world > 1:
+            outs = [o for part in D.gather_objects(outs, self.group) for o in part]
+        if self.rank == 0:
+            for o in outs:
+                record_tabular(o["tabular"])
         return outs
+
+    def policy_state_dicts(self):
+        """every member's policy parameters as K CPU state dicts in member order, on every rank (one gather across ranks):
+        what ``checkpoint.save_state_dict`` / ``load_state_dict`` and ``evaluate.eval_policies`` take"""
+        mine = [{k: v.detach().cpu() for k, v in p.state_dict().items()} for p in self.policies]
+        return [sd for part in D.gather_objects(mine, self.group) for sd in part]
