@@ -16,7 +16,7 @@ CH_FC, CH_FL, CH_IID, CH_GE = 0, 1, 2, 3
 POLICY_COMM, POLICY_DEC, POLICY_CENT = 0, 1, 2
 POLICY_FLAG_RELU = 1
 MAX_AGENTS, MAX_GRID, MAX_LAYERS = 256, 64, 4
-ABI_VERSION = 7
+ABI_VERSION = 8
 MAX_CONDS = 256
 
 EXPORTS = ("cm_abi_version", "cm_strerror", "cm_last_cuda_error", "cm_device_count", "cm_env_reset", "cm_env_step",

@@ -5,7 +5,7 @@ import sys
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(_HERE)
-SOURCES = ["env_kernels.cu", "policy_kernel.cu", "policy_tc_kernel.cu", "policy_attn_kernel.cu", "policy_attn_mma_kernel.cu", "policy_cent_kernel.cu", "host_abi.cu", "ppo_kernels.cu", "ppo_net_kernels.cu", "abi.cu"]
+SOURCES = ["env_kernels.cu", "policy_forward.cu", "policy_tc_kernel.cu", "policy_attn_mma_kernel.cu", "policy_cent_kernel.cu", "host_abi.cu", "ppo_kernels.cu", "ppo_net_kernels.cu", "abi.cu"]
 OUT = os.path.join(_HERE, "lib", "libcommarl_b200.so")
 
 

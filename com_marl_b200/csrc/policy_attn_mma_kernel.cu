@@ -1,13 +1,18 @@
 // policy_attn_mma_kernel.cu — attention + graph convolutions for large teams (64 < n <= 256) on the warp-level tensor
-// path (mma.sync.m16n8k16, SASS HMMA): same stage of the large-team pipeline and same interface as policy_attn_kernel.cu
-// (which stays as the exact-fp32 cross-check, cm_policy_desc.math = 2).
+// path (mma.sync.m16n8k16, SASS HMMA), the middle stage of the large-team pipeline (launch_policy_tc_large at the end of
+// this file):
+//   1. policy_tc_kernel<mode Enc> : obs rows -> E, Q = E Wa^T, H_0 Wg_0          (rows of 64 floats in io.workspace)
+//   2. policy_attn_mma_kernel     : per env  M = softmax_j(Q E^T),  A_l = M * Range * chan_l / (sum + 1e-12),
+//                                   H_{l+1} = tanh(A_l (H_l Wg_l) + bg_l),  X = E + H_L         (comm_base_net.py:80-108,
+//                                   attention_module.py:38-49, graph_conv_module.py:51-72)
+//   3. policy_tc_kernel<mode Head>: X rows -> logits / probs / actions
 //
 // Why mma.sync here and not tcgen05: the unit of work is a 16-row x n-key strip of ONE environment whose softmax, masking
 // and re-normalisation sit between the two products; with mma.sync the strip never leaves the warp's registers — the score
 // accumulators ARE the A operand of the aggregation (the C fragment of two adjacent 8-key tiles is exactly the A fragment of
 // a 16-key slice) — and there is no CTA-wide barrier, TMEM hand-over or shared-memory round trip per strip.  Measured issue
 // rate on B200 (tests/native/mma_sync_probe.cu): one m16n8k16 per 8 cycles per SM sub-partition = 1019 MAC/clk/SM, against
-// ~43 MAC/clk/SM the FFMA kernel reaches.
+// ~43 MAC/clk/SM an FFMA version of this stage reached (DESIGN §3.2).
 //
 // fp32-level accuracy comes from the same error compensation as the tcgen05 kernel: x = hi + lo, hi = fp16(x),
 // lo = fp16(x - hi); a product is hi*hi + hi*lo + lo*hi accumulated in fp32 in ONE accumulator (the dropped lo*lo term is
@@ -523,6 +528,29 @@ int launch_policy_attn_mma(const cm_policy_desc *desc, const cm_policy_io *io, c
     A.envs_per_policy = io->envs_per_policy;
     A.weights_stride = io->weights_stride;
     return launch_attn_mma_n<true>(desc->n_agents, A, stream);
+}
+
+int launch_policy_tc_encode(const cm_policy_desc *desc, const cm_policy_io *io, float *scr_e, float *scr_q, float *scr_hw, cudaStream_t stream);
+int launch_policy_tc_head(const cm_policy_desc *desc, const cm_policy_io *io, const float *x_rows, cudaStream_t stream);
+
+size_t tc_large_ws_floats(int n, int64_t n_envs) { return (size_t)3 * (size_t)n_envs * (size_t)n * kE; }
+
+// Comm-DP forward for teams of 65..256 agents: encoder (tensor cores) -> attention / graph convolutions (here) -> head
+// (tensor cores), three launches on one stream, rows handed over through the caller's workspace.
+int launch_policy_tc_large(const cm_policy_desc *desc, const cm_policy_io *io, cudaStream_t stream)
+{
+    const int n = desc->n_agents;
+    if (n <= 64 || n > CM_MAX_AGENTS) return CM_EUNSUPPORTED;
+    const size_t rows = (size_t)io->n_envs * n;
+    if (!io->workspace || io->workspace_bytes < tc_large_ws_floats(n, io->n_envs) * sizeof(float)) return CM_EINVAL;
+    if ((reinterpret_cast<uintptr_t>(io->workspace) & 15u) != 0) return CM_EINVAL;
+    float *scr_e = io->workspace, *scr_q = scr_e + rows * kE, *scr_hw = scr_q + rows * kE;
+    int rc = launch_policy_tc_encode(desc, io, scr_e, scr_q, scr_hw, stream);
+    if (rc) return rc;
+    rc = launch_policy_attn_mma(desc, io, scr_e, scr_q, scr_hw, stream);
+    if (rc) return rc;
+    if (!io->probs && !io->actions && !io->logits) return CM_OK;
+    return launch_policy_tc_head(desc, io, scr_q, stream);
 }
 
 }  // namespace cm

@@ -1,4 +1,4 @@
-// policy_layout.cuh — weight-blob layouts shared by the policy kernels (fp32 FFMA and tcgen05 variants).
+// policy_layout.cuh — weight-blob layouts shared by the policy kernels.
 #pragma once
 #include <stdint.h>
 
@@ -55,14 +55,6 @@ __host__ __device__ inline CentBlob cent_blob_layout(int n, int D)
     o.total = p;
     return o;
 }
-
-struct PolicyArgs {
-    cm_policy_desc d;
-    cm_policy_io io;
-    int envs_per_tile;
-    int64_t n_tiles;
-};
-
 
 // ---- tcgen05 variant.  Every dense product runs on the tensor cores in fp16 with error compensation:
 //   x = x_hi + 2^-12 x_lo,   x_hi = fp16(x),   x_lo = fp16((x - x_hi) * 4096)        (22+ significant bits)

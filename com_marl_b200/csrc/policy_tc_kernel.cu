@@ -1,7 +1,17 @@
-// policy_tc_kernel.cu — CommCategoricalMLPPolicy forward on the 5th-generation tensor cores (tcgen05).
+// policy_tc_kernel.cu — fused CommCategoricalMLPPolicy forward (+ action sampling) on the 5th-generation tensor cores (tcgen05).
 //
-// Same formula and outputs as policy_kernel.cu (see its header for the reference lines), different machine
-// mapping: a CTA of 512 threads owns a tile of 128 agent rows (whole environments, n <= 64); TWO such CTAs are
+// Reference formula (comm_categorical_mlp_policy.py:48-119, comm_base_net.py:80-108,
+// attention_module.py:38-49, graph_conv_module.py:51-72, categorical_mlp_module.py:64-80):
+//   h  = tanh(obs W1^T + b1)            D   -> 128      encoder._layers.0
+//   E  = tanh(h   W2^T + b2)            128 -> 64       encoder._output_layers.0 (output_nonlinearity=tanh)
+//   M  = softmax_j((E Wa^T) E^T)        per env, n x n  attention_layer ('general')
+//   A_l = M * Range * chan_l ; A_l /= (sum_j A_l + 1e-12)
+//   H_{l+1} = tanh(A_l (H_l Wg_l) + bg_l),  H_0 = E      gcn_layers.l   (Wg is (in,out))
+//   X  = E + H_L                                         residual
+//   logits = head(X): tanh 64->128, tanh 128->64, tanh 64->32, linear 32->5
+//   probs  = softmax(logits) * avail / sum ; action ~ Categorical(probs) | argmax
+//
+// Machine mapping: a CTA of 512 threads owns a tile of 128 agent rows (whole environments, n <= 64); TWO such CTAs are
 // resident per SM (256 tensor-memory columns and ~103 KB of shared memory each), so that one tile's epilogue
 // (CUDA cores) runs while the other tile's products (tensor cores) and weight copies (TMA engine) are in flight.
 //   * every row-wise dense layer (encoder, attention query, H_l Wg_l, the categorical head) is a series of
@@ -1348,13 +1358,6 @@ __global__ void tc_prepare_kernel(const float *__restrict__ w, __half *__restric
     }
 }
 
-// experiments / cross-checks only: CM_TC_ATTENTION=cuda keeps the CUDA-core attention loops for every team size
-static bool cm_tc_attention_disabled()
-{
-    static const int off = [] { const char *e = getenv("CM_TC_ATTENTION"); return (e && e[0] == 'c') ? 1 : 0; }();
-    return off != 0;
-}
-
 static size_t tc_smem_bytes() { return (size_t)kActBytes + kWBytes + (64 + 8) * kTPitch * 4 + kBiasFloats * 4 + 64; }   // (4 mbarriers + the TMEM base)
 
 static int launch_tc_mode(const cm_policy_desc *desc, const cm_policy_io *io, int mode, int in_dim, float *scr_e, float *scr_q,
@@ -1373,7 +1376,7 @@ static int launch_tc_mode(const cm_policy_desc *desc, const cm_policy_io *io, in
     A.plan = make_tc_plan(desc->obs_dim, desc->n_layers, mode);
     // Comm-DP teams of 17 .. 64 agents: attention on the tensor cores, an env per slot of 32 / 64 tile rows (a slot is a
     // multiple of the warp size, so a warp's rows share their env's key columns); smaller teams: dense packing, CUDA cores
-    const bool attn_tc = !rows_mode && desc->n_agents > 16 && !cm_tc_attention_disabled();
+    const bool attn_tc = !rows_mode && desc->n_agents > 16;
     A.slot = rows_mode ? 0 : (attn_tc ? (desc->n_agents <= 32 ? 32 : 64) : desc->n_agents);
     A.envs_per_tile = rows_mode ? 0 : kTcRows / A.slot;
     A.n_tiles = rows_mode ? (io->n_envs * desc->n_agents + kTcRows - 1) / kTcRows : (io->n_envs + A.envs_per_tile - 1) / A.envs_per_tile;
@@ -1423,7 +1426,7 @@ static int launch_tc_mode(const cm_policy_desc *desc, const cm_policy_io *io, in
     return CM_OK;
 }
 
-int launch_policy_tc_large(const cm_policy_desc *desc, const cm_policy_io *io, cudaStream_t stream);   // policy_attn_kernel.cu
+int launch_policy_tc_large(const cm_policy_desc *desc, const cm_policy_io *io, cudaStream_t stream);   // policy_attn_mma_kernel.cu
 
 int launch_policy_tc(const cm_policy_desc *desc, const cm_policy_io *io, cudaStream_t stream)
 {
@@ -1432,7 +1435,7 @@ int launch_policy_tc(const cm_policy_desc *desc, const cm_policy_io *io, cudaStr
     return launch_tc_mode(desc, io, mode, desc->obs_dim, nullptr, nullptr, nullptr, stream);
 }
 
-// large-team pipeline halves (policy_attn_kernel.cu drives them): rows -> E, Q, H_0 Wg_0 ; X rows -> logits / actions
+// large-team pipeline halves (launch_policy_tc_large drives them): rows -> E, Q, H_0 Wg_0 ; X rows -> logits / actions
 int launch_policy_tc_encode(const cm_policy_desc *desc, const cm_policy_io *io, float *scr_e, float *scr_q, float *scr_hw, cudaStream_t stream)
 {
     return launch_tc_mode(desc, io, kTcModeEnc, desc->obs_dim, scr_e, scr_q, scr_hw, stream);

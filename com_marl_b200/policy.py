@@ -134,11 +134,9 @@ class CommCategoricalMLPPolicy(nn.Module):
         self._embedding_dim = embedding_dim
         self.n_gcn_layers = int(n_gcn_layers)
         self.seed = int(seed)
-        # kernel variant: 'fp32' = exact FFMA kernels; 'tc' = tcgen05 tensor cores, error-compensated fp16 products with
-        # fp32 accumulation (fp32-level accuracy; teams of n > 64 run encoder / head on the tensor cores and the n x n
-        # attention in exact fp32 between them); 'auto' = 'tc'
-        if math not in ("auto", "fp32", "tc", "tc_fp32attn"):
-            raise ValueError("math must be 'auto', 'fp32', 'tc' or 'tc_fp32attn'")
+        # 'auto' = 'tc': tensor cores, error-compensated fp16 products with fp32 accumulation (fp32-level accuracy)
+        if math not in ("auto", "tc"):
+            raise ValueError(f"math must be 'auto' or 'tc', not {math!r}: the tensor-core kernels are the only Comm-DP forward")
         self.math = math
         self.encoder = _MLP(self._dec_obs_dim, encoder_hidden_sizes, embedding_dim, output_tanh=True)
         self.attention_layer = _Attention(embedding_dim, attention_type)
@@ -190,7 +188,7 @@ class CommCategoricalMLPPolicy(nn.Module):
         return self._blob
 
     def uses_tensor_cores(self):
-        return self.math in ("tc", "auto", "tc_fp32attn")
+        return True
 
     def tc_weight_blob(self):
         """pre-split (hi | lo), pre-laid-out B operands of the tcgen05 variant; rebuilt when a parameter changed"""
@@ -235,7 +233,7 @@ class CommCategoricalMLPPolicy(nn.Module):
         tensor-core kernels read it instead of ``obs`` (24 bytes per agent row instead of 4 D; identical results)."""
         desc, io = self._call_structs(obs, adj_bits, chan_bits, avail_bits, sample_u, tick, episode, greedy, probs, logits,
                                       attention, actions, env_id0, ws_slot)
-        if obs_bits is not None and self.uses_tensor_cores():
+        if obs_bits is not None:
             io.obs_bits, io.obs_nbits = N.ptr(obs_bits), int(obs_nbits)
         with torch.cuda.device(self.device):
             N.check("cm_policy_forward", N.lib().cm_policy_forward(C.byref(desc), C.byref(io), N.stream_ptr()))
@@ -245,17 +243,12 @@ class CommCategoricalMLPPolicy(nn.Module):
         """descriptor + io struct of one cm_policy_forward call on device tensors"""
         n, D, L = self._n_agents, self._dec_obs_dim, self.n_gcn_layers
         B = obs.shape[0]
-        tc = self.uses_tensor_cores()
-        desc = N.PolicyDesc(n, D, L, int(self.residual), int(greedy), (2 if self.math == "tc_fp32attn" else 1) if tc else 0,
-                            self.seed, env_id0, self._kind)
+        desc = N.PolicyDesc(n, D, L, int(self.residual), int(greedy), 1, self.seed, env_id0, self._kind)
         io = N.PolicyIO()
         io.n_envs = B
-        if tc:
-            io.tc_weights = N.ptr(self.tc_weight_blob())      # (refreshes the fp32 blob as well)
-            io.error_flag = N.ptr(self._tc_error)
-            io.weights = N.ptr(self._blob)
-        else:
-            io.weights = N.ptr(self.weight_blob())
+        io.tc_weights = N.ptr(self.tc_weight_blob())          # (refreshes the fp32 blob as well)
+        io.error_flag = N.ptr(self._tc_error)
+        io.weights = N.ptr(self._blob)
         for k, v in (("obs", obs), ("adj_bits", adj_bits), ("chan_bits", chan_bits), ("avail_bits", avail_bits),
                      ("sample_u", sample_u), ("tick", tick), ("episode", episode), ("probs", probs), ("logits", logits),
                      ("attention", attention), ("actions", actions)):
@@ -768,7 +761,7 @@ class PolicySet:
     @staticmethod
     def _arch(p):
         shapes = tuple((k, tuple(v.shape)) for k, v in p.state_dict().items())
-        math = ("tc_fp32attn" if p.math == "tc_fp32attn" else "tc") if p.uses_tensor_cores() else "fp32"   # 'auto' = its kernel
+        math = "tc" if p.uses_tensor_cores() else "fp32"       # CENT's two maths; 'auto' = the kernel it picked
         return (type(p), p._n_agents, p._dec_obs_dim, getattr(p, "n_gcn_layers", 0), getattr(p, "residual", False), math,
                 getattr(p, "_relu", False), shapes)
 

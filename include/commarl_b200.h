@@ -46,10 +46,11 @@
 extern "C" {
 #endif
 
-#define CM_ABI_VERSION 7   /* 2: host_arena / obs_bits members, cm_rollout_step_host; 3: cm_ppo_net; 4: CENT kinds of cm_ppo_net,
+#define CM_ABI_VERSION 8   /* 2: host_arena / obs_bits members, cm_rollout_step_host; 3: cm_ppo_net; 4: CENT kinds of cm_ppo_net,
                               cm_net_desc.flags; 5: cm_channel_cond, per-env channel conditions (cm_env_desc.conds ...);
                               6: several policies in one cm_policy_forward (cm_policy_io.n_policies ...);
-                              7: several networks in one cm_ppo_net (cm_net_io.n_policies ...), cm_adam_step_set */
+                              7: several networks in one cm_ppo_net (cm_net_io.n_policies ...), cm_adam_step_set;
+                              8: Comm-DP / Obs-DP take math = 1 only */
 #define CM_MAX_AGENTS 256   /* n, p */
 #define CM_MAX_GRID 64      /* grid side incl. Coverage's wall border */
 #define CM_MAX_LAYERS 4     /* n_gcn_layers */
@@ -183,11 +184,12 @@ typedef struct cm_policy_desc {
     int32_t n_layers;          /* L */
     int32_t residual;          /* comm_categorical_mlp_policy.py:74-77 */
     int32_t greedy;            /* argmax instead of sampling (:109-112) */
-    int32_t math;              /* 0: exact fp32 FFMA kernels; 1: tensor cores, error-compensated fp16 products (x = hi + lo)
-                                  with fp32 accumulation: fp32-level accuracy; needs io.tc_weights.  Teams with n <= 64: one
-                                  fused tcgen05 kernel; larger teams: tcgen05 encoder -> attention / graph convolutions on
-                                  mma.sync -> tcgen05 head, rows handed over through io.workspace.  2: like 1 with the large-team
-                                  attention in exact fp32 on the CUDA cores (cross-check) */
+    int32_t math;              /* Comm-DP / Obs-DP: 1 only (any other value: CM_EUNSUPPORTED) = tensor cores, error-compensated
+                                  fp16 products (x = hi + lo) with fp32 accumulation: fp32-level accuracy; needs io.tc_weights.
+                                  Teams with n <= 64: one fused tcgen05 kernel; larger teams: tcgen05 encoder -> attention /
+                                  graph convolutions on mma.sync -> tcgen05 head, rows handed over through io.workspace.
+                                  At most 2^23 agent rows (n_envs * n) per call; more return CM_EUNSUPPORTED.
+                                  CENT: 0 or 1, see `kind` */
     uint64_t seed;
     int64_t env_id0;
     int32_t kind;              /* cm_policy_kind: 0 = Comm-DP (CommCategoricalMLPPolicy), 1 = Obs-DP (DecCategoricalMLPPolicy:
@@ -224,7 +226,8 @@ typedef struct cm_policy_io {
     int8_t *actions;           /* [B][n], or NULL */
     const float *tc_weights;   /* math == 1: blob written by cm_policy_tc_prepare() (cm_policy_tc_blob_floats() floats) */
     int32_t *error_flag;       /* DEVICE i32[1], optional: set when a bounded device-side wait times out */
-    float *workspace;          /* teams with n > 64 only: cm_policy_workspace_bytes() bytes of scratch (stays L2 resident) */
+    float *workspace;          /* Comm-DP teams with n > 64 only: cm_policy_workspace_bytes() bytes of scratch, 16-byte aligned:
+                                  the E, Q and H_0 Wg_0 rows the large-team pipeline hands between its launches */
     size_t workspace_bytes;
     const uint32_t *obs_bits;  /* optional [B][n][6]: the packed observation cm_env_step writes (cm_step_io.obs_bits).  When given, the
                                   tensor-core kernels (math = 1) build their first operand from it — 24 bytes per agent row instead of
@@ -240,7 +243,7 @@ typedef struct cm_policy_io {
     int32_t n_policies;
     int64_t envs_per_policy;
     int64_t weights_stride;    /* floats */
-    int64_t tc_weights_stride; /* floats; math = 0 paths do not read it */
+    int64_t tc_weights_stride; /* floats; CENT with math = 0 does not read it */
 } cm_policy_io;
 
 int cm_abi_version(void);
@@ -282,7 +285,8 @@ size_t cm_policy_cent_workspace_bytes(int64_t n_envs);
  * panels, one per tensor-core product, so that the kernel fetches a layer's B operand with one bulk async copy */
 size_t cm_policy_tc_blob_floats(int32_t obs_dim, int32_t n_layers);
 int cm_policy_tc_prepare(const cm_policy_desc *desc, const float *weights, float *tc_weights, cm_stream_t stream);
-/* scratch the forward needs for teams larger than one 64-row tile (0 for n <= 64) */
+/* Comm-DP: bytes of scratch the forward needs for teams larger than one 64-row tile, 3 * n_envs * n_agents * 64 floats
+ * (0 for n <= 64) */
 size_t cm_policy_workspace_bytes(int32_t n_agents, int64_t n_envs);
 
 /* ---- host-buffer calls: the reference-facing form of the three entry points above ------------------------------

@@ -1,26 +1,17 @@
 """Kernel paths of cm_policy_forward (Comm-DP) and the helpers tests/test_gpu_policy_paths.py compares them with.
 
-cm_policy_forward picks one of five paths by team size and math mode:
-  * tc, n <= 16: policy_tc_kernel with the exact CUDA-core attention (kVec = 4 / 2 / 1 by the team's divisibility);
-  * tc, 17 <= n <= 32 and 33 <= n <= 64: policy_tc_kernel with the tcgen05 attention in env slots of 32 / 64 tile rows;
-  * tc, n > 64: encoder and head on policy_tc_kernel, the attention on policy_attn_mma_kernel (mma.sync);
-  * the exact fp32 variants: math 'fp32' (policy_small_kernel / policy_large_kernel) and, for n > 64, 'tc_fp32attn'
-    (policy_attn_kernel between the tensor-core encoder and head).
-``CM_TC_ATTENTION=cuda`` makes teams of 17 .. 64 take the CUDA-core attention instead; the library reads it once per
-process, so that case runs in a spawned child (``run_cuda_attention``).
+cm_policy_forward picks one of four paths by team size:
+  * n <= 16: policy_tc_kernel with the exact CUDA-core attention (kVec = 4 / 2 / 1 by the team's divisibility);
+  * 17 <= n <= 32 and 33 <= n <= 64: policy_tc_kernel with the tcgen05 attention in env slots of 32 / 64 tile rows;
+  * n > 64: encoder and head on policy_tc_kernel, the attention on policy_attn_mma_kernel (mma.sync).
 
 Every comparison is against the float64 oracle (oracle.policy_forward).  Nothing here touches CUDA at import time.
 """
 import os
-import queue
-import sys
-import time
-import traceback
 
 import numpy as np
 
 TESTS = os.path.dirname(os.path.abspath(__file__))
-ROOT = os.path.dirname(TESTS)
 TC_ROWS = 128                                # policy_tc_kernel: agent rows per tile
 
 
@@ -30,11 +21,9 @@ def tc_slot(n):
     return n if n <= 16 else (32 if n <= 32 else 64)
 
 
-def path_of(n, math):
-    if math == "fp32":
-        return "fp32 small" if n <= 64 else "fp32 large"
+def path_of(n):
     if n > 64:
-        return "tc + fp32 attention" if math == "tc_fp32attn" else "tc + mma attention"
+        return "tc + mma attention"
     if n <= 16:
         return f"tc cuda-core attention kVec={4 if n % 4 == 0 else (2 if n % 2 == 0 else 1)}"
     return f"tc tcgen05 attention slot {tc_slot(n)}"
@@ -213,9 +202,7 @@ ARCHS = [dict(L=1, residual=False, gcn_bias=True, attention="general", D=77),
 PATHS = {"small": ("tc", (6, 16, 14, 5)),                 # kVec 2 (teams of 2, 6, 10, 14), 4 and 1
          "slot32": ("tc", (17, 32, 24, 31)),
          "slot64": ("tc", (33, 64, 54, 40)),
-         "mma": ("tc", (72, 200, 129, 256)),
-         "fp32": ("fp32", (6, 40, 72, 200)),
-         "fp32attn": ("tc_fp32attn", (97, 150, 65, 240))}
+         "mma": ("tc", (72, 200, 129, 256))}
 
 
 def arch_cases(path):
@@ -225,11 +212,11 @@ def arch_cases(path):
 
 def arch_label(c):
     return (f"n={c['n']} D={c['D']} L={c['L']} residual={c['residual']} gcn_bias={c['gcn_bias']} {c['attention']} "
-            f"math={c['math']} [{path_of(c['n'], c['math'])}]")
+            f"math={c['math']} [{path_of(c['n'])}]")
 
 
 def arch_batch(c, sms):
-    return ragged_B(c["n"], sms) if c["math"] == "tc" and c["n"] <= 64 else 97
+    return ragged_B(c["n"], sms) if c["n"] <= 64 else 97
 
 
 def arch_run(c, sms, outputs=("logits", "probs", "attention", "actions")):
@@ -238,57 +225,6 @@ def arch_run(c, sms, outputs=("logits", "probs", "attention", "actions")):
     x = inputs(c["n"], c["D"], c["L"], arch_batch(c, sms), seed=c["n"] * 7 + c["L"])
     pol = policy(w, c["n"], c["D"], c["L"], c["math"], c["residual"], c["attention"])
     return w, x, forward(pol, x, outputs)
-
-
-# ---- the child process of CM_TC_ATTENTION=cuda ---------------------------------------------------------------------------
-def cuda_attention_cases():
-    return arch_cases("slot32") + arch_cases("slot64")
-
-
-def worker(q):
-    try:
-        os.environ["CM_TC_ATTENTION"] = "cuda"     # before the first launch: the library reads it once per process
-        for p in (ROOT, TESTS):
-            if p not in sys.path:
-                sys.path.insert(0, p)
-        import torch
-        torch.set_num_threads(1)
-        sms = torch.cuda.get_device_properties(0).multi_processor_count
-        q.put(("ok", {c["id"]: arch_run(c, sms)[2] for c in cuda_attention_cases()}))
-    except BaseException:
-        q.put(("error", traceback.format_exc()))
-
-
-def run_cuda_attention(timeout=600):
-    """-> {case id: kernel outputs} computed by a spawned child with CM_TC_ATTENTION=cuda.  The child is always joined."""
-    import torch.multiprocessing as mp
-    ctx = mp.get_context("spawn")
-    q = ctx.Queue()
-    proc = ctx.Process(target=worker, args=(q,))
-    proc.start()
-    try:
-        deadline = time.monotonic() + timeout
-        while True:
-            try:
-                status, res = q.get(timeout=2)
-                break
-            except queue.Empty:
-                if not proc.is_alive():
-                    raise RuntimeError(f"CM_TC_ATTENTION=cuda child exited with code {proc.exitcode} before reporting")
-                if time.monotonic() > deadline:
-                    raise TimeoutError(f"CM_TC_ATTENTION=cuda child did not finish in {timeout} s")
-        proc.join(timeout=60)
-        if status != "ok":
-            raise RuntimeError(f"CM_TC_ATTENTION=cuda child failed:\n{res}")
-        assert proc.exitcode == 0, proc.exitcode
-        return res
-    finally:
-        if proc.is_alive():
-            proc.terminate()
-            proc.join(timeout=30)
-        if proc.is_alive():
-            proc.kill()
-            proc.join(timeout=30)
 
 
 # ---- peaked attention -----------------------------------------------------------------------------------------------------

@@ -15,10 +15,9 @@ from com_marl_b200.scenario import ScenarioSpec  # noqa: E402
 
 def main():
     cases = [("pp", 10, 1, 0.04, 2, 0.3, 40, "auto", {"max_env_steps": 6}),        # lane groups of 4, tcgen05 policy, IID
-             ("co", 10, 1, 0.03, 2, 0.0, 40, "fp32", {"max_env_steps": 6}),        # Coverage, FFMA policy
+             ("co", 10, 1, 0.03, 2, 0.0, 40, "auto", {"max_env_steps": 6}),        # Coverage
              ("pp", 20, 2, 0.08, 4, 0.2, 9, "auto", {"max_env_steps": 5}),         # n = 32: whole-warp groups
              ("pp", 30, 2, 0.08, 4, 0.0, 3, "auto", {"max_env_steps": 4}),         # n = 72: tc encoder -> attention kernel -> tc head
-             ("pp", 30, 2, 0.08, 4, 0.0, 2, "fp32", {"max_env_steps": 4}),         # n = 72: large-team FFMA kernel
              ("pp", 50, 2, 0.08, 4, 0.0, 2, "auto", {"max_env_steps": 3})]         # n = 200: attention kernel with 13-row groups
     for scen, m, sen, den, cap, loss, B, math, over in cases:
         spec = ScenarioSpec.from_cli(scen, m, sen, den, cap=cap, loss=loss, seed=3, **over)

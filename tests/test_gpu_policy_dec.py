@@ -154,7 +154,8 @@ def test_dec_sampler_paths_contract():
 
 
 def test_policy_kind_error_codes():
-    """C-ABI error behaviour of the new descriptor field: unknown kinds are rejected, Obs-DP needs the tensor-core path."""
+    """C-ABI error behaviour of the new descriptor field: unknown kinds are rejected, Comm-DP and Obs-DP need the tensor-core
+    path (math = 1)."""
     import ctypes as C
     from com_marl_b200 import _native as N
     n, D, B = 3, 29, 8
@@ -164,7 +165,8 @@ def test_policy_kind_error_codes():
     io = N.PolicyIO()
     io.n_envs, io.weights, io.tc_weights = B, N.ptr(pol.weight_blob()), N.ptr(pol.tc_weight_blob())
     io.obs, io.probs = N.ptr(obs), N.ptr(probs)
-    for kind, math, expect in ((7, 1, N.CM_EINVAL), (N.POLICY_DEC, 0, N.CM_EUNSUPPORTED), (N.POLICY_DEC, 1, N.CM_OK)):
+    for kind, math, expect in ((7, 1, N.CM_EINVAL), (N.POLICY_DEC, 0, N.CM_EUNSUPPORTED), (N.POLICY_DEC, 2, N.CM_EUNSUPPORTED),
+                               (N.POLICY_COMM, 0, N.CM_EUNSUPPORTED), (N.POLICY_COMM, 2, N.CM_EUNSUPPORTED), (N.POLICY_DEC, 1, N.CM_OK)):
         desc = N.PolicyDesc(n, D, 1, 0, 1, math, 1, 0, kind)
         assert N.lib().cm_policy_forward(C.byref(desc), C.byref(io), N.stream_ptr()) == expect, (kind, math)
     torch.cuda.synchronize()

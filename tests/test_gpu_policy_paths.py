@@ -2,14 +2,13 @@
 
 tests/test_gpu_policy.py checks the reference's default architecture at a handful of team sizes.  This file covers what
 the kernels branch on (the paths are listed in tests/policy_path_util.py):
-  (a) every team size 1 .. 256 in every math mode, which runs every kVec, env slot, NS / WARPS and (RT, KT) build;
+  (a) every team size 1 .. 256, which runs every kVec, env slot and NS / WARPS build;
   (b) an architecture matrix per path: 1 .. 4 GCN layers, residual on / off, GCN bias on / off, 'general' / 'dot'
       attention, D up to 128, with batches that give every tcgen05 CTA three tiles, the last one ragged;
-  (c) the CUDA-core attention of teams of 17 .. 64 (CM_TC_ATTENTION=cuda, in a spawned child);
-  (d) packed observations (obs_bits) at the word edges of the window, for Comm-DP and Obs-DP;
-  (e) probabilities and actions that do not depend on which optional outputs are requested;
-  (f) peaked attention whose mass the masks remove, down to masked-in sums far below the renormalisation's 1e-12;
-  (g) the device rollout at 1, 3 and 4 layers, recomputed step by step by the oracle.
+  (c) packed observations (obs_bits) at the word edges of the window, for Comm-DP and Obs-DP;
+  (d) probabilities and actions that do not depend on which optional outputs are requested;
+  (e) peaked attention whose mass the masks remove, down to masked-in sums far below the renormalisation's 1e-12;
+  (f) the device rollout at 1, 3 and 4 layers, recomputed step by step by the oracle.
 Tolerances are those of tests/test_gpu_policy.py: logits within 1e-5 * max(1, max|ref|), probabilities and attention
 within 1e-5, sampled actions exactly the inverse-CDF specification on the kernel's own probabilities.
 
@@ -38,7 +37,7 @@ def test_oracle_matches_torch_float64():
     for L, residual, gcn_bias, attention in itertools.product((1, 2, 3, 4), (True, False), (True, False), ("general", "dot")):
         w = U.weights(n, D, L, residual, gcn_bias, attention, seed=L)
         x = U.inputs(n, D, L, B, seed=L + 10)
-        pol = U.policy(w, n, D, L, "fp32", residual, attention, device="cpu").double()
+        pol = U.policy(w, n, D, L, "auto", residual, attention, device="cpu").double()
         assert ("gcn_layers.0.bias" in w) == gcn_bias
         with torch.no_grad():
             dist, M = pol.forward(torch.from_numpy(x["obs"].reshape(B, -1)).double(), torch.from_numpy(x["avail"].reshape(B, -1)).double(),
@@ -50,16 +49,16 @@ def test_oracle_matches_torch_float64():
 
 
 @gpu
-@pytest.mark.parametrize("math", ["fp32", "tc", "tc_fp32attn"])
+@pytest.mark.parametrize("math", ["tc"])
 def test_every_team_size(math):
-    """n = 1 .. 256 (tc_fp32attn: 65 .. 256, where it differs from 'tc') at D = 53, L = 2 and a small ragged batch"""
+    """n = 1 .. 256 at D = 53, L = 2 and a small ragged batch"""
     D, L = 53, 2
-    for n in range(65 if math == "tc_fp32attn" else 1, 257):
+    for n in range(1, 257):
         B = 2 * (U.TC_ROWS // U.tc_slot(n)) + 1 if n <= 64 else 3
         w = U.weights(n, D, L, seed=n)
         x = U.inputs(n, D, L, B, seed=n + 1000)
         got = U.forward(U.policy(w, n, D, L, math), x)
-        U.check(f"n={n} D={D} L={L} B={B} math={math} [{U.path_of(n, math)}]", got, U.oracle(w, x), x["u"])
+        U.check(f"n={n} D={D} L={L} B={B} math={math} [{U.path_of(n)}]", got, U.oracle(w, x), x["u"])
 
 
 @gpu
@@ -74,17 +73,6 @@ def test_architecture_matrix(path):
         U.check(label, got, U.oracle(w, x, c["residual"]), x["u"])
         _, _, lean = U.arch_run(c, sms, outputs=("probs", "actions"))
         U.same(label + " without logits / attention", lean, got)
-
-
-@gpu
-def test_cuda_core_attention_17_to_64():
-    """the architecture matrix of teams of 17 .. 64 with CM_TC_ATTENTION=cuda (the CUDA-core attention in dense slots)"""
-    res = U.run_cuda_attention()
-    sms = _sms()
-    for c in U.cuda_attention_cases():
-        w = U.weights(c["n"], c["D"], c["L"], c["residual"], c["gcn_bias"], c["attention"], seed=c["n"] + 100 * c["L"])
-        x = U.inputs(c["n"], c["D"], c["L"], U.arch_batch(c, sms), seed=c["n"] * 7 + c["L"])
-        U.check(f"CM_TC_ATTENTION=cuda {U.arch_label(c)}", res[c["id"]], U.oracle(w, x, c["residual"]), x["u"])
 
 
 NBITS = (8, 31, 32, 33, 61, 64, 65, 90, 96)
@@ -126,8 +114,7 @@ def test_packed_observations(team):
 # (path, team, math, attention, scales): the scales grow the score path geometrically until the median masked-in mass is
 # far below 1e-6
 PEAKED = [("small", 8, "tc", "general"), ("slot32", 32, "tc", "general"), ("slot64", 64, "tc", "general"),
-          ("slot64", 48, "tc", "dot"), ("mma", 72, "tc", "general"), ("mma", 200, "tc", "dot"),
-          ("fp32", 32, "fp32", "general"), ("fp32", 72, "fp32", "dot"), ("fp32attn", 72, "tc_fp32attn", "general")]
+          ("slot64", 48, "tc", "dot"), ("mma", 72, "tc", "general"), ("mma", 200, "tc", "dot")]
 SCALES = {"general": (1.0, 2.0, 4.0, 8.0, 16.0), "dot": (1.0, 1.5, 2.25, 3.375)}
 
 
@@ -147,8 +134,8 @@ def test_peaked_attention():
             w, x, mass = U.peaked(base_w, base_x, scale, attention, seed=n)
             lowest = min(lowest, float(np.median(mass)))
             ref = U.oracle(w, x)
-            label = f"peaked {path} n={n} {attention} scale={scale} math={math} [{U.path_of(n, math)}]"
-            cpu = U.policy(w, n, D, L, "fp32", attention=attention, device="cpu")
+            label = f"peaked {path} n={n} {attention} scale={scale} math={math} [{U.path_of(n)}]"
+            cpu = U.policy(w, n, D, L, "auto", attention=attention, device="cpu")
             with torch.no_grad():
                 dist, _ = cpu.forward(torch.from_numpy(x["obs"].reshape(B, -1)), torch.from_numpy(x["avail"].reshape(B, -1)).float(),
                                       torch.from_numpy(x["adj"]).float(), torch.from_numpy(x["chan"].reshape(B, L * n, n)).float())

@@ -49,4 +49,4 @@ def test_prescaled_activations_at_the_ends_of_fp16(n):
     w = extreme_weights(n, D, L, seed=n)
     x = U.inputs(n, D, L, B, seed=n + 77)
     got = U.forward(U.policy(w, n, D, L, "tc"), x)
-    U.check(f"n={n} saturated / subnormal activations [{U.path_of(n, 'tc')}]", got, U.oracle(w, x), x["u"])
+    U.check(f"n={n} saturated / subnormal activations [{U.path_of(n)}]", got, U.oracle(w, x), x["u"])

@@ -13,17 +13,15 @@ import pytest
 import policy_set_util as U
 
 # (kind, n, D, math, envs per policy, policies): every kVec / slot size of the Comm-DP tensor-core kernel, the large-team
-# pipeline in both attention maths, the FFMA kernels, Obs-DP (rows mode) and CENT in both maths.  Envs per policy are not
-# multiples of the envs per tile and E n is not a multiple of 128.  With P = 64 the tensor-core cases have more than 296 tiles
-# (2 CTAs x 148 SMs), so persistent CTAs walk tiles of several policies: the weight stream prefetches across a policy switch
-# and the bias table is reloaded.
+# pipeline, Obs-DP (rows mode) and CENT in both maths.  Envs per policy are not multiples of the envs per tile and E n is not
+# a multiple of 128.  With P = 64 the tensor-core cases have more than 296 tiles (2 CTAs x 148 SMs), so persistent CTAs walk
+# tiles of several policies: the weight stream prefetches across a policy switch and the bias table is reloaded.
 CASES = [("comm", n, 13, "tc", 37, 3) for n in (3, 4, 5, 6, 16, 17, 32, 33, 64)] + \
-        [("comm", n, 13, m, 5, 3) for n in (65, 130, 200, 256) for m in ("tc", "tc_fp32attn")] + \
-        [("comm", n, 13, "fp32", 23, 3) for n in (5, 32, 100)] + \
+        [("comm", n, 13, "tc", 5, 3) for n in (65, 130, 200, 256)] + \
         [("dec", n, 13, "tc", E, 3) for n, E in ((4, 11), (32, 11), (200, 3))] + \
         [("cent", n, D, m, E, 3) for n, D, E in ((3, 13, 70), (32, 13, 130), (200, 5, 70)) for m in ("fp32", "tc")] + \
         [("comm", 32, 13, "tc", 37, P) for P in (1, 2, 7, 64)] + \
-        [("dec", 32, 13, "tc", 20, 64), ("comm", 4, 13, "tc", 150, 64), ("comm", 65, 13, "tc", 9, 64), ("comm", 32, 13, "fp32", 37, 64)]
+        [("dec", 32, 13, "tc", 20, 64), ("comm", 4, 13, "tc", 150, 64), ("comm", 65, 13, "tc", 9, 64)]
 
 
 def _ids(c):
@@ -81,7 +79,7 @@ def _raw_call(pset, kind, inp, out, **over):
 
 
 @pytest.mark.gpu
-@pytest.mark.parametrize("kind,math", [("comm", "tc"), ("comm", "fp32"), ("dec", "tc"), ("cent", "tc")])
+@pytest.mark.parametrize("kind,math", [("comm", "tc"), ("dec", "tc"), ("cent", "tc"), ("cent", "fp32")])
 def test_invalid_blocks_and_strides(kind, math):
     import torch
     from com_marl_b200 import _native as N
@@ -124,13 +122,15 @@ def test_host_calls_reject_policy_sets():
 def test_mismatched_architectures_raise():
     from com_marl_b200.policy import PolicySet
     a = U.make_policy("comm", 8, 13, "tc", seed=1)
-    for other in (U.make_policy("comm", 8, 13, "fp32", seed=2), U.make_policy("comm", 8, 13, "tc", seed=2, L=3),
+    for other in (U.make_policy("comm", 8, 13, "tc", seed=2, L=3),
                   U.make_policy("comm", 9, 13, "tc", seed=2), U.make_policy("comm", 8, 12, "tc", seed=2),
                   U.make_policy("dec", 8, 13, "tc", seed=2), U.make_policy("cent", 8, 13, "tc", seed=2)):
         with pytest.raises(ValueError):
             PolicySet([a, other])
     with pytest.raises(ValueError):
         PolicySet([U.make_policy("cent", 8, 13, "fp32", seed=1), U.make_policy("cent", 8, 13, "fp32", seed=2, relu=True)])
+    with pytest.raises(ValueError):                # the same CENT architecture on the other math
+        PolicySet([U.make_policy("cent", 8, 13, "tc", seed=1), U.make_policy("cent", 8, 13, "fp32", seed=2)])
 
 
 def _spec(size):

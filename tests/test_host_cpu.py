@@ -28,7 +28,7 @@ def test_library_exports_every_declared_symbol():
     assert lib.cm_strerror(N.CM_EACTION) == b"Action Not found!"
     assert lib.cm_policy_blob_floats(21, 2) == 42309 and lib.cm_policy_blob_floats(53, 2) == 46405   # SURVEY.md §3.3
     assert lib.cm_policy_cent_blob_floats(4, 21) == 84 * 128 + 128 + 8256 + 2080 + 33 * 20   # n*D -> 128 -> 64 -> 32 -> 5n
-    assert lib.cm_policy_workspace_bytes(32, 100) == 0 and lib.cm_policy_workspace_bytes(200, 4) == 4 * 3 * 64 * 256 * 4
+    assert lib.cm_policy_workspace_bytes(32, 100) == 0 and lib.cm_policy_workspace_bytes(200, 4) == 4 * 3 * 200 * 64 * 4
 
 
 @pytest.mark.skipif(torch.cuda.is_available(), reason="checks the no-GPU behaviour")

@@ -4,7 +4,7 @@
 set -e
 OUT=${1:-tests/native/lib_trace.so}
 cd "$(dirname "$0")/.."
-SRC="env_kernels.cu policy_kernel.cu policy_tc_kernel.cu policy_attn_kernel.cu policy_attn_mma_kernel.cu policy_cent_kernel.cu host_abi.cu ppo_kernels.cu ppo_net_kernels.cu abi.cu"
+SRC="env_kernels.cu policy_forward.cu policy_tc_kernel.cu policy_attn_mma_kernel.cu policy_cent_kernel.cu host_abi.cu ppo_kernels.cu ppo_net_kernels.cu abi.cu"
 mkdir -p /tmp/trace_obj
 for f in $SRC; do
   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 -Xcompiler -fPIC -DCM_ENV_TRACE -DCM_TC_TRACE -I include -I com_marl_b200/csrc -c com_marl_b200/csrc/$f -o /tmp/trace_obj/${f%.cu}.o &
